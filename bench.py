@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — world-steps/sec of the batched rigid-body step (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3] [--dump-outputs DIR]
 
 One "step" = one Ensemble::Step (narrowphase -> rows -> PGS -> integrate) over every world of the
 rank's batch.  Default workload = BASELINE.json configs[2], the configuration the metric's target
@@ -47,6 +47,8 @@ DENSE = {"c4"}                # workloads on the reference's default dense solve
 FIXED_K = 20
 FLOPS_PER_ROW_UPDATE = 54.0   # SURVEY.md §8(d)
 ROW_STREAM_BYTES = 208.0      # bytes of one 3-row block streamed from HBM per Gauss-Seidel pass: 176 B record + 32 B multipliers
+DUMP_WORLDS = 4096            # --dump-outputs: worlds sampled (seed 0) when the batch is larger; 4096 x 64 bodies x 18 doubles = 38 MB
+DUMP_MAX_BYTES = 64 << 20
 
 
 def parse():
@@ -64,7 +66,13 @@ def parse():
     ap.add_argument("--no-fixed-k", action="store_true", help="skip the extra fixed-K (K = 20) measurement of the PGS workloads (and the strong-scaling extra of c3)")
     ap.add_argument("--no-evolving", action="store_true", help="skip the extra evolving-state measurement (the batch stepped on without restore)")
     ap.add_argument("--precision", type=int, default=64, choices=[64, 32], help="32 = opt-in FP32 constraint records (not the headline)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (body state, status, rollout cost) of a fixed "
+                         "seeded sample of rank 0's worlds as DIR/<name>.npy in float64, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != "ours" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl ours and --steps >= 1")
+    return args
 
 
 def peaks():
@@ -148,6 +156,24 @@ def run_reference(args):
         "gpu_launches": 0,
     }
     emit(line)
+
+
+def dump_outputs(path, b, st, costs):
+    """Writes what a caller of the timed step receives -- egg_get_bodies (p, R, v, w), egg_get_status
+    and the rollout cost of every world -- for a fixed seeded sample of the batch's worlds, as float64
+    DIR/<name>.npy.  The scene is seeded, so the same arguments give the same inputs on every run."""
+    W = b.W
+    idx = np.arange(W) if W <= DUMP_WORLDS else np.sort(np.random.default_rng(0).choice(W, DUMP_WORLDS, replace=False))
+    out = dict(zip(("p", "R", "v", "w"), b.bodies()))
+    out.update(st)
+    out["cost"] = costs
+    out = {k: np.ascontiguousarray(a[idx], dtype=np.float64) for k, a in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs would write {total} bytes"
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+    print(f"bench.py: wrote {len(out)} arrays ({total} bytes, {len(idx)} of {W} worlds) to {path}", file=sys.stderr)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -282,6 +308,8 @@ def run_ours(args):
     contacts_mean = float(st["n_contacts"].mean())
     status_or = int(np.bitwise_or.reduce(st["status"]))
     best = float(all_costs.min().item())
+    if args.dump_outputs is not None and rank == 0:   # before the end-to-end leg below overwrites the state
+        dump_outputs(args.dump_outputs, b, st, costs.cpu().numpy())
 
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:
