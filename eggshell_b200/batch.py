@@ -22,7 +22,8 @@ ST_LCP_FAILED, ST_JOINT_CONFLICT, ST_BAD_INIT, ST_CONTACT_OVERFLOW, ST_NONFINITE
 
 EXPORTS = [
     "egg_desc_default", "egg_create", "egg_destroy", "egg_set_bodies", "egg_set_shapes", "egg_set_state", "egg_set_joints",
-    "egg_set_external", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
+    "egg_set_external", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_step_controlled",
+    "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
     "egg_get_status", "egg_get_dense_work", "egg_get_debug_counters", "egg_rollout_costs", "egg_set_stream", "egg_sync", "egg_device_bytes",
     "egg_launch_count", "egg_capacity", "egg_set_profiling", "egg_get_kernel_ms", "egg_fp64_peak_tflops", "egg_host_alloc", "egg_host_free", "egg_last_error", "egg_version",
 ]
@@ -64,6 +65,9 @@ def lib():
         L.egg_host_free.argtypes = [C.c_void_p]
         L.egg_set_stream.argtypes = [C.c_void_p, C.c_void_p]
         L.egg_rollout_costs.argtypes = [C.c_void_p, C.c_void_p]
+        L.egg_step_controlled.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_void_p, C.c_int]
+        L.egg_gather_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+        L.egg_seed_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
         _LIB = L
     return _LIB
 
@@ -113,6 +117,7 @@ class Batch:
         _chk(L.egg_create(C.byref(d), C.byref(self.h)), "egg_create")
         self.W, self.n, self.nj = n_worlds, n_bodies, n_joints
         self.desc = d
+        self.stream = None   # cudaStream_t handed to set_stream; None = the batch's own stream
         self.max_contacts = None
         self._probe_capacity()
 
@@ -181,10 +186,32 @@ class Batch:
 
     def set_stream(self, cuda_stream_ptr):
         _chk(lib().egg_set_stream(self.h, C.c_void_p(cuda_stream_ptr)), "egg_set_stream")
+        self.stream = cuda_stream_ptr
 
     # -- stepping -----------------------------------------------------------------------------
     def step(self, dt, n_steps=1, integrator=OPEN_DYNAMICS_ENGINE):
         _chk(lib().egg_step(self.h, C.c_double(dt), int(integrator), int(n_steps)), "egg_step")
+
+    def step_controlled(self, dt, u_ptr, horizon, integrator=OPEN_DYNAMICS_ENGINE):
+        """`horizon` steps; before step t the f_ext slot takes slice t of the device schedule at u_ptr,
+        float64 [horizon][W][n][6] (egg_step_controlled)."""
+        _chk(lib().egg_step_controlled(self.h, C.c_double(dt), int(integrator), C.c_void_p(u_ptr), int(horizon)),
+             "egg_step_controlled")
+
+    # -- device-side state exchange (MPC) ------------------------------------------------------
+    def gather_state(self, worlds, out_ptr):
+        """Writes the state of the listed worlds to the device buffer at out_ptr, float64
+        [len(worlds)][n][18] = (p, R row-major, v, w) per body (egg_gather_state)."""
+        w64 = np.asarray(worlds, dtype=np.int64).ravel()
+        idx = np.ascontiguousarray(w64, dtype=np.int32)
+        if not np.array_equal(idx, w64):
+            raise EggError("gather_state: world index out of the int32 range")
+        _chk(lib().egg_gather_state(self.h, _p(idx), int(idx.size), C.c_void_p(out_ptr)), "egg_gather_state")
+
+    def seed_state(self, in_ptr, k, first=0):
+        """World w takes row (first + w) % k of the device buffer at in_ptr, float64 [k][n][18]
+        (egg_seed_state).  Call snapshot() to make the seeded state the next horizon's start."""
+        _chk(lib().egg_seed_state(self.h, C.c_void_p(in_ptr), int(k), int(first)), "egg_seed_state")
 
     def update_contacts(self):
         _chk(lib().egg_update_contacts(self.h), "egg_update_contacts")

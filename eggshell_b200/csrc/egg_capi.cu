@@ -64,6 +64,7 @@ struct egg_batch {
   int* level_aux = nullptr;
   int device = 0;
   double* snap = nullptr;        // egg_snapshot copy of dev.dyn
+  int* gather_idx = nullptr;     // [W] world indices of egg_gather_state, allocated by its first call
   bool profiling = false;
   std::vector<cudaEvent_t> ev;   // 4 per profiled step
   std::vector<cudaEvent_t> ev_free;
@@ -523,14 +524,35 @@ int egg_post_stabilize(egg_batch* b, int max_steps, int* steps_out, double* err_
   return relax_report(b, steps_out, err_sq_out);
 }
 
-int egg_step(egg_batch* b, double dt, int integrator, int n_steps) {
+// The argument and call-order checks of egg_step and egg_step_controlled.
+static int step_check(egg_batch* b, double dt, int integrator, int n_steps, const char* what) {
   if (!b || n_steps < 0 || !(dt > 0)) return EGG_ERR_ARG;
-  if (!b->initialised) { g_err = "egg_step before egg_init"; return EGG_ERR_STATE; }
+  if (!b->initialised) { g_err = std::string(what) + " before egg_init"; return EGG_ERR_STATE; }
   if (integrator != EGG_OPEN_DYNAMICS_ENGINE) {
     // ensembles.cc:398-405: EXPLICIT_EULER refuses contacts, IMPLICIT_MIDPOINT panics.
     g_err = "only OPEN_DYNAMICS_ENGINE is supported (as in the reference once contacts exist)";
     return EGG_ERR_UNSUPPORTED;
   }
+  return EGG_OK;
+}
+
+// A _d argument must be device (or managed) memory of the batch's device: a host pointer would
+// reach a kernel as an illegal address.  The length behind the pointer cannot be checked here.
+static int check_device_ptr(egg_batch* b, const void* p, const char* what) {
+  if (!p) { g_err = std::string(what) + ": NULL device pointer"; return EGG_ERR_ARG; }
+  cudaPointerAttributes a;
+  cudaError_t e = cudaPointerGetAttributes(&a, p);
+  if (e != cudaSuccess) { cudaGetLastError(); g_err = std::string(what) + ": not a CUDA pointer"; return EGG_ERR_ARG; }
+  if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != b->device) {
+    g_err = std::string(what) + ": the buffer is not device memory of the batch's device";
+    return EGG_ERR_ARG;
+  }
+  return EGG_OK;
+}
+
+// n_steps x Ensemble::Step.  With a control schedule u_d ([n_steps][W][n][6]), slice s is copied into
+// the f_ext slot before step s (outside the profiled kernel buckets).
+static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d) {
   const int solver = b->dev.prm.solver;
   if (solver < EGG_SOLVER_DENSE_MURTY || solver > EGG_SOLVER_SOR) { g_err = "unknown solver"; return EGG_ERR_ARG; }
   CK(cudaSetDevice(b->device));
@@ -543,7 +565,12 @@ int egg_step(egg_batch* b, double dt, int integrator, int n_steps) {
     b->iso_known = true;
     b->dev.rmax = egg_runs_rmax(b->dev);   // run format of the PGS stream for isotropic bodies, else one block per lane and stage
   }
+  const size_t slice = (size_t)b->dev.W * b->dev.n * 6;
   for (int s = 0; s < n_steps; s++) {
+    if (u_d) {
+      LK(egg_launch_fext_slice(b->dev, u_d + (size_t)s * slice, b->stream));
+      b->launches++;
+    }
     cudaEvent_t e[4] = {nullptr, nullptr, nullptr, nullptr};
     if (b->profiling) {
       for (int k = 0; k < 4; k++) {
@@ -575,6 +602,46 @@ int egg_step(egg_batch* b, double dt, int integrator, int n_steps) {
     b->launches += (solver == EGG_SOLVER_PGS && b->dev.rec_fmt) ? 5 : 3;   // collide, assemble (1 or 3 kernels), solve
   }
   CK(cudaGetLastError());
+  return EGG_OK;
+}
+
+int egg_step(egg_batch* b, double dt, int integrator, int n_steps) {
+  RET(step_check(b, dt, integrator, n_steps, "egg_step"));
+  return step_loop(b, dt, n_steps, nullptr);
+}
+
+int egg_step_controlled(egg_batch* b, double dt, int integrator, const double* u_d, int horizon) {
+  if (!b || !u_d) return EGG_ERR_ARG;
+  if (horizon < 1) { g_err = "egg_step_controlled: horizon must be >= 1"; return EGG_ERR_ARG; }
+  RET(step_check(b, dt, integrator, horizon, "egg_step_controlled"));
+  RET(check_device_ptr(b, u_d, "egg_step_controlled(u_d)"));
+  return step_loop(b, dt, horizon, u_d);
+}
+
+int egg_gather_state(egg_batch* b, const int* worlds, int k, double* out_d) {
+  if (!b || !worlds || !out_d) return EGG_ERR_ARG;
+  const int W = b->dev.W;
+  if (k < 1 || k > W) { g_err = "egg_gather_state: k must be in [1, n_worlds]"; return EGG_ERR_ARG; }
+  for (int i = 0; i < k; i++)
+    if (worlds[i] < 0 || worlds[i] >= W) { g_err = "egg_gather_state: world index out of range"; return EGG_ERR_ARG; }
+  if (!b->initialised) { g_err = "egg_gather_state before egg_init"; return EGG_ERR_STATE; }
+  RET(check_device_ptr(b, out_d, "egg_gather_state(out_d)"));
+  CK(cudaSetDevice(b->device));
+  if (!b->gather_idx) RET(dalloc(b, &b->gather_idx, (size_t)W));
+  CK(cudaMemcpyAsync(b->gather_idx, worlds, (size_t)k * sizeof(int), cudaMemcpyHostToDevice, b->stream));
+  LK(egg_launch_gather_state(b->dev, b->gather_idx, k, out_d, b->stream));
+  b->launches++;
+  return EGG_OK;
+}
+
+int egg_seed_state(egg_batch* b, const double* in_d, int k, int first) {
+  if (!b || !in_d) return EGG_ERR_ARG;
+  if (k < 1 || k > b->dev.W || first < 0) { g_err = "egg_seed_state: k must be in [1, n_worlds] and first >= 0"; return EGG_ERR_ARG; }
+  if (!b->initialised) { g_err = "egg_seed_state before egg_init"; return EGG_ERR_STATE; }
+  RET(check_device_ptr(b, in_d, "egg_seed_state(in_d)"));
+  CK(cudaSetDevice(b->device));
+  LK(egg_launch_seed_state(b->dev, in_d, k, first, b->stream));
+  b->launches++;
   return EGG_OK;
 }
 

@@ -153,6 +153,11 @@ cudaError_t egg_launch_solve_iter(const EggDev& d, double dt, int solver, cudaSt
 cudaError_t egg_launch_costs(const EggDev& d, double* cost_d, cudaStream_t s);
 cudaError_t egg_launch_pack(int W, const double* aos, int per_world, int comps, double* soa, int soa_comps, int comp_off, cudaStream_t s);
 cudaError_t egg_launch_unpack(int W, double* aos, int per_world, int comps, const double* soa, int soa_comps, int comp_off, cudaStream_t s);
+// one control slice u [W][n][6] (device) -> the f_ext slot of stat
+cudaError_t egg_launch_fext_slice(const EggDev& d, const double* u, cudaStream_t s);
+// dyn of worlds[0..k) (device int array) -> out [k][n][18]; dyn of world w <- in [(first + w) mod k][n][18]
+cudaError_t egg_launch_gather_state(const EggDev& d, const int* worlds, int k, double* out, cudaStream_t s);
+cudaError_t egg_launch_seed_state(const EggDev& d, const double* in, int k, int first, cudaStream_t s);
 // Dynamic shared memory each kernel family needs for this batch shape (checked against the device
 // limit in egg_create, so that an unsupported shape fails there with a clear message).
 size_t egg_collide_smem(const EggDev& d);

@@ -163,6 +163,45 @@ __global__ void egg_unpack_kernel(double* aos, int W, int per_world, int comps, 
   aos[gid] = soa[((size_t)w * soa_comps + comp_off + c) * per_world + b];
 }
 
+// One slice of a control schedule, AoS u [W][n][6] -> the f_ext components 10..15 of stat [W][16][n].
+// One thread per (w, component, body) with the body fastest: the writes are coalesced, and the reads
+// of a warp (48-byte stride) share their sectors with the warps of the neighbouring components.
+__global__ void egg_fext_slice_kernel(const double* u, int W, int n, double* stat) {
+  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gid >= (long long)W * 6 * n) return;
+  const int b = (int)(gid % n);
+  const long long t = gid / n;
+  const int c = (int)(t % 6);
+  const long long w = t / 6;
+  stat[((size_t)w * EGG_STAT + 10 + c) * n + b] = u[((size_t)w * n + b) * 6 + c];
+}
+
+// The unpack kernel with a world-index map: dyn [W][18][n] of worlds[i] -> AoS out [k][n][18], the
+// per-body order of egg_get_bodies (p, R row-major, v, w).
+__global__ void egg_gather_state_kernel(const double* dyn, int n, const int* worlds, int k, double* out) {
+  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gid >= (long long)k * n * EGG_DYN) return;
+  const int c = (int)(gid % EGG_DYN);
+  const long long t = gid / EGG_DYN;
+  const int b = (int)(t % n);
+  const int i = (int)(t / n);
+  out[gid] = dyn[((size_t)worlds[i] * EGG_DYN + c) * n + b];
+}
+
+// AoS in [k][n][18] -> dyn of every world, world w from source (first + w) mod k.  One thread per
+// (w, component, body) with the body fastest: the W x 18 x n writes are coalesced, the k x n x 18
+// reads are small and stay in L2.
+__global__ void egg_seed_state_kernel(double* dyn, int W, int n, const double* in, int k, int first) {
+  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gid >= (long long)W * EGG_DYN * n) return;
+  const int b = (int)(gid % n);
+  const long long t = gid / n;
+  const int c = (int)(t % EGG_DYN);
+  const long long w = t / EGG_DYN;
+  const long long src = ((long long)first + w) % k;
+  dyn[gid] = in[((size_t)src * n + b) * EGG_DYN + c];
+}
+
 // FP64 roofline probe: 8 independent DFMA chains per thread.
 __global__ void egg_dfma_kernel(double* out, int iters) {
   double a0 = threadIdx.x * 1e-3, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
@@ -236,5 +275,21 @@ cudaError_t egg_launch_unpack(int W, double* aos, int per_world, int comps, cons
   long long total = (long long)W * per_world * comps;
   if (total == 0) return cudaSuccess;
   egg_unpack_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(aos, W, per_world, comps, soa, soa_comps, comp_off);
+  return cudaGetLastError();
+}
+
+cudaError_t egg_launch_fext_slice(const EggDev& d, const double* u, cudaStream_t s) {
+  const long long total = (long long)d.W * 6 * d.n;
+  egg_fext_slice_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(u, d.W, d.n, d.stat);
+  return cudaGetLastError();
+}
+cudaError_t egg_launch_gather_state(const EggDev& d, const int* worlds, int k, double* out, cudaStream_t s) {
+  const long long total = (long long)k * d.n * EGG_DYN;
+  egg_gather_state_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(d.dyn, d.n, worlds, k, out);
+  return cudaGetLastError();
+}
+cudaError_t egg_launch_seed_state(const EggDev& d, const double* in, int k, int first, cudaStream_t s) {
+  const long long total = (long long)d.W * EGG_DYN * d.n;
+  egg_seed_state_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(d.dyn, d.W, d.n, in, k, first);
   return cudaGetLastError();
 }

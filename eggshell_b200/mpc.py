@@ -1,9 +1,13 @@
 """Multi-GPU host logic: contiguous world shards and the one collective of the path — an allgather
-of per-rollout costs followed by an identical arg-min / top-k on every rank (SURVEY.md §8e).
+of per-rollout costs followed by an identical arg-min / top-k on every rank (SURVEY.md §8e) — and
+the receding-horizon loop built on it: the winners' terminal states are gathered from their owner
+ranks and re-seed every world for the next horizon (`mpc_iteration`).
 
 Worlds are independent (the reference already steps two unrelated ensembles per SimulationStep,
 /root/reference/eggshell/model.cc:67-68), so there is no data-path exchange inside a horizon."""
 import numpy as np
+
+STATE_PER_BODY = 18   # p(3), R(9, row-major), v(3), w(3): a row of egg_gather_state / egg_seed_state
 
 
 def shard_range(n_worlds_total, rank, world_size):
@@ -52,3 +56,67 @@ def owner_of(world_index, n_worlds_total, world_size):
         if lo <= world_index < hi:
             return r, world_index - lo
     raise IndexError(world_index)
+
+
+def gather_winner_states(winners, n_total, pack):
+    """Rows of the winning worlds, in `winners` order, identical on every rank: a [k, F] tensor.
+
+    winners: global world indices (duplicates allowed), the same on every rank (select_best).
+    pack(local_indices): this rank's rows for an int array of its local world indices, a [len, F]
+    tensor on the device of the collective (an empty array gives a [0, F] tensor).  Each rank fills
+    the slots of the winners it owns in a [world_size, k, F] buffer, one all_gather_into_tensor
+    shares it, and every winner is read from its owner's slot: nothing is summed, so the rows
+    (including -0.0) arrive bit for bit."""
+    import torch
+    import torch.distributed as dist
+    winners = np.asarray(winners, dtype=np.int64).ravel()
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
+        return pack(winners)
+    rank, ws = dist.get_rank(), dist.get_world_size()
+    owner = [owner_of(int(g), n_total, ws) for g in winners]
+    mine = np.array([i for i, (r, _) in enumerate(owner) if r == rank], dtype=np.int64)
+    rows = pack(np.array([owner[i][1] for i in mine], dtype=np.int64))
+    k, F = winners.size, rows.shape[1]
+    slot = torch.zeros((k, F), dtype=rows.dtype, device=rows.device)
+    if mine.size:
+        slot[torch.from_numpy(mine).to(rows.device)] = rows
+    buf = torch.empty((ws * k, F), dtype=rows.dtype, device=rows.device)   # [world_size, k, F] (gloo wants it flat)
+    dist.all_gather_into_tensor(buf, slot)
+    src = torch.tensor([r for r, _ in owner], dtype=torch.int64, device=rows.device)
+    return buf.view(ws, k, F)[src, torch.arange(k, device=rows.device)]
+
+
+def mpc_iteration(batch, u, dt, k, n_total, first):
+    """One receding-horizon iteration of a (sharded) random-shooting sweep.
+
+    From the batch's snapshot, every world runs the control schedule u (a contiguous float64 CUDA
+    tensor [H, W, n, 6] on the batch's device: slice t is the f_ext of step t); the per-world costs
+    are gathered over all ranks and the k best worlds win (select_best); their terminal states are
+    fetched from their owner ranks; world w of this shard (global index first + w) is re-seeded from
+    winner (first + w) % k and the seeded state is snapshotted as the next horizon's start.
+    The batch must run on torch's current stream (Batch.set_stream), on which u is produced.
+    Returns (winners, their costs, states [k, n * 18] float64 CUDA tensor)."""
+    import torch
+    dev = torch.device("cuda", int(batch.desc.device))
+    if not (isinstance(u, torch.Tensor) and u.is_cuda and u.device == dev and u.dtype == torch.float64
+            and u.is_contiguous() and u.dim() == 4 and u.shape[0] >= 1 and tuple(u.shape[1:]) == (batch.W, batch.n, 6)):
+        raise ValueError(f"u must be a contiguous float64 tensor [H >= 1, {batch.W}, {batch.n}, 6] on {dev}")
+    if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
+        raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
+    batch.restore()
+    batch.step_controlled(dt, u.data_ptr(), u.shape[0])
+    costs = torch.empty(batch.W, dtype=torch.float64, device=dev)
+    batch.rollout_costs(costs.data_ptr())
+    winners, best = select_best(allgather_costs(costs), k)
+    F = batch.n * STATE_PER_BODY
+
+    def pack(local):
+        out = torch.empty((len(local), F), dtype=torch.float64, device=dev)
+        if len(local):
+            batch.gather_state(local, out.data_ptr())
+        return out
+
+    states = gather_winner_states(winners, n_total, pack)
+    batch.seed_state(states.data_ptr(), len(winners), first)
+    batch.snapshot()
+    return winners, best, states

@@ -155,6 +155,29 @@ int egg_post_stabilize(egg_batch* b, int max_steps, int* steps_out, double* err_
  * the batch stream. */
 int egg_step(egg_batch* b, double dt, int integrator, int n_steps);
 
+/* Receding-horizon MPC (INTEGRATION.md).  The three calls below take DEVICE buffers on the batch's
+ * device (cudaPointerGetAttributes must report device or managed memory there, else EGG_ERR_ARG);
+ * their lengths cannot be checked through a raw pointer and are the caller's responsibility.  They
+ * are asynchronous on the batch stream: keep the buffers alive and unchanged until the next
+ * synchronising call.  Before egg_init they return EGG_ERR_STATE. */
+
+/* horizon x Ensemble::Step(dt, integrator) with a per-step control schedule: before step t the f_ext
+ * slot of every world is replaced by u_d[t], exactly what egg_set_external(u[t]) before
+ * egg_step(b, dt, integrator, 1) does.  u_d is [horizon][W][n_bodies][6], time-major, so every slice
+ * has the layout of egg_set_external.  After the call the slot holds u_d[horizon-1].  horizon >= 1. */
+int egg_step_controlled(egg_batch* b, double dt, int integrator, const double* u_d, int horizon);
+
+/* out_d[k][n_bodies][18] = (p(3), R(9, row-major), v(3), w(3)) of worlds[0..k), element for element
+ * what egg_get_bodies returns for those worlds.  worlds is a HOST int array, each entry in [0, W),
+ * duplicates allowed; 1 <= k <= W. */
+int egg_gather_state(egg_batch* b, const int* worlds, int k, double* out_d);
+
+/* World w takes the state in_d[(first + w) mod k] (the [k][n_bodies][18] layout of egg_gather_state);
+ * 1 <= k <= W, first >= 0.  first is the global index of local world 0 of a sharded sweep, so a
+ * world's seed does not depend on the sharding.  Only the live state is written: call egg_snapshot
+ * to make it the start of the next horizon.  The rollout cost keeps its egg_init reference pose. */
+int egg_seed_state(egg_batch* b, const double* in_d, int k, int first);
+
 /* Ensemble::UpdateContacts + CheckAndCorrectEnsembleState only (ensembles.cc:445-480, 241-329):
  * runs the narrowphase kernel on the current state without stepping; read the result with
  * egg_get_contacts / egg_get_pair_hits. */
