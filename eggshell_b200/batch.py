@@ -23,7 +23,7 @@ ST_LCP_FAILED, ST_JOINT_CONFLICT, ST_BAD_INIT, ST_CONTACT_OVERFLOW, ST_NONFINITE
 EXPORTS = [
     "egg_desc_default", "egg_create", "egg_destroy", "egg_set_bodies", "egg_set_shapes", "egg_set_state", "egg_set_joints",
     "egg_set_external", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_step_controlled",
-    "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
+    "egg_set_cost", "egg_step_controlled_cost", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
     "egg_get_status", "egg_get_dense_work", "egg_get_debug_counters", "egg_rollout_costs", "egg_set_stream", "egg_sync", "egg_device_bytes",
     "egg_launch_count", "egg_capacity", "egg_set_profiling", "egg_get_kernel_ms", "egg_fp64_peak_tflops", "egg_host_alloc", "egg_host_free", "egg_last_error", "egg_version",
 ]
@@ -36,6 +36,13 @@ class EggDesc(C.Structure):
         ("tol", C.c_double), ("cfm", C.c_double), ("erp", C.c_double), ("gravity", C.c_double * 3),
         ("min_constraint_dist", C.c_double),
         ("quirks", C.c_int), ("cfm_mode", C.c_int), ("device", C.c_int), ("taps", C.c_int),
+    ]
+
+
+class EggCost(C.Structure):
+    _fields_ = [
+        ("q_run", C.c_void_p), ("l_run", C.c_void_p), ("u_run", C.c_void_p), ("q_term", C.c_void_p),
+        ("l_term", C.c_void_p), ("x_ref", C.c_void_p), ("ref_steps", C.c_int),
     ]
 
 
@@ -66,6 +73,8 @@ def lib():
         L.egg_set_stream.argtypes = [C.c_void_p, C.c_void_p]
         L.egg_rollout_costs.argtypes = [C.c_void_p, C.c_void_p]
         L.egg_step_controlled.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_void_p, C.c_int]
+        L.egg_set_cost.argtypes = [C.c_void_p, C.c_void_p]
+        L.egg_step_controlled_cost.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_void_p, C.c_int, C.c_void_p]
         L.egg_gather_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.egg_seed_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
         _LIB = L
@@ -118,6 +127,7 @@ class Batch:
         self.W, self.n, self.nj = n_worlds, n_bodies, n_joints
         self.desc = d
         self.stream = None   # cudaStream_t handed to set_stream; None = the batch's own stream
+        self.cost = None     # mpc.QuadraticCost handed to set_cost
         self.max_contacts = None
         self._probe_capacity()
 
@@ -197,6 +207,26 @@ class Batch:
         float64 [horizon][W][n][6] (egg_step_controlled)."""
         _chk(lib().egg_step_controlled(self.h, C.c_double(dt), int(integrator), C.c_void_p(u_ptr), int(horizon)),
              "egg_step_controlled")
+
+    def set_cost(self, cost):
+        """Configures the cost of step_controlled_cost: an mpc.QuadraticCost for this batch's n bodies,
+        or None to clear it (egg_set_cost).  Synchronises the batch stream."""
+        from .mpc import QuadraticCost
+        if cost is None:
+            _chk(lib().egg_set_cost(self.h, None), "egg_set_cost")
+        else:
+            if not isinstance(cost, QuadraticCost) or cost.n != self.n:
+                raise ValueError(f"set_cost takes an mpc.QuadraticCost for n = {self.n} bodies, or None")
+            c = EggCost(_p(cost.q_run), _p(cost.l_run), _p(cost.u_run), _p(cost.q_term), _p(cost.l_term),
+                        _p(cost.x_ref), cost.ref_steps)
+            _chk(lib().egg_set_cost(self.h, C.byref(c)), "egg_set_cost")
+        self.cost = cost
+
+    def step_controlled_cost(self, dt, u_ptr, horizon, cost_ptr, integrator=OPEN_DYNAMICS_ENGINE):
+        """step_controlled that also writes the configured cost J of every world to the device buffer
+        at cost_ptr, float64 [W] (egg_step_controlled_cost)."""
+        _chk(lib().egg_step_controlled_cost(self.h, C.c_double(dt), int(integrator), C.c_void_p(u_ptr), int(horizon),
+                                            C.c_void_p(cost_ptr)), "egg_step_controlled_cost")
 
     # -- device-side state exchange (MPC) ------------------------------------------------------
     def gather_state(self, worlds, out_ptr):

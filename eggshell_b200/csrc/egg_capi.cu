@@ -65,6 +65,9 @@ struct egg_batch {
   int device = 0;
   double* snap = nullptr;        // egg_snapshot copy of dev.dyn
   int* gather_idx = nullptr;     // [W] world indices of egg_gather_state, allocated by its first call
+  double* cost_buf = nullptr;    // egg_set_cost arrays (EggCost layout); null = no cost set
+  size_t cost_bytes = 0;
+  EggCost cost = {};             // pointers into cost_buf
   bool profiling = false;
   std::vector<cudaEvent_t> ev;   // 4 per profiled step
   std::vector<cudaEvent_t> ev_free;
@@ -92,6 +95,14 @@ static int dalloc(egg_batch* b, T** p, size_t count) {
   b->allocs.push_back(q);
   b->bytes += (long long)bytes;
   *p = (T*)q;
+  return EGG_OK;
+}
+// Releases one dalloc'd buffer before egg_destroy, once the work queued on the stream is done with it.
+static int dfree(egg_batch* b, void* p, size_t bytes) {
+  CK(cudaStreamSynchronize(b->stream));
+  CK(cudaFree(p));
+  b->allocs.erase(std::find(b->allocs.begin(), b->allocs.end(), p));
+  b->bytes -= (long long)bytes;
   return EGG_OK;
 }
 #define DA(ptr, count)                                  \
@@ -551,8 +562,10 @@ static int check_device_ptr(egg_batch* b, const void* p, const char* what) {
 }
 
 // n_steps x Ensemble::Step.  With a control schedule u_d ([n_steps][W][n][6]), slice s is copied into
-// the f_ext slot before step s (outside the profiled kernel buckets).
-static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d) {
+// the f_ext slot before step s (outside the profiled kernel buckets).  With cost_d as well, that copy
+// is the kernel that also adds the running cost of step s to cost_d, and the terminal cost follows
+// the last step.
+static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d, double* cost_d) {
   const int solver = b->dev.prm.solver;
   if (solver < EGG_SOLVER_DENSE_MURTY || solver > EGG_SOLVER_SOR) { g_err = "unknown solver"; return EGG_ERR_ARG; }
   CK(cudaSetDevice(b->device));
@@ -568,7 +581,8 @@ static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d) {
   const size_t slice = (size_t)b->dev.W * b->dev.n * 6;
   for (int s = 0; s < n_steps; s++) {
     if (u_d) {
-      LK(egg_launch_fext_slice(b->dev, u_d + (size_t)s * slice, b->stream));
+      if (cost_d) LK(egg_launch_fext_slice_cost(b->dev, u_d + (size_t)s * slice, b->cost, s, cost_d, b->stream));
+      else LK(egg_launch_fext_slice(b->dev, u_d + (size_t)s * slice, b->stream));
       b->launches++;
     }
     cudaEvent_t e[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -601,13 +615,17 @@ static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d) {
     if (b->profiling) CK(cudaEventRecord(e[3], b->stream));
     b->launches += (solver == EGG_SOLVER_PGS && b->dev.rec_fmt) ? 5 : 3;   // collide, assemble (1 or 3 kernels), solve
   }
+  if (cost_d) {
+    LK(egg_launch_cost_terminal(b->dev, b->cost, n_steps, cost_d, b->stream));
+    b->launches++;
+  }
   CK(cudaGetLastError());
   return EGG_OK;
 }
 
 int egg_step(egg_batch* b, double dt, int integrator, int n_steps) {
   RET(step_check(b, dt, integrator, n_steps, "egg_step"));
-  return step_loop(b, dt, n_steps, nullptr);
+  return step_loop(b, dt, n_steps, nullptr, nullptr);
 }
 
 int egg_step_controlled(egg_batch* b, double dt, int integrator, const double* u_d, int horizon) {
@@ -615,7 +633,62 @@ int egg_step_controlled(egg_batch* b, double dt, int integrator, const double* u
   if (horizon < 1) { g_err = "egg_step_controlled: horizon must be >= 1"; return EGG_ERR_ARG; }
   RET(step_check(b, dt, integrator, horizon, "egg_step_controlled"));
   RET(check_device_ptr(b, u_d, "egg_step_controlled(u_d)"));
-  return step_loop(b, dt, horizon, u_d);
+  return step_loop(b, dt, horizon, u_d, nullptr);
+}
+
+int egg_step_controlled_cost(egg_batch* b, double dt, int integrator, const double* u_d, int horizon, double* cost_d) {
+  if (!b || !u_d) return EGG_ERR_ARG;
+  if (horizon < 1) { g_err = "egg_step_controlled_cost: horizon must be >= 1"; return EGG_ERR_ARG; }
+  RET(step_check(b, dt, integrator, horizon, "egg_step_controlled_cost"));
+  RET(check_device_ptr(b, u_d, "egg_step_controlled_cost(u_d)"));
+  RET(check_device_ptr(b, cost_d, "egg_step_controlled_cost(cost_d)"));
+  if (!b->cost_buf) { g_err = "egg_step_controlled_cost without a cost: call egg_set_cost first"; return EGG_ERR_STATE; }
+  if (b->cost.ref_steps > 1 && b->cost.ref_steps < horizon + 1) {
+    g_err = "egg_step_controlled_cost: the cost's reference has " + std::to_string(b->cost.ref_steps) + " rows, fewer than horizon + 1 = " +
+            std::to_string(horizon + 1);
+    return EGG_ERR_ARG;
+  }
+  return step_loop(b, dt, horizon, u_d, cost_d);
+}
+
+int egg_set_cost(egg_batch* b, const egg_cost* c) {
+  if (!b) return EGG_ERR_ARG;
+  const size_t n = (size_t)b->dev.n, nd = (size_t)EGG_DYN * n;
+  std::vector<double> h;   // the EggCost layout: q_run, l_run, q_term, l_term [18][n], u_run [6][n], x_ref [R][18][n]
+  int R = 1;
+  if (c) {
+    if (c->x_ref) R = c->ref_steps;
+    if (R < 1) { g_err = "egg_set_cost: ref_steps must be >= 1"; return EGG_ERR_ARG; }
+    h.assign(4 * nd + 6 * n + (size_t)R * nd, 0.0);
+    struct { const double* src; size_t rows, comps, off; } part[6] = {
+        {c->q_run, 1, EGG_DYN, 0}, {c->l_run, 1, EGG_DYN, nd}, {c->q_term, 1, EGG_DYN, 2 * nd},
+        {c->l_term, 1, EGG_DYN, 3 * nd}, {c->u_run, 1, 6, 4 * nd}, {c->x_ref, (size_t)R, EGG_DYN, 4 * nd + 6 * n}};
+    for (auto& p : part) {
+      if (!p.src) continue;
+      for (size_t r = 0; r < p.rows; r++)
+        for (size_t i = 0; i < n; i++)
+          for (size_t k = 0; k < p.comps; k++) {
+            const double v = p.src[(r * n + i) * p.comps + k];   // host [rows][n][comps] -> [rows][comps][n]
+            if (!std::isfinite(v)) { g_err = "egg_set_cost: non-finite weight or reference value"; return EGG_ERR_ARG; }
+            h[p.off + (r * p.comps + k) * n + i] = v;
+          }
+    }
+  }
+  CK(cudaSetDevice(b->device));
+  if (b->cost_buf) {
+    RET(dfree(b, b->cost_buf, b->cost_bytes));
+    b->cost_buf = nullptr;
+    b->cost_bytes = 0;
+    b->cost = EggCost{};
+  }
+  if (!c) return EGG_OK;
+  RET(dalloc(b, &b->cost_buf, h.size()));
+  b->cost_bytes = h.size() * sizeof(double);
+  CK(cudaMemcpyAsync(b->cost_buf, h.data(), b->cost_bytes, cudaMemcpyHostToDevice, b->stream));
+  CK(cudaStreamSynchronize(b->stream));   // h is a temporary
+  const double* q = b->cost_buf;
+  b->cost = EggCost{q, q + nd, q + 4 * nd, q + 2 * nd, q + 3 * nd, q + 4 * nd + 6 * n, R};
+  return EGG_OK;
 }
 
 int egg_gather_state(egg_batch* b, const int* worlds, int k, double* out_d) {

@@ -158,6 +158,21 @@ cudaError_t egg_launch_fext_slice(const EggDev& d, const double* u, cudaStream_t
 // dyn of worlds[0..k) (device int array) -> out [k][n][18]; dyn of world w <- in [(first + w) mod k][n][18]
 cudaError_t egg_launch_gather_state(const EggDev& d, const int* worlds, int k, double* out, cudaStream_t s);
 cudaError_t egg_launch_seed_state(const EggDev& d, const double* in, int k, int first, cudaStream_t s);
+// Device copy of egg_set_cost, shared by all worlds and stored component-major ([c][n], the body
+// index fastest, like dyn) so that the lanes of a warp read consecutive words.
+struct EggCost {
+  const double* q_run;    // [18][n]
+  const double* l_run;    // [18][n]
+  const double* u_run;    // [6][n]
+  const double* q_term;   // [18][n]
+  const double* l_term;   // [18][n]
+  const double* x_ref;    // [ref_steps][18][n]
+  int ref_steps;
+};
+// egg_launch_fext_slice that also adds the running cost at (x_t, u_t) to cost[W] (stores it at t = 0);
+// the terminal term at x_horizon is added after the last step
+cudaError_t egg_launch_fext_slice_cost(const EggDev& d, const double* u, const EggCost& c, int t, double* cost, cudaStream_t s);
+cudaError_t egg_launch_cost_terminal(const EggDev& d, const EggCost& c, int horizon, double* cost, cudaStream_t s);
 // Dynamic shared memory each kernel family needs for this batch shape (checked against the device
 // limit in egg_create, so that an unsupported shape fails there with a clear message).
 size_t egg_collide_smem(const EggDev& d);

@@ -1,4 +1,5 @@
-// Init, rollout cost, AoS<->SoA staging and the FP64 roofline probe (assembly + PGS: egg_pgs.cu).
+// Init, rollout costs, MPC control slices and state exchange, AoS<->SoA staging and the FP64
+// roofline probe (assembly + PGS: egg_pgs.cu).
 //
 // Replaces (per world):
 //   egg_init_kernel        Ensemble::Init pieces          ensembles.cc:24-29, 202-232
@@ -176,6 +177,68 @@ __global__ void egg_fext_slice_kernel(const double* u, int W, int n, double* sta
   stat[((size_t)w * EGG_STAT + 10 + c) * n + b] = u[((size_t)w * n + b) * 6 + c];
 }
 
+// The configurable MPC cost (egg_set_cost): one warp per world, lane l takes bodies l, l + 32, ...
+// in that order and a fixed shuffle tree sums the lanes, so the summation order depends only on n:
+// a world's cost has the same bits in any batch, shard or launch shape.
+__device__ inline double egg_warp_sum(double s) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+  return s;
+}
+
+// sum_c q[c] d[c]^2 + l[c] d[c] over the 18 state components of body b, d = x - x_ref ([c][n] arrays)
+__device__ inline double egg_state_cost(const double* x, const double* xr, const double* q, const double* l, int n, int b) {
+  double s = 0.0;
+#pragma unroll
+  for (int c = 0; c < EGG_DYN; c++) {
+    const double d = x[c * n + b] - xr[c * n + b];
+    s += (q[c * n + b] * d + l[c * n + b]) * d;
+  }
+  return s;
+}
+
+// egg_fext_slice_kernel fused with the running cost of step t: the same f_ext writes, and
+// cost[w] (= at t = 0, += after) the running term at (x_t, u_t), read in the same pass.  Left alone,
+// ptxas hoists all 84 loads of a body and takes 255 registers with spills; the bound caps it at 64.
+__global__ void __launch_bounds__(256, 4) egg_fext_slice_cost_kernel(const double* __restrict__ u, int W, int n, double* __restrict__ stat,
+                                           const double* __restrict__ dyn, EggCost cc, const double* __restrict__ xr,
+                                           int t, double* __restrict__ cost) {
+  const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (w >= W) return;   // uniform over the warp
+  const int lane = threadIdx.x & 31;
+  const double* x = dyn + (size_t)w * EGG_DYN * n;
+  double* f = stat + ((size_t)w * EGG_STAT + 10) * n;
+  double s = 0.0;
+#pragma unroll 1
+  for (int b = lane; b < n; b += 32) {
+    const double* ub = u + ((size_t)w * n + b) * 6;
+    double r = egg_state_cost(x, xr, cc.q_run, cc.l_run, n, b);
+#pragma unroll
+    for (int j = 0; j < 6; j++) {
+      const double uj = ub[j];
+      f[j * n + b] = uj;
+      r += cc.u_run[j * n + b] * uj * uj;
+    }
+    s += r;
+  }
+  s = egg_warp_sum(s);
+  if (lane == 0) cost[w] = (t == 0) ? s : cost[w] + s;
+}
+
+// The terminal term at x_H: cost[w] += sum_b sum_c q_term d^2 + l_term d.
+__global__ void egg_cost_terminal_kernel(int W, int n, const double* __restrict__ dyn, EggCost cc,
+                                         const double* __restrict__ xr, double* __restrict__ cost) {
+  const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (w >= W) return;
+  const int lane = threadIdx.x & 31;
+  const double* x = dyn + (size_t)w * EGG_DYN * n;
+  double s = 0.0;
+#pragma unroll 1
+  for (int b = lane; b < n; b += 32) s += egg_state_cost(x, xr, cc.q_term, cc.l_term, n, b);
+  s = egg_warp_sum(s);
+  if (lane == 0) cost[w] += s;
+}
+
 // The unpack kernel with a world-index map: dyn [W][18][n] of worlds[i] -> AoS out [k][n][18], the
 // per-body order of egg_get_bodies (p, R row-major, v, w).
 __global__ void egg_gather_state_kernel(const double* dyn, int n, const int* worlds, int k, double* out) {
@@ -281,6 +344,20 @@ cudaError_t egg_launch_unpack(int W, double* aos, int per_world, int comps, cons
 cudaError_t egg_launch_fext_slice(const EggDev& d, const double* u, cudaStream_t s) {
   const long long total = (long long)d.W * 6 * d.n;
   egg_fext_slice_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(u, d.W, d.n, d.stat);
+  return cudaGetLastError();
+}
+// x_ref row of step t (row 0 for a constant reference)
+static const double* cost_ref_row(const EggDev& d, const EggCost& c, int t) {
+  return c.x_ref + (size_t)(c.ref_steps == 1 ? 0 : t) * EGG_DYN * d.n;
+}
+cudaError_t egg_launch_fext_slice_cost(const EggDev& d, const double* u, const EggCost& c, int t, double* cost, cudaStream_t s) {
+  const long long threads = (long long)d.W * 32;   // one warp per world
+  egg_fext_slice_cost_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(u, d.W, d.n, d.stat, d.dyn, c, cost_ref_row(d, c, t), t, cost);
+  return cudaGetLastError();
+}
+cudaError_t egg_launch_cost_terminal(const EggDev& d, const EggCost& c, int horizon, double* cost, cudaStream_t s) {
+  const long long threads = (long long)d.W * 32;
+  egg_cost_terminal_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(d.W, d.n, d.dyn, c, cost_ref_row(d, c, horizon), cost);
   return cudaGetLastError();
 }
 cudaError_t egg_launch_gather_state(const EggDev& d, const int* worlds, int k, double* out, cudaStream_t s) {

@@ -8,6 +8,68 @@ Worlds are independent (the reference already steps two unrelated ensembles per 
 import numpy as np
 
 STATE_PER_BODY = 18   # p(3), R(9, row-major), v(3), w(3): a row of egg_gather_state / egg_seed_state
+CONTROL_PER_BODY = 6  # f(3), tau(3): a row of egg_set_external / a control schedule slice
+
+
+class QuadraticCost:
+    """A quadratic running + terminal cost over a controlled horizon, shared by all worlds
+    (Batch.set_cost, egg_set_cost).  With x_t [n, 18] the state before step t, x_H the state after
+    the last step, u_t [n, 6] the control of step t and d_t = x_t - x_ref[t]:
+
+        J = sum_{t<H} sum_b [ sum_c q_run[b,c] d_t[b,c]^2 + l_run[b,c] d_t[b,c] + sum_j u_run[b,j] u_t[b,j]^2 ]
+          +           sum_b   sum_c q_term[b,c] d_H[b,c]^2 + l_term[b,c] d_H[b,c]
+
+    The weights broadcast to [n, 18] ([n, 6] for u_run); x_ref broadcasts to [n, 18] (one reference
+    for every step) or is [ref_steps, n, 18] with ref_steps >= H + 1 (row t for step t).  The linear
+    terms express progress: l_term[0, 0] = -1 rewards body 0 for moving along +x.  Every value must
+    be finite."""
+
+    def __init__(self, n, q_run=0.0, l_run=0.0, u_run=0.0, q_term=0.0, l_term=0.0, x_ref=0.0):
+        n = int(n)
+        if n < 1:
+            raise ValueError("QuadraticCost: n must be >= 1")
+        self.n = n
+        S, U = STATE_PER_BODY, CONTROL_PER_BODY
+        self.q_run, self.l_run, self.q_term, self.l_term = (self._arr(a, (n, S), name) for a, name in
+                                                            ((q_run, "q_run"), (l_run, "l_run"), (q_term, "q_term"), (l_term, "l_term")))
+        self.u_run = self._arr(u_run, (n, U), "u_run")
+        x = np.asarray(x_ref, dtype=np.float64)
+        if x.ndim == 3:
+            if x.shape[0] < 1:
+                raise ValueError("QuadraticCost: x_ref needs ref_steps >= 1 rows")
+            self.x_ref = self._arr(x, (x.shape[0], n, S), "x_ref")
+        elif x.ndim <= 2:
+            self.x_ref = self._arr(x, (1, n, S), "x_ref")
+        else:
+            raise ValueError(f"QuadraticCost: x_ref must broadcast to [{n}, {S}] or be [ref_steps, {n}, {S}]")
+        self.ref_steps = self.x_ref.shape[0]
+
+    @staticmethod
+    def _arr(a, shape, name):
+        a = np.asarray(a, dtype=np.float64)
+        try:
+            a = np.ascontiguousarray(np.broadcast_to(a, shape))
+        except ValueError:
+            raise ValueError(f"QuadraticCost: {name} of shape {a.shape} does not broadcast to {list(shape)}") from None
+        if not np.isfinite(a).all():
+            raise ValueError(f"QuadraticCost: {name} has non-finite values")
+        return a
+
+    def evaluate(self, states, u):
+        """The float64 numpy reference of J: states [H + 1, W, n, 18] (x_0 ... x_H), u [H, W, n, 6].
+        Returns J [W]."""
+        states, u = np.asarray(states, dtype=np.float64), np.asarray(u, dtype=np.float64)
+        if u.ndim != 4 or u.shape[0] < 1 or u.shape[2:] != (self.n, CONTROL_PER_BODY):
+            raise ValueError(f"u must be [H >= 1, W, {self.n}, {CONTROL_PER_BODY}]")
+        H, W = u.shape[:2]
+        if states.shape != (H + 1, W, self.n, STATE_PER_BODY):
+            raise ValueError(f"states must be [{H + 1}, {W}, {self.n}, {STATE_PER_BODY}] for a horizon of {H}")
+        if 1 < self.ref_steps < H + 1:
+            raise ValueError(f"the reference has {self.ref_steps} rows, fewer than H + 1 = {H + 1}")
+        ref = self.x_ref[np.minimum(np.arange(H + 1), self.ref_steps - 1)]   # [H + 1, n, 18]
+        d = states - ref[:, None]
+        run = (self.q_run * d[:H] ** 2 + self.l_run * d[:H]).sum(axis=(0, 2, 3)) + (self.u_run * u ** 2).sum(axis=(0, 2, 3))
+        return run + (self.q_term * d[H] ** 2 + self.l_term * d[H]).sum(axis=(1, 2))
 
 
 def shard_range(n_worlds_total, rank, world_size):
@@ -91,8 +153,9 @@ def mpc_iteration(batch, u, dt, k, n_total, first):
 
     From the batch's snapshot, every world runs the control schedule u (a contiguous float64 CUDA
     tensor [H, W, n, 6] on the batch's device: slice t is the f_ext of step t); the per-world costs
-    are gathered over all ranks and the k best worlds win (select_best); their terminal states are
-    fetched from their owner ranks; world w of this shard (global index first + w) is re-seeded from
+    (the QuadraticCost of Batch.set_cost, accumulated over the horizon on the device, or without one
+    the built-in egg_rollout_costs) are gathered over all ranks and the k best worlds win
+    (select_best); their terminal states are fetched from their owner ranks; world w of this shard (global index first + w) is re-seeded from
     winner (first + w) % k and the seeded state is snapshotted as the next horizon's start.
     The batch must run on torch's current stream (Batch.set_stream), on which u is produced.
     Returns (winners, their costs, states [k, n * 18] float64 CUDA tensor)."""
@@ -103,10 +166,13 @@ def mpc_iteration(batch, u, dt, k, n_total, first):
         raise ValueError(f"u must be a contiguous float64 tensor [H >= 1, {batch.W}, {batch.n}, 6] on {dev}")
     if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
         raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
-    batch.restore()
-    batch.step_controlled(dt, u.data_ptr(), u.shape[0])
     costs = torch.empty(batch.W, dtype=torch.float64, device=dev)
-    batch.rollout_costs(costs.data_ptr())
+    batch.restore()
+    if batch.cost is None:
+        batch.step_controlled(dt, u.data_ptr(), u.shape[0])
+        batch.rollout_costs(costs.data_ptr())
+    else:
+        batch.step_controlled_cost(dt, u.data_ptr(), u.shape[0], costs.data_ptr())
     winners, best = select_best(allgather_costs(costs), k)
     F = batch.n * STATE_PER_BODY
 

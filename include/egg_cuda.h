@@ -178,6 +178,39 @@ int egg_gather_state(egg_batch* b, const int* worlds, int k, double* out_d);
  * to make it the start of the next horizon.  The rollout cost keeps its egg_init reference pose. */
 int egg_seed_state(egg_batch* b, const double* in_d, int k, int first);
 
+/* A quadratic running + terminal cost over a controlled horizon, shared by all worlds.  A body's
+ * state row is x = (p(3), R(9, row-major), v(3), w(3)) (the egg_gather_state row), its control
+ * u = (f(3), tau(3)) (the egg_set_external row).  With x_t the state before step t, x_H the state
+ * after the last step and d_t = x_t - x_ref[t] (x_ref[t] = x_ref[0] when ref_steps = 1):
+ *   J = sum_{t<H} sum_b [ sum_c q_run[b][c] d_t[b][c]^2 + l_run[b][c] d_t[b][c] + sum_j u_run[b][j] u_t[b][j]^2 ]
+ *     +           sum_b   sum_c q_term[b][c] d_H[b][c]^2 + l_term[b][c] d_H[b][c]
+ * The linear terms express progress (l_term[0][0] = -1: reward body 0 for moving along +x).
+ * Non-finite states or controls propagate into J as computed. */
+typedef struct egg_cost {
+  const double* q_run;  /* [n_bodies][18]; NULL = all zero (every array is a HOST array) */
+  const double* l_run;  /* [n_bodies][18] */
+  const double* u_run;  /* [n_bodies][6] */
+  const double* q_term; /* [n_bodies][18] */
+  const double* l_term; /* [n_bodies][18] */
+  const double* x_ref;  /* [ref_steps][n_bodies][18]; NULL = zeros (ref_steps is then ignored) */
+  int ref_steps;        /* 1 (a constant reference) or >= horizon + 1 of every later rollout */
+} egg_cost;
+
+/* Copies the cost into device memory owned by the batch (counted by egg_device_bytes); c == NULL
+ * clears it and releases that memory.  Non-finite weights or reference values, or ref_steps < 1 with
+ * a reference, return EGG_ERR_ARG and leave the previous cost in place.  Valid before or after
+ * egg_init.  Synchronises the batch stream. */
+int egg_set_cost(egg_batch* b, const egg_cost* c);
+
+/* egg_step_controlled, bit for bit the same state and f_ext slot, that also writes J of every world
+ * (the cost of egg_set_cost) to the DEVICE buffer cost_d[W].  cost_d is overwritten, not added to.
+ * The sum runs in an order that depends only on n_bodies and the step, so a world's J has the same
+ * bits in any batch.  EGG_ERR_STATE without a cost or before egg_init; EGG_ERR_ARG for the arguments
+ * egg_step_controlled refuses, a cost_d that is not device memory of the batch's device, or
+ * 1 < ref_steps < horizon + 1.  Every check runs before the first launch; asynchronous on the
+ * batch stream. */
+int egg_step_controlled_cost(egg_batch* b, double dt, int integrator, const double* u_d, int horizon, double* cost_d);
+
 /* Ensemble::UpdateContacts + CheckAndCorrectEnsembleState only (ensembles.cc:445-480, 241-329):
  * runs the narrowphase kernel on the current state without stepping; read the result with
  * egg_get_contacts / egg_get_pair_hits. */
@@ -231,7 +264,8 @@ int egg_get_debug_counters(egg_batch* b, unsigned long long* out32, int reset);
 
 /* MPC rollout cost per world written to a DEVICE buffer of n_worlds doubles (feeds the NCCL
  * allgather): cost = -(x_body0 - x0_body0) + 10 (z_body0 - z0_body0)^2 with (x0,z0) the pose at
- * egg_init.  The reference has no cost function; this definition is ours (SURVEY.md §8d C5). */
+ * egg_init.  The reference has no cost function; this definition is ours (SURVEY.md §8d C5).
+ * A configurable cost accumulated over the horizon: egg_set_cost / egg_step_controlled_cost. */
 int egg_rollout_costs(egg_batch* b, double* cost_d);
 
 /* Stream plumbing: run the batch on a caller-owned cudaStream_t (e.g. torch's current stream) so
