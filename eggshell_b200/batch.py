@@ -23,7 +23,7 @@ ST_LCP_FAILED, ST_JOINT_CONFLICT, ST_BAD_INIT, ST_CONTACT_OVERFLOW, ST_NONFINITE
 EXPORTS = [
     "egg_desc_default", "egg_create", "egg_destroy", "egg_set_bodies", "egg_set_shapes", "egg_set_state", "egg_set_joints",
     "egg_set_external", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_step_controlled",
-    "egg_set_cost", "egg_step_controlled_cost", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
+    "egg_set_cost", "egg_step_controlled_cost", "egg_set_sampler", "egg_sample_controls", "egg_mppi_reduce", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
     "egg_get_status", "egg_get_dense_work", "egg_get_debug_counters", "egg_rollout_costs", "egg_set_stream", "egg_sync", "egg_device_bytes",
     "egg_launch_count", "egg_capacity", "egg_set_profiling", "egg_get_kernel_ms", "egg_fp64_peak_tflops", "egg_host_alloc", "egg_host_free", "egg_last_error", "egg_version",
 ]
@@ -44,6 +44,10 @@ class EggCost(C.Structure):
         ("q_run", C.c_void_p), ("l_run", C.c_void_p), ("u_run", C.c_void_p), ("q_term", C.c_void_p),
         ("l_term", C.c_void_p), ("x_ref", C.c_void_p), ("ref_steps", C.c_int),
     ]
+
+
+class EggSampler(C.Structure):
+    _fields_ = [("sigma", C.c_void_p), ("u_lo", C.c_void_p), ("u_hi", C.c_void_p)]
 
 
 class EggError(RuntimeError):
@@ -77,6 +81,9 @@ def lib():
         L.egg_step_controlled_cost.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_void_p, C.c_int, C.c_void_p]
         L.egg_gather_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.egg_seed_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
+        L.egg_set_sampler.argtypes = [C.c_void_p, C.c_void_p]
+        L.egg_sample_controls.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_ulonglong, C.c_ulonglong, C.c_int, C.c_void_p]
+        L.egg_mppi_reduce.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
         _LIB = L
     return _LIB
 
@@ -128,6 +135,7 @@ class Batch:
         self.desc = d
         self.stream = None   # cudaStream_t handed to set_stream; None = the batch's own stream
         self.cost = None     # mpc.QuadraticCost handed to set_cost
+        self.sampler = None  # mpc.MPPI handed to set_sampler
         self.max_contacts = None
         self._probe_capacity()
 
@@ -227,6 +235,34 @@ class Batch:
         at cost_ptr, float64 [W] (egg_step_controlled_cost)."""
         _chk(lib().egg_step_controlled_cost(self.h, C.c_double(dt), int(integrator), C.c_void_p(u_ptr), int(horizon),
                                             C.c_void_p(cost_ptr)), "egg_step_controlled_cost")
+
+    # -- MPPI sampling and weighted reduction --------------------------------------------------
+    def set_sampler(self, mppi):
+        """Configures the noise scale and control bounds of sample_controls from an mpc.MPPI for this
+        batch's n bodies, or None to clear them (egg_set_sampler).  Synchronises the batch stream."""
+        from .mpc import MPPI
+        if mppi is None:
+            _chk(lib().egg_set_sampler(self.h, None), "egg_set_sampler")
+        else:
+            if not isinstance(mppi, MPPI) or mppi.n != self.n:
+                raise ValueError(f"set_sampler takes an mpc.MPPI for n = {self.n} bodies, or None")
+            s = EggSampler(_p(mppi.sigma), _p(mppi.u_lo), _p(mppi.u_hi))
+            _chk(lib().egg_set_sampler(self.h, C.byref(s)), "egg_set_sampler")
+        self.sampler = mppi
+
+    def sample_controls(self, u_nom_ptr, horizon, seed, iteration, first, u_ptr):
+        """Writes the perturbed schedules float64 [horizon][W][n][6] to the device buffer at u_ptr from
+        the nominal schedule [horizon][n][6] at u_nom_ptr (egg_sample_controls).  `first` is the global
+        index of local world 0; global world 0 gets no noise."""
+        _chk(lib().egg_sample_controls(self.h, C.c_void_p(u_nom_ptr), int(horizon), C.c_ulonglong(int(seed)),
+                                       C.c_ulonglong(int(iteration)), int(first), C.c_void_p(u_ptr)), "egg_sample_controls")
+
+    def mppi_reduce(self, u_ptr, horizon, cost_ptr, baseline_ptr, lam, out_ptr):
+        """out (device, float64 [horizon n 6 + 2]) = sum_w omega_w u[t][w], sum omega, sum omega^2 with
+        omega_w = exp(-(cost[w] - baseline) / lam), 0 for a non-finite cost (egg_mppi_reduce).
+        baseline_ptr is a device scalar."""
+        _chk(lib().egg_mppi_reduce(self.h, C.c_void_p(u_ptr), int(horizon), C.c_void_p(cost_ptr), C.c_void_p(baseline_ptr),
+                                   C.c_double(lam), C.c_void_p(out_ptr)), "egg_mppi_reduce")
 
     # -- device-side state exchange (MPC) ------------------------------------------------------
     def gather_state(self, worlds, out_ptr):

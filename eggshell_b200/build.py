@@ -20,6 +20,7 @@ UNITS = [
     ("egg_pgs_stream.cu", []),
     ("egg_pgs_runs.cu", []),
     ("egg_dense.cu", ["-fmad=false"]),
+    ("egg_mppi.cu", []),
     ("egg_capi.cu", []),
 ]
 

@@ -10,6 +10,9 @@
 #include <string>
 #include <vector>
 #include <algorithm>
+#include <climits>
+#include <cstdint>
+#include <limits>
 
 cudaError_t egg_launch_solve_dense(const EggDev& d, double dt, cudaStream_t s, void* scratch, size_t scratch_bytes);
 size_t egg_dense_scratch_bytes(const EggDev& d);
@@ -68,6 +71,10 @@ struct egg_batch {
   double* cost_buf = nullptr;    // egg_set_cost arrays (EggCost layout); null = no cost set
   size_t cost_bytes = 0;
   EggCost cost = {};             // pointers into cost_buf
+  double* sampler_buf = nullptr; // egg_set_sampler arrays (EggSampler layout); null = no sampler set
+  EggSampler sampler = {};       // pointers into sampler_buf
+  double* mppi_partial = nullptr;  // stage-1 partials of egg_mppi_reduce, grown on demand
+  size_t mppi_partial_count = 0;
   bool profiling = false;
   std::vector<cudaEvent_t> ev;   // 4 per profiled step
   std::vector<cudaEvent_t> ev_free;
@@ -688,6 +695,88 @@ int egg_set_cost(egg_batch* b, const egg_cost* c) {
   CK(cudaStreamSynchronize(b->stream));   // h is a temporary
   const double* q = b->cost_buf;
   b->cost = EggCost{q, q + nd, q + 4 * nd, q + 2 * nd, q + 3 * nd, q + 4 * nd + 6 * n, R};
+  return EGG_OK;
+}
+
+int egg_set_sampler(egg_batch* b, const egg_sampler* s) {
+  if (!b) return EGG_ERR_ARG;
+  const size_t n = (size_t)b->dev.n, nc = 6 * n;
+  std::vector<double> h;   // the EggSampler layout: sigma, lo, hi, each [6][n]
+  if (s) {
+    if (!s->sigma) { g_err = "egg_set_sampler: sigma is required"; return EGG_ERR_ARG; }
+    h.assign(3 * nc, 0.0);
+    const double inf = std::numeric_limits<double>::infinity();
+    for (size_t i = 0; i < n; i++)
+      for (size_t j = 0; j < 6; j++) {
+        const double sg = s->sigma[i * 6 + j];
+        const double lo = s->u_lo ? s->u_lo[i * 6 + j] : -inf, hi = s->u_hi ? s->u_hi[i * 6 + j] : inf;
+        if (!std::isfinite(sg) || sg < 0) { g_err = "egg_set_sampler: sigma must be finite and >= 0"; return EGG_ERR_ARG; }
+        if (std::isnan(lo) || std::isnan(hi)) { g_err = "egg_set_sampler: NaN bound"; return EGG_ERR_ARG; }
+        if (lo > hi) { g_err = "egg_set_sampler: u_lo > u_hi"; return EGG_ERR_ARG; }
+        h[j * n + i] = sg;   // host [n][6] -> [6][n]
+        h[nc + j * n + i] = lo;
+        h[2 * nc + j * n + i] = hi;
+      }
+  }
+  CK(cudaSetDevice(b->device));
+  double* buf = nullptr;   // the new sampler is in device memory before the old one goes
+  if (s) {
+    RET(dalloc(b, &buf, h.size()));
+    CK(cudaMemcpyAsync(buf, h.data(), h.size() * sizeof(double), cudaMemcpyHostToDevice, b->stream));
+  }
+  CK(cudaStreamSynchronize(b->stream));   // h is a temporary; queued samplers are done with the old buffer
+  if (b->sampler_buf) RET(dfree(b, b->sampler_buf, 3 * nc * sizeof(double)));
+  b->sampler_buf = buf;
+  b->sampler = s ? EggSampler{buf, buf + nc, buf + 2 * nc} : EggSampler{};
+  return EGG_OK;
+}
+
+// The double2 accesses of the sampler need 16-byte aligned schedules.
+static int check_aligned16(const void* p, const char* what) {
+  if ((uintptr_t)p & 15) { g_err = std::string(what) + ": must be 16-byte aligned"; return EGG_ERR_ARG; }
+  return EGG_OK;
+}
+
+int egg_sample_controls(egg_batch* b, const double* u_nom_d, int horizon, unsigned long long seed,
+                        unsigned long long iteration, int first, double* u_d) {
+  if (!b) return EGG_ERR_ARG;
+  if (horizon < 1 || first < 0) { g_err = "egg_sample_controls: horizon must be >= 1 and first >= 0"; return EGG_ERR_ARG; }
+  RET(check_device_ptr(b, u_nom_d, "egg_sample_controls(u_nom_d)"));
+  RET(check_device_ptr(b, u_d, "egg_sample_controls(u_d)"));
+  RET(check_aligned16(u_nom_d, "egg_sample_controls(u_nom_d)"));
+  RET(check_aligned16(u_d, "egg_sample_controls(u_d)"));
+  if (!b->initialised) { g_err = "egg_sample_controls before egg_init"; return EGG_ERR_STATE; }
+  if (!b->sampler_buf) { g_err = "egg_sample_controls without a sampler: call egg_set_sampler first"; return EGG_ERR_STATE; }
+  CK(cudaSetDevice(b->device));
+  LK(egg_launch_mppi_sample(b->dev, b->sampler, u_nom_d, horizon, seed, iteration, first, u_d, b->stream));
+  b->launches++;
+  return EGG_OK;
+}
+
+int egg_mppi_reduce(egg_batch* b, const double* u_d, int horizon, const double* cost_d, const double* baseline_d,
+                    double lambda, double* out_d) {
+  if (!b) return EGG_ERR_ARG;
+  if (!(lambda > 0) || !std::isfinite(lambda)) { g_err = "egg_mppi_reduce: lambda must be finite and > 0"; return EGG_ERR_ARG; }
+  if (horizon < 1) { g_err = "egg_mppi_reduce: horizon must be >= 1"; return EGG_ERR_ARG; }
+  const int chunks = egg_mppi_chunks(b->dev.W);
+  const long long cols = (long long)horizon * b->dev.n * 6 + 2;
+  if (chunks > 65535 || cols > INT_MAX) { g_err = "egg_mppi_reduce: too many worlds or too long a horizon"; return EGG_ERR_ARG; }
+  RET(check_device_ptr(b, u_d, "egg_mppi_reduce(u_d)"));
+  RET(check_device_ptr(b, cost_d, "egg_mppi_reduce(cost_d)"));
+  RET(check_device_ptr(b, baseline_d, "egg_mppi_reduce(baseline_d)"));
+  RET(check_device_ptr(b, out_d, "egg_mppi_reduce(out_d)"));
+  if (!b->initialised) { g_err = "egg_mppi_reduce before egg_init"; return EGG_ERR_STATE; }
+  CK(cudaSetDevice(b->device));
+  const size_t need = (size_t)chunks * (size_t)cols;
+  if (need > b->mppi_partial_count) {
+    if (b->mppi_partial) RET(dfree(b, b->mppi_partial, b->mppi_partial_count * sizeof(double)));
+    b->mppi_partial = nullptr;
+    b->mppi_partial_count = 0;
+    RET(dalloc(b, &b->mppi_partial, need));
+    b->mppi_partial_count = need;
+  }
+  LK(egg_launch_mppi_reduce(b->dev, u_d, horizon, cost_d, baseline_d, lambda, b->mppi_partial, out_d, b->stream));
+  b->launches += 2;
   return EGG_OK;
 }
 

@@ -173,6 +173,19 @@ struct EggCost {
 // the terminal term at x_horizon is added after the last step
 cudaError_t egg_launch_fext_slice_cost(const EggDev& d, const double* u, const EggCost& c, int t, double* cost, cudaStream_t s);
 cudaError_t egg_launch_cost_terminal(const EggDev& d, const EggCost& c, int horizon, double* cost, cudaStream_t s);
+// Device copy of egg_set_sampler: sigma, u_lo, u_hi, each component-major [6][n] (+-inf for no bound).
+struct EggSampler {
+  const double* sigma;
+  const double* lo;
+  const double* hi;
+};
+// MPPI (egg_sample_controls, egg_mppi_reduce): u [H][W][n][6] <- clamp(u_nom [H][n][6] + sigma eps);
+// out [H n 6 + 2] <- sum_w omega_w u[t][w], sum omega, sum omega^2 through partial [chunks][H n 6 + 2]
+cudaError_t egg_launch_mppi_sample(const EggDev& d, const EggSampler& sm, const double* u_nom, int horizon,
+                                   unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s);
+int egg_mppi_chunks(int W);   // stage-1 chunks of egg_launch_mppi_reduce: partial holds chunks x (H n 6 + 2) doubles
+cudaError_t egg_launch_mppi_reduce(const EggDev& d, const double* u, int horizon, const double* cost, const double* baseline,
+                                   double lambda, double* partial, double* out, cudaStream_t s);
 // Dynamic shared memory each kernel family needs for this batch shape (checked against the device
 // limit in egg_create, so that an unsupported shape fails there with a clear message).
 size_t egg_collide_smem(const EggDev& d);

@@ -1,0 +1,123 @@
+// MPPI (model predictive path integral): the two data-heavy steps of the sampling planner, next to
+// the step.  egg_sample_controls writes W perturbed copies of a nominal control schedule;
+// egg_mppi_reduce sums them weighted by exp(-(J - J_min) / lambda).  Both touch the whole
+// [H][W][n][6] schedule (6.3 GB at 131072 legged20 worlds and H = 50) and nothing else of size.
+#include "egg_internal.cuh"
+#include <curand_philox4x32_x.h>   // header-only device code of the toolkit: curand_Philox4x32_10
+
+// Two Philox words -> a uniform in (0, 1]: the top 53 bits of (lo | hi << 32), offset by 2^-54 so
+// that 0 never occurs (ln u is finite, |eps| <= 8.7).  Above 0.5 the sum is a tie that rounds to
+// even, so 1.0 can occur; it is harmless (ln 1 = 0 gives r = 0, sincospi(2) is finite).
+__device__ __forceinline__ double egg_u01(unsigned lo, unsigned hi) {
+  const unsigned long long x = ((unsigned long long)hi << 32) | lo;
+  return (double)(x >> 11) * 0x1p-53 + 0x1p-54;
+}
+
+// clamp that lets NaN through (fmin/fmax would replace it by a bound)
+__device__ __forceinline__ double egg_clamp(double v, double lo, double hi) { return v < lo ? lo : (v > hi ? hi : v); }
+
+// One thread per (step, world, body, component pair): i = (w n + b) 3 + p within step t, so thread i
+// writes the two adjacent doubles u[t][w][b][2p, 2p + 1] as one 16-byte store and a warp writes 512
+// consecutive bytes.  The noise is computed for every element whatever sigma is (sigma = 0 costs what
+// sigma > 0 does); global world 0 and sigma = 0 keep u_nom bit for bit (-0.0 included).
+__global__ void __launch_bounds__(256) egg_mppi_sample_kernel(const double* __restrict__ u_nom, EggSampler sm, int W, int n,
+                                                              int H, unsigned per_step, uint2 key, uint2 iter, int first,
+                                                              double2* __restrict__ u) {
+  const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= per_step) return;
+  const unsigned p = i % 3u, r = i / 3u, b = r % (unsigned)n, w = r / (unsigned)n;
+  const unsigned g = (unsigned)first + w;
+  const int j = 2 * (int)p;
+  const double s0 = sm.sigma[j * n + b], s1 = sm.sigma[(j + 1) * n + b];
+  const double lo0 = sm.lo[j * n + b], lo1 = sm.lo[(j + 1) * n + b];
+  const double hi0 = sm.hi[j * n + b], hi1 = sm.hi[(j + 1) * n + b];
+  for (int t = blockIdx.y; t < H; t += gridDim.y) {
+    const uint4 c = curand_Philox4x32_10(make_uint4(((unsigned)t * (unsigned)n + b) * 3u + p, g, iter.x, iter.y), key);
+    const double u1 = egg_u01(c.x, c.y), u2 = egg_u01(c.z, c.w);
+    const double rad = sqrt(-2.0 * log(u1));
+    double sn, cs;
+    sincospi(2.0 * u2, &sn, &cs);
+    const double2 m = *reinterpret_cast<const double2*>(u_nom + ((size_t)t * n + b) * 6 + j);
+    double v0 = m.x + s0 * (rad * cs), v1 = m.y + s1 * (rad * sn);
+    if (g == 0 || s0 == 0.0) v0 = m.x;
+    if (g == 0 || s1 == 0.0) v1 = m.y;
+    u[(size_t)t * per_step + i] = make_double2(egg_clamp(v0, lo0, hi0), egg_clamp(v1, lo1, hi1));
+  }
+}
+
+// Worlds per stage-1 partial of the reduction (= the block size of its kernel).
+#define EGG_MPPI_CHUNK 256
+
+// Stage 1: block (x, c) sums the worlds [c CHUNK, (c + 1) CHUNK) of columns x*256 ... of the
+// [H n 6 + 2]-column table (u[t][w] flattened over (t, b, j), then omega, then omega^2), in world
+// order.  The chunk's weights are computed once into shared memory.  For a fixed world the 256
+// threads read 256 consecutive doubles of u, so the loads are coalesced; each thread walks down its
+// column.  A zero weight contributes exactly nothing (a NaN control of a discarded world included).
+__global__ void __launch_bounds__(EGG_MPPI_CHUNK) egg_mppi_reduce_kernel(const double* __restrict__ u, int W, int n6, int L,
+                                                                        const double* __restrict__ cost,
+                                                                        const double* __restrict__ baseline, double lambda,
+                                                                        double* __restrict__ partial) {
+  __shared__ double om[EGG_MPPI_CHUNK];
+  const int w0 = blockIdx.y * EGG_MPPI_CHUNK;
+  const int nw = min(EGG_MPPI_CHUNK, W - w0);
+  const double base = *baseline;
+  double o = 0.0;
+  if ((int)threadIdx.x < nw) {
+    const double J = cost[w0 + threadIdx.x];
+    if (isfinite(J) && isfinite(base)) o = exp(-(J - base) / lambda);
+  }
+  om[threadIdx.x] = o;
+  __syncthreads();
+  const int col = blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= L + 2) return;
+  double s = 0.0;
+  if (col < L) {
+    const int t = col / n6, e = col - t * n6;
+    const double* x = u + ((size_t)t * W + w0) * n6 + e;
+#pragma unroll 8
+    for (int k = 0; k < nw; k++) {
+      const double ok = om[k], xk = x[(size_t)k * n6];
+      s += ok != 0.0 ? ok * xk : 0.0;
+    }
+  } else if (col == L) {
+    for (int k = 0; k < nw; k++) s += om[k];
+  } else {
+    for (int k = 0; k < nw; k++) s += om[k] * om[k];
+  }
+  partial[(size_t)blockIdx.y * (L + 2) + col] = s;
+}
+
+// Stage 2: out[col] = the chunk partials of column col added in chunk order.
+__global__ void __launch_bounds__(256) egg_mppi_reduce_final_kernel(const double* __restrict__ partial, int chunks, int L2,
+                                                                    double* __restrict__ out) {
+  const int col = blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= L2) return;
+  double s = 0.0;
+#pragma unroll 8
+  for (int c = 0; c < chunks; c++) s += partial[(size_t)c * L2 + col];
+  out[col] = s;
+}
+
+cudaError_t egg_launch_mppi_sample(const EggDev& d, const EggSampler& sm, const double* u_nom, int horizon,
+                                   unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s) {
+  const unsigned per_step = (unsigned)d.W * (unsigned)d.n * 3u;
+  const dim3 grid((per_step + 255) / 256, (unsigned)min(horizon, 65535));
+  egg_mppi_sample_kernel<<<grid, 256, 0, s>>>(u_nom, sm, d.W, d.n, horizon, per_step,
+                                              make_uint2((unsigned)seed, (unsigned)(seed >> 32)),
+                                              make_uint2((unsigned)iteration, (unsigned)(iteration >> 32)), first,
+                                              reinterpret_cast<double2*>(u));
+  return cudaGetLastError();
+}
+
+int egg_mppi_chunks(int W) { return (W + EGG_MPPI_CHUNK - 1) / EGG_MPPI_CHUNK; }
+
+cudaError_t egg_launch_mppi_reduce(const EggDev& d, const double* u, int horizon, const double* cost, const double* baseline,
+                                   double lambda, double* partial, double* out, cudaStream_t s) {
+  const int n6 = d.n * 6, L = horizon * n6, chunks = egg_mppi_chunks(d.W);
+  egg_mppi_reduce_kernel<<<dim3((unsigned)(L + 2 + EGG_MPPI_CHUNK - 1) / EGG_MPPI_CHUNK, (unsigned)chunks), EGG_MPPI_CHUNK, 0, s>>>(
+      u, d.W, n6, L, cost, baseline, lambda, partial);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  egg_mppi_reduce_final_kernel<<<(unsigned)(L + 2 + 255) / 256, 256, 0, s>>>(partial, chunks, L + 2, out);
+  return cudaGetLastError();
+}

@@ -1,7 +1,8 @@
 """Multi-GPU host logic: contiguous world shards and the one collective of the path — an allgather
 of per-rollout costs followed by an identical arg-min / top-k on every rank (SURVEY.md §8e) — and
 the receding-horizon loop built on it: the winners' terminal states are gathered from their owner
-ranks and re-seed every world for the next horizon (`mpc_iteration`).
+ranks and re-seed every world for the next horizon (`mpc_iteration`) — and an MPPI planner on top of
+the same pieces (`MPPI`, `mppi_iteration`, `mppi_advance`).
 
 Worlds are independent (the reference already steps two unrelated ensembles per SimulationStep,
 /root/reference/eggshell/model.cc:67-68), so there is no data-path exchange inside a horizon."""
@@ -186,3 +187,198 @@ def mpc_iteration(batch, u, dt, k, n_total, first):
     batch.seed_state(states.data_ptr(), len(winners), first)
     batch.snapshot()
     return winners, best, states
+
+
+class MPPI:
+    """Planner state of MPPI (model predictive path integral): a nominal schedule u_nom, float64
+    [horizon, n, 6] on `device`, improved by mppi_iteration and executed by mppi_advance.
+
+    sigma: the standard deviation of the noise per body and control component, broadcast to [n, 6],
+    finite and >= 0.  u_lo / u_hi: bounds of every sampled and nominal control, broadcast to [n, 6]
+    (None = unbounded; +-inf allowed, NaN not; u_lo <= u_hi).  lam: the temperature lambda of the
+    weights exp(-(J - J_min) / lam), finite and > 0.  seed: the Philox key, in [0, 2^64).  u_nom: the
+    initial nominal schedule, broadcast to [horizon, n, 6] (default zeros), finite.  Hand the planner
+    to Batch.set_sampler before mppi_iteration."""
+
+    def __init__(self, n, horizon, sigma, lam, u_lo=None, u_hi=None, seed=0, u_nom=None, device="cuda"):
+        import torch
+        n, horizon = int(n), int(horizon)
+        if n < 1 or horizon < 1:
+            raise ValueError("MPPI: n and horizon must be >= 1")
+        U = CONTROL_PER_BODY
+        self.n, self.horizon = n, horizon
+        self.sigma = self._arr(sigma, (n, U), "sigma")
+        if not np.isfinite(self.sigma).all() or (self.sigma < 0).any():
+            raise ValueError("MPPI: sigma must be finite and >= 0")
+        self.u_lo = None if u_lo is None else self._arr(u_lo, (n, U), "u_lo")
+        self.u_hi = None if u_hi is None else self._arr(u_hi, (n, U), "u_hi")
+        for a, name in ((self.u_lo, "u_lo"), (self.u_hi, "u_hi")):
+            if a is not None and np.isnan(a).any():
+                raise ValueError(f"MPPI: {name} has NaN values")
+        lo = np.full((n, U), -np.inf) if self.u_lo is None else self.u_lo
+        hi = np.full((n, U), np.inf) if self.u_hi is None else self.u_hi
+        if (lo > hi).any():
+            raise ValueError("MPPI: u_lo > u_hi")
+        lam = float(lam)
+        if not (np.isfinite(lam) and lam > 0):
+            raise ValueError("MPPI: lam must be finite and > 0")
+        self.lam = lam
+        seed = int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("MPPI: seed must be in [0, 2^64)")
+        self.seed = seed
+        un = np.zeros((horizon, n, U)) if u_nom is None else self._arr(
+            u_nom.detach().cpu().numpy() if isinstance(u_nom, torch.Tensor) else u_nom, (horizon, n, U), "u_nom")
+        if not np.isfinite(un).all():
+            raise ValueError("MPPI: u_nom has non-finite values")
+        self.device = torch.device(device)
+        self.u_nom = torch.from_numpy(un).to(self.device)
+        self.lo = torch.from_numpy(lo).to(self.device)   # the bounds as tensors, for clamp on the device
+        self.hi = torch.from_numpy(hi).to(self.device)
+        self.iteration = 0
+
+    @staticmethod
+    def _arr(a, shape, name):
+        a = np.asarray(a, dtype=np.float64)
+        try:
+            return np.ascontiguousarray(np.broadcast_to(a, shape))
+        except ValueError:
+            raise ValueError(f"MPPI: {name} of shape {a.shape} does not broadcast to {list(shape)}") from None
+
+    def clamp(self, u):
+        """u clamped to [u_lo, u_hi] (broadcast over leading dimensions)."""
+        import torch
+        return torch.clamp(u, min=self.lo, max=self.hi)
+
+
+def allgather_rows(x):
+    """x: a 1-D tensor of the same length on every rank.  Returns [world_size, len] in rank order with
+    one all_gather_into_tensor (x[None] without a process group)."""
+    import torch
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
+        return x[None]
+    ws = dist.get_world_size()
+    out = torch.empty(ws * x.numel(), dtype=x.dtype, device=x.device)
+    dist.all_gather_into_tensor(out, x.contiguous())
+    return out.view(ws, x.numel())
+
+
+def allgather_rank_sum(x):
+    """The sum over ranks of x, added in rank order ((x_0 + x_1) + x_2 ...), so every rank holds the
+    same bits whatever the collective's own reduction order would be."""
+    rows = allgather_rows(x)
+    acc = rows[0].clone()
+    for r in range(1, rows.shape[0]):
+        acc += rows[r]
+    return acc
+
+
+def _mppi_check(batch, mppi, u, first):
+    import torch
+    import torch.distributed as dist
+    dev = torch.device("cuda", int(batch.desc.device))
+    H = mppi.horizon
+    if not (isinstance(u, torch.Tensor) and u.is_cuda and u.device == dev and u.dtype == torch.float64
+            and u.is_contiguous() and u.dim() == 4 and u.shape[0] == H and tuple(u.shape[1:]) == (batch.W, batch.n, 6)):
+        raise ValueError(f"u must be a contiguous float64 tensor [{H}, {batch.W}, {batch.n}, 6] on {dev}")
+    if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
+        raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
+    if batch.sampler is not mppi:
+        raise ValueError("the batch's sampler is not this planner: call Batch.set_sampler(mppi) first")
+    if mppi.u_nom.device != dev:
+        raise ValueError(f"the planner's u_nom must live on {dev}")
+    rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
+    if (first == 0) != (rank == 0):
+        raise ValueError("rank 0 must own global world 0 (first = 0 exactly on rank 0)")
+    return dev
+
+
+def mppi_sample(batch, mppi, u, first):
+    """Step 1 of mppi_iteration without the restore: the perturbed schedules of this iteration into u."""
+    batch.sample_controls(mppi.u_nom.data_ptr(), mppi.horizon, mppi.seed, mppi.iteration, first, u.data_ptr())
+
+
+def mppi_combine(batch, mppi, u, costs):
+    """Steps 3 to 6 of mppi_iteration, all on the device: the baseline and nominal cost, the weighted
+    sums of this shard, their rank-order sum and the candidate nominal schedule.  Returns
+    (candidate [H, n, 6], stats [nominal J, min J, sum omega, sum omega^2]) without reading anything back."""
+    import torch
+    inf = torch.tensor(float("inf"), dtype=torch.float64, device=costs.device)
+    local_min = torch.where(torch.isfinite(costs), costs, inf).min()
+    g = allgather_rows(torch.stack([local_min, costs[0]]))   # [world_size, 2]; costs[0] of rank 0 is global world 0
+    baseline = g[:, 0].min().contiguous()
+    L = mppi.horizon * batch.n * CONTROL_PER_BODY
+    part = torch.empty(L + 2, dtype=torch.float64, device=costs.device)
+    batch.mppi_reduce(u.data_ptr(), mppi.horizon, costs.data_ptr(), baseline.data_ptr(), mppi.lam, part.data_ptr())
+    total = allgather_rank_sum(part)
+    candidate = mppi.clamp(total[:L].view(mppi.horizon, batch.n, CONTROL_PER_BODY) / total[L])
+    return candidate, torch.stack([g[0, 1], baseline, total[L], total[L + 1]])
+
+
+def mppi_iteration(batch, mppi, dt, u, first):
+    """One MPPI iteration of a (sharded) sweep.  u is the caller's schedule buffer, a contiguous float64
+    CUDA tensor [H, W, n, 6] on the batch's device, overwritten with this iteration's samples; first
+    is the global index of local world 0 (0 on rank 0).  The batch must run on torch's current stream
+    and sample with this planner (Batch.set_sampler(mppi)).
+
+      1. restore the snapshot; sample W perturbed copies of u_nom into u (global world 0: u_nom itself);
+      2. roll them out with the batch's QuadraticCost (step_controlled_cost), or without one with the
+         built-in cost (step_controlled + rollout_costs);
+      3. one allgather of [finite local min J, J of global world 0]: the baseline J_min (kept on the
+         device) and the nominal schedule's cost;
+      4. mppi_reduce: sum_w omega_w u_w, sum omega, sum omega^2 with omega = exp(-(J - J_min) / lam);
+      5. one allgather of those partials, added in rank order (identical bits on every rank);
+      6. u_nom <- clamp(sum omega u / sum omega);  7. iteration += 1.
+
+    Reads back one small tensor.  Returns {nominal_cost, min_cost, weight_sum, ess} with
+    ess = (sum omega)^2 / sum omega^2 the effective number of samples.  If no rollout finished with a
+    finite cost (sum omega = 0) it raises and leaves u_nom and iteration unchanged."""
+    import torch
+    dev = _mppi_check(batch, mppi, u, first)
+    costs = torch.empty(batch.W, dtype=torch.float64, device=dev)
+    batch.restore()
+    mppi_sample(batch, mppi, u, first)
+    if batch.cost is None:
+        batch.step_controlled(dt, u.data_ptr(), mppi.horizon)
+        batch.rollout_costs(costs.data_ptr())
+    else:
+        batch.step_controlled_cost(dt, u.data_ptr(), mppi.horizon, costs.data_ptr())
+    candidate, stats = mppi_combine(batch, mppi, u, costs)
+    nominal, jmin, wsum, w2 = stats.cpu().numpy().tolist()
+    if not wsum > 0:
+        raise RuntimeError(f"mppi_iteration: the weights sum to {wsum} (no rollout finished with a finite cost); u_nom is unchanged")
+    mppi.u_nom.copy_(candidate)
+    mppi.iteration += 1
+    return {"nominal_cost": nominal, "min_cost": jmin, "weight_sum": wsum, "ess": wsum * wsum / w2}
+
+
+def mppi_advance(batch, mppi, dt, n_total):
+    """Executes the plan's first control: from the snapshot every world takes one step with
+    clamp(u_nom[0]); global world 0's new state re-seeds every world of every rank and becomes the
+    snapshot, the start of the next horizon; u_nom shifts by one step (the last row repeats).  This
+    costs one step of the whole batch, 1/H of a horizon.  Returns (the executed control [n, 6], the
+    new start rows [n, 18]), float64 CUDA tensors."""
+    import torch
+    dev = torch.device("cuda", int(batch.desc.device))
+    if mppi.u_nom.device != dev:
+        raise ValueError(f"the planner's u_nom must live on {dev}")
+    if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
+        raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
+    u0 = mppi.clamp(mppi.u_nom[0])
+    batch.restore()
+    batch.step_controlled(dt, u0.expand(1, batch.W, batch.n, CONTROL_PER_BODY).contiguous().data_ptr(), 1)
+    F = batch.n * STATE_PER_BODY
+
+    def pack(local):
+        out = torch.empty((len(local), F), dtype=torch.float64, device=dev)
+        if len(local):
+            batch.gather_state(local, out.data_ptr())
+        return out
+
+    state = gather_winner_states([0], n_total, pack)
+    batch.seed_state(state.data_ptr(), 1, 0)
+    batch.snapshot()
+    if mppi.horizon > 1:
+        mppi.u_nom[:-1] = mppi.u_nom[1:].clone()
+    return u0, state.view(batch.n, STATE_PER_BODY)

@@ -211,6 +211,47 @@ int egg_set_cost(egg_batch* b, const egg_cost* c);
  * batch stream. */
 int egg_step_controlled_cost(egg_batch* b, double dt, int integrator, const double* u_d, int horizon, double* cost_d);
 
+/* MPPI (model predictive path integral, INTEGRATION.md): the two data-heavy steps of a sampling
+ * planner, sampling W perturbed copies of a nominal schedule and their cost-weighted sum.
+ * Per-body noise scale and control bounds, shared by all worlds and steps: */
+typedef struct egg_sampler {
+  const double* sigma; /* [n_bodies][6] standard deviation of the noise, finite and >= 0 (HOST array) */
+  const double* u_lo;  /* [n_bodies][6] lower bound of every sampled control; NULL = unbounded */
+  const double* u_hi;  /* [n_bodies][6] upper bound; NULL = unbounded.  +-inf allowed, NaN not */
+} egg_sampler;
+
+/* Copies the sampler into device memory owned by the batch (counted by egg_device_bytes); s == NULL
+ * clears it and releases that memory.  A non-finite or negative sigma, a NaN bound or u_lo > u_hi
+ * returns EGG_ERR_ARG and leaves the previous sampler in place.  Valid before or after egg_init.
+ * Synchronises the batch stream. */
+int egg_set_sampler(egg_batch* b, const egg_sampler* s);
+
+/* u_d[t][w][b][j] = clamp(u_nom_d[t][b][j] + sigma[b][j] eps, u_lo[b][j], u_hi[b][j]) for t < horizon
+ * and every local world w; u_nom_d is [horizon][n_bodies][6], u_d [horizon][W][n_bodies][6] (the
+ * schedule of egg_step_controlled).  eps is a standard normal from Philox4x32-10 with key
+ * (seed_lo, seed_hi) and counter (q, g, iteration_lo, iteration_hi), g = first + w the global world
+ * index and q = (t n_bodies + b) 3 + p for the component pair (2p, 2p + 1): the four output words
+ * make two uniforms u = ((lo | hi << 32) >> 11) 2^-53 + 2^-54 (words 0, 1 and words 2, 3), and
+ * Box-Muller gives eps_2p = r cos(2 pi u2), eps_2p+1 = r sin(2 pi u2), r = sqrt(-2 ln u1).  The
+ * samples depend on the global index only, not on the sharding.  Global world 0 takes no noise: it
+ * runs clamp(u_nom).  EGG_ERR_STATE without a sampler or before egg_init; EGG_ERR_ARG for
+ * horizon < 1, first < 0, or a pointer that is not device memory of the batch's device.
+ * Asynchronous on the batch stream; one launch. */
+int egg_sample_controls(egg_batch* b, const double* u_nom_d, int horizon, unsigned long long seed,
+                        unsigned long long iteration, int first, double* u_d);
+
+/* The cost-weighted sum of the schedules u_d [horizon][W][n_bodies][6].  World w gets the weight
+ * omega_w = exp(-(cost_d[w] - *baseline_d) / lambda); omega_w = 0 for a non-finite cost_d[w], and every
+ * weight is 0 when *baseline_d (a DEVICE scalar) is not finite.  out_d [horizon n_bodies 6 + 2]
+ * receives sum_w omega_w u_d[t][w] as [horizon][n_bodies][6], then sum omega, then sum omega^2.
+ * Deterministic, without atomics: each fixed chunk of worlds is summed in index order into a scratch
+ * buffer the batch owns (counted by egg_device_bytes), then the chunk sums are added in chunk order,
+ * so the bits depend only on W, n_bodies, horizon and the inputs.  EGG_ERR_ARG for lambda <= 0 or
+ * not finite, horizon < 1, or a pointer that is not device memory of the batch's device;
+ * EGG_ERR_STATE before egg_init.  Asynchronous on the batch stream; two launches. */
+int egg_mppi_reduce(egg_batch* b, const double* u_d, int horizon, const double* cost_d, const double* baseline_d,
+                    double lambda, double* out_d);
+
 /* Ensemble::UpdateContacts + CheckAndCorrectEnsembleState only (ensembles.cc:445-480, 241-329):
  * runs the narrowphase kernel on the current state without stepping; read the result with
  * egg_get_contacts / egg_get_pair_hits. */

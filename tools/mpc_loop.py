@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Cost of the receding-horizon MPC loop (mpc.mpc_iteration) over the plain rollout sweep.
 
-    python tools/mpc_loop.py [--worlds 131072] [--horizon 50] [--repeats 5] [--profile] [--out FILE]
+    python tools/mpc_loop.py [--worlds 131072] [--horizon 50] [--repeats 5] [--legs abcde] [--profile] [--out FILE]
     python -m torch.distributed.run --nproc_per_node N tools/mpc_loop.py ...
 
 One process per GPU; every rank owns `--worlds` legged20 worlds (bench.py's c5mpc scene, seeded per
@@ -19,10 +19,19 @@ the whole overhead of the loop and d - c the cost of accumulating the configured
 (in place of the built-in terminal cost).  Then the loop runs with random time-varying schedules,
 without and with the cost set, and its world-steps/s are reported.  --profile adds the device time
 of the per-step kernels of one c and one d leg from torch.profiler (a separate, untimed pass).
+
+Leg e times only what MPPI adds to a horizon (mpc.mppi_iteration minus the rollout), at sigma = 0 so
+that the schedule is the constant one of leg c: egg_sample_controls, the allgather of the baseline,
+egg_mppi_reduce, the allgather of the partials and the rank-order combine into the new nominal
+schedule.  egg_sample_controls and egg_mppi_reduce are also timed alone, and their achieved GB/s
+(bytes computed from the shapes) are reported against the 6555.8 GB/s copy bandwidth of BASELINE.md.
+Then mppi_iteration runs with sigma > 0 on the torques and the representative cost, and its
+world-steps/s are reported.  --profile adds the device time of the MPPI kernels of one leg e.
+--legs picks the legs to run (b needs a; the overheads need the legs they compare).
 Rank 0 prints one JSON line with the GPU name and power limit.
 
 Memory: a schedule is H x worlds x 20 x 6 doubles, 6.3 GB per GPU at 131072 worlds and H = 50; the
-script holds two (constant and random), plus the batch and one saved start state (0.4 GB).
+script holds three (constant, random and MPPI samples), plus the batch and one saved start state (0.4 GB).
 """
 import argparse
 import json
@@ -47,7 +56,9 @@ def parse():
     ap.add_argument("--repeats", type=int, default=5, help="timed repeats of each leg")
     ap.add_argument("--random-iters", type=int, default=3, help="timed loop iterations with random schedules")
     ap.add_argument("--sigma", type=float, default=0.05, help="std. dev. of the random torques (N m)")
-    ap.add_argument("--profile", action="store_true", help="also record the per-step kernel times of legs c and d with torch.profiler")
+    ap.add_argument("--legs", default="abcde", help="legs to run (default: all)")
+    ap.add_argument("--lam", type=float, default=1.0, help="MPPI temperature lambda of leg e")
+    ap.add_argument("--profile", action="store_true", help="also record the kernel times of legs c, d and e with torch.profiler")
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     return ap.parse_args()
 
@@ -67,11 +78,12 @@ def spread(xs):
     return {"median": float(np.median(xs)), "min": float(xs.min()), "max": float(xs.max()), "n": int(xs.size)}
 
 
-def profile_legs(b, prepare, leg_c, leg_d, sync):
-    """Device milliseconds of the per-step control kernels of one leg c and one leg d."""
+def profile_legs(prepare, legs, sync):
+    """Device milliseconds of the per-step control kernels of one leg c and one leg d, and of the
+    MPPI kernels of one leg e."""
     from torch.profiler import profile, ProfilerActivity
     out = {}
-    for name, fn in (("c", leg_c), ("d", leg_d)):
+    for name, fn in legs.items():
         prepare(name)
         sync()
         with profile(activities=[ProfilerActivity.CUDA]) as prof:
@@ -79,7 +91,7 @@ def profile_legs(b, prepare, leg_c, leg_d, sync):
             sync()
         for e in prof.key_averages():
             kernel = re.search(r"egg_\w+", e.key)
-            if kernel and ("fext_slice" in kernel.group(0) or "egg_cost" in kernel.group(0)):
+            if kernel and any(key in kernel.group(0) for key in ("fext_slice", "egg_cost", "egg_mppi")):
                 out[f"{name}: {kernel.group(0)}"] = {"calls": e.count, "ms": e.device_time_total / 1e3}
     return out
 
@@ -112,6 +124,16 @@ def main():
     gen.manual_seed(1234 + rank)
     u_rand = u_const.clone()
     u_rand[..., 3:6] += args.sigma * torch.randn(u_rand[..., 3:6].shape, generator=gen, device=dev, dtype=torch.float64)
+    u_mppi = torch.empty_like(u_const) if "e" in args.legs else None
+    # MPPI planners around world 0's f_ext: sigma = 0 for the overhead of leg e, sigma on the torques for the loop
+    sigma = np.zeros((n, 6))
+    sigma[:, 3:6] = args.sigma
+    mppi0 = mpc.MPPI(n, H, sigma=0.0, lam=args.lam, seed=11, u_nom=scene["f_ext"][0], device=dev)
+    mppi1 = mpc.MPPI(n, H, sigma=sigma, lam=args.lam, seed=12, u_nom=scene["f_ext"][0], device=dev)
+    L = H * n * 6
+    chunks = -(-W // 256)   # stage-1 chunks of egg_mppi_reduce
+    sample_bytes = 8 * (H * W * n * 6 + L)                                  # write the samples, read u_nom
+    reduce_bytes = 8 * (H * W * n * 6 + W + 2 * chunks * (L + 2) + L + 2)   # read u and J, partials out and in, result
     costs = torch.empty(W, dtype=torch.float64, device=dev)
     all_costs = torch.empty(n_total, dtype=torch.float64, device=dev)
     start = torch.empty((W, n * 18), dtype=torch.float64, device=dev)
@@ -181,11 +203,18 @@ def main():
             if ws > 1:
                 dist.all_gather_into_tensor(all_costs, costs)
 
-        legs = {"a": leg_a, "c": leg_c, "b": leg_b, "d": leg_d}
+        def leg_e():
+            mpc.mppi_sample(b, mppi0, u_mppi, first)
+            mpc.mppi_combine(b, mppi0, u_mppi, costs)
+
+        legs = {name: fn for name, fn in (("a", leg_a), ("c", leg_c), ("b", leg_b), ("d", leg_d), ("e", leg_e)) if name in args.legs}
 
         def prepare(name):   # the cost is set for leg d only (outside the timed region: set_cost synchronises)
             reset()
             b.set_cost(cost if name == "d" else None)
+            if name == "e":   # the costs of a rollout of the constant schedule, which leg e weighs
+                b.set_sampler(mppi0)
+                leg_c()
 
         for name, fn in legs.items():     # warm-up
             prepare(name)
@@ -195,17 +224,48 @@ def main():
             for name, fn in legs.items():
                 prepare(name)
                 t[name].append(timed(fn))
-        a, c, bb, d = np.array(t["a"]), np.array(t["c"]), np.array(t["b"]), np.array(t["d"])
-        entry = {"a_sweep_ms": spread(a), "c_controlled_sweep_ms": spread(c), "b_mpc_iteration_ms": spread(bb),
-                 "d_controlled_cost_sweep_ms": spread(d),
-                 "slice_copy_overhead_ms": spread(c - a), "loop_overhead_ms": spread(bb - a), "cost_overhead_ms": spread(d - c),
-                 "slice_copy_overhead_pct": spread(100.0 * (c - a) / a), "loop_overhead_pct": spread(100.0 * (bb - a) / a),
-                 "cost_overhead_pct": spread(100.0 * (d - c) / c)}
+        t = {name: np.array(x) for name, x in t.items()}
+        entry = {}
+        for name, key in (("a", "a_sweep_ms"), ("c", "c_controlled_sweep_ms"), ("b", "b_mpc_iteration_ms"),
+                          ("d", "d_controlled_cost_sweep_ms"), ("e", "e_mppi_additions_ms")):
+            if name in t:
+                entry[key] = spread(t[name])
+        for key, hi, lo, base in (("slice_copy_overhead", "c", "a", "a"), ("loop_overhead", "b", "a", "a"),
+                                  ("cost_overhead", "d", "c", "c")):
+            if hi in t and lo in t:
+                entry[key + "_ms"] = spread(t[hi] - t[lo])
+                entry[key + "_pct"] = spread(100.0 * (t[hi] - t[lo]) / t[base])
+        if "e" in t and "c" in t:
+            entry["e_mppi_additions_pct_of_c"] = spread(100.0 * t["e"] / t["c"])
+        if "e" in t:   # the two kernels alone, and their bandwidth
+            prepare("e")
+            ks, kr = [], []
+            ub = torch.zeros((), dtype=torch.float64, device=dev)
+            part = torch.empty(L + 2, dtype=torch.float64, device=dev)
+            for _ in range(args.repeats):
+                ks.append(timed(lambda: b.sample_controls(mppi0.u_nom.data_ptr(), H, mppi0.seed, 0, first, u_mppi.data_ptr())))
+                kr.append(timed(lambda: b.mppi_reduce(u_mppi.data_ptr(), H, costs.data_ptr(), ub.data_ptr(), args.lam, part.data_ptr())))
+            ks, kr = np.array(ks), np.array(kr)
+            entry["e_kernels"] = {
+                "copy_bandwidth_GBps": 6555.8,
+                "sample_controls": {"ms": spread(ks), "bytes": sample_bytes, "GBps": spread(sample_bytes / (ks * 1e-3) / 1e9)},
+                "mppi_reduce": {"ms": spread(kr), "bytes": reduce_bytes, "GBps": spread(reduce_bytes / (kr * 1e-3) / 1e9),
+                                "launches": 2, "chunks": chunks}}
         if args.profile:
-            entry["kernel_ms_per_horizon"] = profile_legs(b, prepare, leg_c, leg_d, sync)
+            entry["kernel_ms_per_horizon"] = profile_legs(prepare, {x: legs[x] for x in "cde" if x in legs}, sync)
         # the loop itself with random time-varying schedules (the state evolves from iteration to iteration),
         # with the built-in cost and with the configured one
-        for key, qc in (("random_loop", None), ("random_loop_cost", cost)):
+        loops = [(key, qc) for key, qc, leg in (("random_loop", None, "b"), ("random_loop_cost", cost, "d")) if leg in legs]
+        if "e" in legs:   # MPPI with sigma > 0 and the representative cost
+            reset()
+            b.set_cost(cost)
+            b.set_sampler(mppi1)
+            mpc.mppi_iteration(b, mppi1, dt, u_mppi, first)
+            ms = timed(lambda: [mpc.mppi_iteration(b, mppi1, dt, u_mppi, first) for _ in range(args.random_iters)])
+            entry["mppi_loop_cost"] = {"iterations": args.random_iters, "ms_per_iteration": ms / args.random_iters,
+                                       "world_steps_per_s": n_total * H * args.random_iters / (ms * 1e-3),
+                                       "sigma_torque": args.sigma, "lam": args.lam}
+        for key, qc in loops:
             reset()
             b.set_cost(qc)
             mpc.mpc_iteration(b, u_rand, dt, k, n_total, first)
