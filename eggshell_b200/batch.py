@@ -25,7 +25,7 @@ EXPORTS = [
     "egg_set_external", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_step_controlled",
     "egg_set_cost", "egg_step_controlled_cost", "egg_set_sampler", "egg_sample_controls", "egg_mppi_reduce", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
     "egg_get_status", "egg_get_dense_work", "egg_get_debug_counters", "egg_rollout_costs", "egg_set_stream", "egg_sync", "egg_device_bytes",
-    "egg_launch_count", "egg_capacity", "egg_set_profiling", "egg_get_kernel_ms", "egg_fp64_peak_tflops", "egg_host_alloc", "egg_host_free", "egg_last_error", "egg_version",
+    "egg_launch_count", "egg_capacity", "egg_get_kernel_config", "egg_set_profiling", "egg_get_kernel_ms", "egg_fp64_peak_tflops", "egg_host_alloc", "egg_host_free", "egg_last_error", "egg_version",
 ]
 
 
@@ -349,6 +349,15 @@ class Batch:
 
     def rollout_costs(self, device_ptr):
         _chk(lib().egg_rollout_costs(self.h, C.c_void_p(device_ptr)), "egg_rollout_costs")
+
+    def kernel_config(self):
+        """The kernel instances this batch runs (egg_get_kernel_config): lanes per world, worlds per
+        warp, M^-1 layout (-1 until the first step), record format (-1 until the first step for PGS),
+        run cap, record precision, narrowphase and record-assembly threads per world."""
+        out = (C.c_int * 8)()
+        _chk(lib().egg_get_kernel_config(self.h, out), "egg_get_kernel_config")
+        keys = ("lpw", "worlds_per_warp", "iso", "rec_format", "run_cap", "precision", "collide_threads", "records_threads")
+        return dict(zip(keys, (int(x) for x in out)))
 
     def set_profiling(self, on=True):
         _chk(lib().egg_set_profiling(self.h, int(on)), "egg_set_profiling")

@@ -22,6 +22,10 @@ cudaError_t egg_launch_relax(const EggDev& d, double dt, double step_scale, int 
                              int* prog, double* err2, int* any_active, cudaStream_t s);
 
 static thread_local std::string g_err;
+static int env_int(const char* name, int dflt) {
+  const char* e = getenv(name);
+  return e ? atoi(e) : dflt;
+}
 static void set_err(const char* what, cudaError_t e) {
   char buf[512];
   snprintf(buf, sizeof(buf), "%s: %s", what, cudaGetErrorString(e));
@@ -183,6 +187,17 @@ int egg_create(const egg_desc* dsc, egg_batch** out) {
   d.prm.erp = dsc->erp; d.prm.cfm = dsc->cfm; d.prm.tol = dsc->tol; d.prm.min_dist = dsc->min_constraint_dist;
   for (int k = 0; k < 3; k++) d.prm.g[k] = dsc->gravity[k];
   d.prm.k_max = dsc->k_max; d.prm.solver = dsc->solver; d.prm.quirks = dsc->quirks; d.prm.cfm_mode = dsc->cfm_mode;
+  // kernel-selection overrides: read here, once per batch (egg_get_kernel_config reports the result)
+  d.sel.lpw = env_int("EGG_PGS_LPW", 0);
+  d.sel.min_warps = env_int("EGG_PGS_MIN_WARPS_PER_SM", 3);
+  d.sel.runs = getenv("EGG_PGS_RUNS") ? (env_int("EGG_PGS_RUNS", 0) != 0) : -1;
+  d.sel.run_cap = env_int("EGG_PGS_RUN_CAP", 0);
+  d.sel.target_ctas = env_int("EGG_PGS_TARGET_CTAS", 11);
+  if (d.sel.target_ctas < 1) d.sel.target_ctas = 11;
+  d.sel.collide_nt = env_int("EGG_COLLIDE_NT", 0);
+  d.sel.records_nt = env_int("EGG_RECORDS_NT", 0);
+  d.sel.ctas_per_sm = env_int("EGG_PGS_CTAS_PER_SM", 0);
+  d.sel.pf = env_int("EGG_PGS_PF", 3);
 
   DA(d.dyn, (size_t)W * EGG_DYN * n);
   DA(d.stat, (size_t)W * EGG_STAT * n);
@@ -216,7 +231,7 @@ int egg_create(const egg_desc* dsc, egg_batch** out) {
     DA(d.st_cnt, (size_t)W * d.nrec);
     // run format (egg_pgs_runs.cu): FP64 records, at most 8 lanes per world; whether the bodies are
     // isotropic (its other condition) is known after egg_init, so the choice is made at the first step
-    const bool runs_asked = (dsc->quirks & EGG_OPT_PGS_RUNS) != 0 || (getenv("EGG_PGS_RUNS") && atoi(getenv("EGG_PGS_RUNS")) != 0);
+    const bool runs_asked = (dsc->quirks & EGG_OPT_PGS_RUNS) != 0 || d.sel.runs == 1;
     if (runs_asked && dsc->precision == 64 && d.lpw <= 8) {   // [W][nrec] words: only for batches that asked for the run format
       DA(d.st_runs, (size_t)W * d.nrec);
       d.run_cap = egg_run_cap(d);
@@ -342,6 +357,20 @@ double egg_fp64_peak_tflops(int device) {
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { g_err = "no CUDA device"; return (double)EGG_ERR_NO_DEVICE; }
   if (cudaSetDevice(device) != cudaSuccess) return (double)EGG_ERR_ARG;
   return egg_measure_fp64_tflops();
+}
+int egg_get_kernel_config(const egg_batch* b, int out[8]) {
+  if (!b || !out) return EGG_ERR_ARG;
+  const EggDev& d = b->dev;
+  const bool pgs = b->desc.solver == EGG_SOLVER_PGS;
+  out[0] = d.lpw;                                          // 0 without the group stream
+  out[1] = d.lpw ? 32 / d.lpw : 0;
+  out[2] = b->iso_known ? d.iso : -1;
+  out[3] = !pgs ? 0 : (!b->iso_known ? -1 : (d.rmax > 0 ? 2 : 1));
+  out[4] = (b->iso_known && d.rmax > 0) ? d.run_cap : 0;
+  out[5] = b->desc.precision;
+  out[6] = egg_collide_threads(d);
+  out[7] = egg_assemble_threads(d);
+  return EGG_OK;
 }
 int egg_capacity(const egg_batch* b) { return b ? b->dev.maxc : 0; }
 long long egg_device_bytes(const egg_batch* b) { return b ? b->bytes : 0; }

@@ -591,14 +591,19 @@ __global__ void __launch_bounds__(NT) egg_collide_kernel(EggDev d) {
 
 size_t egg_collide_smem(const EggDev& d) { return (size_t)17 * d.n * sizeof(double) + (size_t)((d.P + 3) & ~3) * 2 + (size_t)((d.P + 7) & ~7); }
 
+// Threads per world by its pair count: one warp for small worlds (every barrier and block scan
+// is paid per warp).  Measured, 131072 x 20 bodies (190 pairs): 3.45 ms at 256 threads, 2.56 at
+// 128, 1.52 at 64, 1.08 at 32; 16384 x 64 bodies (2016 pairs): 2.81 ms at 256, 3.41 at 128.
+// EGG_COLLIDE_NT (d.sel.collide_nt) = 32 / 64 / 128 picks that instance, any other value 256.
+int egg_collide_threads(const EggDev& d) {
+  const int nt = d.sel.collide_nt ? d.sel.collide_nt : (d.P <= 256 ? 32 : (d.P <= 600 ? 64 : (d.P <= 1200 ? 128 : 256)));
+  return (nt == 32 || nt == 64 || nt == 128) ? nt : 256;
+}
+
 cudaError_t egg_launch_collide(const EggDev& d, cudaStream_t s) {
   const size_t smem = egg_collide_smem(d);
   cudaError_t e = cudaSuccess;
-  static const int env_nt = getenv("EGG_COLLIDE_NT") ? atoi(getenv("EGG_COLLIDE_NT")) : 0;   // development override: 64 / 128 / 256
-  // threads per world by its pair count: one warp for small worlds (every barrier and block scan
-  // is paid per warp).  Measured, 131072 x 20 bodies (190 pairs): 3.45 ms at 256 threads, 2.56 at
-  // 128, 1.52 at 64, 1.08 at 32; 16384 x 64 bodies (2016 pairs): 2.81 ms at 256, 3.41 at 128.
-  const int nt = env_nt ? env_nt : (d.P <= 256 ? 32 : (d.P <= 600 ? 64 : (d.P <= 1200 ? 128 : 256)));
+  const int nt = egg_collide_threads(d);
   if (nt == 32) {
     egg_collide_kernel<32><<<d.W, 32, smem, s>>>(d);
   } else if (nt == 64) {

@@ -46,6 +46,22 @@ struct EggParams {
   int k_max, solver, quirks, cfm_mode;
 };
 
+// Development overrides of the kernel selection, read from the environment by egg_create and kept
+// with the batch, so that batches of one process can run different instances.  Unset variables
+// take the defaults below; lpw, run_cap, collide_nt and records_nt = 0 leave the choice to the
+// selection rules of the launchers.
+struct EggSel {
+  int lpw;           // EGG_PGS_LPW: lanes per world 1 / 2 / 4 / 8 / 16 of the group stream
+  int min_warps;     // EGG_PGS_MIN_WARPS_PER_SM: warps per SM the LPW rule aims for (default 3)
+  int runs;          // EGG_PGS_RUNS: -1 unset, 0 off, 1 on (overrides EGG_OPT_PGS_RUNS)
+  int run_cap;       // EGG_PGS_RUN_CAP: runs per world and stage of the run format
+  int target_ctas;   // EGG_PGS_TARGET_CTAS: resident CTAs per SM the run cap is sized for (default 11)
+  int collide_nt;    // EGG_COLLIDE_NT: narrowphase threads per world
+  int records_nt;    // EGG_RECORDS_NT: record-assembly threads per world of the group stream / run format
+  int ctas_per_sm;   // EGG_PGS_CTAS_PER_SM: cap on resident solve CTAs per SM (grid size only)
+  int pf;            // EGG_PGS_PF: L2 prefetch depth of the solve in 4 KB rounds (default 3)
+};
+
 struct EggDev {
   int W, n, nj, maxc, P, nrec;   // P = n(n-1)/2, nrec = nj + maxc
   double* dyn;
@@ -93,6 +109,7 @@ struct EggDev {
   unsigned long long* dbg;    // [32] debug / phase-timing counters (written only by builds with EGG_DENSE_TIMING)
   int rec_fmt;                // 0: D diagonal in REC_DDIAG, multipliers in lam[]; 1: multipliers in REC_DDIAG, next-stage count in slot 29 (stream variant)
   EggParams prm;
+  EggSel sel;
 };
 
 struct d3 {
@@ -149,6 +166,10 @@ cudaError_t egg_launch_assemble_stream(const EggDev& d, double dt, cudaStream_t 
 size_t egg_stream_rec_bytes(int W, int nrec, int lpw);
 int egg_stream_blkb(int precision);
 int egg_stage_cap(const EggDev& d);
+// Threads per world of the instance each pre-solve launcher runs for this batch (egg_get_kernel_config).
+int egg_collide_threads(const EggDev& d);
+int egg_records_threads(const EggDev& d);
+int egg_assemble_threads(const EggDev& d);
 cudaError_t egg_launch_solve_iter(const EggDev& d, double dt, int solver, cudaStream_t s);
 cudaError_t egg_launch_costs(const EggDev& d, double* cost_d, cudaStream_t s);
 cudaError_t egg_launch_pack(int W, const double* aos, int per_world, int comps, double* soa, int soa_comps, int comp_off, cudaStream_t s);

@@ -111,26 +111,21 @@ int num_sms() {
   }
   return g_num_sms;
 }
-int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
 bool stream_variant(const EggDev& d) { return d.rec_fmt != 0; }
 
 }  // namespace
 
-// Lanes per world of the PGS kernel = maximum blocks per stage the assembly may emit.
+// Lanes per world of the PGS kernel = maximum blocks per stage the assembly may emit.  The
+// overrides come from d.sel (read by egg_create).
 int egg_stage_cap(const EggDev& d) {
-  static const int env_lpw = env_int("EGG_PGS_LPW", 0);
-  static const int env_min_warps = env_int("EGG_PGS_MIN_WARPS_PER_SM", 3);
-  int lpw = env_lpw;
+  int lpw = d.sel.lpw;
   if (stream_variant(d)) {
     // narrow worlds expose little parallelism per level: fewer lanes, more worlds per warp
     // (measured: stack10 87 ms at 1 / 101 at 2 / 133 at 4; legged20 95 ms at 4 / 115 at 2 / 123 at 8)
     // -- unless the batch is too small to give every SM a few warps that way
     if (lpw != 1 && lpw != 2 && lpw != 4 && lpw != 8 && lpw != 16) {
       lpw = (d.n <= 12) ? 1 : (d.n <= 24 ? 4 : 8);
-      const long long want = (long long)num_sms() * env_min_warps;
+      const long long want = (long long)num_sms() * d.sel.min_warps;
       while (lpw < 8 && (long long)d.W * lpw / 32 < want) lpw *= 2;
     }
     return lpw;
@@ -142,12 +137,17 @@ size_t egg_assemble_smem(const EggDev& d) {
   return (size_t)(EGG_DYN + EGG_STAT + 6) * d.n * sizeof(double) + (size_t)(7 * d.nrec + d.n + 8) * sizeof(int);
 }
 
+int egg_assemble_threads(const EggDev& d) {
+  if (d.rec_fmt) return egg_records_threads(d);
+  return d.nrec <= 128 ? 64 : 256;
+}
+
 cudaError_t egg_launch_assemble(const EggDev& d, double dt, cudaStream_t s) {
   if (d.rec_fmt) return egg_launch_assemble_stream(d, dt, s);
   const size_t smem = egg_assemble_smem(d);
   const int cap = egg_stage_cap(d);
   cudaError_t e = cudaSuccess;
-  if (d.nrec <= 128) {
+  if (egg_assemble_threads(d) == 64) {
     if (smem > 48 * 1024) e = cudaFuncSetAttribute(egg_assemble_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     egg_assemble_kernel<64><<<d.W, 64, smem, s>>>(d, dt, cap);

@@ -589,11 +589,6 @@ __global__ void __launch_bounds__(32, 11) egg_pgs_runs_kernel(EggDev d, double d
   }
 }
 
-int env_i(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
 // Staging bytes for cap runs per world and stage: worst case every run is full.
 size_t staging_bytes(int G, int cap) { return (size_t)HDRB + (size_t)G * cap * (RUNB + RUN_MAX * (LAMB + RBLKB)) + 32; }
 
@@ -604,7 +599,6 @@ cudaError_t launch(const EggDev& d, double dt, cudaStream_t s) {
   const size_t smem = 64 + (size_t)G * 48 * d.n + stg;
   static thread_local size_t c_smem = ~(size_t)0;
   static thread_local int c_dev = -1, c_per_sm = 0, c_sms = 148;
-  static const int env_cap = env_i("EGG_PGS_CTAS_PER_SM", 0), env_pf = env_i("EGG_PGS_PF", 3);
   cudaError_t e = cudaSuccess;
   int dev = 0;
   EGG_FIRST(e, cudaGetDevice(&dev));
@@ -618,12 +612,12 @@ cudaError_t launch(const EggDev& d, double dt, cudaStream_t s) {
     c_smem = smem; c_dev = dev;
   }
   int per_sm = c_per_sm;
-  if (env_cap > 0 && env_cap < per_sm) per_sm = env_cap;
+  if (d.sel.ctas_per_sm > 0 && d.sel.ctas_per_sm < per_sm) per_sm = d.sel.ctas_per_sm;
   const int groups = (d.W + G - 1) / G;
   const int grid = groups < c_sms * per_sm ? groups : c_sms * per_sm;
   e = cudaMemsetAsync(d.work_ctr, 0, sizeof(int), s);
   if (e != cudaSuccess) return e;
-  egg_pgs_runs_kernel<LPW, ISO><<<grid, 32, smem, s>>>(d, dt, env_pf, (int)(stg - 32));
+  egg_pgs_runs_kernel<LPW, ISO><<<grid, 32, smem, s>>>(d, dt, d.sel.pf, (int)(stg - 32));
   return cudaGetLastError();
 }
 
@@ -641,8 +635,8 @@ cudaError_t launch_lpw(const EggDev& d, double dt, cudaStream_t s) {
 
 // The run format applies to FP64 records of isotropic bodies with at most 8 lanes per world.
 int egg_runs_rmax(const EggDev& d) {
-  static const int env_runs = env_i("EGG_PGS_RUNS", -1);   // development override of EGG_OPT_PGS_RUNS (quirks bit 16)
-  const bool want = env_runs >= 0 ? env_runs != 0 : (d.prm.quirks & 16) != 0;
+  // EGG_PGS_RUNS (d.sel.runs) is a development override of EGG_OPT_PGS_RUNS (quirks bit 16)
+  const bool want = d.sel.runs >= 0 ? d.sel.runs != 0 : (d.prm.quirks & 16) != 0;
   if (!want || !d.rec_fmt || !d.st_runs || d.iso < 1 || d.lpw > 8 || d.blkb != RECB64 + LAMB) return 0;
   return RUN_MAX;
 }
@@ -651,10 +645,9 @@ int egg_runs_rmax(const EggDev& d) {
 // resident warps (64-body worlds: 11 one-warp CTAs per SM with 4 x 64 x 48 B of accumulators each
 // leave ~7.7 KB for the staging buffer: 6 runs per world and stage instead of 8).
 int egg_run_cap(const EggDev& d) {
-  static const int env_cap = env_i("EGG_PGS_RUN_CAP", 0), env_ctas = env_i("EGG_PGS_TARGET_CTAS", 11);
   const int G = 32 / d.lpw;
-  if (env_cap > 0) return env_cap < d.lpw ? env_cap : d.lpw;
-  const long long per_cta = 232448 / env_ctas - 1024;
+  if (d.sel.run_cap > 0) return d.sel.run_cap < d.lpw ? d.sel.run_cap : d.lpw;
+  const long long per_cta = 232448 / d.sel.target_ctas - 1024;
   const long long avail = per_cta - 64 - (long long)G * 48 * d.n - HDRB - 32;
   int cap = (int)(avail / ((long long)G * (RUNB + RUN_MAX * (LAMB + RBLKB))));
   if (cap > d.lpw) cap = d.lpw;
@@ -672,12 +665,12 @@ cudaError_t egg_launch_assemble_runs_tail(const EggDev& d, double dt, cudaStream
   const int ngroups = (d.W + G - 1) / G;
   egg_rounds_runs_kernel<<<(ngroups + 3) / 4, 128, 0, s>>>(d, G);
   const size_t smem = (size_t)(EGG_DYN + EGG_STAT + 6) * d.n * sizeof(double);
-  const int est = d.nj + 6 * d.n;           // threads per world as in egg_pgs_stream.cu (launch_records)
-  if (est <= 192) {
+  const int nt = egg_records_threads(d);    // 32, 128 or 256, by the rule of the group stream (egg_pgs_stream.cu)
+  if (nt == 32) {
     if (smem > 48 * 1024) EGG_FIRST(e, cudaFuncSetAttribute(egg_records_runs_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (e != cudaSuccess) return e;
     egg_records_runs_kernel<32><<<d.W, 32, smem, s>>>(d, dt, G);
-  } else if (est <= 768) {
+  } else if (nt == 128) {
     if (smem > 48 * 1024) EGG_FIRST(e, cudaFuncSetAttribute(egg_records_runs_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (e != cudaSuccess) return e;
     egg_records_runs_kernel<128><<<d.W, 128, smem, s>>>(d, dt, G);

@@ -661,11 +661,6 @@ __global__ void __launch_bounds__(32, MINB) egg_pgs_stream_kernel(EggDev d, doub
   }
 }
 
-int env_i(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
 template <bool F32>
 size_t stream_smem(const EggDev& d, int lpw) {
   const int G = 32 / lpw;
@@ -676,11 +671,10 @@ template <int LPW, int MINB, int ISO, bool F32>
 cudaError_t launch(const EggDev& d, double dt, cudaStream_t s) {
   constexpr int G = 32 / LPW;
   const size_t smem = stream_smem<F32>(d, LPW);
-  // shared-memory attribute, occupancy and the environment switches are looked up once per
-  // (kernel instance, shared-memory size, device), not on every step
+  // shared-memory attribute and occupancy are looked up once per (kernel instance, shared-memory
+  // size, device), not on every step
   static thread_local size_t c_smem = ~(size_t)0;
   static thread_local int c_dev = -1, c_per_sm = 0, c_sms = 148;
-  static const int env_cap = env_i("EGG_PGS_CTAS_PER_SM", 0), env_pf = env_i("EGG_PGS_PF", 3);
   cudaError_t e = cudaSuccess;
   int dev = 0;
   EGG_FIRST(e, cudaGetDevice(&dev));
@@ -694,12 +688,12 @@ cudaError_t launch(const EggDev& d, double dt, cudaStream_t s) {
     c_smem = smem; c_dev = dev;
   }
   int per_sm = c_per_sm;
-  if (env_cap > 0 && env_cap < per_sm) per_sm = env_cap;
+  if (d.sel.ctas_per_sm > 0 && d.sel.ctas_per_sm < per_sm) per_sm = d.sel.ctas_per_sm;
   const int groups = (d.W + G - 1) / G;
   const int grid = groups < c_sms * per_sm ? groups : c_sms * per_sm;
   e = cudaMemsetAsync(d.work_ctr, 0, sizeof(int), s);
   if (e != cudaSuccess) return e;   // without the reset the persistent kernel would find an exhausted queue and do nothing
-  egg_pgs_stream_kernel<LPW, MINB, ISO, F32><<<grid, 32, smem, s>>>(d, dt, env_pf);
+  egg_pgs_stream_kernel<LPW, MINB, ISO, F32><<<grid, 32, smem, s>>>(d, dt, d.sel.pf);
   return cudaGetLastError();
 }
 
@@ -753,15 +747,25 @@ cudaError_t launch_records_nt(const EggDev& d, double dt, int G, size_t smem, cu
 }
 // Threads per world by the constraints a world typically has (joints + a few contacts per body), not
 // by its capacity.  Measured (131072 x legged20, ~43 constraints): 3.8 ms at 256 threads, 1.8 at 64,
-// 1.6 at 32; 16384 x pile64 (~410): 1.41 ms at 256, 1.24 at 128, 1.27 at 64.
-cudaError_t launch_records(const EggDev& d, double dt, int G, size_t smem, cudaStream_t s) {
-  static const int env_nt = env_i("EGG_RECORDS_NT", 0);
+// 1.6 at 32; 16384 x pile64 (~410): 1.41 ms at 256, 1.24 at 128, 1.27 at 64.  EGG_RECORDS_NT
+// (d.sel.records_nt) is rounded up to an instance: 32 / 64 / 128 / 256, or 32 / 128 / 256 for the
+// record kernel of the run format (egg_pgs_runs.cu).
+int egg_records_threads(const EggDev& d) {
   const int est = d.nj + 6 * d.n;
-  const int nt = env_nt ? env_nt : (est <= 192 ? 32 : (est <= 768 ? 128 : 256));
-  if (nt <= 32) return launch_records_nt<32>(d, dt, G, smem, s);
-  if (nt <= 64) return launch_records_nt<64>(d, dt, G, smem, s);
-  if (nt <= 128) return launch_records_nt<128>(d, dt, G, smem, s);
-  return launch_records_nt<256>(d, dt, G, smem, s);
+  const int nt = d.sel.records_nt ? d.sel.records_nt : (est <= 192 ? 32 : (est <= 768 ? 128 : 256));
+  if (nt <= 32) return 32;
+  if (nt <= 64 && d.rmax == 0) return 64;
+  if (nt <= 128) return 128;
+  return 256;
+}
+
+cudaError_t launch_records(const EggDev& d, double dt, int G, size_t smem, cudaStream_t s) {
+  switch (egg_records_threads(d)) {
+    case 32: return launch_records_nt<32>(d, dt, G, smem, s);
+    case 64: return launch_records_nt<64>(d, dt, G, smem, s);
+    case 128: return launch_records_nt<128>(d, dt, G, smem, s);
+    default: return launch_records_nt<256>(d, dt, G, smem, s);
+  }
 }
 
 // Group-stream assembly: schedule (per world) -> rounds (per group) -> records (per world).
@@ -776,7 +780,7 @@ cudaError_t egg_launch_assemble_stream(const EggDev& d, double dt, cudaStream_t 
     const size_t smem = wpc * per;
     if (smem > 48 * 1024) EGG_FIRST(e, cudaFuncSetAttribute(egg_schedule_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (e != cudaSuccess) return e;
-    egg_schedule_kernel<<<(d.W + wpc - 1) / wpc, 128, smem, s>>>(d, d.rmax > 0 ? egg_run_cap(d) : d.lpw, wpc, d.rmax);
+    egg_schedule_kernel<<<(d.W + wpc - 1) / wpc, 128, smem, s>>>(d, d.rmax > 0 ? d.run_cap : d.lpw, wpc, d.rmax);
   }
   if (d.rmax > 0) return egg_launch_assemble_runs_tail(d, dt, s);   // run headers and run-format records (egg_pgs_runs.cu)
   const int ngroups = (d.W + G - 1) / G;

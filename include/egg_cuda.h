@@ -317,6 +317,19 @@ int egg_sync(egg_batch* b);
 /* Per-world contact capacity actually allocated (max_contacts after rounding / the automatic rule). */
 int egg_capacity(const egg_batch* b);
 
+/* Which kernel instances the batch runs (read-only, no device access).  out[0] lanes per world of
+ * the PGS group stream (0 for the other solvers), out[1] worlds per warp (32 / out[0], or 0),
+ * out[2] M^-1 layout of the PGS kernel: 0 general 3x3, 1 isotropic per body, 2 isotropic and
+ * uniform, -1 before the first step after egg_init decides it, out[3] constraint-record format:
+ * 0 per-world records (dense, Jacobi, SOR), 1 PGS group stream, 2 PGS run format, -1 for PGS before
+ * the first step after egg_init, out[4] runs per world and stage of the run format (0 without it),
+ * out[5] record precision (64 or 32), out[6] narrowphase threads per world, out[7] record-assembly
+ * threads per world (for the run format: after the first step).  The development overrides
+ * EGG_PGS_LPW, EGG_PGS_MIN_WARPS_PER_SM, EGG_PGS_RUNS, EGG_PGS_RUN_CAP, EGG_PGS_TARGET_CTAS,
+ * EGG_COLLIDE_NT, EGG_RECORDS_NT (and EGG_PGS_CTAS_PER_SM, EGG_PGS_PF) are read by egg_create and
+ * apply to that batch only. */
+int egg_get_kernel_config(const egg_batch* b, int out[8]);
+
 /* Bytes of device memory held by the batch; number of kernel launches issued so far. */
 long long egg_device_bytes(const egg_batch* b);
 long long egg_launch_count(const egg_batch* b);

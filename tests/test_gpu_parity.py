@@ -3,59 +3,9 @@ time from shared state.  Discrete outputs bit-exact; p, R, v, w, lambda within 1
 import numpy as np
 import pytest
 
-from tests.helpers import oracle_world, compare_step, rel_err, SCALE
+from tests.helpers import oracle_world, compare_step, rel_err, SCALE, stepwise as _stepwise, stepwise_fp32
 
 pytestmark = pytest.mark.gpu
-
-
-def _stepwise(scene, nsteps, worlds_idx, batch_kw, oracle_kw, tol=1e-9, lam_tol=1e-9):
-    import eggshell_b200 as E
-    b = E.scenes.make_batch(scene, taps=True, **batch_kw)
-    ows = [oracle_world(scene, wi, **oracle_kw)[0] for wi in worlds_idx]
-    dt = scene["dt"]
-    worst_all = {}
-    for s in range(nsteps):
-        # shared state: the oracle adopts the GPU state before every step
-        p, R, v, w = b.bodies()
-        for k, wi in enumerate(worlds_idx):
-            ows[k].set_state(p[wi], R[wi], v[wi], w[wi])
-        b.step(dt)
-        for ow in ows:
-            ow.step(dt)
-        worst = compare_step(b, ows, worlds_idx, tol=tol, lam_tol=lam_tol)
-        st = b.status()
-        for k, wi in enumerate(worlds_idx):
-            os_ = ows[k].stats()
-            assert st["sweeps"][wi] == os_["sweeps"], f"step {s} world {wi}: sweeps {st['sweeps'][wi]} != {os_['sweeps']}"
-            lam, rhs, rs = ows[k].solution()
-            con = b.contacts()
-            con_rs = con["row_state"][wi, :len(rs)]
-            assert np.array_equal(con_rs, rs), f"step {s} world {wi}: row clamp states differ"
-            # Near-tie probe: the CUDA kernels contract multiply-adds, the oracle does not, so equal clamp
-            # states only mean something if no free multiplier sits within rounding distance of a bound.
-            # margin = distance of the closest strictly-inside multiplier to its bound (friction rows
-            # [-1, 1], normal rows [0, inf)); it must dwarf the CUDA-vs-oracle difference of that world.
-            lam = np.asarray(lam); rs = np.asarray(rs)
-            # bounded rows: contact blocks, except the first contact block after joints (quirk q2: block c is
-            # projected with the bounds of block c - 1, sparse_iterations_utils.cc:169,180,229-235)
-            blk = np.arange(len(lam)) // 3
-            bounded = (blk > scene["nj"]) if scene["nj"] else np.ones(len(lam), dtype=bool)
-            free = (rs == 0) & bounded
-            if free.any() and os_["sweeps"] > 0:      # zero sweeps: x is the unprojected initial guess (= rhs)
-                row = np.arange(len(lam)) % 3
-                dist = np.where(row < 2, 1.0 - np.abs(lam), np.abs(lam))[free]
-                diff = float(np.max(np.abs(con["lam"][wi, :len(lam)] - lam)))
-                margin = float(dist.min())
-                worst_all["clamp_margin"] = min(worst_all.get("clamp_margin", np.inf), margin)
-                worst_all["clamp_margin_over_diff"] = min(worst_all.get("clamp_margin_over_diff", np.inf), margin / max(diff, 1e-300))
-        assert worst["lam"] <= lam_tol, f"lambda mismatch {worst['lam']:.3e}"
-        for k_, v_ in worst.items():
-            worst_all[k_] = max(worst_all.get(k_, 0.0), v_)
-    b.close()
-    if "clamp_margin_over_diff" in worst_all:
-        # a free multiplier closer to its bound than ~the rounding difference would make the clamp state a coin toss
-        assert worst_all["clamp_margin_over_diff"] > 10.0, f"near-tie: margin {worst_all['clamp_margin']:.3e} is within 10x of the CUDA-vs-oracle difference"
-    return worst_all
 
 
 def test_stack10_pgs_stepwise():
@@ -343,41 +293,31 @@ def test_pgs_fp32_records_opt_in(name, W, k_max, steps):
     state within 1e-4 relative (north_star's FP32 tolerance; measured ~1e-6), same sweep counts."""
     import eggshell_b200 as E
     scene = getattr(E.scenes, name)(W)
-    b = E.scenes.make_batch(scene, solver=E.SOLVER_PGS, k_max=k_max, taps=True, precision=32)
-    ows = [oracle_world(scene, wi, solver=1, k_max=k_max)[0] for wi in range(W)]
-    worst_all = {}
-    for s in range(steps):
-        p, R, v, w = b.bodies()
-        for k in range(W):
-            ows[k].set_state(p[k], R[k], v[k], w[k])
-        b.step(scene["dt"])
-        for ow in ows:
-            ow.step(scene["dt"])
-        worst = compare_step(b, ows, list(range(W)), tol=1e-4, check_lambda=False)
-        st = b.status()
-        assert int(st["status"].max()) == 0
-        for k in range(W):
-            assert st["sweeps"][k] == ows[k].stats()["sweeps"]
-        for key, val in worst.items():
-            worst_all[key] = max(worst_all.get(key, 0.0), val)
-    b.close()
+    worst_all = stepwise_fp32(scene, steps, list(range(W)), dict(solver=E.SOLVER_PGS, k_max=k_max), dict(solver=1, k_max=k_max))
     print(name, "fp32 records worst", worst_all)
-    assert worst_all["v"] < 1e-4 and worst_all["w"] < 1e-4
 
 
-@pytest.mark.parametrize("name,W,k_max,lpw,opt", [("stack10", 65536, 10, "1", 0), ("stack10", 65536, 10, "", 0), ("pile64", 16384, 5, "", 0), ("pile64", 8192, 5, "16", 0),
-                                                 ("legged20", 131072, 10, "", 0), ("pile64", 16384, 5, "", 16), ("stack10", 65536, 10, "1", 16), ("legged20", 65536, 10, "", 16)])
-def test_full_size_step_is_bit_reproducible(name, W, k_max, lpw, opt, monkeypatch):
+@pytest.mark.parametrize("name,W,k_max,lpw,opt,prec,expect", [
+    ("stack10", 65536, 10, "1", 0, 64, 1), ("stack10", 65536, 10, "", 0, 64, 1), ("pile64", 16384, 5, "", 0, 64, 8),
+    ("pile64", 8192, 5, "16", 0, 64, 16), ("legged20", 131072, 10, "", 0, 64, 4), ("legged20", 65536, 10, "2", 0, 64, 2),
+    ("stack10", 65536, 10, "1", 0, 32, 1), ("pile64", 16384, 5, "", 16, 64, 8), ("stack10", 65536, 10, "1", 16, 64, 1),
+    ("legged20", 65536, 10, "", 16, 64, 4)])
+def test_full_size_step_is_bit_reproducible(name, W, k_max, lpw, opt, prec, expect, monkeypatch):
     """The kernels are deterministic, so the same full-size step from the same state must give the
     same bits every time.  This is the test that exposes ordering bugs between the shared-memory
     loads of a stage and the TMA copy of the next one (a generic fence instead of the cross-proxy
-    fence made 1-2 % of the worlds differ from run to run at 32 worlds per warp).  The last three
-    cases run the opt-in run format (EGG_OPT_PGS_RUNS), which hands its staging buffer back the same way."""
+    fence made 1-2 % of the worlds differ from run to run at 32 worlds per warp; the FP32 case runs
+    there, at LPW 1).  The last three cases run the opt-in run format (EGG_OPT_PGS_RUNS), which hands
+    its staging buffer back the same way.  Every case checks the lanes per world it ran at."""
     import eggshell_b200 as E
     if lpw:
         monkeypatch.setenv("EGG_PGS_LPW", lpw)
+    else:
+        monkeypatch.delenv("EGG_PGS_LPW", raising=False)
     scene = getattr(E.scenes, name)(W)
-    b = E.scenes.make_batch(scene, solver=E.SOLVER_PGS, k_max=k_max, max_contacts=1024 if name == "pile64" else 0, quirks=E.QUIRKS_REFERENCE | opt)   # opt 16 = the run format
+    b = E.scenes.make_batch(scene, solver=E.SOLVER_PGS, k_max=k_max, max_contacts=1024 if name == "pile64" else 0, quirks=E.QUIRKS_REFERENCE | opt,   # opt 16 = the run format
+                            precision=prec)
+    assert b.kernel_config()["lpw"] == expect
     b.snapshot()
     ref = None
     for r in range(3):
@@ -390,6 +330,8 @@ def test_full_size_step_is_bit_reproducible(name, W, k_max, lpw, opt, monkeypatc
             continue
         for a, c in zip(out, ref):
             assert np.array_equal(a.view(np.uint64), c.view(np.uint64)), f"run {r} differs from run 0"
+    cfg = b.kernel_config()
+    assert (cfg["lpw"], cfg["precision"], cfg["rec_format"]) == (expect, prec, 2 if opt & 16 else 1), cfg
     b.close()
 
 
@@ -900,16 +842,20 @@ def test_edge_cases_empty_ragged_capacity_and_errors():
 
 
 @pytest.mark.parametrize("name,W,k_max", [("pile64", 16384, 5), ("stack10", 65536, 10), ("legged20", 131072, 10)])
-def test_full_size_worlds_are_independent_of_the_batch(name, W, k_max):
+def test_full_size_worlds_are_independent_of_the_batch(name, W, k_max, monkeypatch):
     """Size-independent property that ties the full-size batches to the oracle-checked small ones: a
     world's step does not depend on which other worlds share its batch, its warp or its group stream.
     Sampled worlds of a full-occupancy batch (first / middle / last groups included) are stepped again
-    in a batch of their own -- other lanes per world, other neighbours, other stage cuts -- and must
-    give the same bits; the small batch is then compared with the oracle as usual."""
+    in a batch of their own -- other lanes per world (forced, and checked for both batches), other
+    neighbours, other stage cuts -- and must give the same bits; the small batch is then compared
+    with the oracle as usual."""
     import eggshell_b200 as E
+    big_lpw, small_lpw = dict(pile64=(8, 16), stack10=(1, 2), legged20=(4, 1))[name]
+    monkeypatch.delenv("EGG_PGS_LPW", raising=False)
     scene = getattr(E.scenes, name)(W)
     maxc = 1024 if name == "pile64" else 0
     b = E.scenes.make_batch(scene, solver=E.SOLVER_PGS, k_max=k_max, max_contacts=maxc)
+    assert b.kernel_config()["lpw"] == big_lpw
     b.step(scene["dt"])
     big = [x.copy() for x in b.bodies()]
     st_big = b.status()
@@ -921,7 +867,9 @@ def test_full_size_worlds_are_independent_of_the_batch(name, W, k_max):
         if key in scene and isinstance(scene[key], np.ndarray) and scene[key].shape[:1] == (W,):
             sub[key] = scene[key][pick].copy()
     sub["W"] = len(pick)
+    monkeypatch.setenv("EGG_PGS_LPW", str(small_lpw))
     sb = E.scenes.make_batch(sub, solver=E.SOLVER_PGS, k_max=k_max, max_contacts=maxc, taps=True)
+    assert sb.kernel_config()["lpw"] == small_lpw
     ows = [oracle_world(sub, k, solver=1, k_max=k_max)[0] for k in range(len(pick))]
     sb.step(sub["dt"])
     for ow in ows:
