@@ -23,7 +23,7 @@ ST_LCP_FAILED, ST_JOINT_CONFLICT, ST_BAD_INIT, ST_CONTACT_OVERFLOW, ST_NONFINITE
 EXPORTS = [
     "egg_desc_default", "egg_create", "egg_destroy", "egg_set_bodies", "egg_set_shapes", "egg_set_state", "egg_set_joints",
     "egg_set_external", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_step_controlled",
-    "egg_set_cost", "egg_step_controlled_cost", "egg_set_sampler", "egg_sample_controls", "egg_mppi_reduce", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
+    "egg_set_cost", "egg_step_controlled_cost", "egg_set_sampler", "egg_sample_controls", "egg_mppi_reduce", "egg_sample_controls_std", "egg_gather_controls", "egg_control_moments", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
     "egg_get_status", "egg_get_dense_work", "egg_get_debug_counters", "egg_rollout_costs", "egg_set_stream", "egg_sync", "egg_device_bytes",
     "egg_launch_count", "egg_capacity", "egg_get_kernel_config", "egg_set_profiling", "egg_get_kernel_ms", "egg_fp64_peak_tflops", "egg_host_alloc", "egg_host_free", "egg_last_error", "egg_version",
 ]
@@ -84,6 +84,10 @@ def lib():
         L.egg_set_sampler.argtypes = [C.c_void_p, C.c_void_p]
         L.egg_sample_controls.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_ulonglong, C.c_ulonglong, C.c_int, C.c_void_p]
         L.egg_mppi_reduce.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
+        L.egg_sample_controls_std.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_ulonglong, C.c_ulonglong, C.c_int,
+                                              C.c_void_p]
+        L.egg_gather_controls.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]
+        L.egg_control_moments.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
         _LIB = L
     return _LIB
 
@@ -135,7 +139,7 @@ class Batch:
         self.desc = d
         self.stream = None   # cudaStream_t handed to set_stream; None = the batch's own stream
         self.cost = None     # mpc.QuadraticCost handed to set_cost
-        self.sampler = None  # mpc.MPPI handed to set_sampler
+        self.sampler = None  # mpc.MPPI or mpc.CEM handed to set_sampler
         self.max_contacts = None
         self._probe_capacity()
 
@@ -238,14 +242,15 @@ class Batch:
 
     # -- MPPI sampling and weighted reduction --------------------------------------------------
     def set_sampler(self, mppi):
-        """Configures the noise scale and control bounds of sample_controls from an mpc.MPPI for this
-        batch's n bodies, or None to clear them (egg_set_sampler).  Synchronises the batch stream."""
-        from .mpc import MPPI
+        """Configures the noise scale and control bounds of sample_controls from an mpc.MPPI or mpc.CEM
+        (its initial sigma) for this batch's n bodies, or None to clear them (egg_set_sampler).
+        Synchronises the batch stream."""
+        from .mpc import CEM, MPPI
         if mppi is None:
             _chk(lib().egg_set_sampler(self.h, None), "egg_set_sampler")
         else:
-            if not isinstance(mppi, MPPI) or mppi.n != self.n:
-                raise ValueError(f"set_sampler takes an mpc.MPPI for n = {self.n} bodies, or None")
+            if not isinstance(mppi, (MPPI, CEM)) or mppi.n != self.n:
+                raise ValueError(f"set_sampler takes an mpc.MPPI or mpc.CEM for n = {self.n} bodies, or None")
             s = EggSampler(_p(mppi.sigma), _p(mppi.u_lo), _p(mppi.u_hi))
             _chk(lib().egg_set_sampler(self.h, C.byref(s)), "egg_set_sampler")
         self.sampler = mppi
@@ -263,6 +268,31 @@ class Batch:
         baseline_ptr is a device scalar."""
         _chk(lib().egg_mppi_reduce(self.h, C.c_void_p(u_ptr), int(horizon), C.c_void_p(cost_ptr), C.c_void_p(baseline_ptr),
                                    C.c_double(lam), C.c_void_p(out_ptr)), "egg_mppi_reduce")
+
+    # -- CEM sampling and elite refit ----------------------------------------------------------
+    def sample_controls_std(self, mean_ptr, std_ptr, horizon, seed, iteration, first, u_ptr):
+        """sample_controls with a per-step noise scale: u[t][w] = clamp(mean[t] + std[t] eps) from the
+        device arrays float64 [horizon][n][6] at mean_ptr and std_ptr, with the eps of sample_controls
+        (egg_sample_controls_std).  The bounds are the sampler's; its sigma is not used."""
+        _chk(lib().egg_sample_controls_std(self.h, C.c_void_p(mean_ptr), C.c_void_p(std_ptr), int(horizon), C.c_ulonglong(int(seed)),
+                                           C.c_ulonglong(int(iteration)), int(first), C.c_void_p(u_ptr)), "egg_sample_controls_std")
+
+    def gather_controls(self, u_ptr, horizon, worlds, out_ptr):
+        """Copies the schedules of the listed local worlds out of the device buffer at u_ptr, float64
+        [horizon][W][n][6], to the device buffer at out_ptr, [len(worlds)][horizon][n][6]
+        (egg_gather_controls)."""
+        w64 = np.asarray(worlds, dtype=np.int64).ravel()
+        idx = np.ascontiguousarray(w64, dtype=np.int32)
+        if not np.array_equal(idx, w64):
+            raise EggError("gather_controls: world index out of the int32 range")
+        _chk(lib().egg_gather_controls(self.h, C.c_void_p(u_ptr), int(horizon), _p(idx), int(idx.size), C.c_void_p(out_ptr)),
+             "egg_gather_controls")
+
+    def control_moments(self, rows_ptr, k, horizon, out_ptr):
+        """out (device, float64 [2][horizon][n][6]) = the mean and the population standard deviation of
+        the k rows [k][horizon][n][6] at rows_ptr, summed in row order (egg_control_moments)."""
+        _chk(lib().egg_control_moments(self.h, C.c_void_p(rows_ptr), int(k), int(horizon), C.c_void_p(out_ptr)),
+             "egg_control_moments")
 
     # -- device-side state exchange (MPC) ------------------------------------------------------
     def gather_state(self, worlds, out_ptr):

@@ -782,6 +782,57 @@ int egg_sample_controls(egg_batch* b, const double* u_nom_d, int horizon, unsign
   return EGG_OK;
 }
 
+int egg_sample_controls_std(egg_batch* b, const double* mean_d, const double* std_d, int horizon, unsigned long long seed,
+                            unsigned long long iteration, int first, double* u_d) {
+  if (!b) return EGG_ERR_ARG;
+  if (horizon < 1 || first < 0) { g_err = "egg_sample_controls_std: horizon must be >= 1 and first >= 0"; return EGG_ERR_ARG; }
+  RET(check_device_ptr(b, mean_d, "egg_sample_controls_std(mean_d)"));
+  RET(check_device_ptr(b, std_d, "egg_sample_controls_std(std_d)"));
+  RET(check_device_ptr(b, u_d, "egg_sample_controls_std(u_d)"));
+  RET(check_aligned16(mean_d, "egg_sample_controls_std(mean_d)"));
+  RET(check_aligned16(std_d, "egg_sample_controls_std(std_d)"));
+  RET(check_aligned16(u_d, "egg_sample_controls_std(u_d)"));
+  if (!b->initialised) { g_err = "egg_sample_controls_std before egg_init"; return EGG_ERR_STATE; }
+  if (!b->sampler_buf) { g_err = "egg_sample_controls_std without a sampler: call egg_set_sampler first"; return EGG_ERR_STATE; }
+  CK(cudaSetDevice(b->device));
+  LK(egg_launch_sample_std(b->dev, b->sampler, mean_d, std_d, horizon, seed, iteration, first, u_d, b->stream));
+  b->launches++;
+  return EGG_OK;
+}
+
+int egg_gather_controls(egg_batch* b, const double* u_d, int horizon, const int* worlds, int k, double* out_d) {
+  if (!b || !worlds) return EGG_ERR_ARG;
+  const int W = b->dev.W;
+  if (horizon < 1) { g_err = "egg_gather_controls: horizon must be >= 1"; return EGG_ERR_ARG; }
+  if (k < 1 || k > W) { g_err = "egg_gather_controls: k must be in [1, n_worlds]"; return EGG_ERR_ARG; }
+  for (int i = 0; i < k; i++)
+    if (worlds[i] < 0 || worlds[i] >= W) { g_err = "egg_gather_controls: world index out of range"; return EGG_ERR_ARG; }
+  if ((long long)k * horizon * b->dev.n * 6 > 256ll * INT_MAX) { g_err = "egg_gather_controls: too many rows"; return EGG_ERR_ARG; }
+  RET(check_device_ptr(b, u_d, "egg_gather_controls(u_d)"));
+  RET(check_device_ptr(b, out_d, "egg_gather_controls(out_d)"));
+  if (!b->initialised) { g_err = "egg_gather_controls before egg_init"; return EGG_ERR_STATE; }
+  CK(cudaSetDevice(b->device));
+  if (!b->gather_idx) RET(dalloc(b, &b->gather_idx, (size_t)W));
+  CK(cudaMemcpyAsync(b->gather_idx, worlds, (size_t)k * sizeof(int), cudaMemcpyHostToDevice, b->stream));
+  LK(egg_launch_gather_controls(b->dev, u_d, horizon, b->gather_idx, k, out_d, b->stream));
+  b->launches++;
+  return EGG_OK;
+}
+
+int egg_control_moments(egg_batch* b, const double* rows_d, int k, int horizon, double* out_d) {
+  if (!b) return EGG_ERR_ARG;
+  if (k < 1 || horizon < 1) { g_err = "egg_control_moments: k and horizon must be >= 1"; return EGG_ERR_ARG; }
+  const long long L = (long long)horizon * b->dev.n * 6;
+  if (L > INT_MAX) { g_err = "egg_control_moments: too long a horizon"; return EGG_ERR_ARG; }
+  RET(check_device_ptr(b, rows_d, "egg_control_moments(rows_d)"));
+  RET(check_device_ptr(b, out_d, "egg_control_moments(out_d)"));
+  if (!b->initialised) { g_err = "egg_control_moments before egg_init"; return EGG_ERR_STATE; }
+  CK(cudaSetDevice(b->device));
+  LK(egg_launch_control_moments(rows_d, k, (int)L, out_d, b->stream));
+  b->launches++;
+  return EGG_OK;
+}
+
 int egg_mppi_reduce(egg_batch* b, const double* u_d, int horizon, const double* cost_d, const double* baseline_d,
                     double lambda, double* out_d) {
   if (!b) return EGG_ERR_ARG;

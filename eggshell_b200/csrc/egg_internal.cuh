@@ -207,6 +207,14 @@ cudaError_t egg_launch_mppi_sample(const EggDev& d, const EggSampler& sm, const 
 int egg_mppi_chunks(int W);   // stage-1 chunks of egg_launch_mppi_reduce: partial holds chunks x (H n 6 + 2) doubles
 cudaError_t egg_launch_mppi_reduce(const EggDev& d, const double* u, int horizon, const double* cost, const double* baseline,
                                    double lambda, double* partial, double* out, cudaStream_t s);
+// CEM (egg_sample_controls_std, egg_gather_controls, egg_control_moments): the sampler with the
+// per-step std [H][n][6] in place of sm.sigma; out [k][H][n][6] <- u[t][worlds[i]];
+// out [2][L] <- mean and population std of the columns of rows [k][L]
+cudaError_t egg_launch_sample_std(const EggDev& d, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
+                                  unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s);
+cudaError_t egg_launch_gather_controls(const EggDev& d, const double* u, int horizon, const int* worlds, int k, double* out,
+                                       cudaStream_t s);
+cudaError_t egg_launch_control_moments(const double* rows, int k, int L, double* out, cudaStream_t s);
 // Dynamic shared memory each kernel family needs for this batch shape (checked against the device
 // limit in egg_create, so that an unsupported shape fails there with a clear message).
 size_t egg_collide_smem(const EggDev& d);

@@ -2,6 +2,8 @@
 // the step.  egg_sample_controls writes W perturbed copies of a nominal control schedule;
 // egg_mppi_reduce sums them weighted by exp(-(J - J_min) / lambda).  Both touch the whole
 // [H][W][n][6] schedule (6.3 GB at 131072 legged20 worlds and H = 50) and nothing else of size.
+// CEM (cross-entropy method) shares the sampler with a per-step sigma (egg_sample_controls_std) and
+// refits on the elites: egg_gather_controls copies their schedules, egg_control_moments averages them.
 #include "egg_internal.cuh"
 #include <curand_philox4x32_x.h>   // header-only device code of the toolkit: curand_Philox4x32_10
 
@@ -16,10 +18,16 @@ __device__ __forceinline__ double egg_u01(unsigned lo, unsigned hi) {
 // clamp that lets NaN through (fmin/fmax would replace it by a bound)
 __device__ __forceinline__ double egg_clamp(double v, double lo, double hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
+// Where the sampler kernel reads sigma.sigma from: the sampler's per-body [6][n] array, the same for
+// every step (egg_sample_controls), or the caller's per-step [H][n][6] device array read like u_nom
+// (egg_sample_controls_std).  Everything else, the noise included, is the same code.
+enum EggSigmaFrom { EGG_SIGMA_PER_BODY, EGG_SIGMA_PER_STEP };
+
 // One thread per (step, world, body, component pair): i = (w n + b) 3 + p within step t, so thread i
 // writes the two adjacent doubles u[t][w][b][2p, 2p + 1] as one 16-byte store and a warp writes 512
 // consecutive bytes.  The noise is computed for every element whatever sigma is (sigma = 0 costs what
 // sigma > 0 does); global world 0 and sigma = 0 keep u_nom bit for bit (-0.0 included).
+template <EggSigmaFrom kFrom>
 __global__ void __launch_bounds__(256) egg_mppi_sample_kernel(const double* __restrict__ u_nom, EggSampler sm, int W, int n,
                                                               int H, unsigned per_step, uint2 key, uint2 iter, int first,
                                                               double2* __restrict__ u) {
@@ -28,7 +36,8 @@ __global__ void __launch_bounds__(256) egg_mppi_sample_kernel(const double* __re
   const unsigned p = i % 3u, r = i / 3u, b = r % (unsigned)n, w = r / (unsigned)n;
   const unsigned g = (unsigned)first + w;
   const int j = 2 * (int)p;
-  const double s0 = sm.sigma[j * n + b], s1 = sm.sigma[(j + 1) * n + b];
+  double s0 = 0.0, s1 = 0.0;
+  if constexpr (kFrom == EGG_SIGMA_PER_BODY) s0 = sm.sigma[j * n + b], s1 = sm.sigma[(j + 1) * n + b];
   const double lo0 = sm.lo[j * n + b], lo1 = sm.lo[(j + 1) * n + b];
   const double hi0 = sm.hi[j * n + b], hi1 = sm.hi[(j + 1) * n + b];
   for (int t = blockIdx.y; t < H; t += gridDim.y) {
@@ -38,6 +47,10 @@ __global__ void __launch_bounds__(256) egg_mppi_sample_kernel(const double* __re
     double sn, cs;
     sincospi(2.0 * u2, &sn, &cs);
     const double2 m = *reinterpret_cast<const double2*>(u_nom + ((size_t)t * n + b) * 6 + j);
+    if constexpr (kFrom == EGG_SIGMA_PER_STEP) {
+      const double2 sd = *reinterpret_cast<const double2*>(sm.sigma + ((size_t)t * n + b) * 6 + j);
+      s0 = sd.x, s1 = sd.y;
+    }
     double v0 = m.x + s0 * (rad * cs), v1 = m.y + s1 * (rad * sn);
     if (g == 0 || s0 == 0.0) v0 = m.x;
     if (g == 0 || s1 == 0.0) v1 = m.y;
@@ -98,14 +111,70 @@ __global__ void __launch_bounds__(256) egg_mppi_reduce_final_kernel(const double
   out[col] = s;
 }
 
-cudaError_t egg_launch_mppi_sample(const EggDev& d, const EggSampler& sm, const double* u_nom, int horizon,
-                                   unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s) {
+// CEM refit (egg_control_moments): one thread per column of rows [k][L], two passes down the column
+// in row order: mean = sum / k, then std = sqrt(sum (x - mean)^2 / k).  The square is rounded before
+// it is added (no fused multiply-add), so the result is the plain float64 definition bit for bit and
+// depends only on k, L and the rows.  Consecutive threads read consecutive doubles of a row.
+__global__ void __launch_bounds__(256) egg_control_moments_kernel(const double* __restrict__ rows, int k, int L,
+                                                                  double* __restrict__ out) {
+  const int col = blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= L) return;
+  const double* x = rows + col;
+  double s = 0.0;
+  for (int i = 0; i < k; i++) s += x[(size_t)i * L];
+  const double mean = s / k;
+  double q = 0.0;
+  for (int i = 0; i < k; i++) {
+    const double dv = x[(size_t)i * L] - mean;
+    q += __dmul_rn(dv, dv);
+  }
+  out[col] = mean;
+  out[L + col] = sqrt(q / k);
+}
+
+// out[i][t][:] = u[t][worlds[i]][:], the n 6 doubles of a step copied as they are (one thread each).
+__global__ void __launch_bounds__(256) egg_gather_controls_kernel(const double* __restrict__ u, int W, int n6, int H,
+                                                                  const int* __restrict__ worlds, int k,
+                                                                  double* __restrict__ out) {
+  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gid >= (long long)k * H * n6) return;
+  const int e = (int)(gid % n6);
+  const long long r = gid / n6;
+  const int t = (int)(r % H), i = (int)(r / H);
+  out[gid] = u[((size_t)t * W + worlds[i]) * n6 + e];
+}
+
+template <EggSigmaFrom kFrom>
+static cudaError_t launch_sample(const EggDev& d, const EggSampler& sm, const double* u_nom, int horizon, unsigned long long seed,
+                                 unsigned long long iteration, int first, double* u, cudaStream_t s) {
   const unsigned per_step = (unsigned)d.W * (unsigned)d.n * 3u;
   const dim3 grid((per_step + 255) / 256, (unsigned)min(horizon, 65535));
-  egg_mppi_sample_kernel<<<grid, 256, 0, s>>>(u_nom, sm, d.W, d.n, horizon, per_step,
-                                              make_uint2((unsigned)seed, (unsigned)(seed >> 32)),
-                                              make_uint2((unsigned)iteration, (unsigned)(iteration >> 32)), first,
-                                              reinterpret_cast<double2*>(u));
+  egg_mppi_sample_kernel<kFrom><<<grid, 256, 0, s>>>(u_nom, sm, d.W, d.n, horizon, per_step,
+                                                     make_uint2((unsigned)seed, (unsigned)(seed >> 32)),
+                                                     make_uint2((unsigned)iteration, (unsigned)(iteration >> 32)), first,
+                                                     reinterpret_cast<double2*>(u));
+  return cudaGetLastError();
+}
+
+cudaError_t egg_launch_mppi_sample(const EggDev& d, const EggSampler& sm, const double* u_nom, int horizon,
+                                   unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s) {
+  return launch_sample<EGG_SIGMA_PER_BODY>(d, sm, u_nom, horizon, seed, iteration, first, u, s);
+}
+
+cudaError_t egg_launch_sample_std(const EggDev& d, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
+                                  unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s) {
+  return launch_sample<EGG_SIGMA_PER_STEP>(d, EggSampler{std_dev, sm.lo, sm.hi}, mean, horizon, seed, iteration, first, u, s);
+}
+
+cudaError_t egg_launch_gather_controls(const EggDev& d, const double* u, int horizon, const int* worlds, int k, double* out,
+                                       cudaStream_t s) {
+  const long long total = (long long)k * horizon * d.n * 6;
+  egg_gather_controls_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(u, d.W, d.n * 6, horizon, worlds, k, out);
+  return cudaGetLastError();
+}
+
+cudaError_t egg_launch_control_moments(const double* rows, int k, int L, double* out, cudaStream_t s) {
+  egg_control_moments_kernel<<<(unsigned)((L + 255) / 256), 256, 0, s>>>(rows, k, L, out);
   return cudaGetLastError();
 }
 

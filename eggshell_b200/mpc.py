@@ -2,7 +2,8 @@
 of per-rollout costs followed by an identical arg-min / top-k on every rank (SURVEY.md §8e) — and
 the receding-horizon loop built on it: the winners' terminal states are gathered from their owner
 ranks and re-seed every world for the next horizon (`mpc_iteration`) — and an MPPI planner on top of
-the same pieces (`MPPI`, `mppi_iteration`, `mppi_advance`).
+the same pieces (`MPPI`, `mppi_iteration`, `mppi_advance`), and a cross-entropy-method planner whose
+elites' schedules are exchanged like the winners' states (`CEM`, `cem_iteration`, `cem_advance`).
 
 Worlds are independent (the reference already steps two unrelated ensembles per SimulationStep,
 /root/reference/eggshell/model.cc:67-68), so there is no data-path exchange inside a horizon."""
@@ -189,7 +190,59 @@ def mpc_iteration(batch, u, dt, k, n_total, first):
     return winners, best, states
 
 
-class MPPI:
+class _SamplingPlan:
+    """What the sampling planners share: a nominal schedule u_nom, float64 [horizon, n, 6] on `device`,
+    the per-body sigma and bounds handed to Batch.set_sampler, the Philox seed and the iteration
+    counter.  Validated here with the rules that MPPI documents."""
+
+    def __init__(self, n, horizon, sigma, u_lo, u_hi, seed, u_nom, device):
+        import torch
+        name = type(self).__name__
+        n, horizon = int(n), int(horizon)
+        if n < 1 or horizon < 1:
+            raise ValueError(f"{name}: n and horizon must be >= 1")
+        U = CONTROL_PER_BODY
+        self.n, self.horizon = n, horizon
+        self.sigma = self._arr(sigma, (n, U), "sigma")
+        if not np.isfinite(self.sigma).all() or (self.sigma < 0).any():
+            raise ValueError(f"{name}: sigma must be finite and >= 0")
+        self.u_lo = None if u_lo is None else self._arr(u_lo, (n, U), "u_lo")
+        self.u_hi = None if u_hi is None else self._arr(u_hi, (n, U), "u_hi")
+        for a, what in ((self.u_lo, "u_lo"), (self.u_hi, "u_hi")):
+            if a is not None and np.isnan(a).any():
+                raise ValueError(f"{name}: {what} has NaN values")
+        lo = np.full((n, U), -np.inf) if self.u_lo is None else self.u_lo
+        hi = np.full((n, U), np.inf) if self.u_hi is None else self.u_hi
+        if (lo > hi).any():
+            raise ValueError(f"{name}: u_lo > u_hi")
+        seed = int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError(f"{name}: seed must be in [0, 2^64)")
+        self.seed = seed
+        un = np.zeros((horizon, n, U)) if u_nom is None else self._arr(
+            u_nom.detach().cpu().numpy() if isinstance(u_nom, torch.Tensor) else u_nom, (horizon, n, U), "u_nom")
+        if not np.isfinite(un).all():
+            raise ValueError(f"{name}: u_nom has non-finite values")
+        self.device = torch.device(device)
+        self.u_nom = torch.from_numpy(un.copy()).to(self.device)   # own storage: the iterations write to it
+        self.lo = torch.from_numpy(lo).to(self.device)   # the bounds as tensors, for clamp on the device
+        self.hi = torch.from_numpy(hi).to(self.device)
+        self.iteration = 0
+
+    def _arr(self, a, shape, what):
+        a = np.asarray(a, dtype=np.float64)
+        try:
+            return np.ascontiguousarray(np.broadcast_to(a, shape))
+        except ValueError:
+            raise ValueError(f"{type(self).__name__}: {what} of shape {a.shape} does not broadcast to {list(shape)}") from None
+
+    def clamp(self, u):
+        """u clamped to [u_lo, u_hi] (broadcast over leading dimensions)."""
+        import torch
+        return torch.clamp(u, min=self.lo, max=self.hi)
+
+
+class MPPI(_SamplingPlan):
     """Planner state of MPPI (model predictive path integral): a nominal schedule u_nom, float64
     [horizon, n, 6] on `device`, improved by mppi_iteration and executed by mppi_advance.
 
@@ -201,54 +254,39 @@ class MPPI:
     to Batch.set_sampler before mppi_iteration."""
 
     def __init__(self, n, horizon, sigma, lam, u_lo=None, u_hi=None, seed=0, u_nom=None, device="cuda"):
-        import torch
-        n, horizon = int(n), int(horizon)
-        if n < 1 or horizon < 1:
-            raise ValueError("MPPI: n and horizon must be >= 1")
-        U = CONTROL_PER_BODY
-        self.n, self.horizon = n, horizon
-        self.sigma = self._arr(sigma, (n, U), "sigma")
-        if not np.isfinite(self.sigma).all() or (self.sigma < 0).any():
-            raise ValueError("MPPI: sigma must be finite and >= 0")
-        self.u_lo = None if u_lo is None else self._arr(u_lo, (n, U), "u_lo")
-        self.u_hi = None if u_hi is None else self._arr(u_hi, (n, U), "u_hi")
-        for a, name in ((self.u_lo, "u_lo"), (self.u_hi, "u_hi")):
-            if a is not None and np.isnan(a).any():
-                raise ValueError(f"MPPI: {name} has NaN values")
-        lo = np.full((n, U), -np.inf) if self.u_lo is None else self.u_lo
-        hi = np.full((n, U), np.inf) if self.u_hi is None else self.u_hi
-        if (lo > hi).any():
-            raise ValueError("MPPI: u_lo > u_hi")
         lam = float(lam)
         if not (np.isfinite(lam) and lam > 0):
             raise ValueError("MPPI: lam must be finite and > 0")
         self.lam = lam
-        seed = int(seed)
-        if not 0 <= seed < 2 ** 64:
-            raise ValueError("MPPI: seed must be in [0, 2^64)")
-        self.seed = seed
-        un = np.zeros((horizon, n, U)) if u_nom is None else self._arr(
-            u_nom.detach().cpu().numpy() if isinstance(u_nom, torch.Tensor) else u_nom, (horizon, n, U), "u_nom")
-        if not np.isfinite(un).all():
-            raise ValueError("MPPI: u_nom has non-finite values")
-        self.device = torch.device(device)
-        self.u_nom = torch.from_numpy(un).to(self.device)
-        self.lo = torch.from_numpy(lo).to(self.device)   # the bounds as tensors, for clamp on the device
-        self.hi = torch.from_numpy(hi).to(self.device)
-        self.iteration = 0
+        super().__init__(n, horizon, sigma, u_lo, u_hi, seed, u_nom, device)
 
-    @staticmethod
-    def _arr(a, shape, name):
-        a = np.asarray(a, dtype=np.float64)
-        try:
-            return np.ascontiguousarray(np.broadcast_to(a, shape))
-        except ValueError:
-            raise ValueError(f"MPPI: {name} of shape {a.shape} does not broadcast to {list(shape)}") from None
 
-    def clamp(self, u):
-        """u clamped to [u_lo, u_hi] (broadcast over leading dimensions)."""
+class CEM(_SamplingPlan):
+    """Planner state of the cross-entropy method: a mean schedule u_nom and a per-step standard
+    deviation std, both float64 [horizon, n, 6] on `device`, refitted to the n_elite cheapest rollouts
+    by cem_iteration and executed by cem_advance.
+
+    sigma: the initial standard deviation per body and control component, broadcast to [n, 6], finite
+    and >= 0; std starts as sigma in every step, and the row that cem_advance appends takes it again.
+    n_elite: the number of elites, >= 1 (at most the number of worlds of the sweep).  alpha: the
+    smoothing of the refit, u_nom <- clamp(alpha u_nom + (1 - alpha) mean of the elites) and
+    std <- max(alpha std + (1 - alpha) std of the elites, sigma_min); 0 <= alpha < 1.  sigma_min: a
+    floor on std that keeps the search from collapsing, finite and >= 0.  u_lo, u_hi, seed and u_nom
+    follow the rules of MPPI.  Hand the planner to Batch.set_sampler before cem_iteration."""
+
+    def __init__(self, n, horizon, sigma, n_elite, alpha=0.0, sigma_min=0.0, u_lo=None, u_hi=None, seed=0, u_nom=None,
+                 device="cuda"):
         import torch
-        return torch.clamp(u, min=self.lo, max=self.hi)
+        n_elite, alpha, sigma_min = int(n_elite), float(alpha), float(sigma_min)
+        if n_elite < 1:
+            raise ValueError("CEM: n_elite must be >= 1")
+        if not 0.0 <= alpha < 1.0:
+            raise ValueError("CEM: alpha must be in [0, 1)")
+        if not (np.isfinite(sigma_min) and sigma_min >= 0):
+            raise ValueError("CEM: sigma_min must be finite and >= 0")
+        self.n_elite, self.alpha, self.sigma_min = n_elite, alpha, sigma_min
+        super().__init__(n, horizon, sigma, u_lo, u_hi, seed, u_nom, device)
+        self.std = torch.tensor(np.broadcast_to(self.sigma, (self.horizon, self.n, CONTROL_PER_BODY)), device=self.device)
 
 
 def allgather_rows(x):
@@ -274,24 +312,36 @@ def allgather_rank_sum(x):
     return acc
 
 
-def _mppi_check(batch, mppi, u, first):
+def _mppi_check(batch, plan, u, first):
+    """The checks of mppi_iteration and cem_iteration for a plan (MPPI or CEM) and a schedule buffer u."""
     import torch
     import torch.distributed as dist
     dev = torch.device("cuda", int(batch.desc.device))
-    H = mppi.horizon
+    H = plan.horizon
     if not (isinstance(u, torch.Tensor) and u.is_cuda and u.device == dev and u.dtype == torch.float64
             and u.is_contiguous() and u.dim() == 4 and u.shape[0] == H and tuple(u.shape[1:]) == (batch.W, batch.n, 6)):
         raise ValueError(f"u must be a contiguous float64 tensor [{H}, {batch.W}, {batch.n}, 6] on {dev}")
     if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
         raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
-    if batch.sampler is not mppi:
+    if batch.sampler is not plan:
         raise ValueError("the batch's sampler is not this planner: call Batch.set_sampler(mppi) first")
-    if mppi.u_nom.device != dev:
+    if plan.u_nom.device != dev:
         raise ValueError(f"the planner's u_nom must live on {dev}")
     rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
     if (first == 0) != (rank == 0):
         raise ValueError("rank 0 must own global world 0 (first = 0 exactly on rank 0)")
     return dev
+
+
+def _rollout(batch, dt, u, costs):
+    """Every world runs the schedule u [H, W, n, 6] from the current state; costs [W] receives J from
+    the batch's QuadraticCost (step_controlled_cost), or without one from the built-in cost
+    (step_controlled + rollout_costs)."""
+    if batch.cost is None:
+        batch.step_controlled(dt, u.data_ptr(), u.shape[0])
+        batch.rollout_costs(costs.data_ptr())
+    else:
+        batch.step_controlled_cost(dt, u.data_ptr(), u.shape[0], costs.data_ptr())
 
 
 def mppi_sample(batch, mppi, u, first):
@@ -339,11 +389,7 @@ def mppi_iteration(batch, mppi, dt, u, first):
     costs = torch.empty(batch.W, dtype=torch.float64, device=dev)
     batch.restore()
     mppi_sample(batch, mppi, u, first)
-    if batch.cost is None:
-        batch.step_controlled(dt, u.data_ptr(), mppi.horizon)
-        batch.rollout_costs(costs.data_ptr())
-    else:
-        batch.step_controlled_cost(dt, u.data_ptr(), mppi.horizon, costs.data_ptr())
+    _rollout(batch, dt, u, costs)
     candidate, stats = mppi_combine(batch, mppi, u, costs)
     nominal, jmin, wsum, w2 = stats.cpu().numpy().tolist()
     if not wsum > 0:
@@ -353,19 +399,19 @@ def mppi_iteration(batch, mppi, dt, u, first):
     return {"nominal_cost": nominal, "min_cost": jmin, "weight_sum": wsum, "ess": wsum * wsum / w2}
 
 
-def mppi_advance(batch, mppi, dt, n_total):
-    """Executes the plan's first control: from the snapshot every world takes one step with
-    clamp(u_nom[0]); global world 0's new state re-seeds every world of every rank and becomes the
-    snapshot, the start of the next horizon; u_nom shifts by one step (the last row repeats).  This
-    costs one step of the whole batch, 1/H of a horizon.  Returns (the executed control [n, 6], the
-    new start rows [n, 18]), float64 CUDA tensors."""
+def mppi_advance(batch, plan, dt, n_total):
+    """Executes the plan's first control (plan: an MPPI or a CEM): from the snapshot every world takes
+    one step with clamp(u_nom[0]); global world 0's new state re-seeds every world of every rank and
+    becomes the snapshot, the start of the next horizon; u_nom shifts by one step (the last row
+    repeats).  This costs one step of the whole batch, 1/H of a horizon.  Returns (the executed control
+    [n, 6], the new start rows [n, 18]), float64 CUDA tensors."""
     import torch
     dev = torch.device("cuda", int(batch.desc.device))
-    if mppi.u_nom.device != dev:
+    if plan.u_nom.device != dev:
         raise ValueError(f"the planner's u_nom must live on {dev}")
     if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
         raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
-    u0 = mppi.clamp(mppi.u_nom[0])
+    u0 = plan.clamp(plan.u_nom[0])
     batch.restore()
     batch.step_controlled(dt, u0.expand(1, batch.W, batch.n, CONTROL_PER_BODY).contiguous().data_ptr(), 1)
     F = batch.n * STATE_PER_BODY
@@ -379,6 +425,100 @@ def mppi_advance(batch, mppi, dt, n_total):
     state = gather_winner_states([0], n_total, pack)
     batch.seed_state(state.data_ptr(), 1, 0)
     batch.snapshot()
-    if mppi.horizon > 1:
-        mppi.u_nom[:-1] = mppi.u_nom[1:].clone()
+    if plan.horizon > 1:
+        plan.u_nom[:-1] = plan.u_nom[1:].clone()
     return u0, state.view(batch.n, STATE_PER_BODY)
+
+
+def cem_sample(batch, cem, u, first):
+    """Step 2 of cem_iteration: the schedules of this iteration, clamp(u_nom + std eps), into u."""
+    batch.sample_controls_std(cem.u_nom.data_ptr(), cem.std.data_ptr(), cem.horizon, cem.seed, cem.iteration, first, u.data_ptr())
+
+
+def cem_select(cem, costs, n_total, pack):
+    """Steps 4 and 5 of cem_iteration: the cost allgather, the n_elite cheapest rollouts among those
+    with a finite cost (select_best: ties by the lowest global world index) and their schedules from
+    their owner ranks (gather_winner_states with `pack`), so every rank holds the same rows, bit for
+    bit, in elite order.  Returns (all costs, elite indices, elite costs, rows [n_elite, F]).  Raises
+    before the exchange if fewer than n_elite rollouts finished with a finite cost."""
+    import torch
+    all_costs = allgather_costs(costs)
+    finite = torch.where(torch.isfinite(all_costs), all_costs, torch.full_like(all_costs, float("inf")))
+    elites, ecost = select_best(finite, cem.n_elite)
+    n_finite = int(np.isfinite(ecost).sum())
+    if n_finite < cem.n_elite:
+        raise RuntimeError(f"cem_iteration: {n_finite} rollouts finished with a finite cost, fewer than n_elite = {cem.n_elite}; "
+                           "the plan is unchanged")
+    return all_costs, elites, ecost, gather_winner_states(elites, n_total, pack)
+
+
+def cem_refit(cem, moments):
+    """Step 7 of cem_iteration without committing it: from the elites' moments [2, H, n, 6] (mean,
+    population std), the candidate (clamp(alpha u_nom + (1 - alpha) mean),
+    max(alpha std + (1 - alpha) std_e, sigma_min)).  Elementwise, so every rank computes the same bits."""
+    import torch
+    a = cem.alpha
+    u_nom = cem.clamp(a * cem.u_nom + (1.0 - a) * moments[0])
+    std = torch.clamp(a * cem.std + (1.0 - a) * moments[1], min=cem.sigma_min)
+    return u_nom, std
+
+
+def cem_iteration(batch, cem, dt, u, first, n_total):
+    """One CEM iteration of a (sharded) sweep of n_total worlds.  u is the caller's schedule buffer, a
+    contiguous float64 CUDA tensor [H, W, n, 6] on the batch's device, overwritten with this
+    iteration's samples; first is the global index of local world 0 (0 on rank 0).  The batch must run
+    on torch's current stream and sample with this planner (Batch.set_sampler(cem)).
+
+      1. restore the snapshot;  2. sample clamp(u_nom + std eps) into u (global world 0: clamp(u_nom));
+      3. roll them out with the batch's QuadraticCost, or without one with the built-in cost;
+      4. allgather the costs and pick the n_elite cheapest finite ones (identical on every rank);
+      5. fetch the elites' schedules from their owner ranks (gather_controls, one allgather);
+      6. control_moments: their mean and population std, computed identically on every rank;
+      7. u_nom <- clamp(alpha u_nom + (1 - alpha) mean), std <- max(alpha std + (1 - alpha) std_e,
+         sigma_min);  iteration += 1.
+
+    Every rank holds the same plan bits, whatever the sharding.  Returns {nominal_cost, min_cost,
+    elite_max_cost, mean_std}: the cost of global world 0 (the plan itself), the cheapest and the most
+    expensive elite, and the mean of the new std.  If fewer than n_elite rollouts finished with a finite
+    cost, or the refit is not finite, it raises and leaves the plan and iteration unchanged."""
+    import torch
+    dev = _mppi_check(batch, cem, u, first)
+    if cem.std.device != dev:
+        raise ValueError(f"the planner's std must live on {dev}")
+    H, U = cem.horizon, CONTROL_PER_BODY
+    costs = torch.empty(batch.W, dtype=torch.float64, device=dev)
+    batch.restore()
+    cem_sample(batch, cem, u, first)
+    _rollout(batch, dt, u, costs)
+    F = H * batch.n * U
+
+    def pack(local):
+        out = torch.empty((len(local), F), dtype=torch.float64, device=dev)
+        if len(local):
+            batch.gather_controls(u.data_ptr(), H, local, out.data_ptr())
+        return out
+
+    all_costs, elites, ecost, rows = cem_select(cem, costs, n_total, pack)
+    moments = torch.empty((2, H, batch.n, U), dtype=torch.float64, device=dev)
+    batch.control_moments(rows.contiguous().data_ptr(), len(elites), H, moments.data_ptr())
+    u_nom, std = cem_refit(cem, moments)
+    ok = torch.isfinite(u_nom).all() & torch.isfinite(std).all()
+    nominal, mean_std, ok = torch.stack([all_costs[0], std.mean(), ok.double()]).cpu().numpy().tolist()
+    if not ok:
+        raise RuntimeError("cem_iteration: the refitted plan is not finite; the plan is unchanged")
+    cem.u_nom.copy_(u_nom)
+    cem.std.copy_(std)
+    cem.iteration += 1
+    return {"nominal_cost": nominal, "min_cost": float(ecost[0]), "elite_max_cost": float(ecost[-1]), "mean_std": mean_std}
+
+
+def cem_advance(batch, cem, dt, n_total):
+    """Executes the plan's first control with mppi_advance (every world steps with clamp(u_nom[0]) and
+    is re-seeded from global world 0, u_nom shifts by one step), then shifts std by one step; its new
+    last row is the initial sigma.  Returns what mppi_advance returns."""
+    import torch
+    executed = mppi_advance(batch, cem, dt, n_total)
+    if cem.horizon > 1:
+        cem.std[:-1] = cem.std[1:].clone()
+    cem.std[-1] = torch.tensor(cem.sigma, device=cem.std.device)
+    return executed

@@ -252,6 +252,38 @@ int egg_sample_controls(egg_batch* b, const double* u_nom_d, int horizon, unsign
 int egg_mppi_reduce(egg_batch* b, const double* u_d, int horizon, const double* cost_d, const double* baseline_d,
                     double lambda, double* out_d);
 
+/* CEM (cross-entropy method, INTEGRATION.md): sample around a mean schedule with a per-step standard
+ * deviation, keep the k cheapest rollouts (the elites) and refit mean and standard deviation to them.
+ *
+ * u_d[t][w][b][j] = clamp(mean_d[t][b][j] + std_d[t][b][j] eps, u_lo[b][j], u_hi[b][j]) for t < horizon
+ * and every local world w; mean_d and std_d are DEVICE [horizon][n_bodies][6] arrays, u_d is
+ * [horizon][W][n_bodies][6].  eps is exactly the eps of egg_sample_controls for the same seed,
+ * iteration and global world first + w (the same Philox key and counter, uniforms and Box-Muller), so
+ * with std_d[t] = sigma for every t the output is that of egg_sample_controls bit for bit.  Global
+ * world 0 and std = 0 keep clamp(mean) bit for bit.  The bounds come from egg_set_sampler; its sigma is
+ * not used.  std_d values are the caller's: finite and >= 0 give a clamped normal sample.
+ * EGG_ERR_STATE without a sampler or before egg_init; EGG_ERR_ARG for horizon < 1, first < 0, a
+ * pointer that is not device memory of the batch's device, or one that is not 16-byte aligned.
+ * Asynchronous on the batch stream; one launch. */
+int egg_sample_controls_std(egg_batch* b, const double* mean_d, const double* std_d, int horizon, unsigned long long seed,
+                            unsigned long long iteration, int first, double* u_d);
+
+/* out_d[i] ([k][horizon][n_bodies][6], device) = the schedule of local world worlds[i] in u_d
+ * ([horizon][W][n_bodies][6]), copied bit for bit.  worlds is a HOST int array, each entry in [0, W),
+ * duplicates allowed; 1 <= k <= W (the rules of egg_gather_state).  EGG_ERR_ARG for those, horizon < 1
+ * or a pointer that is not device memory of the batch's device; EGG_ERR_STATE before egg_init.
+ * Asynchronous on the batch stream; one launch. */
+int egg_gather_controls(egg_batch* b, const double* u_d, int horizon, const int* worlds, int k, double* out_d);
+
+/* The moments of k schedules rows_d [k][horizon][n_bodies][6] (device), per element:
+ * out_d[0] = mean = (the rows added in row order) / k and out_d[1] = the population standard
+ * deviation sqrt(sum_i (x_i - mean)^2 / k), a second pass in row order with every square rounded
+ * before it is added; out_d is [2][horizon][n_bodies][6] (device).  No atomics: the bits depend only
+ * on k, n_bodies, horizon and the rows, and NaN propagates.  EGG_ERR_ARG for k < 1, horizon < 1 or a
+ * pointer that is not device memory of the batch's device; EGG_ERR_STATE before egg_init.
+ * Asynchronous on the batch stream; one launch. */
+int egg_control_moments(egg_batch* b, const double* rows_d, int k, int horizon, double* out_d);
+
 /* Ensemble::UpdateContacts + CheckAndCorrectEnsembleState only (ensembles.cc:445-480, 241-329):
  * runs the narrowphase kernel on the current state without stepping; read the result with
  * egg_get_contacts / egg_get_pair_hits. */

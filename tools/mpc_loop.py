@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Cost of the receding-horizon MPC loop (mpc.mpc_iteration) over the plain rollout sweep.
 
-    python tools/mpc_loop.py [--worlds 131072] [--horizon 50] [--repeats 5] [--legs abcde] [--profile] [--out FILE]
+    python tools/mpc_loop.py [--worlds 131072] [--horizon 50] [--repeats 5] [--legs abcdef] [--profile] [--out FILE]
     python -m torch.distributed.run --nproc_per_node N tools/mpc_loop.py ...
 
 One process per GPU; every rank owns `--worlds` legged20 worlds (bench.py's c5mpc scene, seeded per
@@ -27,11 +27,19 @@ schedule.  egg_sample_controls and egg_mppi_reduce are also timed alone, and the
 (bytes computed from the shapes) are reported against the 6555.8 GB/s copy bandwidth of BASELINE.md.
 Then mppi_iteration runs with sigma > 0 on the torques and the representative cost, and its
 world-steps/s are reported.  --profile adds the device time of the MPPI kernels of one leg e.
+
+Leg f times only what CEM adds to a horizon (mpc.cem_iteration minus the rollout), at std = 0 so that
+the schedule is the constant one of leg c: egg_sample_controls_std, the cost allgather with the
+top-k selection, the elite schedules' gather (egg_gather_controls) and exchange, egg_control_moments
+and the refit of u_nom and std.  Each of those parts is also timed on its own.  Then
+egg_sample_controls_std and egg_sample_controls are timed alone, alternating in the same call, with
+their GB/s against the same copy bandwidth, and cem_iteration runs with sigma > 0 on the torques and
+the representative cost, and its world-steps/s are reported.
 --legs picks the legs to run (b needs a; the overheads need the legs they compare).
 Rank 0 prints one JSON line with the GPU name and power limit.
 
 Memory: a schedule is H x worlds x 20 x 6 doubles, 6.3 GB per GPU at 131072 worlds and H = 50; the
-script holds three (constant, random and MPPI samples), plus the batch and one saved start state (0.4 GB).
+script holds three (constant, random and MPPI or CEM samples), plus the batch and one saved start state (0.4 GB).
 """
 import argparse
 import json
@@ -56,9 +64,10 @@ def parse():
     ap.add_argument("--repeats", type=int, default=5, help="timed repeats of each leg")
     ap.add_argument("--random-iters", type=int, default=3, help="timed loop iterations with random schedules")
     ap.add_argument("--sigma", type=float, default=0.05, help="std. dev. of the random torques (N m)")
-    ap.add_argument("--legs", default="abcde", help="legs to run (default: all)")
+    ap.add_argument("--legs", default="abcdef", help="legs to run (default: all)")
     ap.add_argument("--lam", type=float, default=1.0, help="MPPI temperature lambda of leg e")
-    ap.add_argument("--profile", action="store_true", help="also record the kernel times of legs c, d and e with torch.profiler")
+    ap.add_argument("--elites", type=int, default=128, help="CEM elites of leg f (n_elite, over all GPUs)")
+    ap.add_argument("--profile", action="store_true", help="also record the kernel times of legs c, d, e and f with torch.profiler")
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     return ap.parse_args()
 
@@ -80,7 +89,7 @@ def spread(xs):
 
 def profile_legs(prepare, legs, sync):
     """Device milliseconds of the per-step control kernels of one leg c and one leg d, and of the
-    MPPI kernels of one leg e."""
+    MPPI kernels of one leg e and the CEM kernels of one leg f."""
     from torch.profiler import profile, ProfilerActivity
     out = {}
     for name, fn in legs.items():
@@ -91,7 +100,7 @@ def profile_legs(prepare, legs, sync):
             sync()
         for e in prof.key_averages():
             kernel = re.search(r"egg_\w+", e.key)
-            if kernel and any(key in kernel.group(0) for key in ("fext_slice", "egg_cost", "egg_mppi")):
+            if kernel and any(key in kernel.group(0) for key in ("fext_slice", "egg_cost", "egg_mppi", "egg_gather_controls", "egg_control_moments")):
                 out[f"{name}: {kernel.group(0)}"] = {"calls": e.count, "ms": e.device_time_total / 1e3}
     return out
 
@@ -124,16 +133,20 @@ def main():
     gen.manual_seed(1234 + rank)
     u_rand = u_const.clone()
     u_rand[..., 3:6] += args.sigma * torch.randn(u_rand[..., 3:6].shape, generator=gen, device=dev, dtype=torch.float64)
-    u_mppi = torch.empty_like(u_const) if "e" in args.legs else None
+    u_mppi = torch.empty_like(u_const) if ("e" in args.legs or "f" in args.legs) else None   # MPPI or CEM samples
     # MPPI planners around world 0's f_ext: sigma = 0 for the overhead of leg e, sigma on the torques for the loop
     sigma = np.zeros((n, 6))
     sigma[:, 3:6] = args.sigma
     mppi0 = mpc.MPPI(n, H, sigma=0.0, lam=args.lam, seed=11, u_nom=scene["f_ext"][0], device=dev)
     mppi1 = mpc.MPPI(n, H, sigma=sigma, lam=args.lam, seed=12, u_nom=scene["f_ext"][0], device=dev)
+    # CEM planners the same way: std = 0 for the overhead of leg f, sigma on the torques for the loop
+    cem0 = mpc.CEM(n, H, sigma=0.0, n_elite=args.elites, seed=13, u_nom=scene["f_ext"][0], device=dev)
+    cem1 = mpc.CEM(n, H, sigma=sigma, n_elite=args.elites, seed=14, u_nom=scene["f_ext"][0], device=dev)
     L = H * n * 6
     chunks = -(-W // 256)   # stage-1 chunks of egg_mppi_reduce
     sample_bytes = 8 * (H * W * n * 6 + L)                                  # write the samples, read u_nom
     reduce_bytes = 8 * (H * W * n * 6 + W + 2 * chunks * (L + 2) + L + 2)   # read u and J, partials out and in, result
+    sample_std_bytes = 8 * (H * W * n * 6 + 2 * L)                          # write the samples, read mean and std
     costs = torch.empty(W, dtype=torch.float64, device=dev)
     all_costs = torch.empty(n_total, dtype=torch.float64, device=dev)
     start = torch.empty((W, n * 18), dtype=torch.float64, device=dev)
@@ -207,13 +220,30 @@ def main():
             mpc.mppi_sample(b, mppi0, u_mppi, first)
             mpc.mppi_combine(b, mppi0, u_mppi, costs)
 
-        legs = {name: fn for name, fn in (("a", leg_a), ("c", leg_c), ("b", leg_b), ("d", leg_d), ("e", leg_e)) if name in args.legs}
+        def pack_controls(local):   # the elites' schedules of this rank, as cem_iteration fetches them
+            out = torch.empty((len(local), L), dtype=torch.float64, device=dev)
+            if len(local):
+                b.gather_controls(u_mppi.data_ptr(), H, local, out.data_ptr())
+            return out
+
+        moments = torch.empty((2, H, n, 6), dtype=torch.float64, device=dev)
+
+        def cem_moments(rows):
+            b.control_moments(rows.data_ptr(), rows.shape[0], H, moments.data_ptr())
+
+        def leg_f():
+            mpc.cem_sample(b, cem0, u_mppi, first)
+            cem_moments(mpc.cem_select(cem0, costs, n_total, pack_controls)[3])
+            mpc.cem_refit(cem0, moments)
+
+        legs = {name: fn for name, fn in (("a", leg_a), ("c", leg_c), ("b", leg_b), ("d", leg_d), ("e", leg_e), ("f", leg_f))
+                if name in args.legs}
 
         def prepare(name):   # the cost is set for leg d only (outside the timed region: set_cost synchronises)
             reset()
             b.set_cost(cost if name == "d" else None)
-            if name == "e":   # the costs of a rollout of the constant schedule, which leg e weighs
-                b.set_sampler(mppi0)
+            if name in "ef":   # the costs of a rollout of the constant schedule, which legs e and f weigh
+                b.set_sampler(mppi0 if name == "e" else cem0)
                 leg_c()
 
         for name, fn in legs.items():     # warm-up
@@ -227,7 +257,7 @@ def main():
         t = {name: np.array(x) for name, x in t.items()}
         entry = {}
         for name, key in (("a", "a_sweep_ms"), ("c", "c_controlled_sweep_ms"), ("b", "b_mpc_iteration_ms"),
-                          ("d", "d_controlled_cost_sweep_ms"), ("e", "e_mppi_additions_ms")):
+                          ("d", "d_controlled_cost_sweep_ms"), ("e", "e_mppi_additions_ms"), ("f", "f_cem_additions_ms")):
             if name in t:
                 entry[key] = spread(t[name])
         for key, hi, lo, base in (("slice_copy_overhead", "c", "a", "a"), ("loop_overhead", "b", "a", "a"),
@@ -235,8 +265,9 @@ def main():
             if hi in t and lo in t:
                 entry[key + "_ms"] = spread(t[hi] - t[lo])
                 entry[key + "_pct"] = spread(100.0 * (t[hi] - t[lo]) / t[base])
-        if "e" in t and "c" in t:
-            entry["e_mppi_additions_pct_of_c"] = spread(100.0 * t["e"] / t["c"])
+        for name in "ef":
+            if name in t and "c" in t:
+                entry[f"{name}_{'mppi' if name == 'e' else 'cem'}_additions_pct_of_c"] = spread(100.0 * t[name] / t["c"])
         if "e" in t:   # the two kernels alone, and their bandwidth
             prepare("e")
             ks, kr = [], []
@@ -251,8 +282,30 @@ def main():
                 "sample_controls": {"ms": spread(ks), "bytes": sample_bytes, "GBps": spread(sample_bytes / (ks * 1e-3) / 1e9)},
                 "mppi_reduce": {"ms": spread(kr), "bytes": reduce_bytes, "GBps": spread(reduce_bytes / (kr * 1e-3) / 1e9),
                                 "launches": 2, "chunks": chunks}}
+        if "f" in t:   # the parts of leg f one by one, then the two samplers alone, alternating
+            prepare("f")
+            parts = {"sample_std": [], "cost_allgather_topk": [], "elite_gather_exchange": [], "moments": [], "update": []}
+            got = {}
+            for _ in range(args.repeats):
+                parts["sample_std"].append(timed(lambda: mpc.cem_sample(b, cem0, u_mppi, first)))
+                parts["cost_allgather_topk"].append(timed(lambda: got.update(
+                    el=mpc.select_best(mpc.allgather_costs(costs), cem0.n_elite)[0])))
+                parts["elite_gather_exchange"].append(timed(lambda: got.update(rows=mpc.gather_winner_states(got["el"], n_total, pack_controls))))
+                parts["moments"].append(timed(lambda: cem_moments(got["rows"])))
+                parts["update"].append(timed(lambda: mpc.cem_refit(cem0, moments)))
+            entry["f_parts_ms"] = {key: spread(x) for key, x in parts.items()}
+            kstd, kbody = [], []
+            for _ in range(args.repeats):
+                kstd.append(timed(lambda: b.sample_controls_std(cem0.u_nom.data_ptr(), cem0.std.data_ptr(), H, cem0.seed, 0, first,
+                                                                u_mppi.data_ptr())))
+                kbody.append(timed(lambda: b.sample_controls(cem0.u_nom.data_ptr(), H, cem0.seed, 0, first, u_mppi.data_ptr())))
+            kstd, kbody = np.array(kstd), np.array(kbody)
+            entry["f_kernels"] = {
+                "copy_bandwidth_GBps": 6555.8, "elites": cem0.n_elite,
+                "sample_controls_std": {"ms": spread(kstd), "bytes": sample_std_bytes, "GBps": spread(sample_std_bytes / (kstd * 1e-3) / 1e9)},
+                "sample_controls": {"ms": spread(kbody), "bytes": sample_bytes, "GBps": spread(sample_bytes / (kbody * 1e-3) / 1e9)}}
         if args.profile:
-            entry["kernel_ms_per_horizon"] = profile_legs(prepare, {x: legs[x] for x in "cde" if x in legs}, sync)
+            entry["kernel_ms_per_horizon"] = profile_legs(prepare, {x: legs[x] for x in "cdef" if x in legs}, sync)
         # the loop itself with random time-varying schedules (the state evolves from iteration to iteration),
         # with the built-in cost and with the configured one
         loops = [(key, qc) for key, qc, leg in (("random_loop", None, "b"), ("random_loop_cost", cost, "d")) if leg in legs]
@@ -265,6 +318,15 @@ def main():
             entry["mppi_loop_cost"] = {"iterations": args.random_iters, "ms_per_iteration": ms / args.random_iters,
                                        "world_steps_per_s": n_total * H * args.random_iters / (ms * 1e-3),
                                        "sigma_torque": args.sigma, "lam": args.lam}
+        if "f" in legs:   # CEM with sigma > 0 and the representative cost
+            reset()
+            b.set_cost(cost)
+            b.set_sampler(cem1)
+            mpc.cem_iteration(b, cem1, dt, u_mppi, first, n_total)
+            ms = timed(lambda: [mpc.cem_iteration(b, cem1, dt, u_mppi, first, n_total) for _ in range(args.random_iters)])
+            entry["cem_loop_cost"] = {"iterations": args.random_iters, "ms_per_iteration": ms / args.random_iters,
+                                      "world_steps_per_s": n_total * H * args.random_iters / (ms * 1e-3),
+                                      "sigma_torque": args.sigma, "elites": cem1.n_elite}
         for key, qc in loops:
             reset()
             b.set_cost(qc)
