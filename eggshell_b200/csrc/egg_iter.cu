@@ -176,7 +176,7 @@ __global__ void __launch_bounds__(32) egg_iter_kernel(EggDev d, double dt, int s
     }
     if (lane == 0) {
       int* stt = d.stats + (size_t)w * 8;
-      stt[4] = it; stt[5] = 0; stt[6] = (cfm != 0.0); stt[7] = 0;
+      stt[4] = it; stt[5] = 0; stt[6] = (nc > 0 && cfm != 0.0); stt[7] = 0;   // no rows: ComputeVDot is never reached
       d.resid[w] = err;
     }
     // integrate: v' = v + dt (M^-1 f + a) etc. (ensembles.cc:535,572-591)

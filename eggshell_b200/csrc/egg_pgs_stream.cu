@@ -651,7 +651,7 @@ __global__ void __launch_bounds__(32, MINB) egg_pgs_stream_kernel(EggDev d, doub
         int* stt = d.stats + (size_t)w * 8;
         stt[4] = it;
         stt[5] = 0;
-        stt[6] = (cfm != 0.0);
+        stt[6] = (nc > 0 && cfm != 0.0);       // no rows: ComputeVDot is never reached (ensembles.cc:498-538)
         stt[7] = d.n_levels[w];
         d.resid[w] = err;
       }

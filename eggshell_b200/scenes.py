@@ -2,7 +2,7 @@
 
 Every scene is a dict of world-major numpy arrays ready for ``Batch.set_bodies/set_joints``:
 p,v,w [W,n,3]; R,I [W,n,3,3]; m [W,n]; optional joints i0,i1 [nj], c0,c1 [W,nj,3]; f_ext [W,n,6];
-plus ``dt`` and ``solver``.  All bodies are cubes of side 0.3, the only collider the reference has
+optional box side lengths side [W,n,3] (default 0.3 on every axis); plus ``dt`` and ``solver``.  All bodies are cubes of side 0.3, the only collider the reference has
 (/root/reference/eggshell/body.h:90-91).  Randomness is a seeded numpy PCG64 stream per
 (config, base seed), so the same arrays feed the GPU batch and the CPU oracle.
 """
@@ -234,7 +234,7 @@ def make_batch(scene, **kw):
     """Creates, fills and initialises a ``Batch`` from a scene dict."""
     from .batch import Batch
     b = Batch(scene["W"], scene["n"], scene["nj"], **kw)
-    b.set_bodies(scene["p"], scene["R"], scene["v"], scene["w"], scene["m"], scene["I"])
+    b.set_bodies(scene["p"], scene["R"], scene["v"], scene["w"], scene["m"], scene["I"], side=scene.get("side"))
     if "shape" in scene:
         b.set_shapes(scene["shape"], scene["dims"])
     if scene["nj"]:

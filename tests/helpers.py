@@ -7,7 +7,8 @@ from oracle import pyoracle as O
 
 def oracle_world(scene, w, **params):
     W = O.World()
-    W.set_bodies(scene["p"][w], scene["R"][w], scene["v"][w], scene["w"][w], scene["m"][w], scene["I"][w])
+    W.set_bodies(scene["p"][w], scene["R"][w], scene["v"][w], scene["w"][w], scene["m"][w], scene["I"][w],
+                 None if "side" not in scene else scene["side"][w])
     if "shape" in scene:
         W.set_shapes(scene["shape"][w], scene["dims"][w])
     if scene["nj"]:
