@@ -108,6 +108,15 @@ def _p(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
+def _world_list(worlds, what):
+    """A list of world indices as the contiguous int32 array the C ABI takes."""
+    w64 = np.asarray(worlds, dtype=np.int64).ravel()
+    idx = np.ascontiguousarray(w64, dtype=np.int32)
+    if not np.array_equal(idx, w64):
+        raise EggError(f"{what}: world index out of the int32 range")
+    return idx
+
+
 def pinned_empty(shape, dtype=np.float64):
     """numpy array backed by page-locked host memory (cudaHostAlloc)."""
     n = int(np.prod(shape)) * np.dtype(dtype).itemsize
@@ -281,10 +290,7 @@ class Batch:
         """Copies the schedules of the listed local worlds out of the device buffer at u_ptr, float64
         [horizon][W][n][6], to the device buffer at out_ptr, [len(worlds)][horizon][n][6]
         (egg_gather_controls)."""
-        w64 = np.asarray(worlds, dtype=np.int64).ravel()
-        idx = np.ascontiguousarray(w64, dtype=np.int32)
-        if not np.array_equal(idx, w64):
-            raise EggError("gather_controls: world index out of the int32 range")
+        idx = _world_list(worlds, "gather_controls")
         _chk(lib().egg_gather_controls(self.h, C.c_void_p(u_ptr), int(horizon), _p(idx), int(idx.size), C.c_void_p(out_ptr)),
              "egg_gather_controls")
 
@@ -298,10 +304,7 @@ class Batch:
     def gather_state(self, worlds, out_ptr):
         """Writes the state of the listed worlds to the device buffer at out_ptr, float64
         [len(worlds)][n][18] = (p, R row-major, v, w) per body (egg_gather_state)."""
-        w64 = np.asarray(worlds, dtype=np.int64).ravel()
-        idx = np.ascontiguousarray(w64, dtype=np.int32)
-        if not np.array_equal(idx, w64):
-            raise EggError("gather_state: world index out of the int32 range")
+        idx = _world_list(worlds, "gather_state")
         _chk(lib().egg_gather_state(self.h, _p(idx), int(idx.size), C.c_void_p(out_ptr)), "egg_gather_state")
 
     def seed_state(self, in_ptr, k, first=0):

@@ -13,6 +13,7 @@
 #include <climits>
 #include <cstdint>
 #include <limits>
+#include <initializer_list>
 
 cudaError_t egg_launch_solve_dense(const EggDev& d, double dt, cudaStream_t s, void* scratch, size_t scratch_bytes);
 size_t egg_dense_scratch_bytes(const EggDev& d);
@@ -73,9 +74,10 @@ struct egg_batch {
   double* snap = nullptr;        // egg_snapshot copy of dev.dyn
   int* gather_idx = nullptr;     // [W] world indices of egg_gather_state, allocated by its first call
   double* cost_buf = nullptr;    // egg_set_cost arrays (EggCost layout); null = no cost set
-  size_t cost_bytes = 0;
+  size_t cost_count = 0;
   EggCost cost = {};             // pointers into cost_buf
   double* sampler_buf = nullptr; // egg_set_sampler arrays (EggSampler layout); null = no sampler set
+  size_t sampler_count = 0;
   EggSampler sampler = {};       // pointers into sampler_buf
   double* mppi_partial = nullptr;  // stage-1 partials of egg_mppi_reduce, grown on demand
   size_t mppi_partial_count = 0;
@@ -83,16 +85,6 @@ struct egg_batch {
   std::vector<cudaEvent_t> ev;   // 4 per profiled step
   std::vector<cudaEvent_t> ev_free;
 };
-
-// LK(wrapper call): a launch wrapper's cudaError_t -> EGG_ERR_CUDA with the wrapper named
-#define LK(call)                                \
-  do {                                          \
-    cudaError_t e__ = (call);                   \
-    if (e__ != cudaSuccess) {                   \
-      set_err(#call, e__);                      \
-      return EGG_ERR_CUDA;                      \
-    }                                           \
-  } while (0)
 
 template <class T>
 static int dalloc(egg_batch* b, T** p, size_t count) {
@@ -114,6 +106,22 @@ static int dfree(egg_batch* b, void* p, size_t bytes) {
   CK(cudaFree(p));
   b->allocs.erase(std::find(b->allocs.begin(), b->allocs.end(), p));
   b->bytes -= (long long)bytes;
+  return EGG_OK;
+}
+#define RET(x) do { int r__ = (x); if (r__ != EGG_OK) return r__; } while (0)
+// Replaces the batch-owned buffer buf of count doubles with a new one of new_count doubles (none if 0),
+// filled from host if given.  The new buffer is in place before the old one goes, so a failed
+// allocation keeps the old buffer; the stream is synchronised before the old one is freed.
+static int replace_dbuf(egg_batch* b, double*& buf, size_t& count, size_t new_count, const double* host) {
+  double* q = nullptr;
+  if (new_count) {
+    RET(dalloc(b, &q, new_count));
+    if (host) CK(cudaMemcpyAsync(q, host, new_count * sizeof(double), cudaMemcpyHostToDevice, b->stream));
+  }
+  CK(cudaStreamSynchronize(b->stream));   // host may be a temporary
+  if (buf) RET(dfree(b, buf, count * sizeof(double)));
+  buf = q;
+  count = new_count;
   return EGG_OK;
 }
 #define DA(ptr, count)                                  \
@@ -388,21 +396,20 @@ static int upload(egg_batch* b, const double* host, int per_world, int comps, do
   size_t bytes = (size_t)b->dev.W * per_world * comps * sizeof(double);
   if (bytes == 0) return EGG_OK;
   CK(cudaMemcpyAsync(b->stage, host, bytes, cudaMemcpyHostToDevice, b->stream));
-  LK(egg_launch_pack(b->dev.W, b->stage, per_world, comps, soa, soa_comps, comp_off, b->stream));
+  CK(egg_launch_pack(b->dev.W, b->stage, per_world, comps, soa, soa_comps, comp_off, b->stream));
   b->launches++;
   return EGG_OK;
 }
 static int download(egg_batch* b, double* host, int per_world, int comps, const double* soa, int soa_comps, int comp_off) {
   size_t bytes = (size_t)b->dev.W * per_world * comps * sizeof(double);
   if (bytes == 0) return EGG_OK;
-  LK(egg_launch_unpack(b->dev.W, b->stage, per_world, comps, soa, soa_comps, comp_off, b->stream));
+  CK(egg_launch_unpack(b->dev.W, b->stage, per_world, comps, soa, soa_comps, comp_off, b->stream));
   b->launches++;
   CK(cudaMemcpyAsync(host, b->stage, bytes, cudaMemcpyDeviceToHost, b->stream));
   // the staging buffer is reused by the next call
   CK(cudaStreamSynchronize(b->stream));
   return EGG_OK;
 }
-#define RET(x) do { int r__ = (x); if (r__ != EGG_OK) return r__; } while (0)
 
 int egg_set_state(egg_batch* b, const double* p, const double* R, const double* v, const double* w) {
   if (!b) return EGG_ERR_ARG;
@@ -475,13 +482,13 @@ int egg_set_external(egg_batch* b, const double* f_ext) {
 int egg_init(egg_batch* b) {
   if (!b) return EGG_ERR_ARG;
   CK(cudaSetDevice(b->device));
-  LK(egg_launch_init(b->dev, b->stream));
+  CK(egg_launch_init(b->dev, b->stream));
   b->launches += (b->dev.nj > 0) ? 3 : 2;
   // Ensemble::Init ends with CheckAndCorrectEnsembleState (ensembles.cc:28): the joint-joint
   // conflict scan lives in the narrowphase kernel, so run it once here -- EGG_ST_JOINT_CONFLICT is
   // then visible right after egg_init, as the reference's Panic would be.
-  LK(egg_launch_collide(b->dev, b->stream));
-  LK(egg_launch_clear_contacts(b->dev, b->stream));   // the contact list stays empty until the first Step / UpdateContacts, as in the reference
+  CK(egg_launch_collide(b->dev, b->stream));
+  CK(egg_launch_clear_contacts(b->dev, b->stream));   // the contact list stays empty until the first Step / UpdateContacts, as in the reference
   b->launches += 2;
   b->initialised = true;
   b->iso_known = false;
@@ -532,17 +539,17 @@ int egg_init_stabilize(egg_batch* b, int max_steps, int* steps_out, double* err_
   nodedup.level_start = nullptr;
   const double dt = 0.001 * 500;   // kSimTimeStep * 500 (ensembles.cc:611)
   for (int it = 0; it <= max_steps; it++) {
-    LK(egg_launch_collide(nodedup, b->stream));
-    LK(egg_launch_assemble(nodedup, dt, b->stream));
+    CK(egg_launch_collide(nodedup, b->stream));
+    CK(egg_launch_assemble(nodedup, dt, b->stream));
     CK(cudaMemsetAsync(b->relax_any, 0, sizeof(int), b->stream));
-    LK(egg_launch_relax(nodedup, dt, 0.2, max_steps, 0, b->dense_scratch, b->dense_scratch_bytes, b->relax_prog, b->relax_err2, b->relax_any, b->stream));
+    CK(egg_launch_relax(nodedup, dt, 0.2, max_steps, 0, b->dense_scratch, b->dense_scratch_bytes, b->relax_prog, b->relax_err2, b->relax_any, b->stream));
     b->launches += 3;
     int h_any = 0;
     CK(cudaMemcpyAsync(&h_any, b->relax_any, sizeof(int), cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
     if (!h_any) break;
   }
-  LK(egg_launch_collide(b->dev, b->stream));   // CheckAndCorrectEnsembleState (ensembles.cc:618)
+  CK(egg_launch_collide(b->dev, b->stream));   // CheckAndCorrectEnsembleState (ensembles.cc:618)
   b->launches++;
   return relax_report(b, steps_out, err_sq_out);
 }
@@ -559,9 +566,9 @@ int egg_post_stabilize(egg_batch* b, int max_steps, int* steps_out, double* err_
   // ensembles.cc:624-645: the contact list is NOT refreshed inside this loop; the rows are rebuilt
   // from the current body state and the stored contact geometry every iteration
   for (int it = 0; it <= max_steps; it++) {
-    LK(egg_launch_assemble(pw, dt, b->stream));
+    CK(egg_launch_assemble(pw, dt, b->stream));
     CK(cudaMemsetAsync(b->relax_any, 0, sizeof(int), b->stream));
-    LK(egg_launch_relax(pw, dt, 0.2, max_steps, 1, b->dense_scratch, b->dense_scratch_bytes, b->relax_prog, b->relax_err2, b->relax_any, b->stream));
+    CK(egg_launch_relax(pw, dt, 0.2, max_steps, 1, b->dense_scratch, b->dense_scratch_bytes, b->relax_prog, b->relax_err2, b->relax_any, b->stream));
     b->launches += 2;
     int h_any = 0;
     CK(cudaMemcpyAsync(&h_any, b->relax_any, sizeof(int), cudaMemcpyDeviceToHost, b->stream));
@@ -571,10 +578,19 @@ int egg_post_stabilize(egg_batch* b, int max_steps, int* steps_out, double* err_
   return relax_report(b, steps_out, err_sq_out);
 }
 
+static int arg_err(const char* what, const char* name, const char* msg) {
+  g_err = std::string(what) + "(" + name + "): " + msg;
+  return EGG_ERR_ARG;
+}
+static int check_initialised(egg_batch* b, const char* what) {
+  if (!b->initialised) { g_err = std::string(what) + " before egg_init"; return EGG_ERR_STATE; }
+  return EGG_OK;
+}
+
 // The argument and call-order checks of egg_step and egg_step_controlled.
 static int step_check(egg_batch* b, double dt, int integrator, int n_steps, const char* what) {
   if (!b || n_steps < 0 || !(dt > 0)) return EGG_ERR_ARG;
-  if (!b->initialised) { g_err = std::string(what) + " before egg_init"; return EGG_ERR_STATE; }
+  RET(check_initialised(b, what));
   if (integrator != EGG_OPEN_DYNAMICS_ENGINE) {
     // ensembles.cc:398-405: EXPLICIT_EULER refuses contacts, IMPLICIT_MIDPOINT panics.
     g_err = "only OPEN_DYNAMICS_ENGINE is supported (as in the reference once contacts exist)";
@@ -583,17 +599,30 @@ static int step_check(egg_batch* b, double dt, int integrator, int n_steps, cons
   return EGG_OK;
 }
 
-// A _d argument must be device (or managed) memory of the batch's device: a host pointer would
-// reach a kernel as an illegal address.  The length behind the pointer cannot be checked here.
-static int check_device_ptr(egg_batch* b, const void* p, const char* what) {
-  if (!p) { g_err = std::string(what) + ": NULL device pointer"; return EGG_ERR_ARG; }
-  cudaPointerAttributes a;
-  cudaError_t e = cudaPointerGetAttributes(&a, p);
-  if (e != cudaSuccess) { cudaGetLastError(); g_err = std::string(what) + ": not a CUDA pointer"; return EGG_ERR_ARG; }
-  if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != b->device) {
-    g_err = std::string(what) + ": the buffer is not device memory of the batch's device";
-    return EGG_ERR_ARG;
+// Where enter() checks that egg_init has run: before or after the device pointers (each entry point
+// keeps the order in which it has always checked them), or not at all.
+enum InitCheck { INIT_FIRST, INIT_LAST, INIT_NONE };
+struct DevArg { const void* p; const char* name; };
+
+// The prologue of the entry points that take device buffers (what: the entry point's name).  A _d
+// argument must be device (or managed) memory of the batch's device: a host pointer would reach a
+// kernel as an illegal address.  The length behind the pointer cannot be checked here.  align16: the
+// double2 accesses of the sampler need 16-byte aligned schedules.
+static int enter(egg_batch* b, const char* what, InitCheck init, std::initializer_list<DevArg> ptrs, bool align16 = false) {
+  if (!b) return EGG_ERR_ARG;
+  if (init == INIT_FIRST) RET(check_initialised(b, what));
+  for (const DevArg& a : ptrs) {
+    if (!a.p) return arg_err(what, a.name, "NULL device pointer");
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, a.p) != cudaSuccess) { cudaGetLastError(); return arg_err(what, a.name, "not a CUDA pointer"); }
+    if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != b->device)
+      return arg_err(what, a.name, "the buffer is not device memory of the batch's device");
   }
+  if (align16)
+    for (const DevArg& a : ptrs)
+      if ((uintptr_t)a.p & 15) return arg_err(what, a.name, "must be 16-byte aligned");
+  if (init == INIT_LAST) RET(check_initialised(b, what));
+  CK(cudaSetDevice(b->device));
   return EGG_OK;
 }
 
@@ -617,8 +646,8 @@ static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d, do
   const size_t slice = (size_t)b->dev.W * b->dev.n * 6;
   for (int s = 0; s < n_steps; s++) {
     if (u_d) {
-      if (cost_d) LK(egg_launch_fext_slice_cost(b->dev, u_d + (size_t)s * slice, b->cost, s, cost_d, b->stream));
-      else LK(egg_launch_fext_slice(b->dev, u_d + (size_t)s * slice, b->stream));
+      if (cost_d) CK(egg_launch_fext_slice_cost(b->dev, u_d + (size_t)s * slice, b->cost, s, cost_d, b->stream));
+      else CK(egg_launch_fext_slice(b->dev, u_d + (size_t)s * slice, b->stream));
       b->launches++;
     }
     cudaEvent_t e[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -637,22 +666,22 @@ static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d, do
     cudaError_t e__ = cudaStreamSynchronize(b->stream);                                      \
     if (e__ != cudaSuccess) { set_err(what, e__); return EGG_ERR_CUDA; }                      \
   }
-    LK(egg_launch_collide(b->dev, b->stream));
+    CK(egg_launch_collide(b->dev, b->stream));
     DBG_SYNC("egg_collide_kernel")
     if (b->profiling) CK(cudaEventRecord(e[1], b->stream));
-    LK(egg_launch_assemble(b->dev, dt, b->stream));
+    CK(egg_launch_assemble(b->dev, dt, b->stream));
     DBG_SYNC("assembly kernels")
     if (b->profiling) CK(cudaEventRecord(e[2], b->stream));
-    if (solver == EGG_SOLVER_PGS) LK(egg_launch_solve_pgs(b->dev, dt, b->stream));
-    else if (solver == EGG_SOLVER_DENSE_MURTY) LK(egg_launch_solve_dense(b->dev, dt, b->stream, b->dense_scratch, b->dense_scratch_bytes));
-    else LK(egg_launch_solve_iter(b->dev, dt, solver, b->stream));
+    if (solver == EGG_SOLVER_PGS) CK(egg_launch_solve_pgs(b->dev, dt, b->stream));
+    else if (solver == EGG_SOLVER_DENSE_MURTY) CK(egg_launch_solve_dense(b->dev, dt, b->stream, b->dense_scratch, b->dense_scratch_bytes));
+    else CK(egg_launch_solve_iter(b->dev, dt, solver, b->stream));
     DBG_SYNC("solve kernel")
 #undef DBG_SYNC
     if (b->profiling) CK(cudaEventRecord(e[3], b->stream));
     b->launches += (solver == EGG_SOLVER_PGS && b->dev.rec_fmt) ? 5 : 3;   // collide, assemble (1 or 3 kernels), solve
   }
   if (cost_d) {
-    LK(egg_launch_cost_terminal(b->dev, b->cost, n_steps, cost_d, b->stream));
+    CK(egg_launch_cost_terminal(b->dev, b->cost, n_steps, cost_d, b->stream));
     b->launches++;
   }
   CK(cudaGetLastError());
@@ -668,7 +697,7 @@ int egg_step_controlled(egg_batch* b, double dt, int integrator, const double* u
   if (!b || !u_d) return EGG_ERR_ARG;
   if (horizon < 1) { g_err = "egg_step_controlled: horizon must be >= 1"; return EGG_ERR_ARG; }
   RET(step_check(b, dt, integrator, horizon, "egg_step_controlled"));
-  RET(check_device_ptr(b, u_d, "egg_step_controlled(u_d)"));
+  RET(enter(b, "egg_step_controlled", INIT_NONE, {{u_d, "u_d"}}));
   return step_loop(b, dt, horizon, u_d, nullptr);
 }
 
@@ -676,8 +705,7 @@ int egg_step_controlled_cost(egg_batch* b, double dt, int integrator, const doub
   if (!b || !u_d) return EGG_ERR_ARG;
   if (horizon < 1) { g_err = "egg_step_controlled_cost: horizon must be >= 1"; return EGG_ERR_ARG; }
   RET(step_check(b, dt, integrator, horizon, "egg_step_controlled_cost"));
-  RET(check_device_ptr(b, u_d, "egg_step_controlled_cost(u_d)"));
-  RET(check_device_ptr(b, cost_d, "egg_step_controlled_cost(cost_d)"));
+  RET(enter(b, "egg_step_controlled_cost", INIT_NONE, {{u_d, "u_d"}, {cost_d, "cost_d"}}));
   if (!b->cost_buf) { g_err = "egg_step_controlled_cost without a cost: call egg_set_cost first"; return EGG_ERR_STATE; }
   if (b->cost.ref_steps > 1 && b->cost.ref_steps < horizon + 1) {
     g_err = "egg_step_controlled_cost: the cost's reference has " + std::to_string(b->cost.ref_steps) + " rows, fewer than horizon + 1 = " +
@@ -685,6 +713,19 @@ int egg_step_controlled_cost(egg_batch* b, double dt, int integrator, const doub
     return EGG_ERR_ARG;
   }
   return step_loop(b, dt, horizon, u_d, cost_d);
+}
+
+// Host [rows][n][comps] -> component-major [rows][comps][n], the layout of EggCost and EggSampler.
+// With finite_only, returns false at the first value that is not finite.
+static bool to_component_major(const double* src, size_t rows, size_t n, size_t comps, double* dst, bool finite_only = true) {
+  for (size_t r = 0; r < rows; r++)
+    for (size_t i = 0; i < n; i++)
+      for (size_t k = 0; k < comps; k++) {
+        const double v = src[(r * n + i) * comps + k];
+        if (finite_only && !std::isfinite(v)) return false;
+        dst[(r * comps + k) * n + i] = v;
+      }
+  return true;
 }
 
 int egg_set_cost(egg_batch* b, const egg_cost* c) {
@@ -699,31 +740,16 @@ int egg_set_cost(egg_batch* b, const egg_cost* c) {
     struct { const double* src; size_t rows, comps, off; } part[6] = {
         {c->q_run, 1, EGG_DYN, 0}, {c->l_run, 1, EGG_DYN, nd}, {c->q_term, 1, EGG_DYN, 2 * nd},
         {c->l_term, 1, EGG_DYN, 3 * nd}, {c->u_run, 1, 6, 4 * nd}, {c->x_ref, (size_t)R, EGG_DYN, 4 * nd + 6 * n}};
-    for (auto& p : part) {
-      if (!p.src) continue;
-      for (size_t r = 0; r < p.rows; r++)
-        for (size_t i = 0; i < n; i++)
-          for (size_t k = 0; k < p.comps; k++) {
-            const double v = p.src[(r * n + i) * p.comps + k];   // host [rows][n][comps] -> [rows][comps][n]
-            if (!std::isfinite(v)) { g_err = "egg_set_cost: non-finite weight or reference value"; return EGG_ERR_ARG; }
-            h[p.off + (r * p.comps + k) * n + i] = v;
-          }
-    }
+    for (auto& p : part)
+      if (p.src && !to_component_major(p.src, p.rows, n, p.comps, &h[p.off])) {
+        g_err = "egg_set_cost: non-finite weight or reference value";
+        return EGG_ERR_ARG;
+      }
   }
   CK(cudaSetDevice(b->device));
-  if (b->cost_buf) {
-    RET(dfree(b, b->cost_buf, b->cost_bytes));
-    b->cost_buf = nullptr;
-    b->cost_bytes = 0;
-    b->cost = EggCost{};
-  }
-  if (!c) return EGG_OK;
-  RET(dalloc(b, &b->cost_buf, h.size()));
-  b->cost_bytes = h.size() * sizeof(double);
-  CK(cudaMemcpyAsync(b->cost_buf, h.data(), b->cost_bytes, cudaMemcpyHostToDevice, b->stream));
-  CK(cudaStreamSynchronize(b->stream));   // h is a temporary
+  RET(replace_dbuf(b, b->cost_buf, b->cost_count, h.size(), h.data()));
   const double* q = b->cost_buf;
-  b->cost = EggCost{q, q + nd, q + 4 * nd, q + 2 * nd, q + 3 * nd, q + 4 * nd + 6 * n, R};
+  b->cost = c ? EggCost{q, q + nd, q + 4 * nd, q + 2 * nd, q + 3 * nd, q + 4 * nd + 6 * n, R} : EggCost{};
   return EGG_OK;
 }
 
@@ -733,88 +759,74 @@ int egg_set_sampler(egg_batch* b, const egg_sampler* s) {
   std::vector<double> h;   // the EggSampler layout: sigma, lo, hi, each [6][n]
   if (s) {
     if (!s->sigma) { g_err = "egg_set_sampler: sigma is required"; return EGG_ERR_ARG; }
-    h.assign(3 * nc, 0.0);
     const double inf = std::numeric_limits<double>::infinity();
-    for (size_t i = 0; i < n; i++)
-      for (size_t j = 0; j < 6; j++) {
-        const double sg = s->sigma[i * 6 + j];
-        const double lo = s->u_lo ? s->u_lo[i * 6 + j] : -inf, hi = s->u_hi ? s->u_hi[i * 6 + j] : inf;
-        if (!std::isfinite(sg) || sg < 0) { g_err = "egg_set_sampler: sigma must be finite and >= 0"; return EGG_ERR_ARG; }
-        if (std::isnan(lo) || std::isnan(hi)) { g_err = "egg_set_sampler: NaN bound"; return EGG_ERR_ARG; }
-        if (lo > hi) { g_err = "egg_set_sampler: u_lo > u_hi"; return EGG_ERR_ARG; }
-        h[j * n + i] = sg;   // host [n][6] -> [6][n]
-        h[nc + j * n + i] = lo;
-        h[2 * nc + j * n + i] = hi;
-      }
+    h.assign(3 * nc, inf);   // without bounds: lo = -inf, hi = +inf
+    std::fill(h.begin() + nc, h.begin() + 2 * nc, -inf);
+    const bool finite = to_component_major(s->sigma, 1, n, 6, &h[0]);
+    if (s->u_lo) to_component_major(s->u_lo, 1, n, 6, &h[nc], false);
+    if (s->u_hi) to_component_major(s->u_hi, 1, n, 6, &h[2 * nc], false);
+    for (size_t k = 0; k < nc; k++) {
+      const double lo = h[nc + k], hi = h[2 * nc + k];
+      if (!finite || h[k] < 0) { g_err = "egg_set_sampler: sigma must be finite and >= 0"; return EGG_ERR_ARG; }
+      if (std::isnan(lo) || std::isnan(hi)) { g_err = "egg_set_sampler: NaN bound"; return EGG_ERR_ARG; }
+      if (lo > hi) { g_err = "egg_set_sampler: u_lo > u_hi"; return EGG_ERR_ARG; }
+    }
   }
   CK(cudaSetDevice(b->device));
-  double* buf = nullptr;   // the new sampler is in device memory before the old one goes
-  if (s) {
-    RET(dalloc(b, &buf, h.size()));
-    CK(cudaMemcpyAsync(buf, h.data(), h.size() * sizeof(double), cudaMemcpyHostToDevice, b->stream));
-  }
-  CK(cudaStreamSynchronize(b->stream));   // h is a temporary; queued samplers are done with the old buffer
-  if (b->sampler_buf) RET(dfree(b, b->sampler_buf, 3 * nc * sizeof(double)));
-  b->sampler_buf = buf;
-  b->sampler = s ? EggSampler{buf, buf + nc, buf + 2 * nc} : EggSampler{};
+  RET(replace_dbuf(b, b->sampler_buf, b->sampler_count, h.size(), h.data()));
+  const double* q = b->sampler_buf;
+  b->sampler = s ? EggSampler{q, q + nc, q + 2 * nc} : EggSampler{};
   return EGG_OK;
 }
 
-// The double2 accesses of the sampler need 16-byte aligned schedules.
-static int check_aligned16(const void* p, const char* what) {
-  if ((uintptr_t)p & 15) { g_err = std::string(what) + ": must be 16-byte aligned"; return EGG_ERR_ARG; }
+// egg_sample_controls (std_d null: the sampler's sigma per body) and egg_sample_controls_std; ptrs
+// names the entry point's device arguments.
+static int sample_controls(egg_batch* b, const char* what, std::initializer_list<DevArg> ptrs, const double* mean_d, const double* std_d,
+                           int horizon, unsigned long long seed, unsigned long long iteration, int first, double* u_d) {
+  if (!b) return EGG_ERR_ARG;
+  if (horizon < 1 || first < 0) { g_err = std::string(what) + ": horizon must be >= 1 and first >= 0"; return EGG_ERR_ARG; }
+  RET(enter(b, what, INIT_LAST, ptrs, true));
+  if (!b->sampler_buf) { g_err = std::string(what) + " without a sampler: call egg_set_sampler first"; return EGG_ERR_STATE; }
+  CK(egg_launch_sample(b->dev, b->sampler, mean_d, std_d, horizon, seed, iteration, first, u_d, b->stream));
+  b->launches++;
   return EGG_OK;
 }
 
 int egg_sample_controls(egg_batch* b, const double* u_nom_d, int horizon, unsigned long long seed,
                         unsigned long long iteration, int first, double* u_d) {
-  if (!b) return EGG_ERR_ARG;
-  if (horizon < 1 || first < 0) { g_err = "egg_sample_controls: horizon must be >= 1 and first >= 0"; return EGG_ERR_ARG; }
-  RET(check_device_ptr(b, u_nom_d, "egg_sample_controls(u_nom_d)"));
-  RET(check_device_ptr(b, u_d, "egg_sample_controls(u_d)"));
-  RET(check_aligned16(u_nom_d, "egg_sample_controls(u_nom_d)"));
-  RET(check_aligned16(u_d, "egg_sample_controls(u_d)"));
-  if (!b->initialised) { g_err = "egg_sample_controls before egg_init"; return EGG_ERR_STATE; }
-  if (!b->sampler_buf) { g_err = "egg_sample_controls without a sampler: call egg_set_sampler first"; return EGG_ERR_STATE; }
-  CK(cudaSetDevice(b->device));
-  LK(egg_launch_mppi_sample(b->dev, b->sampler, u_nom_d, horizon, seed, iteration, first, u_d, b->stream));
-  b->launches++;
-  return EGG_OK;
+  return sample_controls(b, "egg_sample_controls", {{u_nom_d, "u_nom_d"}, {u_d, "u_d"}}, u_nom_d, nullptr, horizon, seed, iteration,
+                         first, u_d);
 }
 
 int egg_sample_controls_std(egg_batch* b, const double* mean_d, const double* std_d, int horizon, unsigned long long seed,
                             unsigned long long iteration, int first, double* u_d) {
-  if (!b) return EGG_ERR_ARG;
-  if (horizon < 1 || first < 0) { g_err = "egg_sample_controls_std: horizon must be >= 1 and first >= 0"; return EGG_ERR_ARG; }
-  RET(check_device_ptr(b, mean_d, "egg_sample_controls_std(mean_d)"));
-  RET(check_device_ptr(b, std_d, "egg_sample_controls_std(std_d)"));
-  RET(check_device_ptr(b, u_d, "egg_sample_controls_std(u_d)"));
-  RET(check_aligned16(mean_d, "egg_sample_controls_std(mean_d)"));
-  RET(check_aligned16(std_d, "egg_sample_controls_std(std_d)"));
-  RET(check_aligned16(u_d, "egg_sample_controls_std(u_d)"));
-  if (!b->initialised) { g_err = "egg_sample_controls_std before egg_init"; return EGG_ERR_STATE; }
-  if (!b->sampler_buf) { g_err = "egg_sample_controls_std without a sampler: call egg_set_sampler first"; return EGG_ERR_STATE; }
-  CK(cudaSetDevice(b->device));
-  LK(egg_launch_sample_std(b->dev, b->sampler, mean_d, std_d, horizon, seed, iteration, first, u_d, b->stream));
-  b->launches++;
+  return sample_controls(b, "egg_sample_controls_std", {{mean_d, "mean_d"}, {std_d, "std_d"}, {u_d, "u_d"}}, mean_d, std_d, horizon,
+                         seed, iteration, first, u_d);
+}
+
+// The world list of egg_gather_state and egg_gather_controls: k in [1, W] indices in [0, W).
+static int check_worlds(egg_batch* b, const char* what, const int* worlds, int k) {
+  const int W = b->dev.W;
+  if (k < 1 || k > W) { g_err = std::string(what) + ": k must be in [1, n_worlds]"; return EGG_ERR_ARG; }
+  for (int i = 0; i < k; i++)
+    if (worlds[i] < 0 || worlds[i] >= W) { g_err = std::string(what) + ": world index out of range"; return EGG_ERR_ARG; }
+  return EGG_OK;
+}
+// ... and its copy to the device, into gather_idx (allocated by the first call).
+static int upload_worlds(egg_batch* b, const int* worlds, int k) {
+  if (!b->gather_idx) RET(dalloc(b, &b->gather_idx, (size_t)b->dev.W));
+  CK(cudaMemcpyAsync(b->gather_idx, worlds, (size_t)k * sizeof(int), cudaMemcpyHostToDevice, b->stream));
   return EGG_OK;
 }
 
 int egg_gather_controls(egg_batch* b, const double* u_d, int horizon, const int* worlds, int k, double* out_d) {
   if (!b || !worlds) return EGG_ERR_ARG;
-  const int W = b->dev.W;
   if (horizon < 1) { g_err = "egg_gather_controls: horizon must be >= 1"; return EGG_ERR_ARG; }
-  if (k < 1 || k > W) { g_err = "egg_gather_controls: k must be in [1, n_worlds]"; return EGG_ERR_ARG; }
-  for (int i = 0; i < k; i++)
-    if (worlds[i] < 0 || worlds[i] >= W) { g_err = "egg_gather_controls: world index out of range"; return EGG_ERR_ARG; }
+  RET(check_worlds(b, "egg_gather_controls", worlds, k));
   if ((long long)k * horizon * b->dev.n * 6 > 256ll * INT_MAX) { g_err = "egg_gather_controls: too many rows"; return EGG_ERR_ARG; }
-  RET(check_device_ptr(b, u_d, "egg_gather_controls(u_d)"));
-  RET(check_device_ptr(b, out_d, "egg_gather_controls(out_d)"));
-  if (!b->initialised) { g_err = "egg_gather_controls before egg_init"; return EGG_ERR_STATE; }
-  CK(cudaSetDevice(b->device));
-  if (!b->gather_idx) RET(dalloc(b, &b->gather_idx, (size_t)W));
-  CK(cudaMemcpyAsync(b->gather_idx, worlds, (size_t)k * sizeof(int), cudaMemcpyHostToDevice, b->stream));
-  LK(egg_launch_gather_controls(b->dev, u_d, horizon, b->gather_idx, k, out_d, b->stream));
+  RET(enter(b, "egg_gather_controls", INIT_LAST, {{u_d, "u_d"}, {out_d, "out_d"}}));
+  RET(upload_worlds(b, worlds, k));
+  CK(egg_launch_gather_controls(b->dev, u_d, horizon, b->gather_idx, k, out_d, b->stream));
   b->launches++;
   return EGG_OK;
 }
@@ -824,11 +836,8 @@ int egg_control_moments(egg_batch* b, const double* rows_d, int k, int horizon, 
   if (k < 1 || horizon < 1) { g_err = "egg_control_moments: k and horizon must be >= 1"; return EGG_ERR_ARG; }
   const long long L = (long long)horizon * b->dev.n * 6;
   if (L > INT_MAX) { g_err = "egg_control_moments: too long a horizon"; return EGG_ERR_ARG; }
-  RET(check_device_ptr(b, rows_d, "egg_control_moments(rows_d)"));
-  RET(check_device_ptr(b, out_d, "egg_control_moments(out_d)"));
-  if (!b->initialised) { g_err = "egg_control_moments before egg_init"; return EGG_ERR_STATE; }
-  CK(cudaSetDevice(b->device));
-  LK(egg_launch_control_moments(rows_d, k, (int)L, out_d, b->stream));
+  RET(enter(b, "egg_control_moments", INIT_LAST, {{rows_d, "rows_d"}, {out_d, "out_d"}}));
+  CK(egg_launch_control_moments(rows_d, k, (int)L, out_d, b->stream));
   b->launches++;
   return EGG_OK;
 }
@@ -841,37 +850,20 @@ int egg_mppi_reduce(egg_batch* b, const double* u_d, int horizon, const double* 
   const int chunks = egg_mppi_chunks(b->dev.W);
   const long long cols = (long long)horizon * b->dev.n * 6 + 2;
   if (chunks > 65535 || cols > INT_MAX) { g_err = "egg_mppi_reduce: too many worlds or too long a horizon"; return EGG_ERR_ARG; }
-  RET(check_device_ptr(b, u_d, "egg_mppi_reduce(u_d)"));
-  RET(check_device_ptr(b, cost_d, "egg_mppi_reduce(cost_d)"));
-  RET(check_device_ptr(b, baseline_d, "egg_mppi_reduce(baseline_d)"));
-  RET(check_device_ptr(b, out_d, "egg_mppi_reduce(out_d)"));
-  if (!b->initialised) { g_err = "egg_mppi_reduce before egg_init"; return EGG_ERR_STATE; }
-  CK(cudaSetDevice(b->device));
+  RET(enter(b, "egg_mppi_reduce", INIT_LAST, {{u_d, "u_d"}, {cost_d, "cost_d"}, {baseline_d, "baseline_d"}, {out_d, "out_d"}}));
   const size_t need = (size_t)chunks * (size_t)cols;
-  if (need > b->mppi_partial_count) {
-    if (b->mppi_partial) RET(dfree(b, b->mppi_partial, b->mppi_partial_count * sizeof(double)));
-    b->mppi_partial = nullptr;
-    b->mppi_partial_count = 0;
-    RET(dalloc(b, &b->mppi_partial, need));
-    b->mppi_partial_count = need;
-  }
-  LK(egg_launch_mppi_reduce(b->dev, u_d, horizon, cost_d, baseline_d, lambda, b->mppi_partial, out_d, b->stream));
+  if (need > b->mppi_partial_count) RET(replace_dbuf(b, b->mppi_partial, b->mppi_partial_count, need, nullptr));
+  CK(egg_launch_mppi_reduce(b->dev, u_d, horizon, cost_d, baseline_d, lambda, b->mppi_partial, out_d, b->stream));
   b->launches += 2;
   return EGG_OK;
 }
 
 int egg_gather_state(egg_batch* b, const int* worlds, int k, double* out_d) {
   if (!b || !worlds || !out_d) return EGG_ERR_ARG;
-  const int W = b->dev.W;
-  if (k < 1 || k > W) { g_err = "egg_gather_state: k must be in [1, n_worlds]"; return EGG_ERR_ARG; }
-  for (int i = 0; i < k; i++)
-    if (worlds[i] < 0 || worlds[i] >= W) { g_err = "egg_gather_state: world index out of range"; return EGG_ERR_ARG; }
-  if (!b->initialised) { g_err = "egg_gather_state before egg_init"; return EGG_ERR_STATE; }
-  RET(check_device_ptr(b, out_d, "egg_gather_state(out_d)"));
-  CK(cudaSetDevice(b->device));
-  if (!b->gather_idx) RET(dalloc(b, &b->gather_idx, (size_t)W));
-  CK(cudaMemcpyAsync(b->gather_idx, worlds, (size_t)k * sizeof(int), cudaMemcpyHostToDevice, b->stream));
-  LK(egg_launch_gather_state(b->dev, b->gather_idx, k, out_d, b->stream));
+  RET(check_worlds(b, "egg_gather_state", worlds, k));
+  RET(enter(b, "egg_gather_state", INIT_FIRST, {{out_d, "out_d"}}));
+  RET(upload_worlds(b, worlds, k));
+  CK(egg_launch_gather_state(b->dev, b->gather_idx, k, out_d, b->stream));
   b->launches++;
   return EGG_OK;
 }
@@ -879,10 +871,8 @@ int egg_gather_state(egg_batch* b, const int* worlds, int k, double* out_d) {
 int egg_seed_state(egg_batch* b, const double* in_d, int k, int first) {
   if (!b || !in_d) return EGG_ERR_ARG;
   if (k < 1 || k > b->dev.W || first < 0) { g_err = "egg_seed_state: k must be in [1, n_worlds] and first >= 0"; return EGG_ERR_ARG; }
-  if (!b->initialised) { g_err = "egg_seed_state before egg_init"; return EGG_ERR_STATE; }
-  RET(check_device_ptr(b, in_d, "egg_seed_state(in_d)"));
-  CK(cudaSetDevice(b->device));
-  LK(egg_launch_seed_state(b->dev, in_d, k, first, b->stream));
+  RET(enter(b, "egg_seed_state", INIT_FIRST, {{in_d, "in_d"}}));
+  CK(egg_launch_seed_state(b->dev, in_d, k, first, b->stream));
   b->launches++;
   return EGG_OK;
 }
@@ -891,7 +881,7 @@ int egg_update_contacts(egg_batch* b) {
   if (!b) return EGG_ERR_ARG;
   if (!b->initialised) { g_err = "egg_update_contacts before egg_init"; return EGG_ERR_STATE; }
   CK(cudaSetDevice(b->device));
-  LK(egg_launch_collide(b->dev, b->stream));
+  CK(egg_launch_collide(b->dev, b->stream));
   b->launches++;
   return EGG_OK;
 }
@@ -962,7 +952,7 @@ int egg_get_contacts_range(egg_batch* b, int first, int nworlds, int* count, int
       const size_t nw = (W - w0 < chunk) ? W - w0 : chunk;
       for (auto& pt : part) {
         if (!pt.host) continue;
-        LK(egg_launch_unpack((int)nw, b->stage, (int)mc, pt.comps, d.c_geom + (f + w0) * 7 * mc, 7, pt.off, b->stream));
+        CK(egg_launch_unpack((int)nw, b->stage, (int)mc, pt.comps, d.c_geom + (f + w0) * 7 * mc, 7, pt.off, b->stream));
         b->launches++;
         CK(cudaMemcpyAsync(pt.host + w0 * mc * pt.comps, b->stage, nw * mc * pt.comps * sizeof(double), cudaMemcpyDeviceToHost, b->stream));
         CK(cudaStreamSynchronize(b->stream));      // the staging buffer is reused by the next part
@@ -1044,9 +1034,8 @@ int egg_get_dense_work(egg_batch* b, double* flops) {
 }
 
 int egg_rollout_costs(egg_batch* b, double* cost_d) {
-  if (!b || !cost_d) return EGG_ERR_ARG;
-  CK(cudaSetDevice(b->device));
-  LK(egg_launch_costs(b->dev, cost_d, b->stream));
+  RET(enter(b, "egg_rollout_costs", INIT_NONE, {{cost_d, "cost_d"}}));
+  CK(egg_launch_costs(b->dev, cost_d, b->stream));
   b->launches++;
   return EGG_OK;
 }

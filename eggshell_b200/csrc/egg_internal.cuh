@@ -200,18 +200,17 @@ struct EggSampler {
   const double* lo;
   const double* hi;
 };
-// MPPI (egg_sample_controls, egg_mppi_reduce): u [H][W][n][6] <- clamp(u_nom [H][n][6] + sigma eps);
-// out [H n 6 + 2] <- sum_w omega_w u[t][w], sum omega, sum omega^2 through partial [chunks][H n 6 + 2]
-cudaError_t egg_launch_mppi_sample(const EggDev& d, const EggSampler& sm, const double* u_nom, int horizon,
-                                   unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s);
+// Sampling (egg_sample_controls, egg_sample_controls_std): u [H][W][n][6] <- clamp(mean [H][n][6] + sigma eps)
+// with sm.sigma per body, or with the per-step std_dev [H][n][6] in its place when std_dev is not null.
+cudaError_t egg_launch_sample(const EggDev& d, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
+                              unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s);
+// MPPI (egg_mppi_reduce): out [H n 6 + 2] <- sum_w omega_w u[t][w], sum omega, sum omega^2 through
+// partial [chunks][H n 6 + 2]
 int egg_mppi_chunks(int W);   // stage-1 chunks of egg_launch_mppi_reduce: partial holds chunks x (H n 6 + 2) doubles
 cudaError_t egg_launch_mppi_reduce(const EggDev& d, const double* u, int horizon, const double* cost, const double* baseline,
                                    double lambda, double* partial, double* out, cudaStream_t s);
-// CEM (egg_sample_controls_std, egg_gather_controls, egg_control_moments): the sampler with the
-// per-step std [H][n][6] in place of sm.sigma; out [k][H][n][6] <- u[t][worlds[i]];
+// CEM (egg_gather_controls, egg_control_moments): out [k][H][n][6] <- u[t][worlds[i]];
 // out [2][L] <- mean and population std of the columns of rows [k][L]
-cudaError_t egg_launch_sample_std(const EggDev& d, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
-                                  unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s);
 cudaError_t egg_launch_gather_controls(const EggDev& d, const double* u, int horizon, const int* worlds, int k, double* out,
                                        cudaStream_t s);
 cudaError_t egg_launch_control_moments(const double* rows, int k, int L, double* out, cudaStream_t s);

@@ -156,13 +156,9 @@ static cudaError_t launch_sample(const EggDev& d, const EggSampler& sm, const do
   return cudaGetLastError();
 }
 
-cudaError_t egg_launch_mppi_sample(const EggDev& d, const EggSampler& sm, const double* u_nom, int horizon,
-                                   unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s) {
-  return launch_sample<EGG_SIGMA_PER_BODY>(d, sm, u_nom, horizon, seed, iteration, first, u, s);
-}
-
-cudaError_t egg_launch_sample_std(const EggDev& d, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
-                                  unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s) {
+cudaError_t egg_launch_sample(const EggDev& d, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
+                              unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s) {
+  if (!std_dev) return launch_sample<EGG_SIGMA_PER_BODY>(d, sm, mean, horizon, seed, iteration, first, u, s);
   return launch_sample<EGG_SIGMA_PER_STEP>(d, EggSampler{std_dev, sm.lo, sm.hi}, mean, horizon, seed, iteration, first, u, s);
 }
 

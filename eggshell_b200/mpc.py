@@ -13,6 +13,19 @@ STATE_PER_BODY = 18   # p(3), R(9, row-major), v(3), w(3): a row of egg_gather_s
 CONTROL_PER_BODY = 6  # f(3), tau(3): a row of egg_set_external / a control schedule slice
 
 
+def _broadcast(a, shape, owner, name, finite=False):
+    """a as a contiguous float64 array of the given shape (numpy broadcasting); the errors name the
+    owner class and the argument.  finite: refuse NaN and +-inf as well."""
+    a = np.asarray(a, dtype=np.float64)
+    try:
+        a = np.ascontiguousarray(np.broadcast_to(a, shape))
+    except ValueError:
+        raise ValueError(f"{owner}: {name} of shape {a.shape} does not broadcast to {list(shape)}") from None
+    if finite and not np.isfinite(a).all():
+        raise ValueError(f"{owner}: {name} has non-finite values")
+    return a
+
+
 class QuadraticCost:
     """A quadratic running + terminal cost over a controlled horizon, shared by all worlds
     (Batch.set_cost, egg_set_cost).  With x_t [n, 18] the state before step t, x_H the state after
@@ -32,30 +45,19 @@ class QuadraticCost:
             raise ValueError("QuadraticCost: n must be >= 1")
         self.n = n
         S, U = STATE_PER_BODY, CONTROL_PER_BODY
-        self.q_run, self.l_run, self.q_term, self.l_term = (self._arr(a, (n, S), name) for a, name in
+        self.q_run, self.l_run, self.q_term, self.l_term = (_broadcast(a, (n, S), "QuadraticCost", name, finite=True) for a, name in
                                                             ((q_run, "q_run"), (l_run, "l_run"), (q_term, "q_term"), (l_term, "l_term")))
-        self.u_run = self._arr(u_run, (n, U), "u_run")
+        self.u_run = _broadcast(u_run, (n, U), "QuadraticCost", "u_run", finite=True)
         x = np.asarray(x_ref, dtype=np.float64)
         if x.ndim == 3:
             if x.shape[0] < 1:
                 raise ValueError("QuadraticCost: x_ref needs ref_steps >= 1 rows")
-            self.x_ref = self._arr(x, (x.shape[0], n, S), "x_ref")
+            self.x_ref = _broadcast(x, (x.shape[0], n, S), "QuadraticCost", "x_ref", finite=True)
         elif x.ndim <= 2:
-            self.x_ref = self._arr(x, (1, n, S), "x_ref")
+            self.x_ref = _broadcast(x, (1, n, S), "QuadraticCost", "x_ref", finite=True)
         else:
             raise ValueError(f"QuadraticCost: x_ref must broadcast to [{n}, {S}] or be [ref_steps, {n}, {S}]")
         self.ref_steps = self.x_ref.shape[0]
-
-    @staticmethod
-    def _arr(a, shape, name):
-        a = np.asarray(a, dtype=np.float64)
-        try:
-            a = np.ascontiguousarray(np.broadcast_to(a, shape))
-        except ValueError:
-            raise ValueError(f"QuadraticCost: {name} of shape {a.shape} does not broadcast to {list(shape)}") from None
-        if not np.isfinite(a).all():
-            raise ValueError(f"QuadraticCost: {name} has non-finite values")
-        return a
 
     def evaluate(self, states, u):
         """The float64 numpy reference of J: states [H + 1, W, n, 18] (x_0 ... x_H), u [H, W, n, 6].
@@ -89,21 +91,14 @@ def allgather_costs(local_costs):
     import torch.distributed as dist
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
         return local_costs.clone()
-    ws = dist.get_world_size()
-    n = torch.tensor([local_costs.numel()], dtype=torch.int64, device=local_costs.device)
-    sizes = [torch.zeros_like(n) for _ in range(ws)]
-    dist.all_gather(sizes, n)
-    sizes = [int(s.item()) for s in sizes]
+    sizes = allgather_rows(torch.tensor([local_costs.numel()], dtype=torch.int64, device=local_costs.device))[:, 0].tolist()
     m = max(sizes)
     if all(s == m for s in sizes):
-        out = torch.empty(ws * m, dtype=local_costs.dtype, device=local_costs.device)
-        dist.all_gather_into_tensor(out, local_costs.contiguous())
-        return out
+        return allgather_rows(local_costs).view(-1)
     pad = torch.full((m,), float("inf"), dtype=local_costs.dtype, device=local_costs.device)
     pad[: local_costs.numel()] = local_costs
-    out = torch.empty(ws * m, dtype=local_costs.dtype, device=local_costs.device)
-    dist.all_gather_into_tensor(out, pad)
-    return torch.cat([out[r * m: r * m + sizes[r]] for r in range(ws)])
+    out = allgather_rows(pad)
+    return torch.cat([out[r, : sizes[r]] for r in range(len(sizes))])
 
 
 def select_best(all_costs, k=1):
@@ -150,6 +145,35 @@ def gather_winner_states(winners, n_total, pack):
     return buf.view(ws, k, F)[src, torch.arange(k, device=rows.device)]
 
 
+def _packer(F, device, fill):
+    """A `pack` for gather_winner_states: a float64 [len(local), F] tensor on device, written by
+    fill(local, out_ptr) unless local is empty."""
+    import torch
+
+    def pack(local):
+        out = torch.empty((len(local), F), dtype=torch.float64, device=device)
+        if len(local):
+            fill(local, out.data_ptr())
+        return out
+    return pack
+
+
+def _checked_device(batch, u=None, horizon=None):
+    """The batch's CUDA device, after the checks shared by the loops and planners: u, if given, is a
+    contiguous float64 schedule [horizon, W, n, 6] on that device (any H >= 1 without a horizon), and
+    the batch runs on torch's current stream."""
+    import torch
+    dev = torch.device("cuda", int(batch.desc.device))
+    if u is not None and not (isinstance(u, torch.Tensor) and u.is_cuda and u.device == dev and u.dtype == torch.float64
+                              and u.is_contiguous() and u.dim() == 4 and tuple(u.shape[1:]) == (batch.W, batch.n, 6)
+                              and (u.shape[0] >= 1 if horizon is None else u.shape[0] == horizon)):
+        H = "H >= 1" if horizon is None else horizon
+        raise ValueError(f"u must be a contiguous float64 tensor [{H}, {batch.W}, {batch.n}, 6] on {dev}")
+    if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
+        raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
+    return dev
+
+
 def mpc_iteration(batch, u, dt, k, n_total, first):
     """One receding-horizon iteration of a (sharded) random-shooting sweep.
 
@@ -162,29 +186,12 @@ def mpc_iteration(batch, u, dt, k, n_total, first):
     The batch must run on torch's current stream (Batch.set_stream), on which u is produced.
     Returns (winners, their costs, states [k, n * 18] float64 CUDA tensor)."""
     import torch
-    dev = torch.device("cuda", int(batch.desc.device))
-    if not (isinstance(u, torch.Tensor) and u.is_cuda and u.device == dev and u.dtype == torch.float64
-            and u.is_contiguous() and u.dim() == 4 and u.shape[0] >= 1 and tuple(u.shape[1:]) == (batch.W, batch.n, 6)):
-        raise ValueError(f"u must be a contiguous float64 tensor [H >= 1, {batch.W}, {batch.n}, 6] on {dev}")
-    if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
-        raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
+    dev = _checked_device(batch, u)
     costs = torch.empty(batch.W, dtype=torch.float64, device=dev)
     batch.restore()
-    if batch.cost is None:
-        batch.step_controlled(dt, u.data_ptr(), u.shape[0])
-        batch.rollout_costs(costs.data_ptr())
-    else:
-        batch.step_controlled_cost(dt, u.data_ptr(), u.shape[0], costs.data_ptr())
+    _rollout(batch, dt, u, costs)
     winners, best = select_best(allgather_costs(costs), k)
-    F = batch.n * STATE_PER_BODY
-
-    def pack(local):
-        out = torch.empty((len(local), F), dtype=torch.float64, device=dev)
-        if len(local):
-            batch.gather_state(local, out.data_ptr())
-        return out
-
-    states = gather_winner_states(winners, n_total, pack)
+    states = gather_winner_states(winners, n_total, _packer(batch.n * STATE_PER_BODY, dev, batch.gather_state))
     batch.seed_state(states.data_ptr(), len(winners), first)
     batch.snapshot()
     return winners, best, states
@@ -203,11 +210,11 @@ class _SamplingPlan:
             raise ValueError(f"{name}: n and horizon must be >= 1")
         U = CONTROL_PER_BODY
         self.n, self.horizon = n, horizon
-        self.sigma = self._arr(sigma, (n, U), "sigma")
+        self.sigma = _broadcast(sigma, (n, U), name, "sigma")
         if not np.isfinite(self.sigma).all() or (self.sigma < 0).any():
             raise ValueError(f"{name}: sigma must be finite and >= 0")
-        self.u_lo = None if u_lo is None else self._arr(u_lo, (n, U), "u_lo")
-        self.u_hi = None if u_hi is None else self._arr(u_hi, (n, U), "u_hi")
+        self.u_lo = None if u_lo is None else _broadcast(u_lo, (n, U), name, "u_lo")
+        self.u_hi = None if u_hi is None else _broadcast(u_hi, (n, U), name, "u_hi")
         for a, what in ((self.u_lo, "u_lo"), (self.u_hi, "u_hi")):
             if a is not None and np.isnan(a).any():
                 raise ValueError(f"{name}: {what} has NaN values")
@@ -219,22 +226,13 @@ class _SamplingPlan:
         if not 0 <= seed < 2 ** 64:
             raise ValueError(f"{name}: seed must be in [0, 2^64)")
         self.seed = seed
-        un = np.zeros((horizon, n, U)) if u_nom is None else self._arr(
-            u_nom.detach().cpu().numpy() if isinstance(u_nom, torch.Tensor) else u_nom, (horizon, n, U), "u_nom")
-        if not np.isfinite(un).all():
-            raise ValueError(f"{name}: u_nom has non-finite values")
+        un = np.zeros((horizon, n, U)) if u_nom is None else _broadcast(
+            u_nom.detach().cpu().numpy() if isinstance(u_nom, torch.Tensor) else u_nom, (horizon, n, U), name, "u_nom", finite=True)
         self.device = torch.device(device)
         self.u_nom = torch.from_numpy(un.copy()).to(self.device)   # own storage: the iterations write to it
         self.lo = torch.from_numpy(lo).to(self.device)   # the bounds as tensors, for clamp on the device
         self.hi = torch.from_numpy(hi).to(self.device)
         self.iteration = 0
-
-    def _arr(self, a, shape, what):
-        a = np.asarray(a, dtype=np.float64)
-        try:
-            return np.ascontiguousarray(np.broadcast_to(a, shape))
-        except ValueError:
-            raise ValueError(f"{type(self).__name__}: {what} of shape {a.shape} does not broadcast to {list(shape)}") from None
 
     def clamp(self, u):
         """u clamped to [u_lo, u_hi] (broadcast over leading dimensions)."""
@@ -312,17 +310,10 @@ def allgather_rank_sum(x):
     return acc
 
 
-def _mppi_check(batch, plan, u, first):
+def _plan_check(batch, plan, u, first):
     """The checks of mppi_iteration and cem_iteration for a plan (MPPI or CEM) and a schedule buffer u."""
-    import torch
     import torch.distributed as dist
-    dev = torch.device("cuda", int(batch.desc.device))
-    H = plan.horizon
-    if not (isinstance(u, torch.Tensor) and u.is_cuda and u.device == dev and u.dtype == torch.float64
-            and u.is_contiguous() and u.dim() == 4 and u.shape[0] == H and tuple(u.shape[1:]) == (batch.W, batch.n, 6)):
-        raise ValueError(f"u must be a contiguous float64 tensor [{H}, {batch.W}, {batch.n}, 6] on {dev}")
-    if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
-        raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
+    dev = _checked_device(batch, u, plan.horizon)
     if batch.sampler is not plan:
         raise ValueError("the batch's sampler is not this planner: call Batch.set_sampler(mppi) first")
     if plan.u_nom.device != dev:
@@ -385,7 +376,7 @@ def mppi_iteration(batch, mppi, dt, u, first):
     ess = (sum omega)^2 / sum omega^2 the effective number of samples.  If no rollout finished with a
     finite cost (sum omega = 0) it raises and leaves u_nom and iteration unchanged."""
     import torch
-    dev = _mppi_check(batch, mppi, u, first)
+    dev = _plan_check(batch, mppi, u, first)
     costs = torch.empty(batch.W, dtype=torch.float64, device=dev)
     batch.restore()
     mppi_sample(batch, mppi, u, first)
@@ -405,24 +396,13 @@ def mppi_advance(batch, plan, dt, n_total):
     becomes the snapshot, the start of the next horizon; u_nom shifts by one step (the last row
     repeats).  This costs one step of the whole batch, 1/H of a horizon.  Returns (the executed control
     [n, 6], the new start rows [n, 18]), float64 CUDA tensors."""
-    import torch
-    dev = torch.device("cuda", int(batch.desc.device))
+    dev = _checked_device(batch)
     if plan.u_nom.device != dev:
         raise ValueError(f"the planner's u_nom must live on {dev}")
-    if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
-        raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
     u0 = plan.clamp(plan.u_nom[0])
     batch.restore()
     batch.step_controlled(dt, u0.expand(1, batch.W, batch.n, CONTROL_PER_BODY).contiguous().data_ptr(), 1)
-    F = batch.n * STATE_PER_BODY
-
-    def pack(local):
-        out = torch.empty((len(local), F), dtype=torch.float64, device=dev)
-        if len(local):
-            batch.gather_state(local, out.data_ptr())
-        return out
-
-    state = gather_winner_states([0], n_total, pack)
+    state = gather_winner_states([0], n_total, _packer(batch.n * STATE_PER_BODY, dev, batch.gather_state))
     batch.seed_state(state.data_ptr(), 1, 0)
     batch.snapshot()
     if plan.horizon > 1:
@@ -472,7 +452,7 @@ def cem_iteration(batch, cem, dt, u, first, n_total):
       1. restore the snapshot;  2. sample clamp(u_nom + std eps) into u (global world 0: clamp(u_nom));
       3. roll them out with the batch's QuadraticCost, or without one with the built-in cost;
       4. allgather the costs and pick the n_elite cheapest finite ones (identical on every rank);
-      5. fetch the elites' schedules from their owner ranks (gather_controls, one allgather);
+      5. fetch the elites' schedules from their owner ranks (gather_winner_states, one allgather);
       6. control_moments: their mean and population std, computed identically on every rank;
       7. u_nom <- clamp(alpha u_nom + (1 - alpha) mean), std <- max(alpha std + (1 - alpha) std_e,
          sigma_min);  iteration += 1.
@@ -482,7 +462,7 @@ def cem_iteration(batch, cem, dt, u, first, n_total):
     expensive elite, and the mean of the new std.  If fewer than n_elite rollouts finished with a finite
     cost, or the refit is not finite, it raises and leaves the plan and iteration unchanged."""
     import torch
-    dev = _mppi_check(batch, cem, u, first)
+    dev = _plan_check(batch, cem, u, first)
     if cem.std.device != dev:
         raise ValueError(f"the planner's std must live on {dev}")
     H, U = cem.horizon, CONTROL_PER_BODY
@@ -490,14 +470,7 @@ def cem_iteration(batch, cem, dt, u, first, n_total):
     batch.restore()
     cem_sample(batch, cem, u, first)
     _rollout(batch, dt, u, costs)
-    F = H * batch.n * U
-
-    def pack(local):
-        out = torch.empty((len(local), F), dtype=torch.float64, device=dev)
-        if len(local):
-            batch.gather_controls(u.data_ptr(), H, local, out.data_ptr())
-        return out
-
+    pack = _packer(H * batch.n * U, dev, lambda local, out_ptr: batch.gather_controls(u.data_ptr(), H, local, out_ptr))
     all_costs, elites, ecost, rows = cem_select(cem, costs, n_total, pack)
     moments = torch.empty((2, H, batch.n, U), dtype=torch.float64, device=dev)
     batch.control_moments(rows.contiguous().data_ptr(), len(elites), H, moments.data_ptr())

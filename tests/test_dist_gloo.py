@@ -1,14 +1,10 @@
 """world_size-2 CPU (gloo) test of the N>1 host path: contiguous world shards + the cost allgather
 + identical selection on every rank (SURVEY.md §8e)."""
-import os
-import socket
-
 import numpy as np
 import torch
-import torch.distributed as dist
-import torch.multiprocessing as mp
 
 from eggshell_b200 import mpc
+from tests.mpc_helpers import run_ranks
 
 
 def test_shard_range_partitions_exactly():
@@ -24,47 +20,24 @@ def test_shard_range_partitions_exactly():
                 assert spans[r][0] + l == g
 
 
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    p = s.getsockname()[1]
-    s.close()
-    return p
-
-
-def _worker(rank, ws, port, total, q):
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=ws)
+def _worker(rank, ws, total):
     lo, hi = mpc.shard_range(total, rank, ws)
     # deterministic per-world "rollout cost" that depends only on the global world index
     g = np.arange(lo, hi, dtype=np.float64)
     local = torch.from_numpy(np.cos(g * 0.37) + 1e-3 * g)
     allc = mpc.allgather_costs(local)
     idx, val = mpc.select_best(allc, k=3)
-    q.put((rank, allc.numpy().copy(), idx.copy(), val.copy()))
-    dist.barrier()
-    dist.destroy_process_group()
+    return allc.numpy().copy(), idx.copy(), val.copy()
 
 
 def _run(total):
-    ws = 2
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, ws, port, total, q)) for r in range(ws)]
-    for p in procs:
-        p.start()
-    res = [q.get(timeout=120) for _ in range(ws)]
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    res = run_ranks(_worker, 2, "gloo", total, timeout=120)
     g = np.arange(total, dtype=np.float64)
     expect = np.cos(g * 0.37) + 1e-3 * g
-    for rank, allc, idx, val in res:
+    for allc, idx, val in res:
         assert np.array_equal(allc, expect)
         assert np.array_equal(idx, np.argsort(expect, kind="stable")[:3])
-    assert np.array_equal(res[0][2], res[1][2])
+    assert np.array_equal(res[0][1], res[1][1])
 
 
 def test_allgather_even_shards_gloo():

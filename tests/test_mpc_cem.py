@@ -2,15 +2,13 @@
 scale), egg_gather_controls (the elites' schedules), egg_control_moments (their mean and standard
 deviation) and mpc.CEM, cem_iteration and cem_advance.  The first tests run on the CPU; the rest need
 a CUDA device."""
-import os
-
 import numpy as np
 import pytest
 import torch
 
 from eggshell_b200 import mpc
-from tests.test_mpc_mppi import (_batch, _bits, _boxes, _clamp, _code, _costs_of, _cuda, _free_port, _reach_cost, _rows,
-                                 noise)
+from tests.mpc_helpers import (ZERO_G_PGS, batch_on_current_stream, bits, boxes, clamp, costs_of, cuda, err_code, noise, reach_cost,
+                               run_ranks, state_rows)
 
 gpu = pytest.mark.gpu
 S, U = mpc.STATE_PER_BODY, mpc.CONTROL_PER_BODY
@@ -35,7 +33,7 @@ def moments_numpy(rows):
 
 def refit_numpy(u_nom, std, mean, std_e, alpha, sigma_min, lo, hi):
     """The update of cem_iteration: (clamp(alpha u_nom + (1 - alpha) mean), max(alpha std + (1 - alpha) std_e, sigma_min))."""
-    return _clamp(alpha * u_nom + (1.0 - alpha) * mean, lo, hi), np.maximum(alpha * std + (1.0 - alpha) * std_e, sigma_min)
+    return clamp(alpha * u_nom + (1.0 - alpha) * mean, lo, hi), np.maximum(alpha * std + (1.0 - alpha) * std_e, sigma_min)
 
 
 def _np(t):
@@ -81,7 +79,7 @@ def test_moments_definition():
     assert np.all(np.abs(mean - rows.mean(axis=0)) <= 1e-14 * scale)
     assert np.all(np.abs(std - rows.std(axis=0)) <= 1e-14 * scale)
     m1, s1 = moments_numpy(rows[:1])
-    assert np.array_equal(_bits(m1), _bits(rows[0])) and not s1.any()   # one row: itself, and std 0
+    assert np.array_equal(bits(m1), bits(rows[0])) and not s1.any()   # one row: itself, and std 0
     r = rows.copy()
     r[7, 1, 0, 2] = np.nan
     m, s = moments_numpy(r)
@@ -92,7 +90,7 @@ def test_moments_definition():
                 u_nom=rng.uniform(-1.0, 1.0, size=(H, n, U)), device="cpu")
     un, sd = mpc.cem_refit(c, torch.from_numpy(np.stack([mean, std])))
     eu, es = refit_numpy(_np(c.u_nom), _np(c.std), mean, std, 0.3, 0.5, -1.0, 1.0)
-    assert np.array_equal(_bits(_np(un)), _bits(eu)) and np.array_equal(_bits(_np(sd)), _bits(es))
+    assert np.array_equal(bits(_np(un)), bits(eu)) and np.array_equal(bits(_np(sd)), bits(es))
     assert (_np(un) == 1.0).any() and (_np(un) == -1.0).any() and (_np(sd) == 0.5).any()   # both bounds and the floor reached
 
 
@@ -119,38 +117,18 @@ def _refit_on_shard(rank, ws, n_elite=9):
     return elites, ecost, got.numpy().copy(), _np(un).copy(), _np(sd).copy()
 
 
-def _gloo_worker(rank, ws, port, q):
-    import torch.distributed as dist
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=ws)
-    q.put((rank, _refit_on_shard(rank, ws)))
-    dist.barrier()
-    dist.destroy_process_group()
-
-
 def test_refit_on_two_gloo_ranks_matches_one_rank():
-    import torch.multiprocessing as mp
     ws = 2
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_gloo_worker, args=(r, ws, port, q)) for r in range(ws)]
-    for p in procs:
-        p.start()
-    res = dict(q.get(timeout=120) for _ in range(ws))
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    res = run_ranks(_refit_on_shard, ws, "gloo", timeout=120)
     one = _refit_on_shard(0, 1)
     rows, cost = _pool()
     order = [i for i in np.lexsort((np.arange(cost.size), cost)) if np.isfinite(cost[i])][:9]
     assert list(one[0]) == order and order[:2] == [11, 30]
-    assert np.array_equal(_bits(one[2]), _bits(rows[order]))
+    assert np.array_equal(bits(one[2]), bits(rows[order]))
     for r in range(ws):
         assert list(res[r][0]) == order
         for a, b in zip(res[r][1:], one[1:]):
-            assert np.array_equal(_bits(np.asarray(a)), _bits(np.asarray(b)))
+            assert np.array_equal(bits(np.asarray(a)), bits(np.asarray(b)))
     # fewer finite costs than elites: raises before the exchange
     with pytest.raises(RuntimeError, match="fewer than n_elite = 39"):
         _refit_on_shard(0, 1, n_elite=39)
@@ -182,14 +160,14 @@ def _sample(b, c, first=0, iteration=None):
 @gpu
 def test_std_sampler_with_a_constant_std_is_the_mppi_sampler():
     W, n, H, first = 300, 3, 4, 1000
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     rng = np.random.default_rng(9)
     lo, hi = rng.uniform(-1.5, -0.5, size=(n, U)), rng.uniform(0.5, 1.5, size=(n, U))
     c = _plan(n, H, u_lo=lo, u_hi=hi)
     b.set_sampler(c)
     for f, it in ((first, 2 ** 32 + 5), (0, 3)):
         got, ref = _sample_std(b, c, first=f, iteration=it), _sample(b, c, first=f, iteration=it)
-        assert np.array_equal(_bits(got), _bits(ref)), (f, it)
+        assert np.array_equal(bits(got), bits(ref)), (f, it)
         assert (got == lo).any() and (got == hi).any()
     b.close()
 
@@ -197,13 +175,13 @@ def test_std_sampler_with_a_constant_std_is_the_mppi_sampler():
 @gpu
 def test_std_sampler_matches_numpy():
     W, n, H, first = 300, 3, 3, 1000
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     rng = np.random.default_rng(8)
     c = _plan(n, H)
     c.iteration = 2 ** 32 + 5   # both counter words of the iteration in use
     std = rng.uniform(0.2, 2.0, size=(H, n, U))
     b.set_sampler(c)
-    u = _sample_std(b, c, std=_cuda(std), first=first)
+    u = _sample_std(b, c, std=cuda(std), first=first)
     eps = noise(H, n, np.arange(first, first + W), c.seed, c.iteration)
     got = (u - c.u_nom.cpu().numpy()[:, None]) / std[:, None]
     assert np.max(np.abs(got - eps)) <= 1e-13, np.max(np.abs(got - eps))
@@ -214,7 +192,7 @@ def test_std_sampler_matches_numpy():
 @gpu
 def test_std_sampler_exact_cases():
     W, n, H = 256, 2, 3
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     rng = np.random.default_rng(3)
     lo, hi = rng.uniform(-1.5, -0.5, size=(n, U)), rng.uniform(0.5, 1.5, size=(n, U))
     lo[0, 0], hi[1, 5] = -np.inf, np.inf
@@ -224,41 +202,41 @@ def test_std_sampler_exact_cases():
     std = rng.uniform(0.5, 2.0, size=(H, n, U))
     std[1, 1, 3] = 0.0   # one element without noise
     b.set_sampler(c)
-    sd = _cuda(std)
+    sd = cuda(std)
     u = _sample_std(b, c, std=sd)
-    c_nom = _clamp(un, lo, hi)
-    assert np.array_equal(_bits(u[:, 0]), _bits(c_nom)), "global world 0 runs clamp(mean)"
-    assert np.array_equal(_bits(u[1, :, 1, 3]), _bits(np.full(W, c_nom[1, 1, 3]))), "std = 0 keeps clamp(mean)"
+    c_nom = clamp(un, lo, hi)
+    assert np.array_equal(bits(u[:, 0]), bits(c_nom)), "global world 0 runs clamp(mean)"
+    assert np.array_equal(bits(u[1, :, 1, 3]), bits(np.full(W, c_nom[1, 1, 3]))), "std = 0 keeps clamp(mean)"
     assert (u >= lo).all() and (u <= hi).all()
     at_lo, at_hi = u == lo, u == hi
     assert at_lo.sum() > 100 and at_hi.sum() > 100
     eps = noise(H, n, np.arange(W), c.seed, c.iteration)
-    free = _clamp(un[:, None] + std[:, None] * eps, lo, hi)
+    free = clamp(un[:, None] + std[:, None] * eps, lo, hi)
     assert np.array_equal(at_lo[:, 1:], (free == lo)[:, 1:]) and np.array_equal(at_hi[:, 1:], (free == hi)[:, 1:])
-    assert np.array_equal(_bits(_sample_std(b, c, std=sd)), _bits(u)), "two calls"
+    assert np.array_equal(bits(_sample_std(b, c, std=sd)), bits(u)), "two calls"
     # std = 0 everywhere: clamp(mean) in every world, bit for bit (-0.0 included)
     zero = torch.zeros((H, n, U), dtype=torch.float64, device="cuda")
-    assert np.array_equal(_bits(_sample_std(b, c, std=zero)), _bits(np.broadcast_to(c_nom[:, None], (H, W, n, U))))
+    assert np.array_equal(bits(_sample_std(b, c, std=zero)), bits(np.broadcast_to(c_nom[:, None], (H, W, n, U))))
     # one batch of W against two batches of W / 2 with first = 0 and first = W / 2
     halves = []
     for first in (0, W // 2):
-        h = _batch(_boxes(W // 2, n))
+        h = batch_on_current_stream(boxes(W // 2, n), defaults=ZERO_G_PGS)
         h.set_sampler(c)
         halves.append(_sample_std(h, c, std=sd, first=first))
         h.close()
-    assert np.array_equal(_bits(np.concatenate(halves, axis=1)), _bits(u))
+    assert np.array_equal(bits(np.concatenate(halves, axis=1)), bits(u))
     b.close()
 
 
 @gpu
 def test_std_sampler_honours_the_per_step_std():
     W, n, H = 50000, 2, 4   # 600000 samples per step
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     c = mpc.CEM(n, H, sigma=1.0, n_elite=1, seed=99)
     b.set_sampler(c)
     std = 0.5 * (1.0 + np.arange(H))[:, None, None] * np.ones((H, n, U))
     std[:, 1, 3:] *= 3.0   # and per body and component
-    x = _sample_std(b, c, std=_cuda(std))[:, 1:]
+    x = _sample_std(b, c, std=cuda(std))[:, 1:]
     for t in range(H):
         for sl, scale in (((0, slice(None)), 0.5 * (t + 1)), ((1, slice(0, 3)), 0.5 * (t + 1)), ((1, slice(3, 6)), 1.5 * (t + 1))):
             e = x[t][:, sl[0], sl[1]] / scale
@@ -269,33 +247,33 @@ def test_std_sampler_honours_the_per_step_std():
 @gpu
 def test_gather_controls_copies_rows_bit_for_bit():
     W, n, H = 77, 3, 5
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     rng = np.random.default_rng(12)
     raw = rng.integers(0, 2 ** 63, size=(H, W, n, U), dtype=np.int64).view(np.float64)   # any bits, NaN payloads included
     raw[0, W - 1, 0, 0], raw[2, 5, 1, 1] = -0.0, np.inf
-    ud = _cuda(raw)
+    ud = cuda(raw)
     worlds = [W - 1, 5, 0, 5, 40, W - 1]
     out = torch.full((len(worlds), H, n, U), 7.0, dtype=torch.float64, device="cuda")
     launches = b.launch_count
     b.gather_controls(ud.data_ptr(), H, worlds, out.data_ptr())
     assert b.launch_count - launches == 1
     got = out.cpu().numpy()
-    assert np.array_equal(_bits(got), _bits(raw[:, worlds].transpose(1, 0, 2, 3)))
+    assert np.array_equal(bits(got), bits(raw[:, worlds].transpose(1, 0, 2, 3)))
     # a shorter horizon reads the first steps of a [H][W][n][6] buffer with the same W
     short = torch.full((2, 2, n, U), 7.0, dtype=torch.float64, device="cuda")
     b.gather_controls(ud.data_ptr(), 2, [3, 76], short.data_ptr())
-    assert np.array_equal(_bits(short.cpu().numpy()), _bits(raw[:2, [3, 76]].transpose(1, 0, 2, 3)))
+    assert np.array_equal(bits(short.cpu().numpy()), bits(raw[:2, [3, 76]].transpose(1, 0, 2, 3)))
     b.close()
 
 
 @gpu
 def test_control_moments_match_numpy():
     W, n, H = 64, 3, 7
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     rng = np.random.default_rng(13)
     for k in (1, 2, 37, 300):
         rows = rng.normal(size=(k, H, n, U)) * 10.0 ** rng.integers(-6, 6, size=(1, H, n, U)) + rng.normal(size=(1, H, n, U))
-        rd = _cuda(rows)
+        rd = cuda(rows)
         out = torch.full((2, H, n, U), 7.0, dtype=torch.float64, device="cuda")
         launches = b.launch_count
         b.control_moments(rd.data_ptr(), k, H, out.data_ptr())
@@ -305,13 +283,13 @@ def test_control_moments_match_numpy():
         assert np.all(np.abs(got[0] - rows.mean(axis=0)) <= 1e-14 * scale), k
         assert np.all(np.abs(got[1] - rows.std(axis=0)) <= 1e-14 * scale), k
         mean, std = moments_numpy(rows)
-        assert np.array_equal(_bits(got[0]), _bits(mean)) and np.array_equal(_bits(got[1]), _bits(std)), k
+        assert np.array_equal(bits(got[0]), bits(mean)) and np.array_equal(bits(got[1]), bits(std)), k
         again = torch.empty_like(out)
         b.control_moments(rd.data_ptr(), k, H, again.data_ptr())
-        assert np.array_equal(_bits(again.cpu().numpy()), _bits(got)), "two calls"
+        assert np.array_equal(bits(again.cpu().numpy()), bits(got)), "two calls"
     rows[5, 2, 1, 4] = np.nan
     out = torch.empty((2, H, n, U), dtype=torch.float64, device="cuda")
-    b.control_moments(_cuda(rows).data_ptr(), rows.shape[0], H, out.data_ptr())
+    b.control_moments(cuda(rows).data_ptr(), rows.shape[0], H, out.data_ptr())
     got = out.cpu().numpy()
     assert np.isnan(got[:, 2, 1, 4]).all() and np.isfinite(got).sum() == got.size - 2
     b.close()
@@ -322,10 +300,10 @@ def test_bad_arguments_are_refused_on_the_host():
     import eggshell_b200 as E
     from eggshell_b200.batch import EggError
     W, n, H = 64, 2, 3
-    scene = _boxes(W, n)
-    b = _batch(scene)
+    scene = boxes(W, n)
+    b = batch_on_current_stream(scene, defaults=ZERO_G_PGS)
     b.step(scene["dt"])
-    before = _rows(b)
+    before = state_rows(b)
     c = _plan(n, H)
     u = torch.full((H, W, n, U), 7.0, dtype=torch.float64, device="cuda")
     out = torch.full((W * H * n * U + 2,), 7.0, dtype=torch.float64, device="cuda")
@@ -337,7 +315,7 @@ def test_bad_arguments_are_refused_on_the_host():
     def refused(call, code, what):
         with pytest.raises(EggError) as ei:
             call()
-        assert _code(ei) == code, f"{what}: {ei.value}"
+        assert err_code(ei) == code, f"{what}: {ei.value}"
 
     refused(lambda: b.sample_controls_std(mp, sp, H, 1, 0, 0, up), -4, "no sampler")
     b.set_sampler(c)
@@ -358,7 +336,7 @@ def test_bad_arguments_are_refused_on_the_host():
         refused(lambda: b.control_moments(r_, k, h_, o_), -1, what)
     assert b.launch_count == launches
     assert bool((u == 7.0).all()) and bool((out == 7.0).all())
-    assert np.array_equal(_bits(_rows(b)), _bits(before))
+    assert np.array_equal(bits(state_rows(b)), bits(before))
     b.close()
     # before egg_init: set_sampler is accepted, the three calls are not
     raw = E.Batch(W, n, 0, solver=E.SOLVER_PGS)
@@ -372,7 +350,7 @@ def test_bad_arguments_are_refused_on_the_host():
 
 
 def _reach(W, seed=5):
-    scene = _boxes(W, 1, seed=seed)
+    scene = boxes(W, 1, seed=seed)
     for key in ("p", "R", "v", "w"):
         scene[key] = np.broadcast_to(scene[key][:1], scene[key].shape).copy()
     return scene
@@ -385,10 +363,10 @@ def test_cem_lowers_the_cost_of_a_reaching_task():
     W, H = 1024, 10
     scene = _reach(W)
     dt = scene["dt"]
-    b = _batch(scene)
+    b = batch_on_current_stream(scene, defaults=ZERO_G_PGS)
     b.snapshot()
-    x0 = _rows(b)[0]
-    b.set_cost(_reach_cost(x0, x0[0, 0:3] + [1.0, -0.5, 0.5]))
+    x0 = state_rows(b)[0]
+    b.set_cost(reach_cost(x0, x0[0, 0:3] + [1.0, -0.5, 0.5]))
     c = mpc.CEM(1, H, sigma=[4.0, 4.0, 4.0, 0.0, 0.0, 0.0], n_elite=64, alpha=0.1, sigma_min=0.05, u_lo=-20.0, u_hi=20.0, seed=2024)
     b.set_sampler(c)
     u = torch.empty((H, W, 1, U), dtype=torch.float64, device="cuda")
@@ -404,13 +382,13 @@ def test_cem_lowers_the_cost_of_a_reaching_task():
         old_u, old_s = c.u_nom.cpu().numpy(), c.std.cpu().numpy()
         r = mpc.cem_iteration(b, c, dt, u, 0, W)
         ub = u.cpu().numpy()
-        J = _costs_of(b, u, H, dt)
+        J = costs_of(b, u, H, dt)
         order = np.lexsort((np.arange(W), J))[:64]
         assert r["nominal_cost"] == J[0] and r["min_cost"] == J[order[0]] and r["elite_max_cost"] == J[order[-1]]
-        assert np.array_equal(_bits(ub[:, 0]), _bits(_clamp(old_u, -20.0, 20.0)))
+        assert np.array_equal(bits(ub[:, 0]), bits(clamp(old_u, -20.0, 20.0)))
         mean, std = moments_numpy(ub[:, order].transpose(1, 0, 2, 3))
         eu, es = refit_numpy(old_u, old_s, mean, std, 0.1, 0.05, -20.0, 20.0)
-        assert np.array_equal(_bits(c.u_nom.cpu().numpy()), _bits(eu)) and np.array_equal(_bits(c.std.cpu().numpy()), _bits(es))
+        assert np.array_equal(bits(c.u_nom.cpu().numpy()), bits(eu)) and np.array_equal(bits(c.std.cpu().numpy()), bits(es))
         assert r["mean_std"] == pytest.approx(es.mean(), rel=1e-12)
         assert (es >= 0.05).all()
     last = mpc.cem_iteration(b, c, dt, u, 0, W)
@@ -422,11 +400,11 @@ def test_cem_lowers_the_cost_of_a_reaching_task():
 @gpu
 def test_cem_iteration_raises_without_enough_finite_rollouts():
     W, H = 64, 3
-    scene = _boxes(W, 1)
+    scene = boxes(W, 1)
     dt = scene["dt"]
-    b = _batch(scene)
+    b = batch_on_current_stream(scene, defaults=ZERO_G_PGS)
     b.snapshot()
-    x0 = _rows(b)[0]
+    x0 = state_rows(b)[0]
     c = _plan(1, H, alpha=0.5, sigma_min=0.1)
     b.set_sampler(c)
     u = torch.empty((H, W, 1, U), dtype=torch.float64, device="cuda")
@@ -435,7 +413,7 @@ def test_cem_iteration_raises_without_enough_finite_rollouts():
     b.set_cost(mpc.QuadraticCost(1, q_term=1e308, x_ref=x0 + 10.0))
     with pytest.raises(RuntimeError, match="0 rollouts finished with a finite cost"):
         mpc.cem_iteration(b, c, dt, u, 0, W)
-    assert np.isinf(_costs_of(b, u, H, dt)).all()
+    assert np.isinf(costs_of(b, u, H, dt)).all()
     b.set_cost(mpc.QuadraticCost(1, q_term=1.0, x_ref=x0))
     big = _plan(1, H, n_elite=W + 1)
     b.set_sampler(big)
@@ -478,35 +456,24 @@ def test_cem_advance_steps_every_world_from_the_plan():
     plan, std = c.u_nom.cpu().numpy(), c.std.cpu().numpy()
     assert not np.array_equal(std[-1], sigma)
     executed, start = mpc.cem_advance(b, c, dt, W)
-    c0 = _clamp(plan[0], -0.3, 0.3)
-    assert np.array_equal(_bits(executed.cpu().numpy()), _bits(c0))
+    c0 = clamp(plan[0], -0.3, 0.3)
+    assert np.array_equal(bits(executed.cpu().numpy()), bits(c0))
     fresh = E.scenes.make_batch(scene, **kw)
     fresh.set_external(np.broadcast_to(c0, (W, n, U)))
     fresh.step(dt, 1)
-    expect = _rows(fresh)[0]
+    expect = state_rows(fresh)[0]
     fresh.close()
-    assert np.array_equal(_bits(_rows(b)), _bits(np.broadcast_to(expect, (W, n, S))))
-    assert np.array_equal(_bits(start.cpu().numpy()), _bits(expect))
+    assert np.array_equal(bits(state_rows(b)), bits(np.broadcast_to(expect, (W, n, S))))
+    assert np.array_equal(bits(start.cpu().numpy()), bits(expect))
     b.restore()   # the new start is the snapshot
-    assert np.array_equal(_bits(_rows(b)), _bits(np.broadcast_to(expect, (W, n, S))))
+    assert np.array_equal(bits(state_rows(b)), bits(np.broadcast_to(expect, (W, n, S))))
     got_u, got_s = c.u_nom.cpu().numpy(), c.std.cpu().numpy()
-    assert np.array_equal(_bits(got_u[:-1]), _bits(plan[1:])) and np.array_equal(_bits(got_u[-1]), _bits(plan[-1]))
-    assert np.array_equal(_bits(got_s[:-1]), _bits(std[1:])) and np.array_equal(_bits(got_s[-1]), _bits(sigma))
+    assert np.array_equal(bits(got_u[:-1]), bits(plan[1:])) and np.array_equal(bits(got_u[-1]), bits(plan[-1]))
+    assert np.array_equal(bits(got_s[:-1]), bits(std[1:])) and np.array_equal(bits(got_s[-1]), bits(sigma))
     b.close()
 
 
-def _nccl_worker(rank, ws, port, W, H, iters, q):
-    import torch.distributed as dist
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    torch.cuda.set_device(rank)
-    dist.init_process_group("nccl", rank=rank, world_size=ws, device_id=torch.device("cuda", rank))
-    q.put((rank, _run_planner(W, H, iters, rank, ws)))
-    dist.barrier()
-    dist.destroy_process_group()
-
-
-def _run_planner(W, H, iters, rank, ws):
+def _run_planner(rank, ws, W, H, iters):
     """`iters` CEM iterations of the reaching task on this rank's shard of W worlds; returns the first
     iteration's samples of the shard and every iteration's u_nom and std."""
     lo, hi = mpc.shard_range(W, rank, ws)
@@ -514,10 +481,10 @@ def _run_planner(W, H, iters, rank, ws):
     for key in ("p", "R", "v", "w", "m", "I"):
         scene[key] = scene[key][lo:hi].copy()
     scene["W"] = hi - lo
-    b = _batch(scene, device=torch.cuda.current_device())
+    b = batch_on_current_stream(scene, defaults=ZERO_G_PGS, device=torch.cuda.current_device())
     b.snapshot()
-    x0 = _rows(b)[0]
-    b.set_cost(_reach_cost(x0, x0[0, 0:3] + [1.0, -0.5, 0.5]))
+    x0 = state_rows(b)[0]
+    b.set_cost(reach_cost(x0, x0[0, 0:3] + [1.0, -0.5, 0.5]))
     c = mpc.CEM(1, H, sigma=[4.0, 4.0, 4.0, 0.0, 0.0, 0.0], n_elite=32, alpha=0.2, sigma_min=0.05, seed=77)
     b.set_sampler(c)
     u = torch.empty((H, hi - lo, 1, U), dtype=torch.float64, device=torch.device("cuda", torch.cuda.current_device()))
@@ -536,19 +503,9 @@ def _run_planner(W, H, iters, rank, ws):
 def test_one_rank_against_two_nccl_ranks():
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
-    import torch.multiprocessing as mp
     W, H, iters = 513, 6, 3   # uneven shards
-    one = _run_planner(W, H, iters, 0, 1)
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_nccl_worker, args=(r, 2, port, W, H, iters, q)) for r in range(2)]
-    for p in procs:
-        p.start()
-    res = dict(q.get(timeout=300) for _ in range(2))
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
-    assert np.array_equal(_bits(np.concatenate([res[0][0], res[1][0]], axis=1)), _bits(one[0]))
+    one = _run_planner(0, 1, W, H, iters)
+    res = run_ranks(_run_planner, 2, "nccl", W, H, iters, timeout=300)
+    assert np.array_equal(bits(np.concatenate([res[0][0], res[1][0]], axis=1)), bits(one[0]))
     for r in range(2):
-        assert np.array_equal(_bits(res[r][1]), _bits(one[1])) and np.array_equal(_bits(res[r][2]), _bits(one[2])), r
+        assert np.array_equal(bits(res[r][1]), bits(one[1])) and np.array_equal(bits(res[r][2]), bits(one[2])), r

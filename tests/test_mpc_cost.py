@@ -3,13 +3,13 @@ egg_step_controlled_cost (the running cost added on the device before every step
 after the last one) and mpc.mpc_iteration with a cost.  The first tests run on the CPU; the rest
 need a CUDA device."""
 import ctypes as C
-import re
 
 import numpy as np
 import pytest
 import torch
 
 from eggshell_b200 import mpc
+from tests.mpc_helpers import batch_on_current_stream, bits, cuda, err_code, state_rows
 
 gpu = pytest.mark.gpu
 S, U = mpc.STATE_PER_BODY, mpc.CONTROL_PER_BODY
@@ -89,34 +89,11 @@ def test_evaluate_by_hand():
 
 
 # ---- GPU ------------------------------------------------------------------------------------------
-def _batch(scene, **kw):
-    """A batch on torch's current stream, so that torch-side buffers and the batch's kernels are ordered."""
-    import eggshell_b200 as E
-    b = E.scenes.make_batch(scene, **kw)
-    b.set_stream(torch.cuda.current_stream().cuda_stream)
-    return b
-
-
 def _scene(name, W):
     import eggshell_b200 as E
     if name == "legged20":
         return E.scenes.legged20(W), dict(solver=E.SOLVER_PGS, k_max=100), 5
     return E.scenes.chain(W, links=10, seed=3, anchor_jitter=0.1, v_jitter=0.2), dict(solver=E.SOLVER_DENSE_MURTY), 3
-
-
-def _rows(b):
-    """bodies() as [W, n, 18] rows (p, R row-major, v, w)."""
-    p, R, v, w = b.bodies()
-    W, n = p.shape[:2]
-    return np.concatenate([p, R.reshape(W, n, 9), v, w], axis=-1)
-
-
-def _bits(a):
-    return np.ascontiguousarray(a).view(np.uint64)
-
-
-def _cuda(a):
-    return torch.from_numpy(np.ascontiguousarray(a)).cuda()
 
 
 def _schedule(f_ext, H, seed, sigma=0.2):
@@ -130,11 +107,11 @@ def _schedule(f_ext, H, seed, sigma=0.2):
 def _host_rollout(b, u, dt):
     """x_0 ... x_H [H + 1, W, n, 18] with set_external(u[t]) + step before every step t (bit-identical to
     the controlled path, test_mpc_loop.test_time_varying_schedule_equals_host_loop)."""
-    states = [_rows(b)]
+    states = [state_rows(b)]
     for t in range(u.shape[0]):
         b.set_external(u[t])
         b.step(dt, 1)
-        states.append(_rows(b))
+        states.append(state_rows(b))
     return np.stack(states)
 
 
@@ -181,13 +158,13 @@ def _assert_matches(got, cost, states, u, what=""):
 def test_cost_matches_numpy(name, W, H):
     scene, kw, _ = _scene(name, W)
     dt = scene["dt"]
-    b = _batch(scene, **kw)
+    b = batch_on_current_stream(scene, **kw)
     b.snapshot()
     u = _schedule(b.static()[2], H, seed=51)
     states = _host_rollout(b, u, dt)
     cost = _random_cost(scene["n"], states, seed=52)
-    got = _device_cost(b, cost, _cuda(u), H, dt)
-    assert np.array_equal(_bits(_rows(b)), _bits(states[H])), "the host loop and the controlled path disagree"
+    got = _device_cost(b, cost, cuda(u), H, dt)
+    assert np.array_equal(bits(state_rows(b)), bits(states[H])), "the host loop and the controlled path disagree"
     assert np.all(got != 0)
     _assert_matches(got, cost, states, u)
     b.close()
@@ -200,23 +177,23 @@ def test_cost_path_steps_like_step_controlled(name):
     W, H = 16, 6
     scene, kw, step_launches = _scene(name, W)
     dt = scene["dt"]
-    b = _batch(scene, **kw)
+    b = batch_on_current_stream(scene, **kw)
     b.snapshot()
     f0 = b.static()[2]
     u = _schedule(f0, H, seed=61)
-    ud = _cuda(u)
+    ud = cuda(u)
     b.step_controlled(dt, ud.data_ptr(), H)
-    ref_rows, ref_f = _rows(b), b.static()[2]
+    ref_rows, ref_f = state_rows(b), b.static()[2]
     b.restore()
     b.set_external(f0)
-    b.set_cost(_random_cost(scene["n"], np.stack([_rows(b)] * (H + 1)), seed=62))
+    b.set_cost(_random_cost(scene["n"], np.stack([state_rows(b)] * (H + 1)), seed=62))
     cost = torch.empty(W, dtype=torch.float64, device="cuda")
     launches = b.launch_count
     b.step_controlled_cost(dt, ud.data_ptr(), H, cost.data_ptr())
     assert b.launch_count - launches == H * (step_launches + 1) + 1
-    assert np.array_equal(_bits(_rows(b)), _bits(ref_rows))
-    assert np.array_equal(_bits(b.static()[2]), _bits(ref_f))
-    assert np.array_equal(_bits(ref_f), _bits(u[-1]))
+    assert np.array_equal(bits(state_rows(b)), bits(ref_rows))
+    assert np.array_equal(bits(b.static()[2]), bits(ref_f))
+    assert np.array_equal(bits(ref_f), bits(u[-1]))
     b.close()
 
 
@@ -227,10 +204,10 @@ def test_each_term_alone():
     W, H = 16, 5
     scene, kw, _ = _scene("legged20", W)
     dt = scene["dt"]
-    b = _batch(scene, **kw)
+    b = batch_on_current_stream(scene, **kw)
     b.snapshot()
     u = _schedule(b.static()[2], H, seed=71)
-    ud = _cuda(u)
+    ud = cuda(u)
     states = _host_rollout(b, u, dt)
     for i, term in enumerate(TERMS):
         cost = _random_cost(scene["n"], states, seed=72 + i, terms=(term,))
@@ -245,10 +222,10 @@ def test_constant_reference_equals_repeated_rows():
     W, H = 16, 4
     scene, kw, _ = _scene("legged20", W)
     dt, n = scene["dt"], scene["n"]
-    b = _batch(scene, **kw)
+    b = batch_on_current_stream(scene, **kw)
     b.snapshot()
-    ud = _cuda(_schedule(b.static()[2], H, seed=81))
-    one = _random_cost(n, np.stack([_rows(b)] * (H + 1)), seed=82, per_step=False)
+    ud = cuda(_schedule(b.static()[2], H, seed=81))
+    one = _random_cost(n, np.stack([state_rows(b)] * (H + 1)), seed=82, per_step=False)
     rep = mpc.QuadraticCost(n, x_ref=np.repeat(one.x_ref, H + 1, axis=0), **{t: getattr(one, t) for t in TERMS})
     assert one.ref_steps == 1 and rep.ref_steps == H + 1
     base = b.device_bytes
@@ -256,7 +233,7 @@ def test_constant_reference_equals_repeated_rows():
     assert b.device_bytes - base == (4 * n * S + n * U + n * S) * 8
     c = _device_cost(b, rep, ud, H, dt)
     assert b.device_bytes - base == (4 * n * S + n * U + (H + 1) * n * S) * 8
-    assert np.array_equal(_bits(a), _bits(c))
+    assert np.array_equal(bits(a), bits(c))
     b.set_cost(None)
     assert b.device_bytes == base and b.cost is None
     b.close()
@@ -277,20 +254,20 @@ def test_cost_is_deterministic_and_shard_independent():
     scene, kw, _ = _scene("legged20", W)
     dt, n = scene["dt"], scene["n"]
     u = _schedule(scene["f_ext"], H, seed=91)
-    full = _batch(scene, **kw)
+    full = batch_on_current_stream(scene, **kw)
     full.snapshot()
-    cost = _random_cost(n, np.stack([_rows(full)] * (H + 1)), seed=92)
-    ud = _cuda(u)
+    cost = _random_cost(n, np.stack([state_rows(full)] * (H + 1)), seed=92)
+    ud = cuda(u)
     c_full = _device_cost(full, cost, ud, H, dt)
-    rows_full = _rows(full)
-    assert np.array_equal(_bits(_device_cost(full, cost, ud, H, dt)), _bits(c_full)), "two runs of one batch"
+    rows_full = state_rows(full)
+    assert np.array_equal(bits(_device_cost(full, cost, ud, H, dt)), bits(c_full)), "two runs of one batch"
     full.close()
     for lo, hi in ((0, W // 2), (W // 2, W), (13, 14)):
-        part = _batch(_shard(scene, lo, hi), **kw)
+        part = batch_on_current_stream(_shard(scene, lo, hi), **kw)
         part.snapshot()
-        c = _device_cost(part, cost, _cuda(u[:, lo:hi]), H, dt)
-        assert np.array_equal(_bits(_rows(part)), _bits(rows_full[lo:hi])), f"physics of worlds [{lo}, {hi})"
-        assert np.array_equal(_bits(c), _bits(c_full[lo:hi])), f"costs of worlds [{lo}, {hi})"
+        c = _device_cost(part, cost, cuda(u[:, lo:hi]), H, dt)
+        assert np.array_equal(bits(state_rows(part)), bits(rows_full[lo:hi])), f"physics of worlds [{lo}, {hi})"
+        assert np.array_equal(bits(c), bits(c_full[lo:hi])), f"costs of worlds [{lo}, {hi})"
         part.close()
 
 
@@ -302,12 +279,12 @@ def test_expresses_the_built_in_cost():
     dt, n = scene["dt"], scene["n"]
     for key in ("p", "R", "v", "w"):
         scene[key] = np.broadcast_to(scene[key][:1], scene[key].shape).copy()
-    b = _batch(scene, **kw)
+    b = batch_on_current_stream(scene, **kw)
     b.snapshot()
-    x0 = _rows(b)[0]
+    x0 = state_rows(b)[0]
     l_term, q_term = np.zeros((n, S)), np.zeros((n, S))
     l_term[0, 0], q_term[0, 2] = -1.0, 10.0
-    ud = _cuda(_schedule(scene["f_ext"], H, seed=101))
+    ud = cuda(_schedule(scene["f_ext"], H, seed=101))
     got = _device_cost(b, mpc.QuadraticCost(n, l_term=l_term, q_term=q_term, x_ref=x0), ud, H, dt)
     built_in = torch.empty(W, dtype=torch.float64, device="cuda")
     b.rollout_costs(built_in.data_ptr())
@@ -322,17 +299,17 @@ def test_mpc_iteration_with_a_cost():
     W, H, k = 16, 4, 3
     scene, kw, step_launches = _scene("legged20", W)
     dt, n = scene["dt"], scene["n"]
-    b = _batch(scene, **kw)
+    b = batch_on_current_stream(scene, **kw)
     b.snapshot()
-    ud = _cuda(_schedule(scene["f_ext"], H, seed=111))
-    cost = _random_cost(n, np.stack([_rows(b)] * (H + 1)), seed=112)
+    ud = cuda(_schedule(scene["f_ext"], H, seed=111))
+    cost = _random_cost(n, np.stack([state_rows(b)] * (H + 1)), seed=112)
     configured = _device_cost(b, cost, ud, H, dt)
     launches = b.launch_count
     winners, best, states = mpc.mpc_iteration(b, ud, dt, k, W, 0)
     # H controlled steps with the running cost, the terminal cost, gather_state, seed_state
     assert b.launch_count - launches == H * (step_launches + 1) + 3
     ew, eb = mpc.select_best(configured, k)
-    assert np.array_equal(winners, ew) and np.array_equal(_bits(best), _bits(eb))
+    assert np.array_equal(winners, ew) and np.array_equal(bits(best), bits(eb))
     assert states.shape == (k, n * S)
     # cleared: the built-in cost of egg_rollout_costs again, with the launches of the old path
     b.set_cost(None)
@@ -345,12 +322,8 @@ def test_mpc_iteration_with_a_cost():
     winners, best, _ = mpc.mpc_iteration(b, ud, dt, k, W, 0)
     assert b.launch_count - launches == H * (step_launches + 1) + 3   # controlled steps, rollout costs, gather, seed
     ew, eb = mpc.select_best(built_in, k)
-    assert np.array_equal(winners, ew) and np.array_equal(_bits(best), _bits(eb))
+    assert np.array_equal(winners, ew) and np.array_equal(bits(best), bits(eb))
     b.close()
-
-
-def _code(excinfo):
-    return int(re.search(r"failed \((-?\d+)\)", str(excinfo.value)).group(1))
 
 
 @gpu
@@ -360,10 +333,10 @@ def test_bad_cost_arguments_are_refused_on_the_host():
     W, H = 8, 3
     scene, kw, _ = _scene("legged20", W)
     dt, n = scene["dt"], scene["n"]
-    b = _batch(scene, **dict(kw, k_max=20))
+    b = batch_on_current_stream(scene, **dict(kw, k_max=20))
     b.step(dt)
-    ud = _cuda(_schedule(scene["f_ext"], H, seed=121))
-    before = _rows(b)
+    ud = cuda(_schedule(scene["f_ext"], H, seed=121))
+    before = state_rows(b)
     f_before = b.static()[2].copy()
     good = _random_cost(n, np.stack([before] * (H + 1)), seed=122)
     b.set_cost(good)
@@ -374,7 +347,7 @@ def test_bad_cost_arguments_are_refused_on_the_host():
     def refused(call, code, what):
         with pytest.raises(EggError) as ei:
             call()
-        assert _code(ei) == code, f"{what}: {ei.value}"
+        assert err_code(ei) == code, f"{what}: {ei.value}"
 
     refused(lambda: b.step_controlled_cost(dt, ud.data_ptr(), H, host.ctypes.data), -1, "host cost_d")
     refused(lambda: b.step_controlled_cost(dt, ud.data_ptr(), H, 0), -1, "NULL cost_d")
@@ -393,8 +366,8 @@ def test_bad_cost_arguments_are_refused_on_the_host():
         refused(lambda: b.step_controlled_cost(dt, ud.data_ptr(), H, cbuf.data_ptr()), -1, f"{R} reference rows")
     b.set_cost(None)
     refused(lambda: b.step_controlled_cost(dt, ud.data_ptr(), H, cbuf.data_ptr()), -4, "no cost")
-    assert np.array_equal(_bits(_rows(b)), _bits(before))
-    assert np.array_equal(_bits(b.static()[2]), _bits(f_before))
+    assert np.array_equal(bits(state_rows(b)), bits(before))
+    assert np.array_equal(bits(b.static()[2]), bits(f_before))
     assert bool((cbuf == 7.0).all())
     b.set_cost(good)   # and an accepted call still runs
     b.step_controlled_cost(dt, ud.data_ptr(), H, cbuf.data_ptr())

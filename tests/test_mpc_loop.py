@@ -2,27 +2,14 @@
 states fetched on the device (egg_gather_state, mpc.gather_winner_states) and every world re-seeded
 from them (egg_seed_state, mpc.mpc_iteration).  The first test runs on CPU ranks (gloo); the rest
 need a CUDA device."""
-import os
-import re
-import socket
-
 import numpy as np
 import pytest
 import torch
-import torch.distributed as dist
-import torch.multiprocessing as mp
 
 from eggshell_b200 import mpc
+from tests.mpc_helpers import batch_on_current_stream, bits, cuda, err_code, run_ranks, state_rows
 
 gpu = pytest.mark.gpu
-
-
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    p = s.getsockname()[1]
-    s.close()
-    return p
 
 
 # ---- CPU: gather_winner_states over 2 gloo ranks ---------------------------------------------------
@@ -47,33 +34,18 @@ def _winner_sets(total):
     ]
 
 
-def _gather_worker(rank, ws, port, q):
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=ws)
+def _gather_worker(rank, ws):
     out = []
     for total in (37, 64):
         lo, _ = mpc.shard_range(total, rank, ws)
         for winners in _winner_sets(total):
             rows = mpc.gather_winner_states(np.array(winners), total, lambda local: torch.from_numpy(_fake_rows(lo + np.asarray(local))))
             out.append((total, winners, rows.numpy().copy()))
-    q.put((rank, out))
-    dist.barrier()
-    dist.destroy_process_group()
+    return out
 
 
 def test_gather_winner_states_gloo_bit_exact():
-    ws = 2
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_gather_worker, args=(r, ws, port, q)) for r in range(ws)]
-    for p in procs:
-        p.start()
-    res = dict(q.get(timeout=120) for _ in range(ws))
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    res = run_ranks(_gather_worker, 2, "gloo", timeout=120)
     assert len(res[0]) == len(res[1]) == 6
     for (total, winners, a), (_, _, b) in zip(res[0], res[1]):
         expect = _fake_rows(winners)
@@ -96,25 +68,6 @@ def test_gather_winner_states_single_process_calls_pack_directly():
 
 
 # ---- GPU ------------------------------------------------------------------------------------------
-def _batch(scene, **kw):
-    """A batch on torch's current stream, so that torch-side buffers and the batch's kernels are ordered."""
-    import eggshell_b200 as E
-    b = E.scenes.make_batch(scene, **kw)
-    b.set_stream(torch.cuda.current_stream().cuda_stream)
-    return b
-
-
-def _state_rows(b):
-    """bodies() as [W, n, 18] rows (p, R row-major, v, w)."""
-    p, R, v, w = b.bodies()
-    W, n = p.shape[:2]
-    return np.concatenate([p, R.reshape(W, n, 9), v, w], axis=-1)
-
-
-def _bits(a):
-    return np.ascontiguousarray(a).view(np.uint64)
-
-
 def _schedule(f_ext, H, seed, sigma=0.05):
     """A time-varying schedule around f_ext: random torques on every body, slice by slice."""
     rng = np.random.default_rng(seed)
@@ -123,23 +76,19 @@ def _schedule(f_ext, H, seed, sigma=0.05):
     return u
 
 
-def _cuda(a):
-    return torch.from_numpy(np.ascontiguousarray(a)).cuda()
-
-
 @gpu
 @pytest.mark.parametrize("name,W", [("pile64", 16), ("legged20", 64)])
 def test_gather_state_matches_bodies(name, W):
     import eggshell_b200 as E
     scene = getattr(E.scenes, name)(W)
-    b = _batch(scene, solver=E.SOLVER_PGS, k_max=50)
+    b = batch_on_current_stream(scene, solver=E.SOLVER_PGS, k_max=50)
     b.step(scene["dt"], n_steps=3)
     rng = np.random.default_rng(11)
     idx = np.concatenate([[0, W - 1], rng.integers(0, W, size=9), [W - 1]])
     out = torch.full((idx.size, scene["n"] * 18), np.nan, dtype=torch.float64, device="cuda")
     b.gather_state(idx, out.data_ptr())
     rows = out.cpu().numpy().reshape(idx.size, scene["n"], 18)
-    assert np.array_equal(_bits(rows), _bits(_state_rows(b)[idx]))
+    assert np.array_equal(bits(rows), bits(state_rows(b)[idx]))
     b.close()
 
 
@@ -149,15 +98,15 @@ def test_seed_state_assigns_source_first_plus_w_mod_k(k, first):
     import eggshell_b200 as E
     W = 16
     scene = E.scenes.legged20(W)
-    b = _batch(scene, solver=E.SOLVER_PGS, k_max=20)
+    b = batch_on_current_stream(scene, solver=E.SOLVER_PGS, k_max=20)
     n = scene["n"]
     rng = np.random.default_rng(100 + k)
     src = rng.normal(size=(k, n, 18))
     src[:, ::3, 4] = -0.0
-    b.seed_state(_cuda(src).data_ptr(), k, first)
-    rows = _state_rows(b)
+    b.seed_state(cuda(src).data_ptr(), k, first)
+    rows = state_rows(b)
     for w in range(W):
-        assert np.array_equal(_bits(rows[w]), _bits(src[(first + w) % k])), f"world {w}"
+        assert np.array_equal(bits(rows[w]), bits(src[(first + w) % k])), f"world {w}"
     b.close()
 
 
@@ -169,7 +118,7 @@ def test_seeded_batch_steps_like_a_fresh_batch():
     W = 8
     scene = E.scenes.legged20(W)
     kw = dict(solver=E.SOLVER_PGS, k_max=100)
-    b = _batch(scene, **kw)
+    b = batch_on_current_stream(scene, **kw)
     b.step(scene["dt"], n_steps=4)
     winners = np.array([5, 2, 7])
     states = torch.empty((3, scene["n"] * 18), dtype=torch.float64, device="cuda")
@@ -178,10 +127,10 @@ def test_seeded_batch_steps_like_a_fresh_batch():
     p, R, v, w = [x.copy() for x in b.bodies()]
     b.step(scene["dt"])
     fresh_scene = dict(scene, p=p, R=R, v=v, w=w)
-    fb = _batch(fresh_scene, **kw)
+    fb = batch_on_current_stream(fresh_scene, **kw)
     fb.step(scene["dt"])
     for a, c in zip(b.bodies(), fb.bodies()):
-        assert np.array_equal(_bits(a), _bits(c))
+        assert np.array_equal(bits(a), bits(c))
     assert np.array_equal(b.status()["n_contacts"], fb.status()["n_contacts"])
     b.close()
     fb.close()
@@ -196,16 +145,16 @@ def test_constant_schedule_equals_step(name):
         scene, kw, H = E.scenes.legged20(16), dict(solver=E.SOLVER_PGS, k_max=100), 6
     else:
         scene, kw, H = E.scenes.chain(4, links=10, seed=3, anchor_jitter=0.1, v_jitter=0.2), dict(solver=E.SOLVER_DENSE_MURTY), 4
-    b = _batch(scene, **kw)
+    b = batch_on_current_stream(scene, **kw)
     b.snapshot()
     b.step(scene["dt"], n_steps=H)
     ref = [x.copy() for x in b.bodies()]
     f_ext = b.static()[2]
     b.restore()
-    u = _cuda(np.broadcast_to(f_ext, (H,) + f_ext.shape))
+    u = cuda(np.broadcast_to(f_ext, (H,) + f_ext.shape))
     b.step_controlled(scene["dt"], u.data_ptr(), H)
     for a, c in zip(b.bodies(), ref):
-        assert np.array_equal(_bits(a), _bits(c))
+        assert np.array_equal(bits(a), bits(c))
     b.close()
 
 
@@ -214,7 +163,7 @@ def test_time_varying_schedule_equals_host_loop():
     import eggshell_b200 as E
     W, H = 16, 5
     scene = E.scenes.legged20(W)
-    b = _batch(scene, solver=E.SOLVER_PGS, k_max=100)
+    b = batch_on_current_stream(scene, solver=E.SOLVER_PGS, k_max=100)
     b.snapshot()
     u = _schedule(scene["f_ext"], H, seed=21)
     for t in range(H):
@@ -224,13 +173,13 @@ def test_time_varying_schedule_equals_host_loop():
     b.set_external(scene["f_ext"])
     b.restore()
     launches = b.launch_count
-    ud = _cuda(u)
+    ud = cuda(u)
     b.step_controlled(scene["dt"], ud.data_ptr(), H)
     step_launches = 5   # collide, three assembly kernels, solve (PGS group stream)
     assert b.launch_count - launches == H * (step_launches + 1)
     for a, c in zip(b.bodies(), ref):
-        assert np.array_equal(_bits(a), _bits(c))
-    assert np.array_equal(_bits(b.static()[2]), _bits(u[-1])), "the f_ext slot holds the last slice"
+        assert np.array_equal(bits(a), bits(c))
+    assert np.array_equal(bits(b.static()[2]), bits(u[-1])), "the f_ext slot holds the last slice"
     b.close()
 
 
@@ -241,10 +190,10 @@ def test_time_varying_schedule_matches_oracle():
     from tests.helpers import oracle_world, compare_step
     W, H = 4, 3
     scene = E.scenes.legged20(W)
-    b = _batch(scene, solver=E.SOLVER_PGS, k_max=100, taps=True)
+    b = batch_on_current_stream(scene, solver=E.SOLVER_PGS, k_max=100, taps=True)
     ows = [oracle_world(scene, wi, solver=1, k_max=100)[0] for wi in range(W)]
     u = _schedule(scene["f_ext"], H, seed=31, sigma=0.2)
-    ud = _cuda(u)
+    ud = cuda(u)
     for t in range(H):
         p, R, v, w = b.bodies()
         for wi, ow in enumerate(ows):
@@ -263,9 +212,9 @@ def test_rollout_costs_match_numpy():
     import eggshell_b200 as E
     W = 64
     scene = E.scenes.legged20(W)
-    b = _batch(scene, solver=E.SOLVER_PGS, k_max=100)
+    b = batch_on_current_stream(scene, solver=E.SOLVER_PGS, k_max=100)
     p0 = b.bodies()[0]
-    b.step_controlled(scene["dt"], _cuda(_schedule(scene["f_ext"], 8, seed=41, sigma=1.0)).data_ptr(), 8)
+    b.step_controlled(scene["dt"], cuda(_schedule(scene["f_ext"], 8, seed=41, sigma=1.0)).data_ptr(), 8)
     costs = torch.empty(W, dtype=torch.float64, device="cuda")
     b.rollout_costs(costs.data_ptr())
     c = costs.cpu().numpy()
@@ -278,10 +227,6 @@ def test_rollout_costs_match_numpy():
     b.close()
 
 
-def _code(excinfo):
-    return int(re.search(r"failed \((-?\d+)\)", str(excinfo.value)).group(1))
-
-
 @gpu
 def test_bad_arguments_are_refused_on_the_host():
     import eggshell_b200 as E
@@ -289,17 +234,18 @@ def test_bad_arguments_are_refused_on_the_host():
     W = 8
     scene = E.scenes.legged20(W)
     n, dt = scene["n"], scene["dt"]
-    b = _batch(scene, solver=E.SOLVER_PGS, k_max=20)
+    b = batch_on_current_stream(scene, solver=E.SOLVER_PGS, k_max=20)
     b.step(dt)
     before = [x.copy() for x in b.bodies()]
     f_before = b.static()[2].copy()
     host = np.zeros((W + 1) * n * 18 * 4)
     dbuf = torch.full((W + 1, n * 18), 7.0, dtype=torch.float64, device="cuda")
-    useq = _cuda(np.broadcast_to(scene["f_ext"], (2, W, n, 6)))
+    useq = cuda(np.broadcast_to(scene["f_ext"], (2, W, n, 6)))
     calls = [
         lambda: b.seed_state(host.ctypes.data, 1),
         lambda: b.gather_state([0], host.ctypes.data),
         lambda: b.step_controlled(dt, host.ctypes.data, 1),
+        lambda: b.rollout_costs(host.ctypes.data),
         lambda: b.seed_state(dbuf.data_ptr(), 0),
         lambda: b.gather_state([], dbuf.data_ptr()),
         lambda: b.seed_state(dbuf.data_ptr(), W + 1),
@@ -313,13 +259,13 @@ def test_bad_arguments_are_refused_on_the_host():
     for i, call in enumerate(calls):
         with pytest.raises(EggError) as ei:
             call()
-        assert _code(ei) == -1, f"call {i}: {ei.value}"
+        assert err_code(ei) == -1, f"call {i}: {ei.value}"
     with pytest.raises(EggError) as ei:
         b.step_controlled(dt, useq.data_ptr(), 1, integrator=EXPLICIT_EULER)
-    assert _code(ei) == -5
+    assert err_code(ei) == -5
     for a, c in zip(b.bodies(), before):
-        assert np.array_equal(_bits(a), _bits(c))
-    assert np.array_equal(_bits(b.static()[2]), _bits(f_before))
+        assert np.array_equal(bits(a), bits(c))
+    assert np.array_equal(bits(b.static()[2]), bits(f_before))
     assert bool((dbuf == 7.0).all())
     b.close()
     # before egg_init
@@ -329,7 +275,7 @@ def test_bad_arguments_are_refused_on_the_host():
                  lambda: raw.step_controlled(dt, useq.data_ptr(), 1)):
         with pytest.raises(EggError) as ei:
             call()
-        assert _code(ei) == -4
+        assert err_code(ei) == -4
     raw.close()
 
 
@@ -338,17 +284,17 @@ def test_mpc_iteration_checks_its_schedule():
     import eggshell_b200 as E
     W = 8
     scene = E.scenes.legged20(W)
-    b = _batch(scene, solver=E.SOLVER_PGS, k_max=20)
+    b = batch_on_current_stream(scene, solver=E.SOLVER_PGS, k_max=20)
     b.snapshot()
-    good = _cuda(np.broadcast_to(scene["f_ext"], (2, W, scene["n"], 6)))
+    good = cuda(np.broadcast_to(scene["f_ext"], (2, W, scene["n"], 6)))
     for bad in (good.float(), good.cpu(), good[:, :W - 1].contiguous(), good.transpose(0, 1), good[0]):
         with pytest.raises(ValueError):
             mpc.mpc_iteration(b, bad, scene["dt"], 2, W, 0)
     winners, costs, states = mpc.mpc_iteration(b, good, scene["dt"], 2, W, 0)
     assert len(winners) == 2 and states.shape == (2, scene["n"] * 18)
-    rows = _state_rows(b)
+    rows = state_rows(b)
     for w in range(W):
-        assert np.array_equal(_bits(rows[w].ravel()), _bits(states[w % 2].cpu().numpy()))
+        assert np.array_equal(bits(rows[w].ravel()), bits(states[w % 2].cpu().numpy()))
     b.close()
 
 
@@ -376,45 +322,26 @@ def _run_iterations(rank, ws):
     import eggshell_b200 as E
     scene, u = _two_gpu_inputs()
     lo, hi = mpc.shard_range(TOTAL, rank, ws)
-    b = _batch(_shard(scene, lo, hi), solver=E.SOLVER_PGS, k_max=20, device=rank)
+    b = batch_on_current_stream(_shard(scene, lo, hi), solver=E.SOLVER_PGS, k_max=20, device=rank)
     b.snapshot()
     out = {}
     for it in range(ITERS):
-        winners, costs, _ = mpc.mpc_iteration(b, _cuda(u[it, :, lo:hi]), scene["dt"], K2, TOTAL, lo)
+        winners, costs, _ = mpc.mpc_iteration(b, cuda(u[it, :, lo:hi]), scene["dt"], K2, TOTAL, lo)
         out[f"winners{it}"], out[f"costs{it}"] = np.asarray(winners), np.asarray(costs)
-    out["state"] = _state_rows(b)
+    out["state"] = state_rows(b)
     b.close()
     return out
 
 
-def _nccl_worker(rank, ws, port, path):
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    torch.cuda.set_device(rank)
-    dist.init_process_group("nccl", rank=rank, world_size=ws, device_id=torch.device("cuda", rank))
-    out = _run_iterations(rank, ws)
-    np.savez(os.path.join(path, f"rank{rank}.npz"), **out)
-    dist.barrier()
-    dist.destroy_process_group()
-
-
 @gpu
 @pytest.mark.skipif(not torch.cuda.is_available() or torch.cuda.device_count() < 2, reason="needs 2 GPUs")
-def test_two_ranks_equal_one_rank(tmp_path):
+def test_two_ranks_equal_one_rank():
     ws = 2
-    ctx = mp.get_context("spawn")
-    port = _free_port()
-    procs = [ctx.Process(target=_nccl_worker, args=(r, ws, port, str(tmp_path))) for r in range(ws)]
-    for p in procs:
-        p.start()
-    for p in procs:
-        p.join(timeout=600)
-        assert p.exitcode == 0
-    ranks = [dict(np.load(os.path.join(tmp_path, f"rank{r}.npz"))) for r in range(ws)]
+    ranks = run_ranks(_run_iterations, ws, "nccl", timeout=600)
     one = _run_iterations(0, 1)
     for it in range(ITERS):
         for key in (f"winners{it}", f"costs{it}"):
             for r in range(ws):
                 assert np.array_equal(ranks[r][key].view(np.uint64), one[key].view(np.uint64)), f"rank {r} {key}"
     state2 = np.concatenate([ranks[r]["state"] for r in range(ws)])
-    assert np.array_equal(_bits(state2), _bits(one["state"]))
+    assert np.array_equal(bits(state2), bits(one["state"]))

@@ -2,59 +2,17 @@
 nominal schedule), egg_mppi_reduce (the cost-weighted sum) and mpc.MPPI, mppi_iteration and
 mppi_advance.  The first tests run on the CPU; the rest need a CUDA device."""
 import ctypes as C
-import os
-import re
-import socket
 
 import numpy as np
 import pytest
 import torch
 
 from eggshell_b200 import mpc
+from tests.mpc_helpers import (ZERO_G_PGS, batch_on_current_stream, bits, boxes, clamp, costs_of, cuda, err_code, noise,
+                               philox4x32_10, reach_cost, run_ranks, state_rows)
 
 gpu = pytest.mark.gpu
 S, U = mpc.STATE_PER_BODY, mpc.CONTROL_PER_BODY
-M32 = np.uint64(0xffffffff)
-
-
-# ---- the numpy definition of the noise ------------------------------------------------------------
-def philox4x32_10(ctr, key):
-    """Philox4x32-10 (Salmon et al., SC'11) on arrays: ctr [4, ...], key [2, ...] of uint32 values.
-    Returns the four output words as uint64 arrays holding uint32 values."""
-    c = [np.asarray(x, dtype=np.uint64) & M32 for x in ctr]
-    k = [np.asarray(x, dtype=np.uint64) & M32 for x in key]
-    for r in range(10):
-        p0 = np.uint64(0xD2511F53) * c[0]
-        p1 = np.uint64(0xCD9E8D57) * c[2]
-        c = [((p1 >> np.uint64(32)) ^ c[1] ^ k[0]) & M32, p1 & M32, ((p0 >> np.uint64(32)) ^ c[3] ^ k[1]) & M32, p0 & M32]
-        k = [(k[0] + np.uint64(0x9E3779B9)) & M32, (k[1] + np.uint64(0xBB67AE85)) & M32]
-    return c
-
-
-def _u01(lo, hi):
-    x = (hi << np.uint64(32)) | lo
-    return (x >> np.uint64(11)).astype(np.float64) * 2.0 ** -53 + 2.0 ** -54
-
-
-def noise(H, n, g, seed, iteration):
-    """eps [H, len(g), n, 6] of the global worlds g, as egg_sample_controls defines it."""
-    t, w, b, p = np.meshgrid(np.arange(H), np.arange(len(g)), np.arange(n), np.arange(3), indexing="ij")
-    q = ((t * n + b) * 3 + p).astype(np.uint64)
-    gg = np.asarray(g, dtype=np.uint64)[w]
-    c = philox4x32_10([q, gg, np.uint64(iteration & 0xffffffff), np.uint64(iteration >> 32)],
-                      [np.uint64(seed & 0xffffffff), np.uint64(seed >> 32)])
-    u1, u2 = _u01(c[0], c[1]), _u01(c[2], c[3])
-    r = np.sqrt(-2.0 * np.log(u1))
-    eps = np.stack([r * np.cos(2 * np.pi * u2), r * np.sin(2 * np.pi * u2)], axis=-1)   # [H, W, n, 3, 2]
-    return eps.reshape(H, len(g), n, 6)
-
-
-def _clamp(v, lo, hi):
-    return np.where(v < lo, lo, np.where(v > hi, hi, v))
-
-
-def _bits(a):
-    return np.ascontiguousarray(a).view(np.uint64)
 
 
 # ---- CPU ------------------------------------------------------------------------------------------
@@ -94,75 +52,24 @@ def test_mppi_validates_and_broadcasts():
             mpc.MPPI(n, H, sigma=1.0, lam=1.0, device="cpu")
 
 
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    p = s.getsockname()[1]
-    s.close()
-    return p
-
-
 def _partials(rank, L=37):
     """Per-rank partial sums whose rank-order sum rounds differently from other orders."""
     rng = np.random.default_rng(100 + rank)
     return rng.normal(size=L) * 10.0 ** rng.integers(-8, 8, size=L)
 
 
-def _gloo_worker(rank, ws, port, q):
-    import torch.distributed as dist
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=ws)
-    total = mpc.allgather_rank_sum(torch.from_numpy(_partials(rank)))
-    q.put((rank, total.numpy().copy()))
-    dist.barrier()
-    dist.destroy_process_group()
+def _gloo_worker(rank, ws):
+    return mpc.allgather_rank_sum(torch.from_numpy(_partials(rank))).numpy().copy()
 
 
 def test_rank_order_combine_gloo():
-    import torch.multiprocessing as mp
-    ws = 2
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_gloo_worker, args=(r, ws, port, q)) for r in range(ws)]
-    for p in procs:
-        p.start()
-    res = dict(q.get(timeout=120) for _ in range(ws))
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    res = run_ranks(_gloo_worker, 2, "gloo", timeout=120)
     expect = _partials(0) + _partials(1)
-    assert np.array_equal(_bits(res[0]), _bits(res[1]))
-    assert np.array_equal(_bits(res[0]), _bits(expect))
+    assert np.array_equal(bits(res[0]), bits(res[1]))
+    assert np.array_equal(bits(res[0]), bits(expect))
 
 
 # ---- GPU ------------------------------------------------------------------------------------------
-def _boxes(W, n, seed=0, dt=0.05):
-    """n unit-mass boxes per world in zero gravity, 2 m apart and 10 m above the ground (no contacts)."""
-    import eggshell_b200 as E
-    s = E.scenes._base(W, n)
-    rng = np.random.default_rng(seed)
-    s["p"][:, :, 0] = 2.0 * np.arange(n)
-    s["p"][:, :, 2] = 10.0
-    s["p"] += rng.uniform(-0.1, 0.1, size=s["p"].shape)
-    s.update(dt=dt, name=f"boxes{n}")
-    return s
-
-
-def _batch(scene, **kw):
-    """A batch on torch's current stream, so that torch-side buffers and the batch's kernels are ordered."""
-    import eggshell_b200 as E
-    kw = dict(dict(solver=E.SOLVER_PGS, gravity=(0.0, 0.0, 0.0)), **kw)
-    b = E.scenes.make_batch(scene, **kw)
-    b.set_stream(torch.cuda.current_stream().cuda_stream)
-    return b
-
-
-def _cuda(a):
-    return torch.from_numpy(np.ascontiguousarray(a)).cuda()
-
-
 def _sample(b, m, first=0, iteration=None, seed=None):
     u = torch.full((m.horizon, b.W, b.n, U), np.nan, dtype=torch.float64, device="cuda")
     b.sample_controls(m.u_nom.data_ptr(), m.horizon, m.seed if seed is None else seed,
@@ -181,7 +88,7 @@ def _planner(n, H, seed=7, **kw):
 @gpu
 def test_sampler_matches_numpy():
     W, n, H, first = 300, 3, 3, 1000
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     m = _planner(n, H)
     m.iteration = 2 ** 32 + 5   # both counter words of the iteration in use
     b.set_sampler(m)
@@ -197,7 +104,7 @@ def test_sampler_matches_numpy():
 @gpu
 def test_sampler_exact_cases():
     W, n, H = 256, 2, 3
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     rng = np.random.default_rng(3)
     lo, hi = rng.uniform(-1.5, -0.5, size=(n, U)), rng.uniform(0.5, 1.5, size=(n, U))
     lo[0, 0], hi[1, 5] = -np.inf, np.inf
@@ -206,41 +113,41 @@ def test_sampler_exact_cases():
     m = _planner(n, H, u_nom=un, u_lo=lo, u_hi=hi, sigma=rng.uniform(0.5, 2.0, size=(n, U)))
     b.set_sampler(m)
     u = _sample(b, m)
-    c_nom = _clamp(un, lo, hi)
-    assert np.array_equal(_bits(u[:, 0]), _bits(c_nom)), "global world 0 runs clamp(u_nom)"
+    c_nom = clamp(un, lo, hi)
+    assert np.array_equal(bits(u[:, 0]), bits(c_nom)), "global world 0 runs clamp(u_nom)"
     assert (u >= lo).all() and (u <= hi).all()
     at_lo, at_hi = u == lo, u == hi
     assert at_lo.sum() > 100 and at_hi.sum() > 100   # bounds reached, and hit exactly
     eps = noise(H, n, np.arange(W), m.seed, m.iteration)
-    free = _clamp(un[:, None] + m.sigma * eps, lo, hi)
+    free = clamp(un[:, None] + m.sigma * eps, lo, hi)
     assert np.array_equal(at_lo[:, 1:], (free == lo)[:, 1:]) and np.array_equal(at_hi[:, 1:], (free == hi)[:, 1:])
-    assert np.array_equal(_bits(_sample(b, m)), _bits(u)), "two calls"
+    assert np.array_equal(bits(_sample(b, m)), bits(u)), "two calls"
     for kw in (dict(iteration=1), dict(seed=m.seed + 1)):
         v = _sample(b, m, **kw)
-        assert np.array_equal(_bits(v[:, 0]), _bits(c_nom))
+        assert np.array_equal(bits(v[:, 0]), bits(c_nom))
         inside = (u > lo) & (u < hi) & (v > lo) & (v < hi)
         inside[:, 0] = False
         assert inside.sum() > 1000 and (v[inside] != u[inside]).all(), kw
     # sigma = 0: clamp(u_nom) in every world, bit for bit (-0.0 included)
     m0 = mpc.MPPI(n, H, sigma=0.0, lam=1.0, u_nom=un, u_lo=lo, u_hi=hi)
     b.set_sampler(m0)
-    assert np.array_equal(_bits(_sample(b, m0)), _bits(np.broadcast_to(c_nom[:, None], (H, W, n, U))))
+    assert np.array_equal(bits(_sample(b, m0)), bits(np.broadcast_to(c_nom[:, None], (H, W, n, U))))
     # one batch of W against two batches of W / 2 with first = 0 and first = W / 2
     b.set_sampler(m)
     halves = []
     for lo_w in (0, W // 2):
-        h = _batch(_boxes(W // 2, n))
+        h = batch_on_current_stream(boxes(W // 2, n), defaults=ZERO_G_PGS)
         h.set_sampler(m)
         halves.append(_sample(h, m, first=lo_w))
         h.close()
-    assert np.array_equal(_bits(np.concatenate(halves, axis=1)), _bits(u))
+    assert np.array_equal(bits(np.concatenate(halves, axis=1)), bits(u))
     b.close()
 
 
 @gpu
 def test_noise_moments():
     W, n, H = 30000, 2, 3   # 1.08e6 samples
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     m = mpc.MPPI(n, H, sigma=1.0, lam=1.0, seed=99)
     b.set_sampler(m)
     eps = _sample(b, m)[:, 1:]
@@ -266,49 +173,39 @@ def _reduce_numpy(u, cost, baseline, lam):
 @gpu
 def test_reduce_matches_numpy():
     W, n, H = 1000, 3, 4   # 4 chunks, the last one partial
-    b = _batch(_boxes(W, n))
+    b = batch_on_current_stream(boxes(W, n), defaults=ZERO_G_PGS)
     rng = np.random.default_rng(11)
     u = rng.normal(0.0, 1.0, size=(H, W, n, U))
     cost = rng.uniform(0.0, 3.0, size=W)
     cost[[5, 17, 300, 999]] = [np.nan, np.inf, -np.inf, np.nan]
     base = np.min(cost[np.isfinite(cost)])
-    ud, cd, bd = _cuda(u), _cuda(cost), _cuda(np.array(base))
+    ud, cd, bd = cuda(u), cuda(cost), cuda(np.array(base))
     lam = 0.7
     got = _reduce(b, ud, H, cd, bd, lam)
     s, so, so2, sabs, om = _reduce_numpy(u, cost, base, lam)
     L = H * n * U
     assert np.all(np.abs(got[:L] - s.ravel()) <= 1e-12 * sabs.ravel())
     assert abs(got[L] - so) <= 1e-12 * so and abs(got[L + 1] - so2) <= 1e-12 * so2
-    assert np.array_equal(_bits(_reduce(b, ud, H, cd, bd, lam)), _bits(got)), "two calls"
+    assert np.array_equal(bits(_reduce(b, ud, H, cd, bd, lam)), bits(got)), "two calls"
     # the non-finite costs get weight 0: the same result as dropping those worlds' schedules
     keep = np.isfinite(cost)
     u0 = u.copy()
     u0[:, ~keep] = np.nan
-    assert np.array_equal(_bits(_reduce(b, _cuda(u0), H, cd, bd, lam)), _bits(got))
+    assert np.array_equal(bits(_reduce(b, cuda(u0), H, cd, bd, lam)), bits(got))
     # NaN-only costs, and a non-finite baseline: every weight is 0
-    nan = _cuda(np.full(W, np.nan))
-    assert not _reduce(b, ud, H, nan, _cuda(np.array(np.inf)), lam).any()
-    assert not _reduce(b, ud, H, cd, _cuda(np.array(np.nan)), lam).any()
+    nan = cuda(np.full(W, np.nan))
+    assert not _reduce(b, ud, H, nan, cuda(np.array(np.inf)), lam).any()
+    assert not _reduce(b, ud, H, cd, cuda(np.array(np.nan)), lam).any()
     # a huge lambda: the plain mean; a tiny one with one clearly best world: that world's schedule
-    fin = _cuda(rng.uniform(0.0, 3.0, size=W))
-    got = _reduce(b, ud, H, fin, _cuda(np.array(0.0)), 1e300)
+    fin = cuda(rng.uniform(0.0, 3.0, size=W))
+    got = _reduce(b, ud, H, fin, cuda(np.array(0.0)), 1e300)
     assert got[L] == W and got[L + 1] == W
     assert np.all(np.abs(got[:L] / W - u.mean(axis=1).ravel()) <= 1e-12 * np.abs(u).mean(axis=1).ravel())
     one = np.ones(W)
     one[417] = 0.0
-    got = _reduce(b, ud, H, _cuda(one), _cuda(np.array(0.0)), 1e-3)
-    assert got[L] == 1.0 and np.array_equal(_bits(got[:L]), _bits(u[:, 417].ravel()))
+    got = _reduce(b, ud, H, cuda(one), cuda(np.array(0.0)), 1e-3)
+    assert got[L] == 1.0 and np.array_equal(bits(got[:L]), bits(u[:, 417].ravel()))
     b.close()
-
-
-def _code(excinfo):
-    return int(re.search(r"failed \((-?\d+)\)", str(excinfo.value)).group(1))
-
-
-def _rows(b):
-    p, R, v, w = b.bodies()
-    W, n = p.shape[:2]
-    return np.concatenate([p, R.reshape(W, n, 9), v, w], axis=-1)
 
 
 @gpu
@@ -316,10 +213,10 @@ def test_bad_arguments_are_refused_on_the_host():
     import eggshell_b200 as E
     from eggshell_b200.batch import EggError, EggSampler, _p
     W, n, H = 64, 2, 3
-    scene = _boxes(W, n)
-    b = _batch(scene)
+    scene = boxes(W, n)
+    b = batch_on_current_stream(scene, defaults=ZERO_G_PGS)
     b.step(scene["dt"])
-    before = _rows(b)
+    before = state_rows(b)
     m = _planner(n, H)
     u = torch.full((H, W, n, U), 7.0, dtype=torch.float64, device="cuda")
     out = torch.full((H * n * U + 2,), 7.0, dtype=torch.float64, device="cuda")
@@ -332,7 +229,7 @@ def test_bad_arguments_are_refused_on_the_host():
     def refused(call, code, what):
         with pytest.raises(EggError) as ei:
             call()
-        assert _code(ei) == code, f"{what}: {ei.value}"
+        assert err_code(ei) == code, f"{what}: {ei.value}"
 
     refused(lambda: b.sample_controls(m.u_nom.data_ptr(), H, 1, 0, 0, u.data_ptr()), -4, "no sampler")
     base_bytes = b.device_bytes
@@ -361,7 +258,7 @@ def test_bad_arguments_are_refused_on_the_host():
     assert b.device_bytes - base_bytes == 3 * n * U * 8
     assert b.launch_count == launches
     assert bool((u == 7.0).all()) and bool((out == 7.0).all())
-    assert np.array_equal(_bits(_rows(b)), _bits(before))
+    assert np.array_equal(bits(state_rows(b)), bits(before))
     ref = noise(H, n, np.arange(W), m.seed, 0)   # the sampler in place still samples with m's sigma
     got = _sample(b, m, iteration=0)
     assert np.max(np.abs((got - m.u_nom.cpu().numpy()[:, None]) / m.sigma - ref)[:, 1:]) <= 1e-13
@@ -378,35 +275,19 @@ def test_bad_arguments_are_refused_on_the_host():
     assert bool((u == 7.0).all()) and bool((out == 7.0).all())
 
 
-def _reach_cost(x0, target):
-    """Terminal cost |p - target|^2 of the single body."""
-    q_term = np.zeros((1, S))
-    q_term[0, 0:3] = 1.0
-    x_ref = x0.copy()
-    x_ref[0, 0:3] = target
-    return mpc.QuadraticCost(1, q_term=q_term, x_ref=x_ref)
-
-
-def _costs_of(b, u, H, dt):
-    c = torch.empty(b.W, dtype=torch.float64, device="cuda")
-    b.restore()
-    b.step_controlled_cost(dt, u.data_ptr(), H, c.data_ptr())
-    return c.cpu().numpy()
-
-
 @gpu
 def test_mppi_lowers_the_cost_of_a_reaching_task():
     """One box in zero gravity, far from the ground, pushed by force controls towards a target 1.2 m
     away within H steps; the terminal cost is the squared distance to the target."""
     W, H = 1024, 10
-    scene = _boxes(W, 1, seed=5)
+    scene = boxes(W, 1, seed=5)
     for key in ("p", "R", "v", "w"):
         scene[key] = np.broadcast_to(scene[key][:1], scene[key].shape).copy()
     dt = scene["dt"]
-    b = _batch(scene)
+    b = batch_on_current_stream(scene, defaults=ZERO_G_PGS)
     b.snapshot()
-    x0 = _rows(b)[0]
-    b.set_cost(_reach_cost(x0, x0[0, 0:3] + [1.0, -0.5, 0.5]))
+    x0 = state_rows(b)[0]
+    b.set_cost(reach_cost(x0, x0[0, 0:3] + [1.0, -0.5, 0.5]))
     m = mpc.MPPI(1, H, sigma=[4.0, 4.0, 4.0, 0.0, 0.0, 0.0], lam=0.05, u_lo=-20.0, u_hi=20.0, seed=2024)
     b.set_sampler(m)
     u = torch.empty((H, W, 1, U), dtype=torch.float64, device="cuda")
@@ -423,9 +304,9 @@ def test_mppi_lowers_the_cost_of_a_reaching_task():
         old = m.u_nom.clone()
         r = mpc.mppi_iteration(b, m, dt, u, 0)
         ub = u.cpu().numpy()
-        J = _costs_of(b, u, H, dt)
+        J = costs_of(b, u, H, dt)
         assert r["min_cost"] == J.min() and r["nominal_cost"] == J[0]
-        assert np.array_equal(_bits(ub[:, 0]), _bits(m.clamp(old).cpu().numpy()))
+        assert np.array_equal(bits(ub[:, 0]), bits(m.clamp(old).cpu().numpy()))
         s, so, so2, sabs, _ = _reduce_numpy(ub, J, J.min(), m.lam)
         expect = np.clip(s / so, -20.0, 20.0)
         got = m.u_nom.cpu().numpy()
@@ -442,11 +323,11 @@ def test_mppi_lowers_the_cost_of_a_reaching_task():
 def test_mppi_iteration_raises_without_a_finite_rollout():
     """A cost whose every rollout overflows to inf: sum omega = 0, u_nom and iteration unchanged."""
     W, H = 64, 3
-    scene = _boxes(W, 1)
+    scene = boxes(W, 1)
     dt = scene["dt"]
-    b = _batch(scene)
+    b = batch_on_current_stream(scene, defaults=ZERO_G_PGS)
     b.snapshot()
-    x0 = _rows(b)[0]
+    x0 = state_rows(b)[0]
     b.set_cost(mpc.QuadraticCost(1, q_term=1e308, x_ref=x0 + 10.0))
     m = _planner(1, H)
     b.set_sampler(m)
@@ -455,7 +336,7 @@ def test_mppi_iteration_raises_without_a_finite_rollout():
     with pytest.raises(RuntimeError, match="weights sum to 0"):
         mpc.mppi_iteration(b, m, dt, u, 0)
     assert torch.equal(m.u_nom, old) and m.iteration == 0
-    assert np.isinf(_costs_of(b, u, H, dt)).all()
+    assert np.isinf(costs_of(b, u, H, dt)).all()
     # the checks of mpc_iteration, and the planner's own
     with pytest.raises(ValueError):
         mpc.mppi_iteration(b, m, dt, u[:2].contiguous(), 0)
@@ -486,45 +367,34 @@ def test_mppi_advance_steps_every_world_from_the_plan():
     mpc.mppi_iteration(b, m, dt, u, 0)
     plan = m.u_nom.cpu().numpy()
     executed, start = mpc.mppi_advance(b, m, dt, W)
-    c0 = _clamp(plan[0], -0.3, 0.3)
-    assert np.array_equal(_bits(executed.cpu().numpy()), _bits(c0))
+    c0 = clamp(plan[0], -0.3, 0.3)
+    assert np.array_equal(bits(executed.cpu().numpy()), bits(c0))
     fresh = E.scenes.make_batch(scene, **kw)
     fresh.set_external(np.broadcast_to(c0, (W, n, U)))
     fresh.step(dt, 1)
-    expect = _rows(fresh)[0]
+    expect = state_rows(fresh)[0]
     fresh.close()
-    assert np.array_equal(_bits(_rows(b)), _bits(np.broadcast_to(expect, (W, n, S))))
-    assert np.array_equal(_bits(start.cpu().numpy()), _bits(expect))
+    assert np.array_equal(bits(state_rows(b)), bits(np.broadcast_to(expect, (W, n, S))))
+    assert np.array_equal(bits(start.cpu().numpy()), bits(expect))
     b.restore()   # the new start is the snapshot
-    assert np.array_equal(_bits(_rows(b)), _bits(np.broadcast_to(expect, (W, n, S))))
+    assert np.array_equal(bits(state_rows(b)), bits(np.broadcast_to(expect, (W, n, S))))
     got = m.u_nom.cpu().numpy()
-    assert np.array_equal(_bits(got[:-1]), _bits(plan[1:])) and np.array_equal(_bits(got[-1]), _bits(plan[-1]))
+    assert np.array_equal(bits(got[:-1]), bits(plan[1:])) and np.array_equal(bits(got[-1]), bits(plan[-1]))
     b.close()
 
 
-def _nccl_worker(rank, ws, port, W, H, iters, q):
-    import torch.distributed as dist
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    torch.cuda.set_device(rank)
-    dist.init_process_group("nccl", rank=rank, world_size=ws, device_id=torch.device("cuda", rank))
-    q.put((rank, _run_planner(W, H, iters, rank, ws)))
-    dist.barrier()
-    dist.destroy_process_group()
-
-
-def _run_planner(W, H, iters, rank, ws):
+def _run_planner(rank, ws, W, H, iters):
     """`iters` MPPI iterations of the reaching task on this rank's shard of W worlds; returns the
     first iteration's samples of the shard and every iteration's u_nom."""
     lo, hi = mpc.shard_range(W, rank, ws)
-    scene = _boxes(W, 1, seed=5)
+    scene = boxes(W, 1, seed=5)
     for key in ("p", "R", "v", "w", "m", "I"):
         scene[key] = np.broadcast_to(scene[key][:1], scene[key].shape)[lo:hi].copy()
     scene["W"] = hi - lo
-    b = _batch(scene, device=torch.cuda.current_device())
+    b = batch_on_current_stream(scene, defaults=ZERO_G_PGS, device=torch.cuda.current_device())
     b.snapshot()
-    x0 = _rows(b)[0]
-    b.set_cost(_reach_cost(x0, x0[0, 0:3] + [1.0, -0.5, 0.5]))
+    x0 = state_rows(b)[0]
+    b.set_cost(reach_cost(x0, x0[0, 0:3] + [1.0, -0.5, 0.5]))
     m = mpc.MPPI(1, H, sigma=[4.0, 4.0, 4.0, 0.0, 0.0, 0.0], lam=0.05, seed=77)
     b.set_sampler(m)
     u = torch.empty((H, hi - lo, 1, U), dtype=torch.float64, device=torch.device("cuda", torch.cuda.current_device()))
@@ -542,19 +412,9 @@ def _run_planner(W, H, iters, rank, ws):
 def test_one_rank_against_two_nccl_ranks():
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
-    import torch.multiprocessing as mp
     W, H, iters = 512, 6, 3
-    one_samples, one_plans = _run_planner(W, H, iters, 0, 1)
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_nccl_worker, args=(r, 2, port, W, H, iters, q)) for r in range(2)]
-    for p in procs:
-        p.start()
-    res = dict(q.get(timeout=300) for _ in range(2))
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
-    assert np.array_equal(_bits(np.concatenate([res[0][0], res[1][0]], axis=1)), _bits(one_samples))
-    assert np.array_equal(_bits(res[0][1]), _bits(res[1][1])), "every rank holds the same plan"
+    one_samples, one_plans = _run_planner(0, 1, W, H, iters)
+    res = run_ranks(_run_planner, 2, "nccl", W, H, iters, timeout=300)
+    assert np.array_equal(bits(np.concatenate([res[0][0], res[1][0]], axis=1)), bits(one_samples))
+    assert np.array_equal(bits(res[0][1]), bits(res[1][1])), "every rank holds the same plan"
     assert np.max(np.abs(res[0][1] - one_plans)) <= 1e-12 * max(1.0, np.abs(one_plans).max())
