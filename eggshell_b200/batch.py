@@ -23,7 +23,7 @@ ST_LCP_FAILED, ST_JOINT_CONFLICT, ST_BAD_INIT, ST_CONTACT_OVERFLOW, ST_NONFINITE
 EXPORTS = [
     "egg_desc_default", "egg_create", "egg_destroy", "egg_set_bodies", "egg_set_shapes", "egg_set_state", "egg_set_joints",
     "egg_set_external", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_step_controlled",
-    "egg_set_cost", "egg_step_controlled_cost", "egg_set_sampler", "egg_sample_controls", "egg_mppi_reduce", "egg_sample_controls_std", "egg_gather_controls", "egg_control_moments", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
+    "egg_set_cost", "egg_step_controlled_cost", "egg_set_actuators", "egg_set_sampler", "egg_sample_controls", "egg_mppi_reduce", "egg_sample_controls_std", "egg_gather_controls", "egg_control_moments", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
     "egg_get_status", "egg_get_dense_work", "egg_get_debug_counters", "egg_rollout_costs", "egg_set_stream", "egg_sync", "egg_device_bytes",
     "egg_launch_count", "egg_capacity", "egg_get_kernel_config", "egg_set_profiling", "egg_get_kernel_ms", "egg_fp64_peak_tflops", "egg_host_alloc", "egg_host_free", "egg_last_error", "egg_version",
 ]
@@ -48,6 +48,10 @@ class EggCost(C.Structure):
 
 class EggSampler(C.Structure):
     _fields_ = [("sigma", C.c_void_p), ("u_lo", C.c_void_p), ("u_hi", C.c_void_p)]
+
+
+class EggActuators(C.Structure):
+    _fields_ = [("m", C.c_int), ("body", C.c_void_p), ("reaction", C.c_void_p), ("frame", C.c_void_p), ("axis", C.c_void_p)]
 
 
 class EggError(RuntimeError):
@@ -82,6 +86,7 @@ def lib():
         L.egg_gather_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.egg_seed_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
         L.egg_set_sampler.argtypes = [C.c_void_p, C.c_void_p]
+        L.egg_set_actuators.argtypes = [C.c_void_p, C.c_void_p]
         L.egg_sample_controls.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_ulonglong, C.c_ulonglong, C.c_int, C.c_void_p]
         L.egg_mppi_reduce.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
         L.egg_sample_controls_std.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_ulonglong, C.c_ulonglong, C.c_int,
@@ -149,6 +154,7 @@ class Batch:
         self.stream = None   # cudaStream_t handed to set_stream; None = the batch's own stream
         self.cost = None     # mpc.QuadraticCost handed to set_cost
         self.sampler = None  # mpc.MPPI or mpc.CEM handed to set_sampler
+        self.actuators = None  # mpc.Actuators handed to set_actuators; None = body wrenches
         self.max_contacts = None
         self._probe_capacity()
 
@@ -225,19 +231,46 @@ class Batch:
 
     def step_controlled(self, dt, u_ptr, horizon, integrator=OPEN_DYNAMICS_ENGINE):
         """`horizon` steps; before step t the f_ext slot takes slice t of the device schedule at u_ptr,
-        float64 [horizon][W][n][6] (egg_step_controlled)."""
+        float64 [horizon][W][n][6] (egg_step_controlled), or with an actuator table [horizon][W][m] and
+        the slot takes the wrench the table defines."""
         _chk(lib().egg_step_controlled(self.h, C.c_double(dt), int(integrator), C.c_void_p(u_ptr), int(horizon)),
              "egg_step_controlled")
 
+    # -- control space ------------------------------------------------------------------------
+    @property
+    def control_shape(self):
+        """The shape of one world's control row: (n, 6) body wrenches, or (m,) with an actuator table."""
+        return (self.n, 6) if self.actuators is None else (self.actuators.m,)
+
+    def set_actuators(self, act):
+        """Makes the batch's control row the m values of an mpc.Actuators table for this batch's n
+        bodies, or with None the (n, 6) body wrenches again (egg_set_actuators).  Refused while a
+        sampler or a cost is set.  Synchronises the batch stream."""
+        from .mpc import Actuators
+        if act is None:
+            _chk(lib().egg_set_actuators(self.h, None), "egg_set_actuators")
+        else:
+            if not isinstance(act, Actuators) or act.n != self.n:
+                raise ValueError(f"set_actuators takes an mpc.Actuators for n = {self.n} bodies, or None")
+            a = EggActuators(act.m, _p(act.body), _p(act.reaction), _p(act.frame), _p(act.axis))
+            _chk(lib().egg_set_actuators(self.h, C.byref(a)), "egg_set_actuators")
+        self.actuators = act
+
+    def _check_control_shape(self, what, obj):
+        if obj.control_shape != self.control_shape:
+            raise ValueError(f"{what}: the batch's control rows are {self.control_shape}, the {type(obj).__name__}'s "
+                             f"{obj.control_shape}")
+
     def set_cost(self, cost):
-        """Configures the cost of step_controlled_cost: an mpc.QuadraticCost for this batch's n bodies,
-        or None to clear it (egg_set_cost).  Synchronises the batch stream."""
+        """Configures the cost of step_controlled_cost: an mpc.QuadraticCost for this batch's n bodies
+        and control shape, or None to clear it (egg_set_cost).  Synchronises the batch stream."""
         from .mpc import QuadraticCost
         if cost is None:
             _chk(lib().egg_set_cost(self.h, None), "egg_set_cost")
         else:
             if not isinstance(cost, QuadraticCost) or cost.n != self.n:
                 raise ValueError(f"set_cost takes an mpc.QuadraticCost for n = {self.n} bodies, or None")
+            self._check_control_shape("set_cost", cost)
             c = EggCost(_p(cost.q_run), _p(cost.l_run), _p(cost.u_run), _p(cost.q_term), _p(cost.l_term),
                         _p(cost.x_ref), cost.ref_steps)
             _chk(lib().egg_set_cost(self.h, C.byref(c)), "egg_set_cost")
@@ -260,6 +293,7 @@ class Batch:
         else:
             if not isinstance(mppi, (MPPI, CEM)) or mppi.n != self.n:
                 raise ValueError(f"set_sampler takes an mpc.MPPI or mpc.CEM for n = {self.n} bodies, or None")
+            self._check_control_shape("set_sampler", mppi)
             s = EggSampler(_p(mppi.sigma), _p(mppi.u_lo), _p(mppi.u_hi))
             _chk(lib().egg_set_sampler(self.h, C.byref(s)), "egg_set_sampler")
         self.sampler = mppi

@@ -81,6 +81,11 @@ struct egg_batch {
   EggSampler sampler = {};       // pointers into sampler_buf
   double* mppi_partial = nullptr;  // stage-1 partials of egg_mppi_reduce, grown on demand
   size_t mppi_partial_count = 0;
+  int* act_ibuf = nullptr;       // egg_set_actuators: body, reaction, frame [m], CSR start [n + 1], list; null = body wrenches
+  size_t act_icount = 0;
+  double* act_dbuf = nullptr;    // ... and axis [m][3]
+  size_t act_dcount = 0;
+  EggAct act = {};               // pointers into act_ibuf / act_dbuf; act.m = 0 without a table
   bool profiling = false;
   std::vector<cudaEvent_t> ev;   // 4 per profiled step
   std::vector<cudaEvent_t> ev_free;
@@ -109,17 +114,18 @@ static int dfree(egg_batch* b, void* p, size_t bytes) {
   return EGG_OK;
 }
 #define RET(x) do { int r__ = (x); if (r__ != EGG_OK) return r__; } while (0)
-// Replaces the batch-owned buffer buf of count doubles with a new one of new_count doubles (none if 0),
-// filled from host if given.  The new buffer is in place before the old one goes, so a failed
+// Replaces the batch-owned buffer buf of count elements with a new one of new_count elements (none if
+// 0), filled from host if given.  The new buffer is in place before the old one goes, so a failed
 // allocation keeps the old buffer; the stream is synchronised before the old one is freed.
-static int replace_dbuf(egg_batch* b, double*& buf, size_t& count, size_t new_count, const double* host) {
-  double* q = nullptr;
+template <class T>
+static int replace_dbuf(egg_batch* b, T*& buf, size_t& count, size_t new_count, const T* host) {
+  T* q = nullptr;
   if (new_count) {
     RET(dalloc(b, &q, new_count));
-    if (host) CK(cudaMemcpyAsync(q, host, new_count * sizeof(double), cudaMemcpyHostToDevice, b->stream));
+    if (host) CK(cudaMemcpyAsync(q, host, new_count * sizeof(T), cudaMemcpyHostToDevice, b->stream));
   }
   CK(cudaStreamSynchronize(b->stream));   // host may be a temporary
-  if (buf) RET(dfree(b, buf, count * sizeof(double)));
+  if (buf) RET(dfree(b, buf, count * sizeof(T)));
   buf = q;
   count = new_count;
   return EGG_OK;
@@ -626,10 +632,13 @@ static int enter(egg_batch* b, const char* what, InitCheck init, std::initialize
   return EGG_OK;
 }
 
-// n_steps x Ensemble::Step.  With a control schedule u_d ([n_steps][W][n][6]), slice s is copied into
-// the f_ext slot before step s (outside the profiled kernel buckets).  With cost_d as well, that copy
-// is the kernel that also adds the running cost of step s to cost_d, and the terminal cost follows
-// the last step.
+// The width of a control row per world: m actuator values with an actuator table, else 6 n.
+static int ctrl_width(const egg_batch* b) { return b->act.m ? b->act.m : 6 * b->dev.n; }
+
+// n_steps x Ensemble::Step.  With a control schedule u_d ([n_steps][W][c]), slice s is copied into
+// the f_ext slot before step s (outside the profiled kernel buckets); with an actuator table the
+// actuation kernel writes the slot from the actuator values instead.  With cost_d as well, that
+// kernel also adds the running cost of step s to cost_d, and the terminal cost follows the last step.
 static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d, double* cost_d) {
   const int solver = b->dev.prm.solver;
   if (solver < EGG_SOLVER_DENSE_MURTY || solver > EGG_SOLVER_SOR) { g_err = "unknown solver"; return EGG_ERR_ARG; }
@@ -643,10 +652,11 @@ static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d, do
     b->iso_known = true;
     b->dev.rmax = egg_runs_rmax(b->dev);   // run format of the PGS stream for isotropic bodies, else one block per lane and stage
   }
-  const size_t slice = (size_t)b->dev.W * b->dev.n * 6;
+  const size_t slice = (size_t)b->dev.W * ctrl_width(b);
   for (int s = 0; s < n_steps; s++) {
     if (u_d) {
-      if (cost_d) CK(egg_launch_fext_slice_cost(b->dev, u_d + (size_t)s * slice, b->cost, s, cost_d, b->stream));
+      if (b->act.m) CK(egg_launch_actuate(b->dev, b->act, u_d + (size_t)s * slice, cost_d ? &b->cost : nullptr, s, cost_d, b->stream));
+      else if (cost_d) CK(egg_launch_fext_slice_cost(b->dev, u_d + (size_t)s * slice, b->cost, s, cost_d, b->stream));
       else CK(egg_launch_fext_slice(b->dev, u_d + (size_t)s * slice, b->stream));
       b->launches++;
     }
@@ -730,18 +740,21 @@ static bool to_component_major(const double* src, size_t rows, size_t n, size_t 
 
 int egg_set_cost(egg_batch* b, const egg_cost* c) {
   if (!b) return EGG_ERR_ARG;
-  const size_t n = (size_t)b->dev.n, nd = (size_t)EGG_DYN * n;
-  std::vector<double> h;   // the EggCost layout: q_run, l_run, q_term, l_term [18][n], u_run [6][n], x_ref [R][18][n]
+  const size_t n = (size_t)b->dev.n, nd = (size_t)EGG_DYN * n, cu = (size_t)ctrl_width(b);
+  // the EggCost layout: q_run, l_run, q_term, l_term [18][n], u_run [6][n] (or [m] with an actuator table), x_ref [R][18][n]
+  std::vector<double> h;
   int R = 1;
   if (c) {
     if (c->x_ref) R = c->ref_steps;
     if (R < 1) { g_err = "egg_set_cost: ref_steps must be >= 1"; return EGG_ERR_ARG; }
-    h.assign(4 * nd + 6 * n + (size_t)R * nd, 0.0);
-    struct { const double* src; size_t rows, comps, off; } part[6] = {
-        {c->q_run, 1, EGG_DYN, 0}, {c->l_run, 1, EGG_DYN, nd}, {c->q_term, 1, EGG_DYN, 2 * nd},
-        {c->l_term, 1, EGG_DYN, 3 * nd}, {c->u_run, 1, 6, 4 * nd}, {c->x_ref, (size_t)R, EGG_DYN, 4 * nd + 6 * n}};
+    h.assign(4 * nd + cu + (size_t)R * nd, 0.0);
+    const bool act = b->act.m > 0;
+    struct { const double* src; size_t rows, n, comps, off; } part[6] = {
+        {c->q_run, 1, n, EGG_DYN, 0}, {c->l_run, 1, n, EGG_DYN, nd}, {c->q_term, 1, n, EGG_DYN, 2 * nd},
+        {c->l_term, 1, n, EGG_DYN, 3 * nd}, {c->u_run, 1, act ? cu : n, act ? 1 : (size_t)6, 4 * nd},
+        {c->x_ref, (size_t)R, n, EGG_DYN, 4 * nd + cu}};
     for (auto& p : part)
-      if (p.src && !to_component_major(p.src, p.rows, n, p.comps, &h[p.off])) {
+      if (p.src && !to_component_major(p.src, p.rows, p.n, p.comps, &h[p.off])) {
         g_err = "egg_set_cost: non-finite weight or reference value";
         return EGG_ERR_ARG;
       }
@@ -749,22 +762,22 @@ int egg_set_cost(egg_batch* b, const egg_cost* c) {
   CK(cudaSetDevice(b->device));
   RET(replace_dbuf(b, b->cost_buf, b->cost_count, h.size(), h.data()));
   const double* q = b->cost_buf;
-  b->cost = c ? EggCost{q, q + nd, q + 4 * nd, q + 2 * nd, q + 3 * nd, q + 4 * nd + 6 * n, R} : EggCost{};
+  b->cost = c ? EggCost{q, q + nd, q + 4 * nd, q + 2 * nd, q + 3 * nd, q + 4 * nd + cu, R} : EggCost{};
   return EGG_OK;
 }
 
 int egg_set_sampler(egg_batch* b, const egg_sampler* s) {
   if (!b) return EGG_ERR_ARG;
-  const size_t n = (size_t)b->dev.n, nc = 6 * n;
-  std::vector<double> h;   // the EggSampler layout: sigma, lo, hi, each [6][n]
+  const size_t nc = (size_t)ctrl_width(b);
+  std::vector<double> h;   // the EggSampler layout: sigma, lo, hi, each one control row [c] as the host gives it
   if (s) {
     if (!s->sigma) { g_err = "egg_set_sampler: sigma is required"; return EGG_ERR_ARG; }
     const double inf = std::numeric_limits<double>::infinity();
     h.assign(3 * nc, inf);   // without bounds: lo = -inf, hi = +inf
     std::fill(h.begin() + nc, h.begin() + 2 * nc, -inf);
-    const bool finite = to_component_major(s->sigma, 1, n, 6, &h[0]);
-    if (s->u_lo) to_component_major(s->u_lo, 1, n, 6, &h[nc], false);
-    if (s->u_hi) to_component_major(s->u_hi, 1, n, 6, &h[2 * nc], false);
+    const bool finite = to_component_major(s->sigma, 1, nc, 1, &h[0]);
+    if (s->u_lo) std::copy(s->u_lo, s->u_lo + nc, h.begin() + nc);
+    if (s->u_hi) std::copy(s->u_hi, s->u_hi + nc, h.begin() + 2 * nc);
     for (size_t k = 0; k < nc; k++) {
       const double lo = h[nc + k], hi = h[2 * nc + k];
       if (!finite || h[k] < 0) { g_err = "egg_set_sampler: sigma must be finite and >= 0"; return EGG_ERR_ARG; }
@@ -779,6 +792,67 @@ int egg_set_sampler(egg_batch* b, const egg_sampler* s) {
   return EGG_OK;
 }
 
+int egg_set_actuators(egg_batch* b, const egg_actuators* a) {
+  if (!b) return EGG_ERR_ARG;
+  if (b->sampler_buf || b->cost_buf) {
+    g_err = "egg_set_actuators while a sampler or a cost is set: their control rows have the width of the current control space; "
+            "clear them first";
+    return EGG_ERR_STATE;
+  }
+  const int n = b->dev.n;
+  std::vector<int> hi;      // body, reaction, frame [m], start [n + 1], list
+  std::vector<double> hd;   // axis [m][3]
+  int m = 0;
+  if (a) {
+    m = a->m;
+    if (m < 1 || m > INT_MAX / 8) { g_err = "egg_set_actuators: m must be in [1, INT_MAX / 8]"; return EGG_ERR_ARG; }
+    if (!a->body || !a->reaction || !a->frame || !a->axis) { g_err = "egg_set_actuators: NULL array"; return EGG_ERR_ARG; }
+    std::vector<int> cnt((size_t)n + 1, 0);
+    for (int k = 0; k < m; k++) {
+      const int bo = a->body[k], re = a->reaction[k], fr = a->frame[k];
+      const double* ax = a->axis + 3 * (size_t)k;
+      if (bo < 0 || bo >= n) { g_err = "egg_set_actuators: body out of range"; return EGG_ERR_ARG; }
+      if (re < -1 || re >= n || re == bo) { g_err = "egg_set_actuators: reaction must be -1 or another body"; return EGG_ERR_ARG; }
+      if (fr != -1 && fr != bo && fr != re) { g_err = "egg_set_actuators: frame must be -1, body or reaction"; return EGG_ERR_ARG; }
+      if (!std::isfinite(ax[0]) || !std::isfinite(ax[1]) || !std::isfinite(ax[2]) || (ax[0] == 0 && ax[1] == 0 && ax[2] == 0)) {
+        g_err = "egg_set_actuators: an axis must be finite and not zero";
+        return EGG_ERR_ARG;
+      }
+      cnt[bo + 1]++;
+      if (re >= 0) cnt[re + 1]++;
+    }
+    for (int k = 0; k < n; k++) cnt[k + 1] += cnt[k];   // CSR start
+    const size_t nnz = (size_t)cnt[n];
+    hi.assign(3 * (size_t)m + (size_t)n + 1 + nnz, 0);
+    std::copy(a->body, a->body + m, hi.begin());
+    std::copy(a->reaction, a->reaction + m, hi.begin() + m);
+    std::copy(a->frame, a->frame + m, hi.begin() + 2 * (size_t)m);
+    std::copy(cnt.begin(), cnt.end(), hi.begin() + 3 * (size_t)m);
+    int* list = hi.data() + 3 * (size_t)m + n + 1;
+    for (int k = 0; k < m; k++) {   // in actuator order: every body's list is in actuator order
+      list[cnt[a->body[k]]++] = k;
+      if (a->reaction[k] >= 0) list[cnt[a->reaction[k]]++] = ~k;
+    }
+    hd.assign(a->axis, a->axis + 3 * (size_t)m);
+  }
+  CK(cudaSetDevice(b->device));
+  // both new buffers are in place before the old ones go: a failed allocation keeps the old table
+  int* qi = nullptr;
+  double* qd = nullptr;
+  size_t ni = 0, nd = 0;
+  int r = replace_dbuf(b, qi, ni, hi.size(), hi.data());
+  if (r == EGG_OK) r = replace_dbuf(b, qd, nd, hd.size(), hd.data());
+  if (r != EGG_OK) {
+    if (qi) dfree(b, qi, ni * sizeof(int));
+    return r;
+  }
+  RET(replace_dbuf<int>(b, b->act_ibuf, b->act_icount, 0, nullptr));
+  RET(replace_dbuf<double>(b, b->act_dbuf, b->act_dcount, 0, nullptr));
+  b->act_ibuf = qi, b->act_icount = ni, b->act_dbuf = qd, b->act_dcount = nd;
+  b->act = a ? EggAct{m, qi, qi + m, qi + 2 * m, qd, qi + 3 * m, qi + 3 * m + n + 1} : EggAct{};
+  return EGG_OK;
+}
+
 // egg_sample_controls (std_d null: the sampler's sigma per body) and egg_sample_controls_std; ptrs
 // names the entry point's device arguments.
 static int sample_controls(egg_batch* b, const char* what, std::initializer_list<DevArg> ptrs, const double* mean_d, const double* std_d,
@@ -787,7 +861,7 @@ static int sample_controls(egg_batch* b, const char* what, std::initializer_list
   if (horizon < 1 || first < 0) { g_err = std::string(what) + ": horizon must be >= 1 and first >= 0"; return EGG_ERR_ARG; }
   RET(enter(b, what, INIT_LAST, ptrs, true));
   if (!b->sampler_buf) { g_err = std::string(what) + " without a sampler: call egg_set_sampler first"; return EGG_ERR_STATE; }
-  CK(egg_launch_sample(b->dev, b->sampler, mean_d, std_d, horizon, seed, iteration, first, u_d, b->stream));
+  CK(egg_launch_sample(b->dev, ctrl_width(b), b->sampler, mean_d, std_d, horizon, seed, iteration, first, u_d, b->stream));
   b->launches++;
   return EGG_OK;
 }
@@ -823,10 +897,10 @@ int egg_gather_controls(egg_batch* b, const double* u_d, int horizon, const int*
   if (!b || !worlds) return EGG_ERR_ARG;
   if (horizon < 1) { g_err = "egg_gather_controls: horizon must be >= 1"; return EGG_ERR_ARG; }
   RET(check_worlds(b, "egg_gather_controls", worlds, k));
-  if ((long long)k * horizon * b->dev.n * 6 > 256ll * INT_MAX) { g_err = "egg_gather_controls: too many rows"; return EGG_ERR_ARG; }
+  if ((long long)k * horizon * ctrl_width(b) > 256ll * INT_MAX) { g_err = "egg_gather_controls: too many rows"; return EGG_ERR_ARG; }
   RET(enter(b, "egg_gather_controls", INIT_LAST, {{u_d, "u_d"}, {out_d, "out_d"}}));
   RET(upload_worlds(b, worlds, k));
-  CK(egg_launch_gather_controls(b->dev, u_d, horizon, b->gather_idx, k, out_d, b->stream));
+  CK(egg_launch_gather_controls(b->dev, ctrl_width(b), u_d, horizon, b->gather_idx, k, out_d, b->stream));
   b->launches++;
   return EGG_OK;
 }
@@ -834,7 +908,7 @@ int egg_gather_controls(egg_batch* b, const double* u_d, int horizon, const int*
 int egg_control_moments(egg_batch* b, const double* rows_d, int k, int horizon, double* out_d) {
   if (!b) return EGG_ERR_ARG;
   if (k < 1 || horizon < 1) { g_err = "egg_control_moments: k and horizon must be >= 1"; return EGG_ERR_ARG; }
-  const long long L = (long long)horizon * b->dev.n * 6;
+  const long long L = (long long)horizon * ctrl_width(b);
   if (L > INT_MAX) { g_err = "egg_control_moments: too long a horizon"; return EGG_ERR_ARG; }
   RET(enter(b, "egg_control_moments", INIT_LAST, {{rows_d, "rows_d"}, {out_d, "out_d"}}));
   CK(egg_launch_control_moments(rows_d, k, (int)L, out_d, b->stream));
@@ -848,12 +922,12 @@ int egg_mppi_reduce(egg_batch* b, const double* u_d, int horizon, const double* 
   if (!(lambda > 0) || !std::isfinite(lambda)) { g_err = "egg_mppi_reduce: lambda must be finite and > 0"; return EGG_ERR_ARG; }
   if (horizon < 1) { g_err = "egg_mppi_reduce: horizon must be >= 1"; return EGG_ERR_ARG; }
   const int chunks = egg_mppi_chunks(b->dev.W);
-  const long long cols = (long long)horizon * b->dev.n * 6 + 2;
+  const long long cols = (long long)horizon * ctrl_width(b) + 2;
   if (chunks > 65535 || cols > INT_MAX) { g_err = "egg_mppi_reduce: too many worlds or too long a horizon"; return EGG_ERR_ARG; }
   RET(enter(b, "egg_mppi_reduce", INIT_LAST, {{u_d, "u_d"}, {cost_d, "cost_d"}, {baseline_d, "baseline_d"}, {out_d, "out_d"}}));
   const size_t need = (size_t)chunks * (size_t)cols;
-  if (need > b->mppi_partial_count) RET(replace_dbuf(b, b->mppi_partial, b->mppi_partial_count, need, nullptr));
-  CK(egg_launch_mppi_reduce(b->dev, u_d, horizon, cost_d, baseline_d, lambda, b->mppi_partial, out_d, b->stream));
+  if (need > b->mppi_partial_count) RET(replace_dbuf<double>(b, b->mppi_partial, b->mppi_partial_count, need, nullptr));
+  CK(egg_launch_mppi_reduce(b->dev, ctrl_width(b), u_d, horizon, cost_d, baseline_d, lambda, b->mppi_partial, out_d, b->stream));
   b->launches += 2;
   return EGG_OK;
 }

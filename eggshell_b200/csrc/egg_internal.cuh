@@ -184,7 +184,7 @@ cudaError_t egg_launch_seed_state(const EggDev& d, const double* in, int k, int 
 struct EggCost {
   const double* q_run;    // [18][n]
   const double* l_run;    // [18][n]
-  const double* u_run;    // [6][n]
+  const double* u_run;    // [6][n], or [m] with an actuator table
   const double* q_term;   // [18][n]
   const double* l_term;   // [18][n]
   const double* x_ref;    // [ref_steps][18][n]
@@ -194,24 +194,42 @@ struct EggCost {
 // the terminal term at x_horizon is added after the last step
 cudaError_t egg_launch_fext_slice_cost(const EggDev& d, const double* u, const EggCost& c, int t, double* cost, cudaStream_t s);
 cudaError_t egg_launch_cost_terminal(const EggDev& d, const EggCost& c, int horizon, double* cost, cudaStream_t s);
-// Device copy of egg_set_sampler: sigma, u_lo, u_hi, each component-major [6][n] (+-inf for no bound).
+// Device copy of egg_set_actuators, shared by all worlds.  start / list: per body b, the actuators
+// that touch it in actuator order, list[start[b] .. start[b + 1]), a for +tau (b = body[a]) and ~a
+// for -tau (b = reaction[a]).
+struct EggAct {
+  int m;
+  const int* body;        // [m]
+  const int* reaction;    // [m], -1 = none
+  const int* frame;       // [m], -1 = world
+  const double* axis;     // [m][3]
+  const int* start;       // [n + 1]
+  const int* list;        // [start[n]]
+};
+// Actuator mode: one control row u [W][m] (device) -> the f_ext slot of stat, m g plus the actuator
+// torques; with c (not null) the running cost of step t as egg_launch_fext_slice_cost adds it, the
+// control term sum_a u_run[a] u_a^2 (c->u_run is [m]).
+cudaError_t egg_launch_actuate(const EggDev& d, const EggAct& a, const double* u, const EggCost* c, int t, double* cost, cudaStream_t s);
+// Device copy of egg_set_sampler: sigma, u_lo, u_hi, each one control row [c] (+-inf for no bound);
+// c = 6 n ([n][6]) with body wrenches, m with an actuator table.
 struct EggSampler {
   const double* sigma;
   const double* lo;
   const double* hi;
 };
-// Sampling (egg_sample_controls, egg_sample_controls_std): u [H][W][n][6] <- clamp(mean [H][n][6] + sigma eps)
-// with sm.sigma per body, or with the per-step std_dev [H][n][6] in its place when std_dev is not null.
-cudaError_t egg_launch_sample(const EggDev& d, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
+// Sampling (egg_sample_controls, egg_sample_controls_std): u [H][W][c] <- clamp(mean [H][c] + sigma eps)
+// with sm.sigma per element of the row, or with the per-step std_dev [H][c] in its place when std_dev
+// is not null.  c is the control row width.
+cudaError_t egg_launch_sample(const EggDev& d, int c, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
                               unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s);
-// MPPI (egg_mppi_reduce): out [H n 6 + 2] <- sum_w omega_w u[t][w], sum omega, sum omega^2 through
-// partial [chunks][H n 6 + 2]
-int egg_mppi_chunks(int W);   // stage-1 chunks of egg_launch_mppi_reduce: partial holds chunks x (H n 6 + 2) doubles
-cudaError_t egg_launch_mppi_reduce(const EggDev& d, const double* u, int horizon, const double* cost, const double* baseline,
+// MPPI (egg_mppi_reduce): out [H c + 2] <- sum_w omega_w u[t][w], sum omega, sum omega^2 through
+// partial [chunks][H c + 2]
+int egg_mppi_chunks(int W);   // stage-1 chunks of egg_launch_mppi_reduce: partial holds chunks x (H c + 2) doubles
+cudaError_t egg_launch_mppi_reduce(const EggDev& d, int c, const double* u, int horizon, const double* cost, const double* baseline,
                                    double lambda, double* partial, double* out, cudaStream_t s);
-// CEM (egg_gather_controls, egg_control_moments): out [k][H][n][6] <- u[t][worlds[i]];
+// CEM (egg_gather_controls, egg_control_moments): out [k][H][c] <- u[t][worlds[i]];
 // out [2][L] <- mean and population std of the columns of rows [k][L]
-cudaError_t egg_launch_gather_controls(const EggDev& d, const double* u, int horizon, const int* worlds, int k, double* out,
+cudaError_t egg_launch_gather_controls(const EggDev& d, int c, const double* u, int horizon, const int* worlds, int k, double* out,
                                        cudaStream_t s);
 cudaError_t egg_launch_control_moments(const double* rows, int k, int L, double* out, cudaStream_t s);
 // Dynamic shared memory each kernel family needs for this batch shape (checked against the device

@@ -1,7 +1,9 @@
 // MPPI (model predictive path integral): the two data-heavy steps of the sampling planner, next to
 // the step.  egg_sample_controls writes W perturbed copies of a nominal control schedule;
 // egg_mppi_reduce sums them weighted by exp(-(J - J_min) / lambda).  Both touch the whole
-// [H][W][n][6] schedule (6.3 GB at 131072 legged20 worlds and H = 50) and nothing else of size.
+// [H][W][c] schedule and nothing else of size: c = 6 n body-wrench components per world (6.3 GB at
+// 131072 legged20 worlds and H = 50), or m actuator values with an actuator table (57 for the joint
+// motors of legged20: 3.0 GB).  Every kernel here works on rows of either width.
 // CEM (cross-entropy method) shares the sampler with a per-step sigma (egg_sample_controls_std) and
 // refits on the elites: egg_gather_controls copies their schedules, egg_control_moments averages them.
 #include "egg_internal.cuh"
@@ -18,55 +20,75 @@ __device__ __forceinline__ double egg_u01(unsigned lo, unsigned hi) {
 // clamp that lets NaN through (fmin/fmax would replace it by a bound)
 __device__ __forceinline__ double egg_clamp(double v, double lo, double hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
-// Where the sampler kernel reads sigma.sigma from: the sampler's per-body [6][n] array, the same for
-// every step (egg_sample_controls), or the caller's per-step [H][n][6] device array read like u_nom
+// Where the sampler kernel reads sigma.sigma from: the sampler's row [c], the same for every step
+// (egg_sample_controls), or the caller's per-step [H][c] device array read like u_nom
 // (egg_sample_controls_std).  Everything else, the noise included, is the same code.
 enum EggSigmaFrom { EGG_SIGMA_PER_BODY, EGG_SIGMA_PER_STEP };
 
-// One thread per (step, world, body, component pair): i = (w n + b) 3 + p within step t, so thread i
-// writes the two adjacent doubles u[t][w][b][2p, 2p + 1] as one 16-byte store and a warp writes 512
-// consecutive bytes.  The noise is computed for every element whatever sigma is (sigma = 0 costs what
-// sigma > 0 does); global world 0 and sigma = 0 keep u_nom bit for bit (-0.0 included).
-template <EggSigmaFrom kFrom>
-__global__ void __launch_bounds__(256) egg_mppi_sample_kernel(const double* __restrict__ u_nom, EggSampler sm, int W, int n,
+// Two adjacent doubles of a control row: one 16-byte access when the row width c is even (every
+// pair then starts 16-byte aligned), 8-byte ones when it is odd; half: the pair is the last of an odd
+// row and has no second element (read as 0).
+template <bool kOdd>
+__device__ __forceinline__ double2 egg_load2(const double* p, bool half) {
+  if constexpr (kOdd) return make_double2(p[0], half ? 0.0 : p[1]);
+  else return *reinterpret_cast<const double2*>(p);
+}
+
+// One thread per (step, world, component pair) of a control row of width c with P = ceil(c / 2) pairs:
+// i = w P + p within step t, so thread i writes the elements (2p, 2p + 1) of u[t][w] and, for even c,
+// a warp writes 512 consecutive bytes with 16-byte stores.  The Philox counter is q = t P + p; for
+// c = 6 n this is (t n + b) 3 + p' of the body-wrench space (p = 3 b + p').  For odd c the last pair
+// discards its second normal.  The noise is computed for every element whatever sigma is (sigma = 0
+// costs what sigma > 0 does); global world 0 and sigma = 0 keep u_nom bit for bit (-0.0 included).
+template <EggSigmaFrom kFrom, bool kOdd>
+__global__ void __launch_bounds__(256) egg_mppi_sample_kernel(const double* __restrict__ u_nom, EggSampler sm, int W, int c,
                                                               int H, unsigned per_step, uint2 key, uint2 iter, int first,
-                                                              double2* __restrict__ u) {
+                                                              double* __restrict__ u) {
   const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= per_step) return;
-  const unsigned p = i % 3u, r = i / 3u, b = r % (unsigned)n, w = r / (unsigned)n;
+  const unsigned P = ((unsigned)c + 1u) >> 1;
+  const unsigned p = i % P, w = i / P;
   const unsigned g = (unsigned)first + w;
   const int j = 2 * (int)p;
+  const bool half = kOdd && j + 1 == c;
+  const int j1 = half ? j : j + 1;   // the bounds of a missing second element are never used
   double s0 = 0.0, s1 = 0.0;
-  if constexpr (kFrom == EGG_SIGMA_PER_BODY) s0 = sm.sigma[j * n + b], s1 = sm.sigma[(j + 1) * n + b];
-  const double lo0 = sm.lo[j * n + b], lo1 = sm.lo[(j + 1) * n + b];
-  const double hi0 = sm.hi[j * n + b], hi1 = sm.hi[(j + 1) * n + b];
+  if constexpr (kFrom == EGG_SIGMA_PER_BODY) s0 = sm.sigma[j], s1 = sm.sigma[j1];
+  const double lo0 = sm.lo[j], lo1 = sm.lo[j1];
+  const double hi0 = sm.hi[j], hi1 = sm.hi[j1];
   for (int t = blockIdx.y; t < H; t += gridDim.y) {
-    const uint4 c = curand_Philox4x32_10(make_uint4(((unsigned)t * (unsigned)n + b) * 3u + p, g, iter.x, iter.y), key);
-    const double u1 = egg_u01(c.x, c.y), u2 = egg_u01(c.z, c.w);
+    const uint4 r = curand_Philox4x32_10(make_uint4((unsigned)t * P + p, g, iter.x, iter.y), key);
+    const double u1 = egg_u01(r.x, r.y), u2 = egg_u01(r.z, r.w);
     const double rad = sqrt(-2.0 * log(u1));
     double sn, cs;
     sincospi(2.0 * u2, &sn, &cs);
-    const double2 m = *reinterpret_cast<const double2*>(u_nom + ((size_t)t * n + b) * 6 + j);
+    const double2 m = egg_load2<kOdd>(u_nom + (size_t)t * c + j, half);
     if constexpr (kFrom == EGG_SIGMA_PER_STEP) {
-      const double2 sd = *reinterpret_cast<const double2*>(sm.sigma + ((size_t)t * n + b) * 6 + j);
+      const double2 sd = egg_load2<kOdd>(sm.sigma + (size_t)t * c + j, half);
       s0 = sd.x, s1 = sd.y;
     }
     double v0 = m.x + s0 * (rad * cs), v1 = m.y + s1 * (rad * sn);
     if (g == 0 || s0 == 0.0) v0 = m.x;
     if (g == 0 || s1 == 0.0) v1 = m.y;
-    u[(size_t)t * per_step + i] = make_double2(egg_clamp(v0, lo0, hi0), egg_clamp(v1, lo1, hi1));
+    double* out = u + ((size_t)t * W + w) * c + j;
+    if constexpr (kOdd) {
+      out[0] = egg_clamp(v0, lo0, hi0);
+      if (!half) out[1] = egg_clamp(v1, lo1, hi1);
+    } else {
+      *reinterpret_cast<double2*>(out) = make_double2(egg_clamp(v0, lo0, hi0), egg_clamp(v1, lo1, hi1));
+    }
   }
 }
 
 // Worlds per stage-1 partial of the reduction (= the block size of its kernel).
 #define EGG_MPPI_CHUNK 256
 
-// Stage 1: block (x, c) sums the worlds [c CHUNK, (c + 1) CHUNK) of columns x*256 ... of the
-// [H n 6 + 2]-column table (u[t][w] flattened over (t, b, j), then omega, then omega^2), in world
+// Stage 1: block (x, y) sums the worlds [y CHUNK, (y + 1) CHUNK) of columns x*256 ... of the
+// [H c + 2]-column table (u[t][w] flattened over (t, row element), then omega, then omega^2), in world
 // order.  The chunk's weights are computed once into shared memory.  For a fixed world the 256
 // threads read 256 consecutive doubles of u, so the loads are coalesced; each thread walks down its
 // column.  A zero weight contributes exactly nothing (a NaN control of a discarded world included).
-__global__ void __launch_bounds__(EGG_MPPI_CHUNK) egg_mppi_reduce_kernel(const double* __restrict__ u, int W, int n6, int L,
+__global__ void __launch_bounds__(EGG_MPPI_CHUNK) egg_mppi_reduce_kernel(const double* __restrict__ u, int W, int c, int L,
                                                                         const double* __restrict__ cost,
                                                                         const double* __restrict__ baseline, double lambda,
                                                                         double* __restrict__ partial) {
@@ -85,11 +107,11 @@ __global__ void __launch_bounds__(EGG_MPPI_CHUNK) egg_mppi_reduce_kernel(const d
   if (col >= L + 2) return;
   double s = 0.0;
   if (col < L) {
-    const int t = col / n6, e = col - t * n6;
-    const double* x = u + ((size_t)t * W + w0) * n6 + e;
+    const int t = col / c, e = col - t * c;
+    const double* x = u + ((size_t)t * W + w0) * c + e;
 #pragma unroll 8
     for (int k = 0; k < nw; k++) {
-      const double ok = om[k], xk = x[(size_t)k * n6];
+      const double ok = om[k], xk = x[(size_t)k * c];
       s += ok != 0.0 ? ok * xk : 0.0;
     }
   } else if (col == L) {
@@ -132,40 +154,44 @@ __global__ void __launch_bounds__(256) egg_control_moments_kernel(const double* 
   out[L + col] = sqrt(q / k);
 }
 
-// out[i][t][:] = u[t][worlds[i]][:], the n 6 doubles of a step copied as they are (one thread each).
-__global__ void __launch_bounds__(256) egg_gather_controls_kernel(const double* __restrict__ u, int W, int n6, int H,
+// out[i][t][:] = u[t][worlds[i]][:], the c doubles of a step's row copied as they are (one thread each).
+__global__ void __launch_bounds__(256) egg_gather_controls_kernel(const double* __restrict__ u, int W, int c, int H,
                                                                   const int* __restrict__ worlds, int k,
                                                                   double* __restrict__ out) {
   const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (gid >= (long long)k * H * n6) return;
-  const int e = (int)(gid % n6);
-  const long long r = gid / n6;
+  if (gid >= (long long)k * H * c) return;
+  const int e = (int)(gid % c);
+  const long long r = gid / c;
   const int t = (int)(r % H), i = (int)(r / H);
-  out[gid] = u[((size_t)t * W + worlds[i]) * n6 + e];
+  out[gid] = u[((size_t)t * W + worlds[i]) * c + e];
 }
 
-template <EggSigmaFrom kFrom>
-static cudaError_t launch_sample(const EggDev& d, const EggSampler& sm, const double* u_nom, int horizon, unsigned long long seed,
+template <EggSigmaFrom kFrom, bool kOdd>
+static cudaError_t launch_sample(const EggDev& d, int c, const EggSampler& sm, const double* u_nom, int horizon, unsigned long long seed,
                                  unsigned long long iteration, int first, double* u, cudaStream_t s) {
-  const unsigned per_step = (unsigned)d.W * (unsigned)d.n * 3u;
+  const unsigned per_step = (unsigned)d.W * (((unsigned)c + 1u) >> 1);
   const dim3 grid((per_step + 255) / 256, (unsigned)min(horizon, 65535));
-  egg_mppi_sample_kernel<kFrom><<<grid, 256, 0, s>>>(u_nom, sm, d.W, d.n, horizon, per_step,
-                                                     make_uint2((unsigned)seed, (unsigned)(seed >> 32)),
-                                                     make_uint2((unsigned)iteration, (unsigned)(iteration >> 32)), first,
-                                                     reinterpret_cast<double2*>(u));
+  egg_mppi_sample_kernel<kFrom, kOdd><<<grid, 256, 0, s>>>(u_nom, sm, d.W, c, horizon, per_step,
+                                                           make_uint2((unsigned)seed, (unsigned)(seed >> 32)),
+                                                           make_uint2((unsigned)iteration, (unsigned)(iteration >> 32)), first, u);
   return cudaGetLastError();
 }
 
-cudaError_t egg_launch_sample(const EggDev& d, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
+cudaError_t egg_launch_sample(const EggDev& d, int c, const EggSampler& sm, const double* mean, const double* std_dev, int horizon,
                               unsigned long long seed, unsigned long long iteration, int first, double* u, cudaStream_t s) {
-  if (!std_dev) return launch_sample<EGG_SIGMA_PER_BODY>(d, sm, mean, horizon, seed, iteration, first, u, s);
-  return launch_sample<EGG_SIGMA_PER_STEP>(d, EggSampler{std_dev, sm.lo, sm.hi}, mean, horizon, seed, iteration, first, u, s);
+  const EggSampler per_step{std_dev, sm.lo, sm.hi};
+  if (c & 1) {
+    if (!std_dev) return launch_sample<EGG_SIGMA_PER_BODY, true>(d, c, sm, mean, horizon, seed, iteration, first, u, s);
+    return launch_sample<EGG_SIGMA_PER_STEP, true>(d, c, per_step, mean, horizon, seed, iteration, first, u, s);
+  }
+  if (!std_dev) return launch_sample<EGG_SIGMA_PER_BODY, false>(d, c, sm, mean, horizon, seed, iteration, first, u, s);
+  return launch_sample<EGG_SIGMA_PER_STEP, false>(d, c, per_step, mean, horizon, seed, iteration, first, u, s);
 }
 
-cudaError_t egg_launch_gather_controls(const EggDev& d, const double* u, int horizon, const int* worlds, int k, double* out,
+cudaError_t egg_launch_gather_controls(const EggDev& d, int c, const double* u, int horizon, const int* worlds, int k, double* out,
                                        cudaStream_t s) {
-  const long long total = (long long)k * horizon * d.n * 6;
-  egg_gather_controls_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(u, d.W, d.n * 6, horizon, worlds, k, out);
+  const long long total = (long long)k * horizon * c;
+  egg_gather_controls_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(u, d.W, c, horizon, worlds, k, out);
   return cudaGetLastError();
 }
 
@@ -176,11 +202,11 @@ cudaError_t egg_launch_control_moments(const double* rows, int k, int L, double*
 
 int egg_mppi_chunks(int W) { return (W + EGG_MPPI_CHUNK - 1) / EGG_MPPI_CHUNK; }
 
-cudaError_t egg_launch_mppi_reduce(const EggDev& d, const double* u, int horizon, const double* cost, const double* baseline,
+cudaError_t egg_launch_mppi_reduce(const EggDev& d, int c, const double* u, int horizon, const double* cost, const double* baseline,
                                    double lambda, double* partial, double* out, cudaStream_t s) {
-  const int n6 = d.n * 6, L = horizon * n6, chunks = egg_mppi_chunks(d.W);
+  const int L = horizon * c, chunks = egg_mppi_chunks(d.W);
   egg_mppi_reduce_kernel<<<dim3((unsigned)(L + 2 + EGG_MPPI_CHUNK - 1) / EGG_MPPI_CHUNK, (unsigned)chunks), EGG_MPPI_CHUNK, 0, s>>>(
-      u, d.W, n6, L, cost, baseline, lambda, partial);
+      u, d.W, c, L, cost, baseline, lambda, partial);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   egg_mppi_reduce_final_kernel<<<(unsigned)(L + 2 + 255) / 256, 256, 0, s>>>(partial, chunks, L + 2, out);

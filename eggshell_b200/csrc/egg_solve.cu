@@ -225,6 +225,69 @@ __global__ void __launch_bounds__(256, 4) egg_fext_slice_cost_kernel(const doubl
   if (lane == 0) cost[w] = (t == 0) ? s : cost[w] + s;
 }
 
+// Actuator mode (egg_set_actuators): the f_ext slot of every body from a control row u [W][m] of
+// actuator values, f = (m_b g, sum of +-tau_a over the actuators that touch b, in actuator order) with
+// tau_a = u_a k_a, k_a = axis[a] or R(frame[a]) axis[a] from the state x_t.  Every product and sum is
+// rounded on its own (no contraction), so the numpy transcription mpc.Actuators.wrench has the same
+// bits.  One warp per world: lanes take bodies l, l + 32, ... and gather over the body's list, so no
+// atomics.  With kCost the same pass adds the running cost of step t: the state part of
+// egg_fext_slice_cost_kernel over the lane's bodies, then u_run[a] u_a^2 over actuators l, l + 32,
+// ..., then the warp tree, so a world's J has the same bits in any batch.
+template <bool kCost>
+__global__ void __launch_bounds__(256, 4) egg_actuate_kernel(const double* __restrict__ u, int W, int n, double* __restrict__ stat,
+                                                             const double* __restrict__ dyn, const double* __restrict__ bpar,
+                                                             double g0, double g1, double g2, EggAct act, EggCost cc,
+                                                             const double* __restrict__ xr, int t, double* __restrict__ cost) {
+  const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (w >= W) return;   // uniform over the warp
+  const int lane = threadIdx.x & 31;
+  const double* x = dyn + (size_t)w * EGG_DYN * n;
+  const double* uw = u + (size_t)w * act.m;
+  const double* mass = bpar + ((size_t)w * EGG_BPAR + 3) * n;
+  double* f = stat + ((size_t)w * EGG_STAT + 10) * n;
+  double s = 0.0;
+#pragma unroll 1
+  for (int b = lane; b < n; b += 32) {
+    const double mb = mass[b];
+    double tx = 0.0, ty = 0.0, tz = 0.0;
+#pragma unroll 1
+    for (int i = act.start[b]; i < act.start[b + 1]; i++) {
+      const int e = act.list[i], a = e >= 0 ? e : ~e;
+      const int fr = act.frame[a];
+      const double ua = uw[a];
+      double kx = act.axis[3 * a], ky = act.axis[3 * a + 1], kz = act.axis[3 * a + 2];
+      if (fr >= 0) {
+        double R[9];
+#pragma unroll
+        for (int c = 0; c < 9; c++) R[c] = x[(3 + c) * n + fr];
+        const double rx = __dadd_rn(__dadd_rn(__dmul_rn(R[0], kx), __dmul_rn(R[1], ky)), __dmul_rn(R[2], kz));
+        const double ry = __dadd_rn(__dadd_rn(__dmul_rn(R[3], kx), __dmul_rn(R[4], ky)), __dmul_rn(R[5], kz));
+        const double rz = __dadd_rn(__dadd_rn(__dmul_rn(R[6], kx), __dmul_rn(R[7], ky)), __dmul_rn(R[8], kz));
+        kx = rx, ky = ry, kz = rz;
+      }
+      const double ax = __dmul_rn(ua, kx), ay = __dmul_rn(ua, ky), az = __dmul_rn(ua, kz);
+      if (e >= 0) tx = __dadd_rn(tx, ax), ty = __dadd_rn(ty, ay), tz = __dadd_rn(tz, az);
+      else tx = __dsub_rn(tx, ax), ty = __dsub_rn(ty, ay), tz = __dsub_rn(tz, az);
+    }
+    f[0 * n + b] = __dmul_rn(mb, g0);
+    f[1 * n + b] = __dmul_rn(mb, g1);
+    f[2 * n + b] = __dmul_rn(mb, g2);
+    f[3 * n + b] = tx;
+    f[4 * n + b] = ty;
+    f[5 * n + b] = tz;
+    if constexpr (kCost) s += egg_state_cost(x, xr, cc.q_run, cc.l_run, n, b);
+  }
+  if constexpr (kCost) {
+#pragma unroll 1
+    for (int a = lane; a < act.m; a += 32) {
+      const double ua = uw[a];
+      s += cc.u_run[a] * ua * ua;
+    }
+    s = egg_warp_sum(s);
+    if (lane == 0) cost[w] = (t == 0) ? s : cost[w] + s;
+  }
+}
+
 // The terminal term at x_H: cost[w] += sum_b sum_c q_term d^2 + l_term d.
 __global__ void egg_cost_terminal_kernel(int W, int n, const double* __restrict__ dyn, EggCost cc,
                                          const double* __restrict__ xr, double* __restrict__ cost) {
@@ -353,6 +416,17 @@ static const double* cost_ref_row(const EggDev& d, const EggCost& c, int t) {
 cudaError_t egg_launch_fext_slice_cost(const EggDev& d, const double* u, const EggCost& c, int t, double* cost, cudaStream_t s) {
   const long long threads = (long long)d.W * 32;   // one warp per world
   egg_fext_slice_cost_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(u, d.W, d.n, d.stat, d.dyn, c, cost_ref_row(d, c, t), t, cost);
+  return cudaGetLastError();
+}
+cudaError_t egg_launch_actuate(const EggDev& d, const EggAct& a, const double* u, const EggCost* c, int t, double* cost, cudaStream_t s) {
+  const long long threads = (long long)d.W * 32;   // one warp per world
+  const unsigned blocks = (unsigned)((threads + 255) / 256);
+  if (c)
+    egg_actuate_kernel<true><<<blocks, 256, 0, s>>>(u, d.W, d.n, d.stat, d.dyn, d.bpar, d.prm.g[0], d.prm.g[1], d.prm.g[2], a, *c,
+                                                    cost_ref_row(d, *c, t), t, cost);
+  else
+    egg_actuate_kernel<false><<<blocks, 256, 0, s>>>(u, d.W, d.n, d.stat, d.dyn, d.bpar, d.prm.g[0], d.prm.g[1], d.prm.g[2], a,
+                                                     EggCost{}, nullptr, t, nullptr);
   return cudaGetLastError();
 }
 cudaError_t egg_launch_cost_terminal(const EggDev& d, const EggCost& c, int horizon, double* cost, cudaStream_t s) {

@@ -13,6 +13,16 @@ STATE_PER_BODY = 18   # p(3), R(9, row-major), v(3), w(3): a row of egg_gather_s
 CONTROL_PER_BODY = 6  # f(3), tau(3): a row of egg_set_external / a control schedule slice
 
 
+def _control_shape(n, m, owner):
+    """(n, 6) body wrenches for m = None, else (m,) actuator values (m >= 1)."""
+    if m is None:
+        return (n, CONTROL_PER_BODY)
+    m = int(m)
+    if m < 1:
+        raise ValueError(f"{owner}: m must be >= 1")
+    return (m,)
+
+
 def _broadcast(a, shape, owner, name, finite=False):
     """a as a contiguous float64 array of the given shape (numpy broadcasting); the errors name the
     owner class and the argument.  finite: refuse NaN and +-inf as well."""
@@ -26,6 +36,80 @@ def _broadcast(a, shape, owner, name, finite=False):
     return a
 
 
+class Actuators:
+    """An actuator table (Batch.set_actuators, egg_set_actuators): the batch's control row becomes the
+    m actuator values.  Actuator a applies +tau_a to body[a] and -tau_a to reaction[a] (-1: none,
+    else another body), tau_a = u_a k_a with k_a = axis[a] in the world frame (frame[a] = -1) or
+    rotated by R of body frame[a] (body[a] or reaction[a]) in the state before the step.  axis[a] is
+    used as given (its length is the gear ratio): finite and not all zero.  Invalid tables raise
+    ValueError with the rules of the C ABI."""
+
+    def __init__(self, n, body, reaction, frame, axis):
+        n = int(n)
+        if n < 1:
+            raise ValueError("Actuators: n must be >= 1")
+        body, reaction, frame = (np.asarray(x) for x in (body, reaction, frame))
+        for x, name in ((body, "body"), (reaction, "reaction"), (frame, "frame")):
+            if x.ndim != 1 or not (np.issubdtype(x.dtype, np.integer) or x.size == 0):
+                raise ValueError(f"Actuators: {name} must be a 1-D integer array")
+        m = body.size
+        if m < 1:
+            raise ValueError("Actuators: m must be >= 1")
+        if reaction.size != m or frame.size != m:
+            raise ValueError("Actuators: body, reaction and frame must have the same length")
+        axis = np.asarray(axis, dtype=np.float64)
+        if axis.shape != (m, 3):
+            raise ValueError(f"Actuators: axis must be [{m}, 3]")
+        if ((body < 0) | (body >= n)).any():
+            raise ValueError("Actuators: body out of range")
+        if ((reaction < -1) | (reaction >= n) | (reaction == body)).any():
+            raise ValueError("Actuators: reaction must be -1 or another body")
+        if ((frame != -1) & (frame != body) & (frame != reaction)).any():
+            raise ValueError("Actuators: frame must be -1, body or reaction")
+        if not np.isfinite(axis).all() or (axis == 0).all(axis=1).any():
+            raise ValueError("Actuators: an axis must be finite and not zero")
+        self.n, self.m = n, m
+        self.body, self.reaction, self.frame = (np.ascontiguousarray(x, dtype=np.int32) for x in (body, reaction, frame))
+        self.axis = np.ascontiguousarray(axis)
+
+    @classmethod
+    def ball_joint_motors(cls, n, i0, i1):
+        """Three motors per ball joint with unit axes x, y, z: for a joint between bodies i0 and i1 the
+        torque acts on the child i1 and reacts on the parent i0, in the parent's frame; a joint anchored
+        to the world (i1 = -1) gives body i0, no reaction and world axes.  Motor 3 j + k is axis k of
+        joint j."""
+        i0, i1 = np.asarray(i0).ravel(), np.asarray(i1).ravel()
+        body = np.repeat(np.where(i1 >= 0, i1, i0), 3)
+        reaction = np.repeat(np.where(i1 >= 0, i0, -1), 3)
+        frame = reaction.copy()
+        axis = np.tile(np.eye(3), (i0.size, 1))
+        return cls(n, body, reaction, frame, axis)
+
+    def wrench(self, states, a, mass, gravity):
+        """The float64 numpy transcription of the slot egg_set_actuators defines, in the same order:
+        states [..., n, 18] (the state before the step), a [..., m] (actuator values), mass [..., n],
+        gravity [3].  Returns f_ext [..., n, 6]: (m_b g, the actuator torques)."""
+        states, a = np.asarray(states, dtype=np.float64), np.asarray(a, dtype=np.float64)
+        mass, g = np.asarray(mass, dtype=np.float64), np.asarray(gravity, dtype=np.float64)
+        lead = np.broadcast_shapes(states.shape[:-2], a.shape[:-1], mass.shape[:-1])
+        if states.shape[-2:] != (self.n, STATE_PER_BODY) or a.shape[-1] != self.m or mass.shape[-1] != self.n or g.shape != (3,):
+            raise ValueError(f"wrench takes states [..., {self.n}, {STATE_PER_BODY}], a [..., {self.m}], mass [..., {self.n}], gravity [3]")
+        f = np.zeros(lead + (self.n, 6))
+        f[..., :3] = mass[..., None] * g
+        tq = np.zeros(lead + (self.n, 3))
+        for k in range(self.m):
+            ax, fr = self.axis[k], int(self.frame[k])
+            if fr >= 0:
+                R = states[..., fr, 3:12].reshape(states.shape[:-2] + (3, 3))
+                ax = (R[..., :, 0] * ax[0] + R[..., :, 1] * ax[1]) + R[..., :, 2] * ax[2]
+            tau = a[..., k, None] * ax
+            tq[..., self.body[k], :] = tq[..., self.body[k], :] + tau
+            if self.reaction[k] >= 0:
+                tq[..., self.reaction[k], :] = tq[..., self.reaction[k], :] - tau
+        f[..., 3:] = tq
+        return f
+
+
 class QuadraticCost:
     """A quadratic running + terminal cost over a controlled horizon, shared by all worlds
     (Batch.set_cost, egg_set_cost).  With x_t [n, 18] the state before step t, x_H the state after
@@ -37,17 +121,19 @@ class QuadraticCost:
     The weights broadcast to [n, 18] ([n, 6] for u_run); x_ref broadcasts to [n, 18] (one reference
     for every step) or is [ref_steps, n, 18] with ref_steps >= H + 1 (row t for step t).  The linear
     terms express progress: l_term[0, 0] = -1 rewards body 0 for moving along +x.  Every value must
-    be finite."""
+    be finite.  With m given the cost is for a batch with an actuator table of m actuators: u_t is the
+    [m] row of actuator values and u_run broadcasts to [m] (control_shape (m,))."""
 
-    def __init__(self, n, q_run=0.0, l_run=0.0, u_run=0.0, q_term=0.0, l_term=0.0, x_ref=0.0):
+    def __init__(self, n, q_run=0.0, l_run=0.0, u_run=0.0, q_term=0.0, l_term=0.0, x_ref=0.0, m=None):
         n = int(n)
         if n < 1:
             raise ValueError("QuadraticCost: n must be >= 1")
         self.n = n
-        S, U = STATE_PER_BODY, CONTROL_PER_BODY
+        self.control_shape = _control_shape(n, m, "QuadraticCost")
+        S = STATE_PER_BODY
         self.q_run, self.l_run, self.q_term, self.l_term = (_broadcast(a, (n, S), "QuadraticCost", name, finite=True) for a, name in
                                                             ((q_run, "q_run"), (l_run, "l_run"), (q_term, "q_term"), (l_term, "l_term")))
-        self.u_run = _broadcast(u_run, (n, U), "QuadraticCost", "u_run", finite=True)
+        self.u_run = _broadcast(u_run, self.control_shape, "QuadraticCost", "u_run", finite=True)
         x = np.asarray(x_ref, dtype=np.float64)
         if x.ndim == 3:
             if x.shape[0] < 1:
@@ -60,11 +146,12 @@ class QuadraticCost:
         self.ref_steps = self.x_ref.shape[0]
 
     def evaluate(self, states, u):
-        """The float64 numpy reference of J: states [H + 1, W, n, 18] (x_0 ... x_H), u [H, W, n, 6].
-        Returns J [W]."""
+        """The float64 numpy reference of J: states [H + 1, W, n, 18] (x_0 ... x_H), u [H, W, n, 6]
+        ([H, W, m] with an actuator table).  Returns J [W]."""
         states, u = np.asarray(states, dtype=np.float64), np.asarray(u, dtype=np.float64)
-        if u.ndim != 4 or u.shape[0] < 1 or u.shape[2:] != (self.n, CONTROL_PER_BODY):
-            raise ValueError(f"u must be [H >= 1, W, {self.n}, {CONTROL_PER_BODY}]")
+        cs = self.control_shape
+        if u.ndim != 2 + len(cs) or u.shape[0] < 1 or u.shape[2:] != cs:
+            raise ValueError(f"u must be [H >= 1, W, {', '.join(map(str, cs))}]")
         H, W = u.shape[:2]
         if states.shape != (H + 1, W, self.n, STATE_PER_BODY):
             raise ValueError(f"states must be [{H + 1}, {W}, {self.n}, {STATE_PER_BODY}] for a horizon of {H}")
@@ -72,7 +159,7 @@ class QuadraticCost:
             raise ValueError(f"the reference has {self.ref_steps} rows, fewer than H + 1 = {H + 1}")
         ref = self.x_ref[np.minimum(np.arange(H + 1), self.ref_steps - 1)]   # [H + 1, n, 18]
         d = states - ref[:, None]
-        run = (self.q_run * d[:H] ** 2 + self.l_run * d[:H]).sum(axis=(0, 2, 3)) + (self.u_run * u ** 2).sum(axis=(0, 2, 3))
+        run = (self.q_run * d[:H] ** 2 + self.l_run * d[:H]).sum(axis=(0, 2, 3)) + (self.u_run * u ** 2).sum(axis=(0,) + tuple(range(2, u.ndim)))
         return run + (self.q_term * d[H] ** 2 + self.l_term * d[H]).sum(axis=(1, 2))
 
 
@@ -160,15 +247,16 @@ def _packer(F, device, fill):
 
 def _checked_device(batch, u=None, horizon=None):
     """The batch's CUDA device, after the checks shared by the loops and planners: u, if given, is a
-    contiguous float64 schedule [horizon, W, n, 6] on that device (any H >= 1 without a horizon), and
-    the batch runs on torch's current stream."""
+    contiguous float64 schedule [horizon, W, *batch.control_shape] on that device (any H >= 1 without a
+    horizon), and the batch runs on torch's current stream."""
     import torch
     dev = torch.device("cuda", int(batch.desc.device))
+    cs = batch.control_shape
     if u is not None and not (isinstance(u, torch.Tensor) and u.is_cuda and u.device == dev and u.dtype == torch.float64
-                              and u.is_contiguous() and u.dim() == 4 and tuple(u.shape[1:]) == (batch.W, batch.n, 6)
+                              and u.is_contiguous() and u.dim() == 2 + len(cs) and tuple(u.shape[1:]) == (batch.W,) + cs
                               and (u.shape[0] >= 1 if horizon is None else u.shape[0] == horizon)):
         H = "H >= 1" if horizon is None else horizon
-        raise ValueError(f"u must be a contiguous float64 tensor [{H}, {batch.W}, {batch.n}, 6] on {dev}")
+        raise ValueError(f"u must be a contiguous float64 tensor [{H}, {batch.W}, {', '.join(map(str, cs))}] on {dev}")
     if batch.stream != torch.cuda.current_stream(dev).cuda_stream:
         raise ValueError("the batch must run on torch's current stream: Batch.set_stream(torch.cuda.current_stream().cuda_stream)")
     return dev
@@ -198,40 +286,41 @@ def mpc_iteration(batch, u, dt, k, n_total, first):
 
 
 class _SamplingPlan:
-    """What the sampling planners share: a nominal schedule u_nom, float64 [horizon, n, 6] on `device`,
-    the per-body sigma and bounds handed to Batch.set_sampler, the Philox seed and the iteration
-    counter.  Validated here with the rules that MPPI documents."""
+    """What the sampling planners share: a nominal schedule u_nom, float64 [horizon, *control_shape] on
+    `device`, the sigma and bounds of a control row handed to Batch.set_sampler, the Philox seed and the
+    iteration counter.  control_shape is (n, 6), or (m,) with m given (a batch with an actuator table).
+    Validated here with the rules that MPPI documents."""
 
-    def __init__(self, n, horizon, sigma, u_lo, u_hi, seed, u_nom, device):
+    def __init__(self, n, horizon, sigma, u_lo, u_hi, seed, u_nom, device, m):
         import torch
         name = type(self).__name__
         n, horizon = int(n), int(horizon)
         if n < 1 or horizon < 1:
             raise ValueError(f"{name}: n and horizon must be >= 1")
-        U = CONTROL_PER_BODY
+        U = self.control_shape = _control_shape(n, m, name)
         self.n, self.horizon = n, horizon
-        self.sigma = _broadcast(sigma, (n, U), name, "sigma")
+        self.sigma = _broadcast(sigma, U, name, "sigma")
         if not np.isfinite(self.sigma).all() or (self.sigma < 0).any():
             raise ValueError(f"{name}: sigma must be finite and >= 0")
-        self.u_lo = None if u_lo is None else _broadcast(u_lo, (n, U), name, "u_lo")
-        self.u_hi = None if u_hi is None else _broadcast(u_hi, (n, U), name, "u_hi")
+        self.u_lo = None if u_lo is None else _broadcast(u_lo, U, name, "u_lo")
+        self.u_hi = None if u_hi is None else _broadcast(u_hi, U, name, "u_hi")
         for a, what in ((self.u_lo, "u_lo"), (self.u_hi, "u_hi")):
             if a is not None and np.isnan(a).any():
                 raise ValueError(f"{name}: {what} has NaN values")
-        lo = np.full((n, U), -np.inf) if self.u_lo is None else self.u_lo
-        hi = np.full((n, U), np.inf) if self.u_hi is None else self.u_hi
+        lo = np.full(U, -np.inf) if self.u_lo is None else self.u_lo
+        hi = np.full(U, np.inf) if self.u_hi is None else self.u_hi
         if (lo > hi).any():
             raise ValueError(f"{name}: u_lo > u_hi")
         seed = int(seed)
         if not 0 <= seed < 2 ** 64:
             raise ValueError(f"{name}: seed must be in [0, 2^64)")
         self.seed = seed
-        un = np.zeros((horizon, n, U)) if u_nom is None else _broadcast(
-            u_nom.detach().cpu().numpy() if isinstance(u_nom, torch.Tensor) else u_nom, (horizon, n, U), name, "u_nom", finite=True)
+        un = np.zeros((horizon,) + U) if u_nom is None else _broadcast(
+            u_nom.detach().cpu().numpy() if isinstance(u_nom, torch.Tensor) else u_nom, (horizon,) + U, name, "u_nom", finite=True)
         self.device = torch.device(device)
         self.u_nom = torch.from_numpy(un.copy()).to(self.device)   # own storage: the iterations write to it
-        self.lo = torch.from_numpy(lo).to(self.device)   # the bounds as tensors, for clamp on the device
-        self.hi = torch.from_numpy(hi).to(self.device)
+        self.lo = torch.from_numpy(np.array(lo)).to(self.device)   # the bounds as tensors (own copies), for clamp on the device
+        self.hi = torch.from_numpy(np.array(hi)).to(self.device)
         self.iteration = 0
 
     def clamp(self, u):
@@ -249,14 +338,15 @@ class MPPI(_SamplingPlan):
     (None = unbounded; +-inf allowed, NaN not; u_lo <= u_hi).  lam: the temperature lambda of the
     weights exp(-(J - J_min) / lam), finite and > 0.  seed: the Philox key, in [0, 2^64).  u_nom: the
     initial nominal schedule, broadcast to [horizon, n, 6] (default zeros), finite.  Hand the planner
-    to Batch.set_sampler before mppi_iteration."""
+    to Batch.set_sampler before mppi_iteration.  With m given the planner works in the control space of
+    an actuator table of m actuators: sigma, u_lo and u_hi broadcast to [m] and u_nom to [horizon, m]."""
 
-    def __init__(self, n, horizon, sigma, lam, u_lo=None, u_hi=None, seed=0, u_nom=None, device="cuda"):
+    def __init__(self, n, horizon, sigma, lam, u_lo=None, u_hi=None, seed=0, u_nom=None, device="cuda", m=None):
         lam = float(lam)
         if not (np.isfinite(lam) and lam > 0):
             raise ValueError("MPPI: lam must be finite and > 0")
         self.lam = lam
-        super().__init__(n, horizon, sigma, u_lo, u_hi, seed, u_nom, device)
+        super().__init__(n, horizon, sigma, u_lo, u_hi, seed, u_nom, device, m)
 
 
 class CEM(_SamplingPlan):
@@ -270,10 +360,12 @@ class CEM(_SamplingPlan):
     smoothing of the refit, u_nom <- clamp(alpha u_nom + (1 - alpha) mean of the elites) and
     std <- max(alpha std + (1 - alpha) std of the elites, sigma_min); 0 <= alpha < 1.  sigma_min: a
     floor on std that keeps the search from collapsing, finite and >= 0.  u_lo, u_hi, seed and u_nom
-    follow the rules of MPPI.  Hand the planner to Batch.set_sampler before cem_iteration."""
+    follow the rules of MPPI.  Hand the planner to Batch.set_sampler before cem_iteration.  With m given
+    the planner works in the control space of an actuator table of m actuators, as MPPI does; std is
+    then [horizon, m]."""
 
     def __init__(self, n, horizon, sigma, n_elite, alpha=0.0, sigma_min=0.0, u_lo=None, u_hi=None, seed=0, u_nom=None,
-                 device="cuda"):
+                 device="cuda", m=None):
         import torch
         n_elite, alpha, sigma_min = int(n_elite), float(alpha), float(sigma_min)
         if n_elite < 1:
@@ -283,8 +375,8 @@ class CEM(_SamplingPlan):
         if not (np.isfinite(sigma_min) and sigma_min >= 0):
             raise ValueError("CEM: sigma_min must be finite and >= 0")
         self.n_elite, self.alpha, self.sigma_min = n_elite, alpha, sigma_min
-        super().__init__(n, horizon, sigma, u_lo, u_hi, seed, u_nom, device)
-        self.std = torch.tensor(np.broadcast_to(self.sigma, (self.horizon, self.n, CONTROL_PER_BODY)), device=self.device)
+        super().__init__(n, horizon, sigma, u_lo, u_hi, seed, u_nom, device, m)
+        self.std = torch.tensor(np.broadcast_to(self.sigma, (self.horizon,) + self.control_shape), device=self.device)
 
 
 def allgather_rows(x):
@@ -343,17 +435,19 @@ def mppi_sample(batch, mppi, u, first):
 def mppi_combine(batch, mppi, u, costs):
     """Steps 3 to 6 of mppi_iteration, all on the device: the baseline and nominal cost, the weighted
     sums of this shard, their rank-order sum and the candidate nominal schedule.  Returns
-    (candidate [H, n, 6], stats [nominal J, min J, sum omega, sum omega^2]) without reading anything back."""
+    (candidate [H, *control_shape], stats [nominal J, min J, sum omega, sum omega^2]) without reading
+    anything back."""
     import torch
     inf = torch.tensor(float("inf"), dtype=torch.float64, device=costs.device)
     local_min = torch.where(torch.isfinite(costs), costs, inf).min()
     g = allgather_rows(torch.stack([local_min, costs[0]]))   # [world_size, 2]; costs[0] of rank 0 is global world 0
     baseline = g[:, 0].min().contiguous()
-    L = mppi.horizon * batch.n * CONTROL_PER_BODY
+    cs = batch.control_shape
+    L = mppi.horizon * int(np.prod(cs))
     part = torch.empty(L + 2, dtype=torch.float64, device=costs.device)
     batch.mppi_reduce(u.data_ptr(), mppi.horizon, costs.data_ptr(), baseline.data_ptr(), mppi.lam, part.data_ptr())
     total = allgather_rank_sum(part)
-    candidate = mppi.clamp(total[:L].view(mppi.horizon, batch.n, CONTROL_PER_BODY) / total[L])
+    candidate = mppi.clamp(total[:L].view((mppi.horizon,) + cs) / total[L])
     return candidate, torch.stack([g[0, 1], baseline, total[L], total[L + 1]])
 
 
@@ -395,13 +489,13 @@ def mppi_advance(batch, plan, dt, n_total):
     one step with clamp(u_nom[0]); global world 0's new state re-seeds every world of every rank and
     becomes the snapshot, the start of the next horizon; u_nom shifts by one step (the last row
     repeats).  This costs one step of the whole batch, 1/H of a horizon.  Returns (the executed control
-    [n, 6], the new start rows [n, 18]), float64 CUDA tensors."""
+    [*control_shape], the new start rows [n, 18]), float64 CUDA tensors."""
     dev = _checked_device(batch)
     if plan.u_nom.device != dev:
         raise ValueError(f"the planner's u_nom must live on {dev}")
     u0 = plan.clamp(plan.u_nom[0])
     batch.restore()
-    batch.step_controlled(dt, u0.expand(1, batch.W, batch.n, CONTROL_PER_BODY).contiguous().data_ptr(), 1)
+    batch.step_controlled(dt, u0.expand((1, batch.W) + batch.control_shape).contiguous().data_ptr(), 1)
     state = gather_winner_states([0], n_total, _packer(batch.n * STATE_PER_BODY, dev, batch.gather_state))
     batch.seed_state(state.data_ptr(), 1, 0)
     batch.snapshot()
@@ -465,14 +559,14 @@ def cem_iteration(batch, cem, dt, u, first, n_total):
     dev = _plan_check(batch, cem, u, first)
     if cem.std.device != dev:
         raise ValueError(f"the planner's std must live on {dev}")
-    H, U = cem.horizon, CONTROL_PER_BODY
+    H, cs = cem.horizon, batch.control_shape
     costs = torch.empty(batch.W, dtype=torch.float64, device=dev)
     batch.restore()
     cem_sample(batch, cem, u, first)
     _rollout(batch, dt, u, costs)
-    pack = _packer(H * batch.n * U, dev, lambda local, out_ptr: batch.gather_controls(u.data_ptr(), H, local, out_ptr))
+    pack = _packer(H * int(np.prod(cs)), dev, lambda local, out_ptr: batch.gather_controls(u.data_ptr(), H, local, out_ptr))
     all_costs, elites, ecost, rows = cem_select(cem, costs, n_total, pack)
-    moments = torch.empty((2, H, batch.n, U), dtype=torch.float64, device=dev)
+    moments = torch.empty((2, H) + cs, dtype=torch.float64, device=dev)
     batch.control_moments(rows.contiguous().data_ptr(), len(elites), H, moments.data_ptr())
     u_nom, std = cem_refit(cem, moments)
     ok = torch.isfinite(u_nom).all() & torch.isfinite(std).all()

@@ -166,6 +166,14 @@ def legged20(W, seed=5000, dt=0.005, sigma=0.05):
     return s
 
 
+def legged20_motors():
+    """The joint motors of legged20 (mpc.Actuators.ball_joint_motors): three per ball joint, 57 for its
+    19 joints, acting on the child link and reacting on the parent, with axes in the parent's frame."""
+    from .mpc import Actuators
+    s = legged20(1)
+    return Actuators.ball_joint_motors(s["n"], s["i0"], s["i1"])
+
+
 def cairn(W, rocks=4, xb=(-0.2, 0.2), yb=(-0.2, 0.2), zb=(1.0, 8.0), seed=7, dt=0.005):
     """Cairn(rocks, bounds) (/root/reference/eggshell/ensembles.cc:709-728) with a seeded stream
     instead of the reference's unseeded std::rand(): random p in the box, uniform random R,

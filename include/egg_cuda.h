@@ -164,8 +164,49 @@ int egg_step(egg_batch* b, double dt, int integrator, int n_steps);
 /* horizon x Ensemble::Step(dt, integrator) with a per-step control schedule: before step t the f_ext
  * slot of every world is replaced by u_d[t], exactly what egg_set_external(u[t]) before
  * egg_step(b, dt, integrator, 1) does.  u_d is [horizon][W][n_bodies][6], time-major, so every slice
- * has the layout of egg_set_external.  After the call the slot holds u_d[horizon-1].  horizon >= 1. */
+ * has the layout of egg_set_external.  After the call the slot holds u_d[horizon-1].  horizon >= 1.
+ * With an actuator table (egg_set_actuators) u_d is [horizon][W][m] and the slot takes the wrench the
+ * table defines from u_d[t] and the state before step t. */
 int egg_step_controlled(egg_batch* b, double dt, int integrator, const double* u_d, int horizon);
+
+/* Actuators: a control space of m actuator values per world in place of the n_bodies x 6 body wrenches,
+ * shared by all worlds of the batch (INTEGRATION.md, "Actuators").  Actuator a applies the torque
+ * +tau_a to body[a] (in [0, n_bodies)) and -tau_a to reaction[a] (in [-1, n_bodies), != body[a]; -1 =
+ * none).  Its axis axis[a][3] (finite, not all zero, used as given: its length is the gear ratio) is
+ * given in the rotation of body frame[a] (-1, body[a] or reaction[a]; -1 = the world frame).  With x_t
+ * the state before step t (the row the running cost reads) and u_a the actuator value of step t:
+ *   k_a = axis[a]                         if frame[a] = -1
+ *       = R k, (R k)_i = (R_i0 k_0 + R_i1 k_1) + R_i2 k_2,   R = R of body frame[a] in x_t
+ *   tau_a = u_a k_a                       (component-wise)
+ *   f_ext[b] = (m_b g_x, m_b g_y, m_b g_z, 0, 0, 0), then for a = 0 .. m-1 in order:
+ *              torque += tau_a if body[a] = b;  torque -= tau_a if reaction[a] = b
+ * Every product and sum is rounded on its own (no fused multiply-add), so a float64 transcription in
+ * the same order (mpc.Actuators.wrench) has the same bits.  The base wrench is the force part of the
+ * slot egg_init writes (m g from the mass and egg_desc.gravity, the same product); the gyroscopic
+ * torque egg_init freezes into the slot is NOT included.  It is zero for worlds at rest at egg_init.
+ * The wrench is held over step t (zero-order hold, like f_ext in the reference); after a controlled
+ * call the slot holds the wrench of the last step.  An actuator table adds no forces: body-force
+ * controls stay available in the default control space. */
+typedef struct egg_actuators {
+  int m;               /* number of actuators, >= 1 */
+  const int* body;     /* [m] (every array is a HOST array) */
+  const int* reaction; /* [m] */
+  const int* frame;    /* [m] */
+  const double* axis;  /* [m][3] */
+} egg_actuators;
+
+/* Sets the batch's actuator table: copies it to device memory owned by the batch (counted by
+ * egg_device_bytes), with a per-body list of the actuators that touch each body, in actuator order.
+ * a == NULL returns to body wrenches and releases that memory.  From then on the control row per world
+ * of every call below is the m actuator values: u_d [H][W][m] (egg_step_controlled,
+ * egg_step_controlled_cost, egg_sample_controls, egg_sample_controls_std, egg_mppi_reduce,
+ * egg_gather_controls), u_nom_d / mean_d / std_d [H][m], egg_sampler sigma, u_lo, u_hi [m], egg_cost
+ * u_run [m], egg_mppi_reduce out_d [H m + 2], egg_gather_controls out_d [k][H][m] and
+ * egg_control_moments rows_d [k][H][m], out_d [2][H][m]; their checks apply to that width.  A
+ * malformed table returns EGG_ERR_ARG and keeps the previous one.  EGG_ERR_STATE while a sampler or a
+ * cost is set: their arrays have the width of the current control space, clear them first.  Valid
+ * before or after egg_init.  Synchronises the batch stream. */
+int egg_set_actuators(egg_batch* b, const egg_actuators* a);
 
 /* out_d[k][n_bodies][18] = (p(3), R(9, row-major), v(3), w(3)) of worlds[0..k), element for element
  * what egg_get_bodies returns for those worlds.  worlds is a HOST int array, each entry in [0, W),
@@ -189,7 +230,7 @@ int egg_seed_state(egg_batch* b, const double* in_d, int k, int first);
 typedef struct egg_cost {
   const double* q_run;  /* [n_bodies][18]; NULL = all zero (every array is a HOST array) */
   const double* l_run;  /* [n_bodies][18] */
-  const double* u_run;  /* [n_bodies][6] */
+  const double* u_run;  /* [n_bodies][6]; [m] with an actuator table (egg_set_actuators) */
   const double* q_term; /* [n_bodies][18] */
   const double* l_term; /* [n_bodies][18] */
   const double* x_ref;  /* [ref_steps][n_bodies][18]; NULL = zeros (ref_steps is then ignored) */
@@ -215,7 +256,7 @@ int egg_step_controlled_cost(egg_batch* b, double dt, int integrator, const doub
  * planner, sampling W perturbed copies of a nominal schedule and their cost-weighted sum.
  * Per-body noise scale and control bounds, shared by all worlds and steps: */
 typedef struct egg_sampler {
-  const double* sigma; /* [n_bodies][6] standard deviation of the noise, finite and >= 0 (HOST array) */
+  const double* sigma; /* [n_bodies][6] standard deviation of the noise, finite and >= 0 (HOST array); [m] with an actuator table */
   const double* u_lo;  /* [n_bodies][6] lower bound of every sampled control; NULL = unbounded */
   const double* u_hi;  /* [n_bodies][6] upper bound; NULL = unbounded.  +-inf allowed, NaN not */
 } egg_sampler;
@@ -230,7 +271,9 @@ int egg_set_sampler(egg_batch* b, const egg_sampler* s);
  * and every local world w; u_nom_d is [horizon][n_bodies][6], u_d [horizon][W][n_bodies][6] (the
  * schedule of egg_step_controlled).  eps is a standard normal from Philox4x32-10 with key
  * (seed_lo, seed_hi) and counter (q, g, iteration_lo, iteration_hi), g = first + w the global world
- * index and q = (t n_bodies + b) 3 + p for the component pair (2p, 2p + 1): the four output words
+ * index and q = (t n_bodies + b) 3 + p for the component pair (2p, 2p + 1) (in general q = t ceil(c / 2)
+ * + p for the elements (2p, 2p + 1) of a control row of width c; with an actuator table c = m, and for
+ * odd m the last pair discards its second normal): the four output words
  * make two uniforms u = ((lo | hi << 32) >> 11) 2^-53 + 2^-54 (words 0, 1 and words 2, 3), and
  * Box-Muller gives eps_2p = r cos(2 pi u2), eps_2p+1 = r sin(2 pi u2), r = sqrt(-2 ln u1).  The
  * samples depend on the global index only, not on the sharding.  Global world 0 takes no noise: it

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Cost of the receding-horizon MPC loop (mpc.mpc_iteration) over the plain rollout sweep.
 
-    python tools/mpc_loop.py [--worlds 131072] [--horizon 50] [--repeats 5] [--legs abcdef] [--profile] [--out FILE]
+    python tools/mpc_loop.py [--worlds 131072] [--horizon 50] [--repeats 5] [--legs abcdefg] [--profile] [--out FILE]
     python -m torch.distributed.run --nproc_per_node N tools/mpc_loop.py ...
 
 One process per GPU; every rank owns `--worlds` legged20 worlds (bench.py's c5mpc scene, seeded per
@@ -35,11 +35,20 @@ and the refit of u_nom and std.  Each of those parts is also timed on its own.  
 egg_sample_controls_std and egg_sample_controls are timed alone, alternating in the same call, with
 their GB/s against the same copy bandwidth, and cem_iteration runs with sigma > 0 on the torques and
 the representative cost, and its world-steps/s are reported.
+Leg g runs MPPI in joint space: a second batch of the same worlds with the 57 motors of legged20's 19
+ball joints as its actuator table (scenes.legged20_motors, Batch.set_actuators), in gravity (the
+actuation kernel adds m g to every body; the nominal plan starts at zero torques).  It times whole
+mppi_iterations with the representative cost (its control term on the 57 motor torques), so ms per
+horizon compares with the body-wrench mppi_loop_cost of leg e.  egg_sample_controls and
+egg_mppi_reduce are timed alone at the row width c = 57 with their GB/s.  --profile adds the device
+time of the actuation kernel (egg_actuate_kernel) per horizon against egg_fext_slice_cost_kernel of
+a body-wrench rollout with the same cost.
 --legs picks the legs to run (b needs a; the overheads need the legs they compare).
 Rank 0 prints one JSON line with the GPU name and power limit.
 
 Memory: a schedule is H x worlds x 20 x 6 doubles, 6.3 GB per GPU at 131072 worlds and H = 50; the
 script holds three (constant, random and MPPI or CEM samples), plus the batch and one saved start state (0.4 GB).
+Leg g adds a second batch and a joint-space schedule of H x worlds x 57 doubles (3.0 GB).
 """
 import argparse
 import json
@@ -64,9 +73,10 @@ def parse():
     ap.add_argument("--repeats", type=int, default=5, help="timed repeats of each leg")
     ap.add_argument("--random-iters", type=int, default=3, help="timed loop iterations with random schedules")
     ap.add_argument("--sigma", type=float, default=0.05, help="std. dev. of the random torques (N m)")
-    ap.add_argument("--legs", default="abcdef", help="legs to run (default: all)")
+    ap.add_argument("--legs", default="abcdefg", help="legs to run (default: all)")
     ap.add_argument("--lam", type=float, default=1.0, help="MPPI temperature lambda of leg e")
     ap.add_argument("--elites", type=int, default=128, help="CEM elites of leg f (n_elite, over all GPUs)")
+    ap.add_argument("--sigma-motor", type=float, default=0.5, help="std. dev. of the joint-motor torques of leg g (N m)")
     ap.add_argument("--profile", action="store_true", help="also record the kernel times of legs c, d, e and f with torch.profiler")
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     return ap.parse_args()
@@ -100,7 +110,8 @@ def profile_legs(prepare, legs, sync):
             sync()
         for e in prof.key_averages():
             kernel = re.search(r"egg_\w+", e.key)
-            if kernel and any(key in kernel.group(0) for key in ("fext_slice", "egg_cost", "egg_mppi", "egg_gather_controls", "egg_control_moments")):
+            if kernel and any(key in kernel.group(0) for key in ("fext_slice", "egg_actuate", "egg_cost", "egg_mppi", "egg_gather_controls",
+                                                                 "egg_control_moments")):
                 out[f"{name}: {kernel.group(0)}"] = {"calls": e.count, "ms": e.device_time_total / 1e3}
     return out
 
@@ -142,25 +153,33 @@ def main():
     # CEM planners the same way: std = 0 for the overhead of leg f, sigma on the torques for the loop
     cem0 = mpc.CEM(n, H, sigma=0.0, n_elite=args.elites, seed=13, u_nom=scene["f_ext"][0], device=dev)
     cem1 = mpc.CEM(n, H, sigma=sigma, n_elite=args.elites, seed=14, u_nom=scene["f_ext"][0], device=dev)
+    motors = E.scenes.legged20_motors()
+    c_joint = motors.m
+    u_joint = torch.empty((H, W, c_joint), dtype=torch.float64, device=dev) if "g" in args.legs else None
+    mppi_joint = mpc.MPPI(n, H, sigma=args.sigma_motor, lam=args.lam, seed=15, m=c_joint, device=dev)
     L = H * n * 6
+    Lj = H * c_joint
     chunks = -(-W // 256)   # stage-1 chunks of egg_mppi_reduce
     sample_bytes = 8 * (H * W * n * 6 + L)                                  # write the samples, read u_nom
     reduce_bytes = 8 * (H * W * n * 6 + W + 2 * chunks * (L + 2) + L + 2)   # read u and J, partials out and in, result
     sample_std_bytes = 8 * (H * W * n * 6 + 2 * L)                          # write the samples, read mean and std
+    sample_joint_bytes = 8 * (H * W * c_joint + Lj)                             # the same at the row width of the motors
+    reduce_joint_bytes = 8 * (H * W * c_joint + W + 2 * chunks * (Lj + 2) + Lj + 2)
     costs = torch.empty(W, dtype=torch.float64, device=dev)
     all_costs = torch.empty(n_total, dtype=torch.float64, device=dev)
     start = torch.empty((W, n * 18), dtype=torch.float64, device=dev)
 
-    def representative_cost(x0):
+    def representative_cost(x0, m=None):
         """x0: world 0's start rows [n, 18].  Tracks a reference that moves every body along +x at
-        0.5 m/s from x0, with small velocities and small controls, and rewards progress of body 0."""
+        0.5 m/s from x0, with small velocities and small controls, and rewards progress of body 0.
+        m: the cost for a batch with an actuator table of m actuators."""
         q_run = np.zeros((n, mpc.STATE_PER_BODY))
         q_run[:, 0:3], q_run[:, 12:15] = 1.0, 0.1
         l_term = np.zeros((n, mpc.STATE_PER_BODY))
         l_term[0, 0] = -1.0
         x_ref = np.repeat(x0[None], H + 1, axis=0)
         x_ref[:, :, 0] += 0.5 * dt * np.arange(H + 1)[:, None]
-        return mpc.QuadraticCost(n, q_run=q_run, u_run=1e-3, l_term=l_term, x_ref=x_ref)
+        return mpc.QuadraticCost(n, q_run=q_run, u_run=1e-3, l_term=l_term, x_ref=x_ref, m=m)
 
     def sync():
         if ws > 1:
@@ -188,10 +207,19 @@ def main():
         b.snapshot()
         b.gather_state(np.arange(W), start.data_ptr())   # the common start of every timed leg
         cost = representative_cost(start[0].view(n, mpc.STATE_PER_BODY).cpu().numpy())
+        bj = None
+        if "g" in args.legs:   # the same worlds with the joint motors as the control space
+            bj = E.scenes.make_batch(scene, solver=E.SOLVER_PGS, k_max=k_max, device=local)
+            bj.set_stream(stream.cuda_stream)
+            bj.set_actuators(motors)
+            bj.set_cost(representative_cost(start[0].view(n, mpc.STATE_PER_BODY).cpu().numpy(), m=c_joint))
+            bj.set_sampler(mppi_joint)
 
         def reset():
-            b.seed_state(start.data_ptr(), W, 0)
-            b.snapshot()
+            for x in (b, bj):
+                if x is not None:
+                    x.seed_state(start.data_ptr(), W, 0)
+                    x.snapshot()
 
         def leg_a():
             b.restore()
@@ -236,8 +264,11 @@ def main():
             cem_moments(mpc.cem_select(cem0, costs, n_total, pack_controls)[3])
             mpc.cem_refit(cem0, moments)
 
-        legs = {name: fn for name, fn in (("a", leg_a), ("c", leg_c), ("b", leg_b), ("d", leg_d), ("e", leg_e), ("f", leg_f))
-                if name in args.legs}
+        def leg_g():
+            mpc.mppi_iteration(bj, mppi_joint, dt, u_joint, first)
+
+        legs = {name: fn for name, fn in (("a", leg_a), ("c", leg_c), ("b", leg_b), ("d", leg_d), ("e", leg_e), ("f", leg_f),
+                                          ("g", leg_g)) if name in args.legs}
 
         def prepare(name):   # the cost is set for leg d only (outside the timed region: set_cost synchronises)
             reset()
@@ -257,7 +288,8 @@ def main():
         t = {name: np.array(x) for name, x in t.items()}
         entry = {}
         for name, key in (("a", "a_sweep_ms"), ("c", "c_controlled_sweep_ms"), ("b", "b_mpc_iteration_ms"),
-                          ("d", "d_controlled_cost_sweep_ms"), ("e", "e_mppi_additions_ms"), ("f", "f_cem_additions_ms")):
+                          ("d", "d_controlled_cost_sweep_ms"), ("e", "e_mppi_additions_ms"), ("f", "f_cem_additions_ms"),
+                          ("g", "g_joint_mppi_iteration_ms")):
             if name in t:
                 entry[key] = spread(t[name])
         for key, hi, lo, base in (("slice_copy_overhead", "c", "a", "a"), ("loop_overhead", "b", "a", "a"),
@@ -304,8 +336,29 @@ def main():
                 "copy_bandwidth_GBps": 6555.8, "elites": cem0.n_elite,
                 "sample_controls_std": {"ms": spread(kstd), "bytes": sample_std_bytes, "GBps": spread(sample_std_bytes / (kstd * 1e-3) / 1e9)},
                 "sample_controls": {"ms": spread(kbody), "bytes": sample_bytes, "GBps": spread(sample_bytes / (kbody * 1e-3) / 1e9)}}
+        if "g" in t:   # the two MPPI kernels alone at the motors' row width, and their bandwidth
+            prepare("g")
+            costs.fill_(1.0)   # finite costs for the reduction (weights exp(-1 / lam))
+            ks, kr = [], []
+            ub = torch.zeros((), dtype=torch.float64, device=dev)
+            part = torch.empty(Lj + 2, dtype=torch.float64, device=dev)
+            for _ in range(args.repeats):
+                ks.append(timed(lambda: bj.sample_controls(mppi_joint.u_nom.data_ptr(), H, mppi_joint.seed, 0, first, u_joint.data_ptr())))
+                kr.append(timed(lambda: bj.mppi_reduce(u_joint.data_ptr(), H, costs.data_ptr(), ub.data_ptr(), args.lam, part.data_ptr())))
+            ks, kr = np.array(ks), np.array(kr)
+            entry["g_joint_space"] = {
+                "actuators": c_joint, "sigma_motor": args.sigma_motor, "lam": args.lam, "gravity": list(b.desc.gravity),
+                "ms_per_horizon": spread(t["g"]), "world_steps_per_s": spread(n_total * H / (t["g"] * 1e-3)),
+                "schedule_GB": H * W * c_joint * 8 / 1e9, "body_wrench_schedule_GB": H * W * n * 6 * 8 / 1e9,
+                "copy_bandwidth_GBps": 6555.8,
+                "sample_controls": {"ms": spread(ks), "bytes": sample_joint_bytes, "GBps": spread(sample_joint_bytes / (ks * 1e-3) / 1e9)},
+                "mppi_reduce": {"ms": spread(kr), "bytes": reduce_joint_bytes, "GBps": spread(reduce_joint_bytes / (kr * 1e-3) / 1e9),
+                                "launches": 2, "chunks": chunks}}
         if args.profile:
-            entry["kernel_ms_per_horizon"] = profile_legs(prepare, {x: legs[x] for x in "cdef" if x in legs}, sync)
+            prof = {x: legs[x] for x in "cdefg" if x in legs}
+            if "g" in legs:   # the body-wrench rollout with a cost, for egg_fext_slice_cost_kernel against egg_actuate_kernel
+                prof.setdefault("d", leg_d)
+            entry["kernel_ms_per_horizon"] = profile_legs(prepare, prof, sync)
         # the loop itself with random time-varying schedules (the state evolves from iteration to iteration),
         # with the built-in cost and with the configured one
         loops = [(key, qc) for key, qc, leg in (("random_loop", None, "b"), ("random_loop_cost", cost, "d")) if leg in legs]
@@ -336,6 +389,9 @@ def main():
                           "world_steps_per_s": n_total * H * args.random_iters / (ms * 1e-3)}
         st = b.status()
         entry["status_or"] = int(np.bitwise_or.reduce(st["status"]))
+        if bj is not None:
+            entry["g_status_or"] = int(np.bitwise_or.reduce(bj.status()["status"]))
+            bj.close()
         result[f"k_max_{k_max}"] = entry
         b.close()
     if rank == 0:
