@@ -22,7 +22,7 @@ ST_LCP_FAILED, ST_JOINT_CONFLICT, ST_BAD_INIT, ST_CONTACT_OVERFLOW, ST_NONFINITE
 
 EXPORTS = [
     "egg_desc_default", "egg_create", "egg_destroy", "egg_set_bodies", "egg_set_shapes", "egg_set_state", "egg_set_joints",
-    "egg_set_external", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_step_controlled",
+    "egg_set_external", "egg_set_friction", "egg_init", "egg_init_stabilize", "egg_post_stabilize", "egg_step", "egg_step_controlled",
     "egg_set_cost", "egg_step_controlled_cost", "egg_set_actuators", "egg_set_sampler", "egg_sample_controls", "egg_mppi_reduce", "egg_sample_controls_std", "egg_gather_controls", "egg_control_moments", "egg_gather_state", "egg_seed_state", "egg_snapshot", "egg_restore", "egg_update_contacts", "egg_get_static", "egg_get_bodies", "egg_get_contacts", "egg_get_contacts_range", "egg_get_pair_hits", "egg_get_pair_hits_range",
     "egg_get_status", "egg_get_dense_work", "egg_get_debug_counters", "egg_rollout_costs", "egg_set_stream", "egg_sync", "egg_device_bytes",
     "egg_launch_count", "egg_capacity", "egg_get_kernel_config", "egg_set_profiling", "egg_get_kernel_ms", "egg_fp64_peak_tflops", "egg_host_alloc", "egg_host_free", "egg_last_error", "egg_version",
@@ -155,6 +155,7 @@ class Batch:
         self.cost = None     # mpc.QuadraticCost handed to set_cost
         self.sampler = None  # mpc.MPPI or mpc.CEM handed to set_sampler
         self.actuators = None  # mpc.Actuators handed to set_actuators; None = body wrenches
+        self._mu = None        # [W] friction coefficients handed to set_friction; None = BOX friction
         self.max_contacts = None
         self._probe_capacity()
 
@@ -203,6 +204,23 @@ class Batch:
     def set_external(self, f):
         f = _d(f, (self.W, self.n, 6))
         _chk(lib().egg_set_external(self.h, _p(f)), "egg_set_external")
+
+    def set_friction(self, mu):
+        """Coulomb-pyramid friction (egg_set_friction, INTEGRATION.md "Friction"): a scalar for every
+        world or a [W] array of coefficients, each finite and >= 0; None returns to the reference's BOX
+        friction.  PGS solver only.  A refused table leaves the previous one in place."""
+        if mu is None:
+            _chk(lib().egg_set_friction(self.h, None), "egg_set_friction")
+            self._mu = None
+            return
+        m = _d(mu, (self.W,))
+        _chk(lib().egg_set_friction(self.h, _p(m)), "egg_set_friction")
+        self._mu = m.copy()
+
+    @property
+    def friction(self):
+        """A copy of the [W] friction coefficients, or None with BOX friction."""
+        return None if self._mu is None else self._mu.copy()
 
     def init(self):
         _chk(lib().egg_init(self.h), "egg_init")

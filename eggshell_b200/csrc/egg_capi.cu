@@ -86,6 +86,8 @@ struct egg_batch {
   double* act_dbuf = nullptr;    // ... and axis [m][3]
   size_t act_dcount = 0;
   EggAct act = {};               // pointers into act_ibuf / act_dbuf; act.m = 0 without a table
+  double* mu = nullptr;          // egg_set_friction: [W] Coulomb friction coefficients; null = BOX friction
+  size_t mu_count = 0;
   bool profiling = false;
   std::vector<cudaEvent_t> ev;   // 4 per profiled step
   std::vector<cudaEvent_t> ev_free;
@@ -650,8 +652,10 @@ static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d, do
     b->dev.iso = !(flag & 1) ? 0 : ((flag & 2) ? 2 : 1);   // 0 general, 1 isotropic, 2 isotropic and uniform
     if (getenv("EGG_PGS_ISO") && atoi(getenv("EGG_PGS_ISO")) < b->dev.iso) b->dev.iso = atoi(getenv("EGG_PGS_ISO"));
     b->iso_known = true;
-    b->dev.rmax = egg_runs_rmax(b->dev);   // run format of the PGS stream for isotropic bodies, else one block per lane and stage
   }
+  // run format of the PGS stream for isotropic bodies, else one block per lane and stage; never with a
+  // friction table (BOX friction only).  Decided here, per step, so assembly and solve agree.
+  b->dev.rmax = b->mu ? 0 : egg_runs_rmax(b->dev);
   const size_t slice = (size_t)b->dev.W * ctrl_width(b);
   for (int s = 0; s < n_steps; s++) {
     if (u_d) {
@@ -682,7 +686,7 @@ static int step_loop(egg_batch* b, double dt, int n_steps, const double* u_d, do
     CK(egg_launch_assemble(b->dev, dt, b->stream));
     DBG_SYNC("assembly kernels")
     if (b->profiling) CK(cudaEventRecord(e[2], b->stream));
-    if (solver == EGG_SOLVER_PGS) CK(egg_launch_solve_pgs(b->dev, dt, b->stream));
+    if (solver == EGG_SOLVER_PGS) CK(egg_launch_solve_pgs(b->dev, dt, b->mu, b->stream));
     else if (solver == EGG_SOLVER_DENSE_MURTY) CK(egg_launch_solve_dense(b->dev, dt, b->stream, b->dense_scratch, b->dense_scratch_bytes));
     else CK(egg_launch_solve_iter(b->dev, dt, solver, b->stream));
     DBG_SYNC("solve kernel")
@@ -723,6 +727,25 @@ int egg_step_controlled_cost(egg_batch* b, double dt, int integrator, const doub
     return EGG_ERR_ARG;
   }
   return step_loop(b, dt, horizon, u_d, cost_d);
+}
+
+int egg_set_friction(egg_batch* b, const double* mu) {
+  if (!b) return EGG_ERR_ARG;
+  if (b->desc.solver != EGG_SOLVER_PGS) {
+    g_err = "egg_set_friction: Coulomb friction exists for the PGS solver only (dense, Jacobi and SOR keep BOX friction)";
+    return EGG_ERR_UNSUPPORTED;
+  }
+  const size_t W = (size_t)b->dev.W;
+  std::vector<double> h;
+  if (mu) {
+    h.resize(W);
+    for (size_t w = 0; w < W; w++) {
+      if (!std::isfinite(mu[w]) || mu[w] < 0) { g_err = "egg_set_friction: every mu must be finite and >= 0"; return EGG_ERR_ARG; }
+      h[w] = mu[w] + 0.0;   // -0.0 -> +0.0
+    }
+  }
+  CK(cudaSetDevice(b->device));
+  return replace_dbuf(b, b->mu, b->mu_count, h.size(), h.data());
 }
 
 // Host [rows][n][comps] -> component-major [rows][comps][n], the layout of EggCost and EggSampler.

@@ -155,8 +155,11 @@ cudaError_t egg_launch_collide(const EggDev& d, cudaStream_t s);
 cudaError_t egg_launch_init(const EggDev& d, cudaStream_t s);
 cudaError_t egg_launch_clear_contacts(const EggDev& d, cudaStream_t s);
 cudaError_t egg_launch_assemble(const EggDev& d, double dt, cudaStream_t s);
-cudaError_t egg_launch_solve_pgs(const EggDev& d, double dt, cudaStream_t s);
-cudaError_t egg_launch_solve_pgs_stream(const EggDev& d, double dt, cudaStream_t s);
+// mu: the [W] Coulomb friction coefficients of egg_set_friction (device), null = BOX friction.  A
+// kernel argument of its own rather than a member of EggDev: the parameter layout of the kernels
+// that do not read it stays put.
+cudaError_t egg_launch_solve_pgs(const EggDev& d, double dt, const double* mu, cudaStream_t s);
+cudaError_t egg_launch_solve_pgs_stream(const EggDev& d, double dt, const double* mu, cudaStream_t s);
 cudaError_t egg_launch_solve_pgs_runs(const EggDev& d, double dt, cudaStream_t s);
 int egg_run_cap(const EggDev& d);
 int egg_runs_rmax(const EggDev& d);

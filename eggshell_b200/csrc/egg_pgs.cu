@@ -159,4 +159,4 @@ cudaError_t egg_launch_assemble(const EggDev& d, double dt, cudaStream_t s) {
   return cudaGetLastError();
 }
 
-cudaError_t egg_launch_solve_pgs(const EggDev& d, double dt, cudaStream_t s) { return egg_launch_solve_pgs_stream(d, dt, s); }
+cudaError_t egg_launch_solve_pgs(const EggDev& d, double dt, const double* mu, cudaStream_t s) { return egg_launch_solve_pgs_stream(d, dt, mu, s); }

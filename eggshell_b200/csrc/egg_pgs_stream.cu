@@ -283,8 +283,16 @@ enum { PH_INIT = 0, PH_PROBE = 1, PH_EXACT = 2, PH_UPDATE = 3 };
 // inverse inertias, see egg_solve.cu) and comes as one 16-byte load per body.  ISO == 2: all
 // bodies of the batch share the same (1/m, 1/c) (every body of the reference is the same cube,
 // body.h:91) and the pair is a kernel constant.
-template <int LPW, int MINB, int ISO, bool F32>
-__global__ void __launch_bounds__(32, MINB) egg_pgs_stream_kernel(EggDev d, double dt, int pf) {
+//
+// COULOMB (egg_set_friction): the tangent rows of a block projected as a contact are bounded by
+// [-b, b], b = mu[w] max(x_n, 0), x_n = the block's normal multiplier before its update (x2), instead
+// of [-1, 1].  Such a bound moves with the normal, so "x equals its bound" is recorded by each update
+// as a clamp flag per tangent row (0 free, 1 at -b, 2 at +b) in bits PK_FLAGS.. of the packed word of
+// the multiplier sector; the residual and the row_state taps read the flags.  Every decode of the
+// packed word reads (int)(pk >> 21), i.e. bits 21..52, so the flags never reach an index.
+constexpr int PK_FLAGS = 56;
+template <int LPW, int MINB, int ISO, bool F32, bool COULOMB>
+__global__ void __launch_bounds__(32, MINB) egg_pgs_stream_kernel(EggDev d, double dt, int pf, const double* __restrict__ mu_w) {
   constexpr int G = 32 / LPW;
   constexpr int RECB = F32 ? RECB32 : RECB64;   // bytes of one staged record
   constexpr int SPIECES = RECB / 16;
@@ -327,6 +335,7 @@ __global__ void __launch_bounds__(32, MINB) egg_pgs_stream_kernel(EggDev d, doub
     const double* maos = ISO ? d.minv_iso + (size_t)wc * (n + 1) * 2      // [n+1][2], row n = 0 (ground / world anchor)
                              : d.minv_aos + (size_t)wc * (n + 1) * 10;    // [n+1][10]
     const int nc = valid ? nj + d.c_count[wc] : 0;
+    const double mu = COULOMB ? mu_w[wc] : 0.0;
     char* gs = reinterpret_cast<char*>(d.rec) + (size_t)grp * group_stride_bytes(d.nrec, G);
     const int R = d.grp_info[(size_t)grp * 4];                // rounds of the group
     const int tot0 = d.grp_info[(size_t)grp * 4 + 1];         // blocks in round 0
@@ -435,7 +444,15 @@ __global__ void __launch_bounds__(32, MINB) egg_pgs_stream_kernel(EggDev d, doub
           const double q0s = e0 * e0, q1s = e1 * e1, q2s = e2 * e2;
           double c;
           if (eq) { c = q0s + q1s + q2s; se += c; }
-          else {
+          else if (COULOMB) {
+            // the tangent rows by the clamp flags of the update that produced x_k (none for x_0: free)
+            const unsigned f0 = (unsigned)(pk_lam >> PK_FLAGS) & 3u, f1 = (unsigned)(pk_lam >> (PK_FLAGS + 2)) & 3u;
+            const double c1 = ((f0 == 1u && e0 > 0) ? q0s : 0.0) + ((f1 == 1u && e1 > 0) ? q1s : 0.0) + ((x2 == 0.0 && e2 > 0) ? q2s : 0.0);
+            const double c2 = ((f0 == 2u && e0 < 0) ? q0s : 0.0) + ((f1 == 2u && e1 < 0) ? q1s : 0.0);
+            const double c3 = ((f0 == 0u) ? q0s : 0.0) + ((f1 == 0u) ? q1s : 0.0) + ((x2 > 0.0) ? q2s : 0.0);
+            s1 += c1; s2 += c2; s3 += c3;
+            c = c1 + c2 + c3;
+          } else {
             // w = -e: at lo with w < 0, at hi with w > 0, strictly inside (sparse_iterations.cc:51-69)
             const double c1 = ((x0 == -1.0 && e0 > 0) ? q0s : 0.0) + ((x1 == -1.0 && e1 > 0) ? q1s : 0.0) + ((x2 == 0.0 && e2 > 0) ? q2s : 0.0);
             const double c2 = ((x0 == 1.0 && e0 < 0) ? q0s : 0.0) + ((x1 == 1.0 && e1 < 0) ? q1s : 0.0);
@@ -448,25 +465,39 @@ __global__ void __launch_bounds__(32, MINB) egg_pgs_stream_kernel(EggDev d, doub
             double* lo = lam_out + 3 * orig;
             int* rs = row_state + 3 * orig;
             lo[0] = x0; lo[1] = x1; lo[2] = x2;
-            rs[0] = eq ? 3 : (x0 == -1.0 ? 1 : (x0 == 1.0 ? 2 : 0));
-            rs[1] = eq ? 3 : (x1 == -1.0 ? 1 : (x1 == 1.0 ? 2 : 0));
+            if (COULOMB) {
+              rs[0] = eq ? 3 : (int)((pk_lam >> PK_FLAGS) & 3u);
+              rs[1] = eq ? 3 : (int)((pk_lam >> (PK_FLAGS + 2)) & 3u);
+            } else {
+              rs[0] = eq ? 3 : (x0 == -1.0 ? 1 : (x0 == 1.0 ? 2 : 0));
+              rs[1] = eq ? 3 : (x1 == -1.0 ? 1 : (x1 == 1.0 ? 2 : 0));
+            }
             rs[2] = eq ? 3 : (x2 == 0.0 ? 1 : 0);
           }
           return;
         }
         // clamp kind of this block (q2 shift already folded in by the assembly kernel)
         const bool contact = ((pk >> 20) & 1u) == KIND_CONTACT;
-        const double lo01 = contact ? -1.0 : -kInf, hi01 = contact ? 1.0 : kInf, lo2 = contact ? 0.0 : -kInf;
+        double lo01 = contact ? -1.0 : -kInf, hi01 = contact ? 1.0 : kInf;
+        const double lo2 = contact ? 0.0 : -kInf;
+        if (COULOMB && contact) {
+          const double bnd = mu * (x2 > 0.0 ? x2 : 0.0);
+          lo01 = -bnd; hi01 = bnd;
+        }
         double n0 = x0 + e0 * IA0;
+        unsigned long long flags = 0ull;
+        if (COULOMB) flags = (n0 < lo01) ? 1ull : ((n0 > hi01) ? 2ull : 0ull);
         n0 = clamp_sel(n0, lo01, hi01);
         d0 = n0 - x0;
         double n1 = x1 + (e1 - DO0 * d0) * IA1;
+        if (COULOMB) flags |= ((n1 < lo01) ? 1ull : ((n1 > hi01) ? 2ull : 0ull)) << 2;
         n1 = clamp_sel(n1, lo01, hi01);
         d1 = n1 - x1;
         double n2 = x2 + ((e2 - DO1 * d0) - DO2 * d1) * IA2;
         n2 = (n2 < lo2) ? lo2 : n2;
         d2 = n2 - x2;
-        st_sector(reinterpret_cast<double*>(gs + lam_off), n0, n1, n2, __longlong_as_double((long long)pk_lam));
+        const unsigned long long pk_out = COULOMB ? ((pk_lam & ~(15ull << PK_FLAGS)) | (flags << PK_FLAGS)) : pk_lam;
+        st_sector(reinterpret_cast<double*>(gs + lam_off), n0, n1, n2, __longlong_as_double((long long)pk_out));
       }
       // impulse scatter: a += M^-1 J^T delta
       const double ix = RC0 * d0 + RC3 * d1 + RC6 * d2, iy = RC1 * d0 + RC4 * d1 + RC7 * d2, iz = RC2 * d0 + RC5 * d1 + RC8 * d2;
@@ -667,8 +698,8 @@ size_t stream_smem(const EggDev& d, int lpw) {
   return 64 + (size_t)G * 48 * d.n + (size_t)(HDRB + 32 * ((F32 ? RECB32 : RECB64) + LAMB));   // FP64, 64 bodies: 19072 B, 11 CTAs per SM
 }
 
-template <int LPW, int MINB, int ISO, bool F32>
-cudaError_t launch(const EggDev& d, double dt, cudaStream_t s) {
+template <int LPW, int MINB, int ISO, bool F32, bool COULOMB>
+cudaError_t launch(const EggDev& d, double dt, const double* mu, cudaStream_t s) {
   constexpr int G = 32 / LPW;
   const size_t smem = stream_smem<F32>(d, LPW);
   // shared-memory attribute and occupancy are looked up once per (kernel instance, shared-memory
@@ -680,9 +711,9 @@ cudaError_t launch(const EggDev& d, double dt, cudaStream_t s) {
   EGG_FIRST(e, cudaGetDevice(&dev));
   if (e != cudaSuccess) return e;
   if (smem != c_smem || dev != c_dev) {
-    EGG_FIRST(e, cudaFuncSetAttribute(egg_pgs_stream_kernel<LPW, MINB, ISO, F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    EGG_FIRST(e, cudaFuncSetAttribute(egg_pgs_stream_kernel<LPW, MINB, ISO, F32, COULOMB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     EGG_FIRST(e, cudaDeviceGetAttribute(&c_sms, cudaDevAttrMultiProcessorCount, dev));
-    EGG_FIRST(e, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c_per_sm, egg_pgs_stream_kernel<LPW, MINB, ISO, F32>, 32, smem));
+    EGG_FIRST(e, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c_per_sm, egg_pgs_stream_kernel<LPW, MINB, ISO, F32, COULOMB>, 32, smem));
     if (e != cudaSuccess) return e;
     if (c_per_sm < 1) return cudaErrorLaunchOutOfResources;   // the kernel does not fit an SM with this much shared memory
     c_smem = smem; c_dev = dev;
@@ -693,29 +724,33 @@ cudaError_t launch(const EggDev& d, double dt, cudaStream_t s) {
   const int grid = groups < c_sms * per_sm ? groups : c_sms * per_sm;
   e = cudaMemsetAsync(d.work_ctr, 0, sizeof(int), s);
   if (e != cudaSuccess) return e;   // without the reset the persistent kernel would find an exhausted queue and do nothing
-  egg_pgs_stream_kernel<LPW, MINB, ISO, F32><<<grid, 32, smem, s>>>(d, dt, d.sel.pf);
+  egg_pgs_stream_kernel<LPW, MINB, ISO, F32, COULOMB><<<grid, 32, smem, s>>>(d, dt, d.sel.pf, mu);
   return cudaGetLastError();
 }
 
 // Registers are allocated per scheduler (16384 each): 12 one-warp CTAs per SM = 3 per scheduler
 // = 168 registers.
-template <int MINB, int ISO, bool F32>
-cudaError_t launch_lpw(const EggDev& d, double dt, cudaStream_t s) {
+template <int MINB, int ISO, bool F32, bool COULOMB>
+cudaError_t launch_lpw(const EggDev& d, double dt, const double* mu, cudaStream_t s) {
   switch (d.lpw) {
-    case 1: return launch<1, MINB, ISO, F32>(d, dt, s);
-    case 2: return launch<2, MINB, ISO, F32>(d, dt, s);
-    case 4: return launch<4, MINB, ISO, F32>(d, dt, s);
-    case 16: return launch<16, MINB, ISO, F32>(d, dt, s);
-    default: return launch<8, MINB, ISO, F32>(d, dt, s);
+    case 1: return launch<1, MINB, ISO, F32, COULOMB>(d, dt, mu, s);
+    case 2: return launch<2, MINB, ISO, F32, COULOMB>(d, dt, mu, s);
+    case 4: return launch<4, MINB, ISO, F32, COULOMB>(d, dt, mu, s);
+    case 16: return launch<16, MINB, ISO, F32, COULOMB>(d, dt, mu, s);
+    default: return launch<8, MINB, ISO, F32, COULOMB>(d, dt, mu, s);
   }
 }
 // One staging buffer per warp.  A second buffer (two rounds in flight) was measured no better
 // anywhere -- stack10 4096 worlds 26.9 vs 26.2 ms, legged20 106 vs 90 ms, pile64 8.8 vs 8.1 ms --
 // and was removed again.
 template <int MINB, int ISO>
-cudaError_t launch_nbuf(const EggDev& d, double dt, cudaStream_t s) {
-  if (d.blkb == RECB32 + LAMB) return launch_lpw<MINB, ISO, true>(d, dt, s);
-  return launch_lpw<MINB, ISO, false>(d, dt, s);
+cudaError_t launch_nbuf(const EggDev& d, double dt, const double* mu, cudaStream_t s) {
+  if (mu) {   // Coulomb friction (egg_set_friction): the twins of the BOX instances
+    if (d.blkb == RECB32 + LAMB) return launch_lpw<MINB, ISO, true, true>(d, dt, mu, s);
+    return launch_lpw<MINB, ISO, false, true>(d, dt, mu, s);
+  }
+  if (d.blkb == RECB32 + LAMB) return launch_lpw<MINB, ISO, true, false>(d, dt, mu, s);
+  return launch_lpw<MINB, ISO, false, false>(d, dt, mu, s);
 }
 
 size_t schedule_per_world(const EggDev& d) { return ((size_t)(d.n + 4 * d.nrec + 2 + 7) & ~(size_t)7) * sizeof(unsigned short); }
@@ -789,9 +824,10 @@ cudaError_t egg_launch_assemble_stream(const EggDev& d, double dt, cudaStream_t 
   return launch_records(d, dt, G, smem, s);
 }
 
-cudaError_t egg_launch_solve_pgs_stream(const EggDev& d, double dt, cudaStream_t s) {
+// With a friction table the caller keeps d.rmax = 0 (egg_capi.cu): the run format has BOX friction only.
+cudaError_t egg_launch_solve_pgs_stream(const EggDev& d, double dt, const double* mu, cudaStream_t s) {
   if (d.rmax > 0) return egg_launch_solve_pgs_runs(d, dt, s);
-  if (d.iso == 2) return launch_nbuf<12, 2>(d, dt, s);
-  if (d.iso == 1) return launch_nbuf<12, 1>(d, dt, s);
-  return launch_nbuf<8, 0>(d, dt, s);
+  if (d.iso == 2) return launch_nbuf<12, 2>(d, dt, mu, s);
+  if (d.iso == 1) return launch_nbuf<12, 1>(d, dt, mu, s);
+  return launch_nbuf<8, 0>(d, dt, mu, s);
 }

@@ -2,7 +2,8 @@
 
 Every scene is a dict of world-major numpy arrays ready for ``Batch.set_bodies/set_joints``:
 p,v,w [W,n,3]; R,I [W,n,3,3]; m [W,n]; optional joints i0,i1 [nj], c0,c1 [W,nj,3]; f_ext [W,n,6];
-optional box side lengths side [W,n,3] (default 0.3 on every axis); plus ``dt`` and ``solver``.  All bodies are cubes of side 0.3, the only collider the reference has
+optional box side lengths side [W,n,3] (default 0.3 on every axis); optional Coulomb friction
+coefficients mu [W] or a scalar (``Batch.set_friction``); plus ``dt`` and ``solver``.  All bodies are cubes of side 0.3, the only collider the reference has
 (/root/reference/eggshell/body.h:90-91).  Randomness is a seeded numpy PCG64 stream per
 (config, base seed), so the same arrays feed the GPU batch and the CPU oracle.
 """
@@ -250,6 +251,8 @@ def make_batch(scene, **kw):
     b.init()
     if "f_ext" in scene:
         b.set_external(scene["f_ext"])
+    if "mu" in scene:
+        b.set_friction(scene["mu"])
     return b
 
 

@@ -58,7 +58,8 @@ enum egg_quirk {
   /* Not a reference quirk: the run format of the PGS record stream (egg_pgs_runs.cu): a lane carries
    * the consecutive contacts of one manifold through a stage, records shrink to 80 B per block +
    * 64 B per run.  Same sweep in the same row order; measured faster only for stack-like scenes
-   * (DESIGN.md section 4), so it is opt-in.  Isotropic bodies, FP64 records only (else ignored). */
+   * (DESIGN.md section 4), so it is opt-in.  Isotropic bodies, FP64 records only, and no friction
+   * table (egg_set_friction): else ignored, decided at every step. */
   EGG_OPT_PGS_RUNS = 16
 };
 #define EGG_QUIRKS_REFERENCE 3
@@ -131,6 +132,18 @@ int egg_set_state(egg_batch* b, const double* p, const double* R, const double* 
 int egg_set_joints(egg_batch* b, const int* i0, const int* i1, const double* c0, const double* c1);
 /* Overrides Ensemble::external_force_torque_ (ensembles.h:88-89) after egg_init; 6 per body. */
 int egg_set_external(egg_batch* b, const double* f_ext);
+
+/* Coulomb-pyramid friction with one coefficient per world (INTEGRATION.md, "Friction").  mu is a HOST
+ * [n_worlds] array, each entry finite and >= 0; it is copied to device memory owned by the batch
+ * (counted by egg_device_bytes).  With a table, the PGS solve bounds the two tangent rows of a block
+ * projected as a contact by [-b, b], b = mu[w] max(x_n, 0), x_n the block's normal multiplier before
+ * its update, instead of the reference's BOX bounds [-1, 1]; a tangent row is "at its bound" in the
+ * residual and in the row_state taps when that projection clamped it.  mu == NULL returns to BOX
+ * friction, bit for bit, and releases the memory.  EGG_ERR_ARG for a NaN, infinite or negative entry
+ * (the previous table is kept); EGG_ERR_UNSUPPORTED unless the solver is EGG_SOLVER_PGS (the dense
+ * path, Jacobi and SOR keep BOX friction).  While a table is set the run format (EGG_OPT_PGS_RUNS) is
+ * not used.  Valid before or after egg_init.  Synchronises the batch stream. */
+int egg_set_friction(egg_batch* b, const double* mu);
 
 /* Ensemble::Init (ensembles.cc:24-29): M^-1 blocks, f_ext, initial-condition check and
  * CheckAndCorrectEnsembleState (a joint-joint conflict sets EGG_ST_JOINT_CONFLICT here, where the
